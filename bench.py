@@ -5,6 +5,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...      # CPU restatement of the reference path on the host cores
+    python bench.py ... --dump-outputs DIR    # also write the last timed step's result rows to DIR/*.npy (dump_outputs)
 
 Default = the north_star configuration (BASELINE.json configs[3], C4): the 1 B-row synthetic table with a
 sorted-int-codec `id` column, `select id from test_1b where (id > L and id < H)` (1 % window), the canonical segment
@@ -80,6 +81,7 @@ AGG_SPECS = {  # workload -> (predicates, aggregates as (op, col) with op 0 = co
 SECONDARY = [("c4_pruned_1b", "c4", None), ("agg_100m", "agg", 100_000_000), ("c2_100m", "c2", 100_000_000), ("c3_100m", "c3", 100_000_000), ("c4_limit10_1b", "c4_limit10", None),
              ("c5_rare_1b", "c5_rare", None), ("c5p_lt10_1b", "c5p_lt10", None)]
 WINDOW_FRAC = {"c5w_001": 1e-4, "c5w_01": 1e-3, "c5w_1": 1e-2, "c5w_10": 0.1, "c5w_50": 0.5, "c5w_100": 1.0}
+DUMP_BYTES = 64_000_000  # --dump-outputs writes at most this much in all
 
 
 def query_spec(workload: str, total_rows: int):
@@ -255,6 +257,32 @@ def crc_columns(cols):
     return [(int(len(c)), zlib.crc32(np.ascontiguousarray(c).view(np.uint8).reshape(-1).tobytes())) for c in cols]
 
 
+def dump_outputs(out_dir, names, cols, result_rows, suffix=""):
+    """--dump-outputs: one query's result as out_dir/<column><suffix>.npy in float64 (a STRING(k) column as n x k byte
+    codes) and its row count as result_rows<suffix>.npy.  A result above DUMP_BYTES is cut to one seeded sample of rows,
+    the same in every column, whose positions go to sample_rows<suffix>.npy: two builds run with the same arguments
+    can then be compared array for array."""
+    import numpy as np
+
+    arrays = {"result_rows": np.array([result_rows], np.float64)}
+    per_row = sum(c.dtype.itemsize if c.dtype.kind == "S" else 1 for c in cols)  # float64 values per result row
+    n = len(cols[0]) if cols else 0
+    cap = (DUMP_BYTES - 4096) // (8 * (per_row + 1))  # (+1: the sample's positions; 4096: the .npy headers)
+    rows = None
+    if n > cap:
+        rows = np.sort(np.random.default_rng(0).choice(n, size=cap, replace=False))
+        arrays["sample_rows"] = rows.astype(np.float64)
+    for name, c in zip(names, cols):
+        if rows is not None:
+            c = c[rows]
+        if c.dtype.kind == "S":
+            c = np.ascontiguousarray(c).view(np.uint8).reshape(len(c), c.dtype.itemsize)
+        arrays[name] = c.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a)
+
+
 # ---------------------------------------------------------------------------------------------------
 # CPU side: the oracle (restatement of the reference's Scala path), one task per segment on a pool
 # ---------------------------------------------------------------------------------------------------
@@ -318,6 +346,10 @@ def reference_arm(args):
     d, table, gen_s = ensure_table(kind, total, 0, 1, lambda: None, "oracle")
     cores = os.cpu_count() or 1
     rows, res, times = run_cpu(O, d, table, args.workload, total, cores, args.steps, args.warmup)
+    if args.dump_outputs:
+        agg = AGG_SPECS.get(args.workload)
+        names = (agg[2] + [col + ("_count", "_min", "_max")[op] for op, col in agg[1]]) if agg else query_spec(args.workload, total)[1]
+        dump_outputs(args.dump_outputs, names, res.columns, res.nrows)
     sec = statistics.median(times)
     v = rows / sec
     line = {
@@ -352,7 +384,13 @@ def main():
     ap.add_argument("--no-verify", action="store_true")
     ap.add_argument("--no-tma", action="store_true", help="direct-load variant of the dense kernels (A/B)")
     ap.add_argument("--cpu-steps", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the rows the last timed step computed to DIR/<column>.npy (float64, "
+                    "a seeded sample of them beyond 64 MB) so that two builds can be compared output for output")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.sweep:
+        ap.error("--dump-outputs writes the headline query's result; --sweep has none")
     if args.rows is None:
         args.rows = 1_000_000_000 if WORKLOADS[args.workload][1] == "pfor" else 100_000_000
     if args.warmup < 3 and args.impl == "ours" and not os.environ.get("IMM3_BENCH_ALLOW_SHORT"):
@@ -439,9 +477,10 @@ def main():
             opened[key] = (sm, Engine(sm), d, table, sm.getTable(table), open_s, gen_s)
         return opened[key]
 
-    def measure(workload, rows_total, steps, warmup, sample_clocks=False, prune=False):
+    def measure(workload, rows_total, steps, warmup, sample_clocks=False, prune=False, outputs=None):
         """K timed steps of one query.  Per step: L2 flush + barrier (untimed), then the wall time of imm3_query_begin -
-        launch of every kernel of the query, the on-device count exchange, one synchronisation, counts on the host."""
+        launch of every kernel of the query, the on-device count exchange, one synchronisation, counts on the host.
+        `outputs` (a dict) receives the result of the last step, fetched after its clock stopped."""
         sm, eng, d, table, tinfo, open_s, gen_s = open_table(WORKLOADS[workload][1], rows_total)
         query = build_query(workload, table, rows_total)
         is_agg = workload in AGG_SPECS
@@ -475,6 +514,10 @@ def main():
             phases.append(r.host_us())
             launches += r.kernel_launches
             alg, local_rows, take, gcount = r.algorithmic_bytes, r.local_count, r.take, r.global_count
+            if outputs is not None and i == steps - 1:
+                if not is_agg:
+                    r.fetch(r.take)  # (an aggregate's rows are on the host already)
+                outputs.update(names=[r.col_name(c) for c in range(r.ncols)], cols=r.columns(), result_rows=gcount)
             r.close()
         clocks = sampler.stop() if sampler else None
         barrier()
@@ -583,7 +626,10 @@ def main():
 
     # ---- headline: value = wall (barrier -> query + exchange done), K steps ----
     total = args.rows * (world if args.scaling == "weak" else 1)
-    head, clocks, ctx = measure(args.workload, total, args.steps, args.warmup, sample_clocks=True)
+    outputs = {} if args.dump_outputs else None
+    head, clocks, ctx = measure(args.workload, total, args.steps, args.warmup, sample_clocks=True, outputs=outputs)
+    if outputs is not None:
+        dump_outputs(args.dump_outputs, outputs["names"], outputs["cols"], outputs["result_rows"], f"_rank{rank}" if world > 1 else "")
     sm, eng, d, table, tinfo, query, prep, local_rows, take = ctx
     open_s, gen_s = opened[(WORKLOADS[args.workload][1], total)][5:7]
     agg_head = args.workload in AGG_SPECS
