@@ -1761,15 +1761,24 @@ int imm3_query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int n
     std::unique_ptr<imm3_result> r(new imm3_result());
     r->db = db;
     std::vector<int> gidx, aidx;
+    std::vector<int> pfor_cols;  // distinct sorted-int-codec columns decoded per block (MIN / MAX inputs, group columns)
+    auto pfor_slot = [&](int ci) -> int8_t {
+        for (size_t i = 0; i < pfor_cols.size(); i++)
+            if (pfor_cols[i] == ci) return (int8_t)i;
+        pfor_cols.push_back(ci);
+        return (int8_t)(pfor_cols.size() - 1);
+    };
+    for (int i = 0; i < kMaxAggs; i++) ap.agg_pfor[i] = -1;
+    for (int i = 0; i < kMaxGroupCols; i++) ap.group_pfor[i] = -1;
     int key_bits = 0;
     for (int g = 0; g < ngroup; g++) {
         const int ci = find_col(group_cols[g]);
         if (ci < 0) return fail(IMM3_ERR_NOT_FOUND, "Column %s does not exist in table %s", group_cols[g] ? group_cols[g] : "(null)", t.meta.name.c_str());
         const ColumnStore& c = t.cols[(size_t)ci];
-        if (c.meta.codec == IMM3_CODEC_PFOR_INT) return fail(IMM3_ERR_UNSUPPORTED, "group by a sorted-int-codec column (%s) is not supported", c.meta.name.c_str());
         if (key_bits + 8 * c.meta.width > 56) return fail(IMM3_ERR_UNSUPPORTED, "group-by cells must pack into 7 bytes");
         ap.group[g].width = c.meta.width;
         ap.group[g].key_shift = key_bits;
+        if (c.meta.codec == IMM3_CODEC_PFOR_INT) ap.group_pfor[g] = pfor_slot(ci);
         key_bits += 8 * c.meta.width;
         gidx.push_back(ci);
         r->names.push_back(c.meta.name);
@@ -1786,8 +1795,8 @@ int imm3_query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int n
         } else if (aggs[a].op == IMM3_AGG_MIN || aggs[a].op == IMM3_AGG_MAX) {
             if (c.meta.ctype == IMM3_COL_STRING)
                 return fail(IMM3_ERR_UNSUPPORTED, "min / max on a STRING column (the reference maps both to MaxStringAggr, Engine.scala:137,147)");
-            if (c.meta.codec == IMM3_CODEC_PFOR_INT) return fail(IMM3_ERR_UNSUPPORTED, "min / max on a sorted-int-codec column (%s) is not supported", c.meta.name.c_str());
             ap.agg[a].op = aggs[a].op == IMM3_AGG_MIN ? kAggMin : kAggMax;
+            if (c.meta.codec == IMM3_CODEC_PFOR_INT) ap.agg_pfor[a] = pfor_slot(ci);  // (COUNT never reads its column)
             suffix = aggs[a].op == IMM3_AGG_MIN ? "_min" : "_max";
         } else {
             return fail(IMM3_ERR_UNSUPPORTED, "Unknown Aggregate type (Engine.scala:153: only Min, Max and Count are resolved)");
@@ -1808,6 +1817,13 @@ int imm3_query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int n
             if (t.cols[(size_t)f.col_idx].meta.codec == IMM3_CODEC_PFOR_INT)
                 return fail(IMM3_ERR_UNSUPPORTED, "aggregation with a predicate on a sorted-int-codec column (%s) is not supported yet", t.cols[(size_t)f.col_idx].meta.name.c_str());
     }
+    // A MIN / MAX input or a group column in the sorted-int codec: agg_blocks_kernel decodes them block by block.
+    const bool on_blocks = !pfor_cols.empty();
+    if (pfor_cols.size() > (size_t)kMaxPforCols)
+        return fail(IMM3_ERR_UNSUPPORTED, "aggregation decodes at most %d distinct sorted-int-codec columns, the query reads %zu", kMaxPforCols, pfor_cols.size());
+    if (on_blocks && t.max_block_rows > 1024)
+        return fail(IMM3_ERR_UNSUPPORTED, "aggregation over sorted-int-codec columns decodes blocks of at most 1024 rows, table %s has a block of %d",
+                    t.meta.name.c_str(), t.max_block_rows);
     if ((rc = use_device(db))) return rc;
     int64_t ngroups_out = 0;
     std::vector<AggEntry> groups;
@@ -1840,13 +1856,36 @@ int imm3_query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int n
         ap.ntiles = ntiles;
         for (int g = 0; g < ngroup; g++) ap.group[g].base = t.cols[(size_t)gidx[(size_t)g]].d_arena;
         for (int a = 0; a < naggs; a++) ap.agg[a].base = t.cols[(size_t)aidx[(size_t)a]].d_arena;
+        if (on_blocks) {
+            int64_t cap = 0;  // per-warp scratch for the byte-swapped words of one encoded block
+            ap.npfor = (int)pfor_cols.size();
+            for (int i = 0; i < ap.npfor; i++) {
+                const ColumnStore& c = t.cols[(size_t)pfor_cols[(size_t)i]];
+                ap.pfor[i].words = reinterpret_cast<const uint32_t*>(c.d_arena);
+                ap.pfor[i].word_off = c.d_word_off;
+                cap = std::max<int64_t>(cap, c.max_block_words);
+            }
+            ap.blk_words_cap = (int)std::min<int64_t>(1120, ((cap + 4 + 31) / 32) * 32);
+            ap.nblocks = t.nblocks;
+            ap.row_start = t.d_row_start;
+            int optin = 0;
+            CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, db->device));
+            const size_t smem = agg_blocks_smem_bytes(naggs, ap.npfor, ap.blk_words_cap);
+            if (smem + 1024 > (size_t)optin)  // (1 KB: the kernel's static shared memory)
+                return fail(IMM3_ERR_UNSUPPORTED, "aggregation over %d sorted-int-codec columns with %d aggregates needs %zu bytes of shared memory per CTA, the device has %d",
+                            ap.npfor, naggs, smem + 1024, optin);
+        }
         sp.scan_inline = 1;  // (only the total matters here; the last CTA's scan provides it)
         CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
         CUDA_TRY(launch_agg_init((AggEntry*)db->d_agg_table.p, ap.table_slots, ap, (unsigned int*)db->d_agg_cnt.p, db->stream));
         CUDA_TRY(launch_filter(sp, (uint32_t*)db->d_bitmap.p, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
                                (unsigned long long*)db->d_tile_off.p, db->d_ctrl, pr.grid, pr.dyn_smem, db->stream));
-        CUDA_TRY(launch_agg(ap, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, (AggEntry*)db->d_agg_table.p,
-                            (AggEntry*)db->d_agg_out.p, (unsigned int*)db->d_agg_cnt.p, db->d_ctrl, db->num_sms, db->stream));
+        if (on_blocks)
+            CUDA_TRY(launch_agg_blocks(ap, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, (AggEntry*)db->d_agg_table.p,
+                                       (AggEntry*)db->d_agg_out.p, (unsigned int*)db->d_agg_cnt.p, db->d_ctrl, db->num_sms, db->stream));
+        else
+            CUDA_TRY(launch_agg(ap, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, (AggEntry*)db->d_agg_table.p,
+                                (AggEntry*)db->d_agg_out.p, (unsigned int*)db->d_agg_cnt.p, db->d_ctrl, db->num_sms, db->stream));
         CUDA_TRY(cudaEventRecord(db->ev1, db->stream));
         r->launches = 4;
         unsigned int counters[2] = {0, 0};
@@ -1863,12 +1902,15 @@ int imm3_query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int n
         groups.resize((size_t)ngroups_out);
         if (ngroups_out) CUDA_TRY(cudaMemcpy(groups.data(), db->d_agg_out.p, (size_t)ngroups_out * sizeof(AggEntry), cudaMemcpyDeviceToHost));
         std::sort(groups.begin(), groups.end(), [](const AggEntry& x, const AggEntry& y) { return x.first_row < y.first_row; });
-        // algorithmic bytes: filter columns once + per selected row the cells of the group and aggregate columns
+        // algorithmic bytes: filter columns once + every decoded encoded column once (its words and 4 B of word offsets per
+        // block) + per selected row the cells of the dense group and aggregate columns
         int64_t bytes = 0, per_row = 0;
         for (auto& f2 : pr.lp.filters) bytes += t.cols[(size_t)f2.col_idx].encoded_bytes;
-        for (int ci : gidx) per_row += t.cols[(size_t)ci].meta.width;
+        for (int ci : pfor_cols) bytes += t.cols[(size_t)ci].encoded_bytes + 4 * (int64_t)t.nblocks;
+        for (int g = 0; g < ngroup; g++)
+            if (ap.group_pfor[g] < 0) per_row += t.cols[(size_t)gidx[(size_t)g]].meta.width;
         for (int a = 0; a < naggs; a++)
-            if (ap.agg[a].op != kAggCount) per_row += ap.agg[a].width;
+            if (ap.agg[a].op != kAggCount && ap.agg_pfor[a] < 0) per_row += ap.agg[a].width;
         r->alg_bytes = bytes + per_row * (int64_t)db->h_ctrl->c.total;
     }
     // rows of the result: group cells, then the aggregates (COUNT: int64, MIN / MAX: double)

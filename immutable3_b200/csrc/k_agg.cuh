@@ -14,6 +14,9 @@
 //                            value first and only issue an atomic when the row improves it (after the first rows of a
 //                            group almost never), COUNT is one native 32-bit shared-memory atomic; at the end the CTA
 //                            folds its warps' values per slot and adds the groups to the global table
+//   agg_blocks_kernel        instead of agg_kernel when a MIN / MAX input or a group column is in the sorted-int codec: one
+//                            warp per reference BLOCK with selected rows, the block's encoded columns decoded into the
+//                            warp's shared memory, then agg_kernel's row loop (see below)
 //   agg_compact_kernel       occupied slots of the global table -> a dense array (any order; the host sorts the groups by
 //                            the canonical ordinal of their first row, the order the reference reports them in with one
 //                            worker) and clears the table for the next query
@@ -92,7 +95,9 @@ __device__ __forceinline__ void agg_update(long long* v, int op, long long x) {
 }
 __device__ __forceinline__ long long agg_identity(int op) { return op == kAggCount ? 0ll : (op == kAggMin ? LLONG_MAX : LLONG_MIN); }
 
-// One group's partial (x[a]: a count, or an extreme as int64) into the global table.
+// One group's partial (x[a]: a count, or an extreme as int64) into the global table.  (K: agg_blocks_kernel calls its own
+// copy, K = 1, so that agg_kernel's call graph - and with it agg_kernel's register allocation - is the one it had alone.)
+template <int K = 0>
 __device__ __noinline__ void agg_to_global(AggEntry* table, uint32_t slots, unsigned int* overflow, unsigned long long key, unsigned long long fr,
                                            const long long* x, const AggCol* aggs, int naggs) {
     const int gs = agg_global_slot(table, slots, key);
@@ -276,6 +281,288 @@ __global__ void __launch_bounds__(kComputeThreads, 3) agg_kernel(const __grid_co
         for (int a = 0; a < NA; a++) xl[a] = A.agg[a].op == kAggCount ? (long long)(unsigned int)acc[a] : (long long)(A.agg[a].op == kAggMin ? ~acc[a] : acc[a]);
         agg_to_global(table, A.table_slots, overflow, key, first, xl, s_agg, naggs);
     }
+}
+
+// agg_blocks_kernel's per-row work, as functions of the plan: the same steps as agg_kernel's lambdas (fetch_raw / decode /
+// apply / the fold), which stay written out in agg_kernel - routed through these functions its generated code changes.
+// A CTA's empty state: no dict guesses, no keys, this warp's values at their identities (first row: "never seen").
+template <int NA>
+__device__ __forceinline__ void agg_state_init(const AggPlan& A, uint8_t* dict, unsigned long long* keys, int* V, int tid, int lane) {
+    for (int i = tid; i < (1 << kAggDictBits) / 4; i += kComputeThreads) reinterpret_cast<uint32_t*>(dict)[i] = 0u;
+    for (int i = tid; i < kAggSlots; i += kComputeThreads) keys[i] = kAggEmpty;
+    for (int i = lane; i < kAggSlots; i += 32) {
+#pragma unroll
+        for (int a = 0; a < NA; a++) V[a * kAggSlots + i] = A.agg[a].op == kAggCount ? 0 : INT_MIN;
+        V[NA * kAggSlots + i] = INT_MIN;
+    }
+}
+// The words fetched for row `r` (gw / aw: the aligned 32-bit word holding each cell; gp = the group columns at the row
+// the offsets count from) -> the packed group key and the aggregate inputs (MIN inputs complemented).  Group cells of
+// other widths are gathered byte-wise.
+template <int NG, int NA>
+__device__ __forceinline__ void agg_decode(const AggPlan& A, int ngroup, int naggs, const uint8_t* const (&gp)[NG > 0 ? NG : 1], unsigned r,
+                                           const uint32_t (&gw)[NG > 0 ? NG : 1], const uint32_t (&aw)[NA], unsigned long long& key, int (&x)[NA]) {
+    key = 0;
+#pragma unroll
+    for (int g = 0; g < NG; g++) {
+        if (NG == 4 && g >= ngroup) break;
+        const unsigned w = (unsigned)A.group[g].width;
+        const unsigned off = r * w;
+        unsigned long long cell = 0;
+        if (w <= 4u && (w & (w - 1u)) == 0u) {
+            cell = (gw[g] >> ((off & 3u) * 8u)) & (0xFFFFFFFFu >> (32u - 8u * w));
+        } else {
+            for (unsigned b = 0; b < w; b++) cell |= (unsigned long long)__ldg(gp[g] + off + b) << (8u * b);
+        }
+        key |= cell << A.group[g].key_shift;
+    }
+#pragma unroll
+    for (int a = 0; a < NA; a++) {
+        x[a] = 0;
+        if (NA == 8 && a >= naggs) break;
+        const int op = A.agg[a].op;
+        if (op != kAggCount) {
+            const unsigned w = (unsigned)A.agg[a].width;  // 4 (INT) or 1 (TINYINT, sign-extended)
+            const int v = (int)(aw[a] << ((4u - w - ((r * w) & 3u)) * 8u)) >> ((4u - w) * 8u);
+            x[a] = v ^ (op == kAggMin ? -1 : 0);
+        }
+    }
+}
+// One row into its group: `ord` = the row's ordinal in this warp's own sequence of rows (ascending: a group's first row
+// is the one that creates its entry in the warp's values); `row` = its row ordinal (the cold path's first row).
+template <int NA>
+__device__ __forceinline__ void agg_apply(const AggPlan& A, int naggs, uint8_t* dict, unsigned long long* keys, int* V, AggEntry* table,
+                                          unsigned int* overflow, const AggCol* s_agg, long long row, unsigned ord, unsigned long long key,
+                                          const int (&x)[NA]) {
+    const int slot = agg_cta_slot(dict, keys, key);
+    if (slot >= 0) {
+#pragma unroll
+        for (int a = 0; a < NA; a++) {
+            if (NA == 8 && a >= naggs) break;
+            int* const v = V + a * kAggSlots + slot;
+            if (A.agg[a].op == kAggCount) atomicAdd(reinterpret_cast<unsigned int*>(v), 1u);
+            else if (x[a] > *reinterpret_cast<volatile int*>(v)) atomicMax(v, x[a]);  // (a stale read is only ever too low: at worst one atomic too many)
+        }
+        int* const f = V + NA * kAggSlots + slot;
+        const int fo = ~(int)ord;
+        if (fo > *reinterpret_cast<volatile int*>(f)) atomicMax(f, fo);
+    } else {  // the CTA's table is full
+        long long xl[kMaxAggs];
+#pragma unroll
+        for (int a = 0; a < NA; a++) xl[a] = A.agg[a].op == kAggCount ? 1ll : (long long)(A.agg[a].op == kAggMin ? ~x[a] : x[a]);
+        agg_to_global<1>(table, A.table_slots, overflow, key, (unsigned long long)row, xl, s_agg, naggs);
+    }
+}
+// Thread t folds slot t over the CTA's warps and hands the group to the global table; first_row(w, ord) = the row ordinal
+// of warp w's ordinal `ord`.
+template <int NA, class FirstRow>
+__device__ __forceinline__ void agg_fold(const AggPlan& A, int naggs, const unsigned long long* keys, const int* vals, AggEntry* table,
+                                         unsigned int* overflow, const AggCol* s_agg, int tid, FirstRow first_row) {
+    for (int i = tid; i < kAggSlots; i += kComputeThreads) {
+        const unsigned long long key = keys[i];
+        if (key == kAggEmpty) continue;
+        unsigned long long first = ~0ull;
+        int acc[NA];
+#pragma unroll
+        for (int a = 0; a < NA; a++) acc[a] = A.agg[a].op == kAggCount ? 0 : INT_MIN;
+        for (int w = 0; w < kComputeWarps; w++) {
+            const int* const W = vals + w * (NA + 1) * kAggSlots;
+            const int fo = W[NA * kAggSlots + i];
+            if (fo == INT_MIN) continue;  // warp w never saw this group
+            const unsigned long long r = first_row(w, (unsigned)~fo);
+            first = r < first ? r : first;
+#pragma unroll
+            for (int a = 0; a < NA; a++) {
+                if (NA == 8 && a >= naggs) break;
+                const int v = W[a * kAggSlots + i];
+                acc[a] = A.agg[a].op == kAggCount ? (int)((unsigned)acc[a] + (unsigned)v) : (v > acc[a] ? v : acc[a]);  // (a CTA counts < 2^32 rows)
+            }
+        }
+        if (first == ~0ull) continue;
+        long long xl[kMaxAggs];
+#pragma unroll
+        for (int a = 0; a < NA; a++) xl[a] = A.agg[a].op == kAggCount ? (long long)(unsigned int)acc[a] : (long long)(A.agg[a].op == kAggMin ? ~acc[a] : acc[a]);
+        agg_to_global<1>(table, A.table_slots, overflow, key, first, xl, s_agg, naggs);
+    }
+}
+
+// agg_blocks_kernel: the same aggregation when a MIN / MAX input or a group column is in the sorted-int codec.  The filter
+// is the same row-space filter_kernel (no predicate touches an encoded column); the work unit is a reference block instead
+// of a 1024-row span, because an encoded column can only be decoded block by block:
+//   one warp per block with selected rows (blocks warp0, warp0 + nwarps, ...: round robin, like blocks_emit_kernel<true>);
+//   the block's selection bits = the row-space bitmap funnel-shifted to its first row R0; every encoded column the query
+//   reads is decoded into the warp's own shared memory - the dense sorted shape into dense_prepare's O(1)-per-row form,
+//   anything else by pfor_decode_warp - and never written to HBM; then agg_kernel's row loop: dense cells gathered at
+//   R0 + row, encoded cells read from shared memory, the same key packing, slot cache, per-warp partials and fold.
+// A warp's ordinal of a row is k * 1024 + row-in-block, k = the warp's round-robin position, so the fold recovers the
+// block (warp0 + k * nwarps) and the first row (row_start[block] + row-in-block).
+// Per warp, after agg_kernel's state (without its selection vectors): max(words_cap, 512) words - the block's byte-swapped
+// encoded words while a column is decoded, then the block's selection vector - and per encoded column kBlkVals decoded
+// values + 32 mini-block bases.
+__host__ __device__ constexpr int agg_blocks_warp_words(int npfor, int words_cap) { return (words_cap > 512 ? words_cap : 512) + npfor * (kBlkVals + 32); }
+constexpr size_t agg_blocks_state_bytes(int na) { return agg_smem_bytes(na) - (size_t)kComputeWarps * 1024 * 2; }
+
+template <int NG, int NA>
+__global__ void __launch_bounds__(kComputeThreads, 2) agg_blocks_kernel(const __grid_constant__ AggPlan A, const uint32_t* __restrict__ bitmap,
+                                                                         const uint32_t* __restrict__ span_cnt, AggEntry* __restrict__ table,
+                                                                         unsigned int* __restrict__ overflow, const ScanCtrl* ctrl) {
+    extern __shared__ __align__(128) uint8_t agg_smem[];
+    uint8_t* const dict = agg_smem;
+    unsigned long long* const keys = reinterpret_cast<unsigned long long*>(agg_smem + (1u << kAggDictBits));
+    int* const vals = reinterpret_cast<int*>(agg_smem + (1u << kAggDictBits) + kAggSlots * 8);
+    __shared__ AggCol s_agg[kMaxAggs];
+    __shared__ PforCol s_pfor[kMaxPforCols];
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+#pragma unroll
+    for (int i = 0; i < kMaxAggs; i++)
+        if (tid == i) s_agg[i] = A.agg[i];
+#pragma unroll
+    for (int i = 0; i < kMaxPforCols; i++)
+        if (tid == 32 + i) s_pfor[i] = A.pfor[i];
+    const int naggs = NA == 8 ? A.naggs : NA, ngroup = NG == 4 ? A.ngroup : NG, npfor = A.npfor;
+    int* const V = vals + warp * (NA + 1) * kAggSlots;
+    agg_state_init<NA>(A, dict, keys, V, tid, lane);
+    uint32_t* const Wb = reinterpret_cast<uint32_t*>(agg_smem + agg_blocks_state_bytes(NA)) + warp * agg_blocks_warp_words(npfor, A.blk_words_cap);
+    uint32_t* const dec = Wb + (A.blk_words_cap > 512 ? A.blk_words_cap : 512);  // [slot][kBlkVals]
+    uint32_t* const bases = dec + npfor * kBlkVals;                                 // [slot][mini-block]
+    unsigned short* const sel_w = reinterpret_cast<unsigned short*>(Wb);
+    __syncthreads();
+
+    const long long nblocks = A.nblocks, warp0 = (long long)blockIdx.x * kComputeWarps + warp, nwarps = (long long)gridDim.x * kComputeWarps;
+    // block metadata in ONE round trip: lanes 0,1 = row ordinals, lanes 2+2s, 3+2s = word offsets of encoded column s
+    auto load_meta = [&](long long b) -> unsigned long long {
+        unsigned long long m = 0;
+        if (b < nblocks) {
+            if (lane < 2) m = A.row_start[b + lane];
+            else if (lane < 2 + 2 * npfor) m = s_pfor[(lane - 2) >> 1].word_off[b + (lane & 1)];
+        }
+        return m;
+    };
+    const uint8_t* gp[NG > 0 ? NG : 1];
+    const uint8_t* ap[NA];
+    // One block (its index and metadata): selection bits, decode, then 64 selected rows per iteration as in agg_kernel.
+    auto handle = [&](long long blk, unsigned long long meta) {
+        const long long R0 = (long long)__shfl_sync(0xFFFFFFFFu, meta, 0);
+        const int n = (int)((long long)__shfl_sync(0xFFFFFFFFu, meta, 1) - R0);
+        const long long bit0 = R0 + 32 * lane;
+        const uint32_t lo = __ldg(bitmap + (bit0 >> 5)), hi = __ldg(bitmap + (bit0 >> 5) + 1);
+        uint32_t myword = __funnelshift_r(lo, hi, (uint32_t)(bit0 & 31));
+        const int left = n - lane * 32;
+        myword &= left >= 32 ? 0xFFFFFFFFu : (left <= 0 ? 0u : ((1u << left) - 1u));
+        if (__ballot_sync(0xFFFFFFFFu, myword != 0u) == 0u) return;
+        IMM3_CHECK(ctrl, n > 0 && n <= kBlkRows, 9);  // (the host refuses tables with larger blocks)
+        __syncwarp();  // (the previous block's readers are done with the scratch)
+        unsigned dense_slots = 0;  // encoded columns held in dense_prepare's form
+#pragma unroll 1
+        for (int s = 0; s < npfor; s++) {
+            const uint32_t wo0 = (uint32_t)__shfl_sync(0xFFFFFFFFu, meta, 2 + 2 * s), wo1 = (uint32_t)__shfl_sync(0xFFFFFFFFu, meta, 3 + 2 * s);
+            const DenseRegs dr = dense_issue(s_pfor[s].words, wo0, wo1, n, lane);
+            if (dense_prepare(dr, dec + s * kBlkVals, lane)) {
+                dense_slots |= 1u << s;
+                continue;
+            }
+            IMM3_CHECK(ctrl, wo1 >= wo0 + 3u && (int)(wo1 - wo0) <= A.blk_words_cap, 8);  // the block's words fit the decode scratch
+            bases[s * 32 + lane] = pfor_decode_warp(s_pfor[s].words, wo0, wo1, n, Wb, A.blk_words_cap, dec + s * kBlkVals, lane);
+            __syncwarp();
+        }
+        append_selection(myword, lane, sel_w, 0u);  // (over the encoded words: every column is decoded by now)
+        const unsigned cnt = __reduce_add_sync(0xFFFFFFFFu, (unsigned)__popc(myword));
+        __syncwarp();
+        // value of row r of the block in encoded column s
+        auto enc = [&](int s, unsigned r) -> uint32_t {
+            const uint32_t* const vs = dec + s * kBlkVals;
+            return ((dense_slots >> s) & 1u) ? dense_value(vs, (int)r) : vs[(r >> 5) * kBlkLane + (r & 31u)] + bases[s * 32 + (r >> 5)];
+        };
+        // Dense cells: the words are addressed from the row R0 & ~3 (4-byte aligned whatever the width), row r of the block
+        // is row r + d from there.  An encoded cell is 4 bytes at offset 0 of its word, the form agg_decode expects of it.
+        const long long R0a = R0 & ~3ll;
+        const unsigned d = (unsigned)(R0 - R0a);
+#pragma unroll
+        for (int g = 0; g < NG; g++) gp[g] = A.group[g].base + R0a * A.group[g].width;
+#pragma unroll
+        for (int a = 0; a < NA; a++) ap[a] = A.agg[a].base + R0a * A.agg[a].width;
+        auto fetch_raw = [&](unsigned r, uint32_t (&gw)[NG > 0 ? NG : 1], uint32_t (&aw)[NA]) {
+            const unsigned rd = r + d;
+#pragma unroll
+            for (int g = 0; g < NG; g++) {
+                gw[g] = 0;
+                if (NG == 4 && g >= ngroup) break;
+                const unsigned w = (unsigned)A.group[g].width;
+                if (A.group_pfor[g] >= 0) gw[g] = enc(A.group_pfor[g], r);
+                else if (w <= 4u && (w & (w - 1u)) == 0u) gw[g] = __ldg(reinterpret_cast<const uint32_t*>(gp[g] + ((rd * w) & ~3u)));
+            }
+#pragma unroll
+            for (int a = 0; a < NA; a++) {
+                aw[a] = 0;
+                if (NA == 8 && a >= naggs) break;
+                if (A.agg[a].op == kAggCount) continue;
+                if (A.agg_pfor[a] >= 0) aw[a] = enc(A.agg_pfor[a], r);
+                else aw[a] = __ldg(reinterpret_cast<const uint32_t*>(ap[a] + ((rd * (unsigned)A.agg[a].width) & ~3u)));
+            }
+        };
+        const unsigned ord0 = (unsigned)((blk - warp0) / nwarps) << 10;
+        constexpr int NGW = NG > 0 ? NG : 1;
+        unsigned s0 = lane < cnt ? sel_w[lane] : 0u, s1 = 32u + lane < cnt ? sel_w[32 + lane] : 0u;
+        uint32_t g0[NGW], g1[NGW], a0[NA], a1[NA];
+        fetch_raw(s0, g0, a0);
+        fetch_raw(s1, g1, a1);
+        for (unsigned i0 = 0; i0 < cnt; i0 += 64) {
+            const bool live0 = i0 + lane < cnt, live1 = i0 + 32 + lane < cnt;
+            unsigned long long k0, k1;
+            int x0[NA], x1[NA];
+            agg_decode<NG, NA>(A, ngroup, naggs, gp, s0 + d, g0, a0, k0, x0);
+            agg_decode<NG, NA>(A, ngroup, naggs, gp, s1 + d, g1, a1, k1, x1);
+            const unsigned c0 = s0, c1 = s1;
+            if (i0 + 64 < cnt) {  // (the next rows' loads are in flight during this iteration's updates)
+                s0 = i0 + 64 + lane < cnt ? sel_w[i0 + 64 + lane] : 0u;
+                s1 = i0 + 96 + lane < cnt ? sel_w[i0 + 96 + lane] : 0u;
+                fetch_raw(s0, g0, a0);
+                fetch_raw(s1, g1, a1);
+            }
+            if (live0) agg_apply<NA>(A, naggs, dict, keys, V, table, overflow, s_agg, R0 + c0, ord0 + c0, k0, x0);
+            if (live1) agg_apply<NA>(A, naggs, dict, keys, V, table, overflow, s_agg, R0 + c1, ord0 + c1, k1, x1);
+        }
+    };
+
+    asm volatile("griddepcontrol.wait;" ::: "memory");  // (a no-op unless launched as a programmatic dependent)
+    // 32 of the warp's blocks at a time, a lane each.  Fewer selected rows than blocks (most blocks empty): a lane tests its
+    // block through the counts of the (at most two) 1024-row spans it overlaps; otherwise every block is a candidate.  The
+    // warp then handles the candidates in order, the next one's metadata in flight.  (One call site of `handle`: with two,
+    // the compiler keeps it as a called function and the row loop's arrays in local memory.)
+    const unsigned long long total = __ldcg(&ctrl->total);
+    const bool sparse = total < (unsigned long long)nblocks;
+#pragma unroll 1
+    for (long long b0 = warp0; total != 0ull && b0 < nblocks; b0 += 32 * nwarps) {
+        const long long b = b0 + lane * nwarps;
+        bool cand = b < nblocks;
+        if (cand && sparse) {
+            const unsigned long long r0 = A.row_start[b], r1 = A.row_start[b + 1];
+            const long long q0 = (long long)(r0 >> 10), q1 = (long long)((r1 - 1) >> 10);
+            const unsigned c = __ldg(span_cnt + q0) + (q1 != q0 ? __ldg(span_cnt + q1) : 0u);
+            cand = c != 0u;
+        }
+        unsigned todo = __ballot_sync(0xFFFFFFFFu, cand);
+        if (!todo) continue;
+        int nsrc = __ffs((int)todo) - 1;
+        long long nblk = __shfl_sync(0xFFFFFFFFu, b, nsrc);
+        unsigned long long meta_n = load_meta(nblk);
+#pragma unroll 1
+        while (todo) {
+            todo &= todo - 1u;
+            const unsigned long long meta = meta_n;
+            const long long blk = nblk;
+            if (todo) {
+                nsrc = __ffs((int)todo) - 1;
+                nblk = __shfl_sync(0xFFFFFFFFu, b, nsrc);
+                meta_n = load_meta(nblk);
+            }
+            handle(blk, meta);
+        }
+    }
+    __syncthreads();
+    agg_fold<NA>(A, naggs, keys, vals, table, overflow, s_agg, tid, [&](int w, unsigned ord) -> unsigned long long {
+        return A.row_start[(long long)blockIdx.x * kComputeWarps + w + (long long)(ord >> 10) * nwarps] + (ord & 1023u);
+    });
 }
 
 // Occupied slots -> out[0 .. *nout), in any order (the host sorts the groups by first_row).

@@ -209,25 +209,60 @@ static cudaError_t launch_agg_as(const AggPlan& a, const uint32_t* bitmap, const
     agg_kernel<NG, NA><<<(unsigned)grid, kComputeThreads, smem, stream>>>(a, bitmap, span_cnt, table, overflow, ctrl);
     return cudaGetLastError();
 }
+// the instantiation for this query's shape: exact for <= 2 group-by columns and 1 .. 4 aggregates, the general forms beyond
+#define IMM3_AGG_DISPATCH(LAUNCH)                                                                                                         \
+    do {                                                                                                                                  \
+        const int ng = a.ngroup <= 2 ? a.ngroup : 4, na = (a.naggs >= 1 && a.naggs <= 4) ? a.naggs : 8;                                   \
+        IMM3_AGG_DISPATCH_ROW(LAUNCH, 0) else IMM3_AGG_DISPATCH_ROW(LAUNCH, 1) else IMM3_AGG_DISPATCH_ROW(LAUNCH, 2) else IMM3_AGG_DISPATCH_ROW(LAUNCH, 4) \
+    } while (0)
+#define IMM3_AGG_DISPATCH_ROW(LAUNCH, NG)                                                                                                  \
+    if (ng == NG) {                                                                                                                       \
+        if (na == 1) e = LAUNCH<NG, 1>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                                  \
+        else if (na == 2) e = LAUNCH<NG, 2>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                             \
+        else if (na == 3) e = LAUNCH<NG, 3>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                             \
+        else if (na == 4) e = LAUNCH<NG, 4>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                             \
+        else e = LAUNCH<NG, 8>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                                          \
+    }
 cudaError_t launch_agg(const AggPlan& a, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, AggEntry* out, unsigned int* counters,
                        const ScanCtrl* ctrl, int num_sms, cudaStream_t stream) {
     cudaError_t e = configure_once();
     if (e != cudaSuccess) return e;
-    // the instantiation for this query's shape: exact for <= 2 group-by columns and 1 .. 4 aggregates, the general forms beyond
-    const int ng = a.ngroup <= 2 ? a.ngroup : 4, na = (a.naggs >= 1 && a.naggs <= 4) ? a.naggs : 8;
-#define IMM3_AGG_CASE(NG, NA) \
-    if (ng == NG && na == NA) e = launch_agg_as<NG, NA>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream)
-#define IMM3_AGG_ROW(NG) IMM3_AGG_CASE(NG, 1); else IMM3_AGG_CASE(NG, 2); else IMM3_AGG_CASE(NG, 3); else IMM3_AGG_CASE(NG, 4); else IMM3_AGG_CASE(NG, 8)
-    if (ng == 0) { IMM3_AGG_ROW(0); }
-    else if (ng == 1) { IMM3_AGG_ROW(1); }
-    else if (ng == 2) { IMM3_AGG_ROW(2); }
-    else { IMM3_AGG_ROW(4); }
-#undef IMM3_AGG_ROW
-#undef IMM3_AGG_CASE
+    IMM3_AGG_DISPATCH(launch_agg_as);
     if (e != cudaSuccess) return e;
     agg_compact_kernel<<<(a.table_slots + kComputeThreads - 1) / kComputeThreads, kComputeThreads, 0, stream>>>(table, a.table_slots, out, counters);
     return cudaGetLastError();
 }
+
+// ... the same with agg_blocks_kernel (a MIN / MAX input or a group column in the sorted-int codec; blocks of <= 1024 rows)
+size_t agg_blocks_smem_bytes(int naggs, int npfor, int words_cap) {
+    const int na = (naggs >= 1 && naggs <= 4) ? naggs : 8;
+    return agg_blocks_state_bytes(na) + (size_t)kComputeWarps * (size_t)agg_blocks_warp_words(npfor, words_cap) * 4;
+}
+template <int NG, int NA>
+static cudaError_t launch_agg_blocks_as(const AggPlan& a, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, unsigned int* overflow,
+                                        const ScanCtrl* ctrl, int num_sms, cudaStream_t stream) {
+    const size_t smem = agg_blocks_smem_bytes(NA, a.npfor, a.blk_words_cap);
+    cudaError_t e = cudaSuccess;
+    if (smem > 48 * 1024 && (e = cudaFuncSetAttribute(agg_blocks_kernel<NG, NA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
+    int occ = 0;
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, agg_blocks_kernel<NG, NA>, kComputeThreads, smem);
+    if (e != cudaSuccess) return e;
+    if (occ < 1) return cudaErrorInvalidConfiguration;
+    const long long grid = std::max<long long>(1, std::min<long long>((a.nblocks + kComputeWarps - 1) / kComputeWarps, (long long)num_sms * occ));
+    agg_blocks_kernel<NG, NA><<<(unsigned)grid, kComputeThreads, smem, stream>>>(a, bitmap, span_cnt, table, overflow, ctrl);
+    return cudaGetLastError();
+}
+cudaError_t launch_agg_blocks(const AggPlan& a, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, AggEntry* out, unsigned int* counters,
+                              const ScanCtrl* ctrl, int num_sms, cudaStream_t stream) {
+    cudaError_t e = configure_once();
+    if (e != cudaSuccess) return e;
+    IMM3_AGG_DISPATCH(launch_agg_blocks_as);
+    if (e != cudaSuccess) return e;
+    agg_compact_kernel<<<(a.table_slots + kComputeThreads - 1) / kComputeThreads, kComputeThreads, 0, stream>>>(table, a.table_slots, out, counters);
+    return cudaGetLastError();
+}
+#undef IMM3_AGG_DISPATCH_ROW
+#undef IMM3_AGG_DISPATCH
 
 long long scan_inline_max_tiles() { return kScanInlineMaxTiles; }
 cudaError_t launch_offset_scan(const uint32_t* tile_cnt, unsigned long long* tile_off, long long ntiles, long long limit, uint32_t epoch,

@@ -113,7 +113,8 @@ struct PrunePlan {
 };
 
 // Aggregation (k_agg.cuh; ProjectAggOp, ProjectAggregate.scala:115-226): count / min / max over the rows the filter
-// kernel selected, grouped by up to kMaxGroupCols dense columns whose cells pack into at most 7 key bytes.
+// kernel selected, grouped by up to kMaxGroupCols columns whose cells pack into at most 7 key bytes.  A MIN / MAX input or
+// a group column in the sorted-int codec is decoded per block inside agg_blocks_kernel (its slot in agg_pfor / group_pfor).
 constexpr int kMaxAggs = 8;
 constexpr int kMaxGroupCols = 4;
 enum AggOp : int32_t { kAggCount = 0, kAggMin = 1, kAggMax = 2 };
@@ -135,6 +136,14 @@ struct AggPlan {
     int32_t pad;
     AggCol agg[kMaxAggs];
     GroupCol group[kMaxGroupCols];
+    // agg_blocks_kernel only (after the fields agg_kernel reads, which keep their parameter offsets):
+    int8_t agg_pfor[kMaxAggs];          // index into pfor[] of a MIN / MAX input in the sorted-int codec, -1 = dense
+    int8_t group_pfor[kMaxGroupCols];   // ... of a group column, -1 = dense
+    int32_t npfor;                      // distinct encoded columns decoded per block
+    int32_t blk_words_cap;              // per-warp scratch for one encoded block, in 32-bit words (from the columns' max_block_words)
+    int64_t nblocks;                    // reference blocks of the owned slice
+    const uint64_t* row_start;          // nblocks + 1 row ordinals of the blocks (row space of the dense arenas)
+    PforCol pfor[kMaxPforCols];
 };
 // One group in the global table / in the compacted result.  val[i]: COUNT -> the count, MIN / MAX -> the extreme as int64.
 struct AggEntry {

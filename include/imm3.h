@@ -203,8 +203,10 @@ int imm3_result_wait(imm3_result* r);
  * LinkedHashMaps produce with one worker); columns = the group columns (their own types), then one column per aggregate in
  * select-list order, named <col>_count / <col>_min / <col>_max (Engine.scala:136-152).  imm3_result_format_row prints the
  * aggregates only, as the reference does (Row of the aggregators' repr, ProjectAggregateQueue.scala:48-50).
- * Library limits (IMM3_ERR_UNSUPPORTED): group cells must pack into 7 bytes; aggregate and group columns must be dense;
- * predicates on a sorted-int-codec column cannot be combined with aggregation yet.  On a sharded handle the result holds
+ * Library limits (IMM3_ERR_UNSUPPORTED): group cells must pack into 7 bytes (a sorted-int-codec INT cell takes 4); aggregate
+ * and group columns may be dense or sorted-int-codec (PFOR_INT), but one query decodes at most 4 distinct sorted-int-codec
+ * columns, from blocks of at most 1024 rows; predicates on a sorted-int-codec column cannot be combined with aggregation
+ * yet.  On a sharded handle the result holds
  * this rank's groups (partials); the caller merges ranks in rank order (count: sum, min / max: min / max). */
 typedef enum imm3_agg_op { IMM3_AGG_COUNT = 0, IMM3_AGG_MIN = 1, IMM3_AGG_MAX = 2, IMM3_AGG_SUM = 3, IMM3_AGG_AVG = 4 } imm3_agg_op;
 typedef struct imm3_agg {
