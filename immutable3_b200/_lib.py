@@ -84,6 +84,7 @@ SIGNATURES = {
     "imm3_result_format_row": (C.c_int, [_P, C.c_int64, C.c_char_p, C.c_size_t]),
     "imm3_result_device_ms": (C.c_double, [_P]),
     "imm3_result_kernel_launches": (C.c_int, [_P]),
+    "imm3_result_route": (C.c_char_p, [_P]),
     "imm3_result_stage_ms": (C.c_double, [_P, C.c_int]),
     "imm3_result_host_us": (C.c_double, [_P, C.c_int]),
     "imm3_result_algorithmic_bytes": (C.c_int64, [_P]),

@@ -154,6 +154,8 @@ struct imm3_db {
     // for any result, so a stale hint costs time, never rows.
     std::unordered_map<std::string, int> emit_hint;
     std::string explain_buf;
+    std::string route;         // kernels queued by the query in progress (imm3_result_route), in launch order
+    const char* route_tag = "";  // appended to every name: "/prefix" while the prefix pass of a small LIMIT is queued
 };
 
 struct imm3_result {
@@ -175,6 +177,7 @@ struct imm3_result {
     double stage_ms[2] = {0, 0};
     double host_us[5] = {0, 0, 0, 0, 0};  // wall clock inside imm3_query_begin: plan, buffers + device plan, launches, wait for the GPU, epilogue
     int launches = 0;
+    std::string route;  // imm3_result_route: "kernel[/key=value...];kernel..." in launch order
     int64_t alg_bytes = 0;
 };
 
@@ -193,6 +196,20 @@ int use_device(imm3_db* db) {
     if (db->host_only) return fail(IMM3_ERR_STATE, "handle was opened with IMM3_OPEN_HOST_ONLY: no device work (there is no CPU fallback)");
     CUDA_TRY(cudaSetDevice(db->device));
     return 0;
+}
+
+// Route of the query in progress (imm3_result_route): one entry per queued kernel, recorded on the host only.
+void note_launch(imm3_db* db, int* launches, const std::string& name) {
+    if (launches) (*launches)++;
+    if (!db->route.empty()) db->route += ';';
+    db->route += name;
+    db->route += db->route_tag;
+}
+std::string with_stages(const char* name, int stages) { return std::string(name) + "/s=" + std::to_string(stages); }
+// the kernel launch_filter picks for this plan
+std::string filter_route(const ScanPlan& sp) {
+    if (sp.nfilter == 0) return "select_all";
+    return sp.stages > 0 ? with_stages("filter(tma)", sp.stages) : std::string("filter(direct)");
 }
 
 // ---- SegmentManager upload path: files -> pinned staging -> HBM --------------------------------
@@ -817,6 +834,7 @@ int launch_exchange(imm3_db* db, int64_t limit, int has_count, unsigned long lon
     cp.limit = limit;
     cp.timeout_ns = db->comm_timeout_ns;
     CUDA_TRY(launch_count_exchange(cp, db->d_ctrl, &reinterpret_cast<CtrlBlock*>(db->d_ctrl)->x, db->stream));
+    note_launch(db, nullptr, "count_exchange");  // (the caller counts the launch where it has a count)
     return 0;
 }
 
@@ -868,7 +886,7 @@ int launch_scan_kernel(imm3_db* db, const ScanPlan& sp, int64_t ntiles, int* lau
     (void)nchunks;
     CUDA_TRY(launch_offset_scan((const uint32_t*)db->d_tile_cnt.p, (unsigned long long*)db->d_tile_off.p, ntiles, sp.limit, db->scan_epoch,
                                 (unsigned long long*)db->d_scan_part.p, db->d_ctrl, want_list ? (unsigned int*)db->d_tile_list.p : nullptr, db->stream));
-    (*launches)++;
+    note_launch(db, launches, "offset_scan");
     return 0;
 }
 
@@ -886,7 +904,7 @@ int launch_or_terms(imm3_db* db, Prepared* pr, int scan_inline, int* launches) {
         tm->sp.scan_inline = (i + 1 == pr->or_terms.size()) ? scan_inline : 0;
         CUDA_TRY(launch_filter(tm->sp, tm->sp.bitmap, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p, (unsigned long long*)db->d_tile_off.p,
                                db->d_ctrl, (int)std::max<int64_t>(1, std::min<int64_t>(tm->grid, tm->sp.ntiles)), tm->dyn_smem, db->stream));
-        (*launches)++;
+        note_launch(db, launches, filter_route(tm->sp));
     }
     return 0;
 }
@@ -917,7 +935,7 @@ int run_scan_once(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* la
         CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
         CUDA_TRY(launch_filter(pr->sp, pr->sp.bitmap, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
                                (unsigned long long*)db->d_tile_off.p, db->d_ctrl, pr->grid, pr->dyn_smem, db->stream));
-        *launches = 1;
+        note_launch(db, launches, filter_route(pr->sp));
         if ((rc = launch_or_terms(db, pr, scan_inline_h, launches))) return rc;
         pr->sp.scan_inline = scan_inline_h;
         if (!pr->sp.scan_inline && (rc = launch_scan_kernel(db, pr->sp, ntiles, launches))) return rc;
@@ -930,7 +948,7 @@ int run_scan_once(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* la
             CUDA_TRY(launch_blocks_emit(pr->sp, pr->sp.bitmap, (const uint32_t*)db->d_span_cnt.p, nullptr, (const unsigned long long*)db->d_tile_off.p,
                                         nblocks_use, db->d_ctrl, true, pdl, (int)std::min<int64_t>(pr->grid_blocks_emit, (nblocks_use + 7) / 8),
                                         pr->blocks_emit_smem, db->stream));
-            (*launches)++;
+            note_launch(db, launches, "blocks_emit(rowspace)");
         }
         CUDA_TRY(cudaEventRecord(db->ev1, db->stream));
     } else if (pr->block_mode && pr->blocks_multi) {
@@ -984,14 +1002,16 @@ int run_scan_once(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* la
             CUDA_TRY(cudaMemsetAsync(db->d_work.p, 0, 4, db->stream));
             CUDA_TRY(launch_blocks_prune(pr->pp, t.d_row_start, nblocks, ntiles, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
                                          (unsigned int*)db->d_work.p, db->num_sms, db->stream, grp_sum));
-            (*launches)++;
+            note_launch(db, launches, "blocks_prune");
         }
         CUDA_TRY(launch_blocks_filter(pr->sp, (uint32_t*)db->d_bitmap.p, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
                                       (unsigned long long*)db->d_tile_off.p, db->d_ctrl, nblocks,
                                       pr->lane ? (int)std::max<int64_t>(1, std::min<int64_t>(pr->grid, (nblocks + 32 * pr->lane_warps - 1) / (32 * pr->lane_warps)))
                                                : (pr->quad ? (int)std::max<int64_t>(1, std::min<int64_t>(pr->grid, (nblocks + 31) / 32)) : pr->grid),
                                       pr->dyn_smem, pr->lane ? (2 | (pr->lane_warps << 8)) : (pr->quad ? 1 : 0), work, db->stream, grp_sum));
-        (*launches)++;
+        note_launch(db, launches, pr->lane   ? "blocks_filter_lane/w=" + std::to_string(pr->lane_warps) + "/s=" + std::to_string(pr->sp.stages)
+                                  : pr->quad ? with_stages("blocks_filter_quad", pr->sp.stages)
+                                             : with_stages("blocks_filter", pr->sp.stages));
         if (group_grid > 0) {
             // one encoded column projected, lane kernel in front: every emit warp finds its rows from the group sums - no scan
             const bool pdl = !getenv("IMM3_NO_PDL");
@@ -1002,7 +1022,7 @@ int run_scan_once(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* la
             CUDA_TRY(launch_blocks_group_emit(pr->sp, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, grp_sum, nblocks, ngroups,
                                               db->d_ctrl, pdl, group_grid, db->stream, publish_here ? db->h_ctrl : nullptr, publish_here ? pub_seq : 0));
             published = publish_here;
-            (*launches)++;
+            note_launch(db, launches, "blocks_group_emit/ctas=" + std::to_string(group_grid));
             CUDA_TRY(cudaEventRecord(db->ev1, db->stream));
         } else if (fused_grid > 0) {
             // one encoded column projected: offset scan + emit in one small-footprint kernel, resident while the filter kernel runs
@@ -1016,7 +1036,7 @@ int run_scan_once(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* la
                                              db->d_ctrl, (unsigned int*)db->d_tile_list.p, pdl, fused_grid, db->stream,
                                              publish_here ? db->h_ctrl : nullptr, publish_here ? pub_seq : 0));
             published = publish_here;
-            (*launches)++;
+            note_launch(db, launches, "blocks_scan_emit");
             CUDA_TRY(cudaEventRecord(db->ev1, db->stream));
         } else {
         if (!pr->sp.scan_inline && (rc = launch_scan_kernel(db, pr->sp, ntiles, launches, true))) return rc;
@@ -1030,7 +1050,7 @@ int run_scan_once(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* la
                                         pr->sp.scan_inline ? nullptr : (const unsigned int*)db->d_tile_list.p,
                                         (const unsigned long long*)db->d_tile_off.p, nblocks, db->d_ctrl, false, pdl,
                                         (int)std::min<int64_t>(pr->grid_blocks_emit, (nblocks + 7) / 8), pr->blocks_emit_smem, db->stream));
-            (*launches)++;
+            note_launch(db, launches, "blocks_emit(blocks)");
         }
         CUDA_TRY(cudaEventRecord(db->ev1, db->stream));
         }
@@ -1073,7 +1093,7 @@ int run_scan_once(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* la
         CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
         CUDA_TRY(launch_filter(pr->sp, pr->sp.bitmap, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
                                (unsigned long long*)db->d_tile_off.p, db->d_ctrl, pr->grid, pr->dyn_smem, db->stream));
-        *launches = 1;
+        note_launch(db, launches, filter_route(pr->sp));
         if ((rc = launch_or_terms(db, pr, scan_inline_d, launches))) return rc;
         pr->sp.scan_inline = scan_inline_d;
         if (!pr->sp.scan_inline && (rc = launch_scan_kernel(db, pr->sp, nsub, launches))) return rc;
@@ -1089,13 +1109,13 @@ int run_scan_once(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* la
                 CUDA_TRY(launch_emit_stream(pr->sp, pr->sp.bitmap, (const uint32_t*)db->d_span_cnt.p, (const uint32_t*)db->d_tile_cnt.p,
                                             (const unsigned long long*)db->d_tile_off.p, nsub, pr->emit_ring, pr->emit_stage_bytes,
                                             only_stream ? -1 : 1, pr->grid_emit_stream, pr->emit_smem, db->d_ctrl, pdl, db->stream));
-                (*launches)++;
+                note_launch(db, launches, with_stages("emit_stream", pr->emit_ring));
             }
             if (!only_stream) {
                 CUDA_TRY(launch_emit(pr->sp, pr->sp.bitmap, (const uint32_t*)db->d_span_cnt.p, (const unsigned long long*)db->d_tile_off.p, 8,
                                      nspans, pr->grid_emit, stream_ok && !only_gather, db->d_ctrl, pr->emit_general, pdl && (only_gather || !stream_ok),
                                      db->stream));
-                (*launches)++;
+                note_launch(db, launches, pr->emit_general ? "emit_general" : "emit");
             }
         }
         CUDA_TRY(cudaEventRecord(db->ev1, db->stream));
@@ -1109,7 +1129,7 @@ int run_scan_once(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* la
         CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
         CUDA_TRY(launch_scan_blocks(pr->sp, db->d_ctrl, db->d_status, pr->grid, pr->dyn_smem, db->stream));  // (single-pass block kernel: blocks > 1024 rows, bitmaps)
         CUDA_TRY(cudaEventRecord(db->ev1, db->stream));
-        *launches = 1;
+        note_launch(db, launches, "scan_blocks");
     }
     if (exchange && db->comm_on) {
         // The per-rank counts are exchanged by the GPUs themselves (k_comm.cuh), behind the query's last kernel: no host
@@ -1222,6 +1242,7 @@ int run_scan(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* launche
     const bool block_prefix = pr->block_mode && pr->blocks_multi && pr->prefix_blocks > 0;
     const bool dense_prefix = !pr->block_mode && pr->multipass && pr->prefix_rows > 0;
     const bool two_phase = comm ? small_limit_policy(pr->lp) : (block_prefix || dense_prefix);
+    db->route.clear();
     if (!two_phase) return run_scan_once(db, pr, ms, total, launches, stage_ms, t.nblocks, comm);
     struct EagerGuard {
         EagerGuard() { g_eager_times = true; }
@@ -1247,7 +1268,9 @@ int run_scan(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* launche
     }
     double ms_a = 0, st_a[2] = {0, 0};
     int launches_a = 0;
+    if (local_prefix) db->route_tag = "/prefix";
     int rc = run_scan_once(db, pr, &ms_a, total, &launches_a, st_a, nb, comm);
+    db->route_tag = "";
     pr->sp = full;
     pr->grid = grid_full;
     if (rc) return rc;
@@ -1582,10 +1605,12 @@ static int query_begin_terms(imm3_db* db, const char* table, const std::vector<s
         // Empty slice (more ranks than segments): this rank still takes part in every round of the exchange.  (A predicate
         // that can never hold is a property of the query, known to every rank: nobody exchanges anything.)
         const int64_t lim = limit > 0 ? limit : INT64_MAX;
+        db->route.clear();
         if ((rc = exchange_only(db, lim, 0))) { give_back(); return rc; }
         if (small_limit_policy(pr.lp) && (int64_t)db->h_ctrl->x.counts[0] < pr.lp.limit && (rc = exchange_only(db, lim, 0))) { give_back(); return rc; }
         r->launches = 1;
     }
+    r->route = r->launches > 0 ? db->route : std::string();
     // Global placement of this rank's rows (SURVEY.md 8e): from the on-device exchange, or trivially for a single handle.
     r->world = 1;
     r->g_offset = 0;
@@ -1888,6 +1913,12 @@ int imm3_query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int n
                                 (AggEntry*)db->d_agg_out.p, (unsigned int*)db->d_agg_cnt.p, db->d_ctrl, db->num_sms, db->stream));
         CUDA_TRY(cudaEventRecord(db->ev1, db->stream));
         r->launches = 4;
+        {
+            // the instantiation IMM3_AGG_DISPATCH (kernels.cu) picks: <= 2 group-by columns exact, else 4; 1 .. 4 aggregates exact, else 8
+            const int ng = ngroup <= 2 ? ngroup : 4, na = (naggs >= 1 && naggs <= 4) ? naggs : 8;
+            const std::string inst = "<" + std::to_string(ng) + "," + std::to_string(na) + ">";
+            r->route = "agg_init;" + filter_route(sp) + ";" + (on_blocks ? "agg_blocks" : "agg") + inst + ";agg_compact";
+        }
         unsigned int counters[2] = {0, 0};
         CUDA_TRY(cudaMemcpyAsync(db->h_ctrl, db->d_ctrl, sizeof(CtrlBlock), cudaMemcpyDeviceToHost, db->stream));
         CUDA_TRY(cudaMemcpyAsync(counters, db->d_agg_cnt.p, sizeof counters, cudaMemcpyDeviceToHost, db->stream));
@@ -1981,6 +2012,7 @@ double imm3_result_device_ms(const imm3_result* r) {
     return r->device_ms;
 }
 int imm3_result_kernel_launches(const imm3_result* r) { return r ? r->launches : IMM3_ERR_INVALID_ARG; }
+const char* imm3_result_route(const imm3_result* r) { return r ? r->route.c_str() : nullptr; }
 double imm3_result_host_us(const imm3_result* r, int phase) { return (r && phase >= 0 && phase < 5) ? r->host_us[phase] : -1.0; }
 double imm3_result_stage_ms(const imm3_result* r, int stage) {
     if (!r || stage < 0 || stage >= 2) return -1.0;

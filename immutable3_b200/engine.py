@@ -283,6 +283,11 @@ class Result:
     def kernel_launches(self) -> int:
         return int(self._lib.imm3_result_kernel_launches(self._h))
 
+    @property
+    def route(self) -> str:
+        """The kernels the query queued, in launch order: "blocks_prune;blocks_filter_lane/w=11/s=2;blocks_group_emit/ctas=148"."""
+        return (self._lib.imm3_result_route(self._h) or b"").decode()
+
     def stage_ms(self, stage: int) -> float:
         return float(self._lib.imm3_result_stage_ms(self._h, stage))
 

@@ -230,6 +230,14 @@ const void* imm3_result_col_device(const imm3_result* r, int col); /* device cop
 int imm3_result_format_row(const imm3_result* r, int64_t row, char* buf, size_t buflen);
 double imm3_result_device_ms(const imm3_result* r);         /* CUDA-event time of the kernels of begin  */
 int imm3_result_kernel_launches(const imm3_result* r);      /* kernels launched by begin                */
+/* The kernels imm3_query_begin / imm3_query_agg queued, in launch order, separated by ';' ("" when none ran): kernel names
+ * (select_all, filter(tma|direct), offset_scan, emit_stream, emit, emit_general, blocks_prune, blocks_filter_lane,
+ * blocks_filter_quad, blocks_filter, blocks_group_emit, blocks_scan_emit, blocks_emit(rowspace|blocks), scan_blocks,
+ * count_exchange, agg_init, agg<NG,NA>, agg_blocks<NG,NA>, agg_compact) with "/key=value" parameters: /s= ring stages,
+ * /w= warps per CTA of the lane kernel, /ctas= the group emit kernel's grid; "/prefix" marks the prefix pass of a small
+ * LIMIT.  E.g. "blocks_prune;blocks_filter_lane/w=11/s=2;blocks_group_emit/ctas=148".  Owned by the result (valid until
+ * imm3_result_free). */
+const char* imm3_result_route(const imm3_result* r);
 /* CUDA-event time of one stage of begin: 0 = filter (+scan) kernel, 1 = emit kernel (multi-pass path);
  * the fused single-pass kernels report everything as stage 0. */
 double imm3_result_stage_ms(const imm3_result* r, int stage);

@@ -1,6 +1,7 @@
 """Parity tests proper: the CUDA path (through the C ABI) against the CPU oracle, bit-exact, on the
 same tables and queries — rows, values and order (SURVEY.md §3.4-8).  Every test needs a GPU."""
 import os
+import re
 
 import numpy as np
 import pytest
@@ -15,10 +16,15 @@ from immutable3_b200.loader import synth_write
 
 pytestmark = pytest.mark.gpu
 
-# variant -> (imm3_open flags, IMM3_PATH): the filter -> offset scan -> emit pipeline with TMA staging / direct loads, the
-# single-pass block kernel forced onto dense tables (IMM3_PATH=fused selects it on block tables), and the library's own choice.
-VARIANT_DEFS = {"blocks": (OPEN_FORCE_BLOCKS, "fused"), "blocks_multi": (OPEN_FORCE_BLOCKS, ""),
-                "multi": (0, "multi"), "multi_direct": (OPEN_NO_TMA, "multi"), "auto": (0, "")}
+# variant -> (imm3_open flags, IMM3_PATH): the single-pass block kernel forced onto dense tables (IMM3_PATH=fused selects it
+# on block tables), the block pipeline forced onto dense tables (row-space filter kernel -> block emit kernel) with TMA staging /
+# direct loads, the dense multi-pass pipeline (filter -> offset scan -> emit: what the library picks for a dense table) with TMA
+# staging / direct loads, and the library's own choice.  On the dense tables below "multi" is the same configuration as "auto";
+# it also checks from the route that the multi-pass kernels ran, and "multi_direct" that no TMA kernel did (ROUTE_CHECKS).
+VARIANT_DEFS = {"blocks": (OPEN_FORCE_BLOCKS, "fused"), "blocks_multi": (OPEN_FORCE_BLOCKS, ""), "blocks_no_tma": (OPEN_FORCE_BLOCKS | OPEN_NO_TMA, ""),
+                "multi": (0, ""), "multi_direct": (OPEN_NO_TMA, ""), "auto": (0, "")}
+ROUTE_CHECKS = {"multi": r"^(?!.*(blocks_|scan_blocks))", "multi_direct": r"^(?!.*(blocks_|scan_blocks|filter\(tma\)|emit_stream))",
+                "blocks": r"^(scan_blocks)?$", "blocks_no_tma": r"^(?!.*(filter\(tma\)|emit_stream))"}
 VARIANTS = {k: v[0] for k, v in VARIANT_DEFS.items()}
 
 
@@ -59,10 +65,13 @@ def set_path(variant):
         os.environ.pop("IMM3_PATH", None)
 
 
-def check(orc, sm, table, select, proj, limit=0, variant=""):
+def check(orc, sm, table, select, proj, limit=0, variant="", route=None):
+    """Rows, values and order against the oracle; `route`: a regex the query's kernel route (Result.route) must match."""
     set_path(variant)
     exp = orc.query(table, oracle_preds(select), proj, limit=limit)
     with Engine(sm).execute(Query(table, select, Project(proj, limit))) as got:
+        for want in (route, ROUTE_CHECKS.get(variant.split("/")[0])):
+            assert want is None or re.search(want, got.route), (variant, table, select, proj, limit, got.route, want)
         assert got.nrows == exp.nrows, (variant, table, select, proj, limit, got.nrows, exp.nrows)
         for c in range(len(proj)):
             a, b = got.column(c), exp.columns[c]
@@ -150,22 +159,30 @@ def test_edge_sizes(world, variant):
     check(orc, sms[variant], "t", NoSelect, [], 0, variant)  # empty select list: only the row count
 
 
-@pytest.mark.parametrize("w,stages", [(1, 3), (1, 4), (2, 3), (2, 4), (4, 3), (4, 4)])
-def test_dense_tile_shapes(world, w, stages, monkeypatch):
-    """Every tile size (8192*W rows) and TMA ring depth gives the same rows: multi-round selection vectors
-    (NoSelect fills a tile with matches), partial last tiles, LIMIT cuts inside and across tiles."""
+@pytest.mark.parametrize("filter_stages,emit_stages", [(2, 2), (2, 3), (2, 4), (3, 2), (3, 3), (3, 4), (6, 2), (6, 3), (6, 4)])
+def test_dense_tile_shapes(world, filter_stages, emit_stages, monkeypatch):
+    """Every TMA ring depth of the dense filter kernel (IMM3_FILTER_STAGES, 8192-row stages) and of the streaming emit kernel
+    (IMM3_EMIT_STAGES) gives the same rows: multi-round selection vectors (NoSelect fills a tile with matches), partial last
+    tiles, LIMIT cuts inside and across tiles; the direct-load filter kernel (OPEN_NO_TMA, "multi_direct") alongside."""
     d, tables, orc, sms = world
-    monkeypatch.setenv("IMM3_DENSE_W", str(w))
-    monkeypatch.setenv("IMM3_DENSE_STAGES", str(stages))
+    monkeypatch.setenv("IMM3_FILTER_STAGES", str(filter_stages))
+    monkeypatch.setenv("IMM3_EMIT_STAGES", str(emit_stages))
+    # the filter kernel's ring as asked (every filter below fits 6 stages of 8192 rows in 200 KB); a streaming emit kernel, when
+    # the result density makes it run, with its ring as asked
+    route = rf"^(?!.*emit_stream/s=(?!{emit_stages}(;|$))).*(^|;)filter\(tma\)/s={filter_stages}(;|$)"
     for variant in ("multi", "multi_direct"):
         for sel, proj in QUERIES_T[:5] + [(NoSelect, ["id", "state", "age"])]:
             for limit in (0, 10, 8191, 8193, 20_000):
-                check(orc, sms[variant], "t", sel, proj, limit, f"{variant}/W{w}/S{stages}")
-        check(orc, sms[variant], "wide", Select("name", Match(["carol"])), ["id", "name", "zip"], 0, f"{variant}/W{w}")
+                check(orc, sms[variant], "t", sel, proj, limit, f"{variant}/F{filter_stages}/E{emit_stages}",
+                      route=route if variant == "multi" and sel is not NoSelect else None)
+        check(orc, sms[variant], "wide", Select("name", Match(["carol"])), ["id", "name", "zip"], 0, f"{variant}/F{filter_stages}")
         set_path(variant)
         got, nsel = Engine(sms[variant]).filter_bitmap("t", Select("age", LT(50)))
         want, wsel = orc.filter_bitmap("t", oracle_preds(Select("age", LT(50))))
         assert nsel == wsel and np.array_equal(got, want)
+    monkeypatch.setenv("IMM3_EMIT", "stream")  # the streaming emit kernel takes every result
+    for limit in (0, 8193):
+        check(orc, sms["multi"], "t", QUERIES_T[0][0], QUERIES_T[0][1], limit, "multi/stream", route=rf";emit_stream/s={emit_stages}$")
 
 
 def test_readme_cli_query_and_row_format(world):
@@ -312,8 +329,8 @@ def test_full_size_synthetic_properties(tmp_path_factory):
     age = np.concatenate([np.fromfile(d / "syn" / f"age_{i}.dat", np.int8) for i in order])
     ids = np.concatenate([np.fromfile(d / "syn" / f"id_{i}.dat", "<i4") for i in order])
     st = np.concatenate([np.fromfile(d / "syn" / f"state_{i}.dat", "S2") for i in order])
-    for flags, path in ((0, "multi"), (OPEN_NO_TMA, "multi"), (0, "")):
-        set_path({"multi": "multi", "": "auto"}[path])
+    set_path("auto")
+    for flags in (0, OPEN_NO_TMA):
         with SegmentManager(d, flags=flags) as sm:
             eng = Engine(sm)
             m = (age > 18) & (age < 30)
