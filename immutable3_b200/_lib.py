@@ -73,6 +73,7 @@ SIGNATURES = {
     "imm3_result_fetch_async": (C.c_int, [_P, C.c_int64]),
     "imm3_result_wait": (C.c_int, [_P]),
     "imm3_query_agg": (C.c_int, [_P, C.c_char_p, C.POINTER(Pred), C.c_int, C.POINTER(Agg), C.c_int, _STRS, C.c_int, _PP]),
+    "imm3_query_agg_global": (C.c_int, [_P, C.c_char_p, C.POINTER(Pred), C.c_int, C.POINTER(Agg), C.c_int, _STRS, C.c_int, _PP]),
     "imm3_query_sql": (C.c_int, [_P, C.c_char_p, _PP]),
     "imm3_result_nrows": (C.c_int64, [_P]),
     "imm3_result_ncols": (C.c_int, [_P]),

@@ -133,6 +133,7 @@ struct imm3_db {
     unsigned long long* comm_peer[kMaxWorld] = {};
     bool comm_on = false;
     uint32_t comm_epoch = 0;
+    uint32_t agg_seq = 0;  // global aggregates exchanged since imm3_comm_connect (identical on all ranks): exchange buffer agg_seq & 1
     unsigned long long comm_timeout_ns = 30000000000ull;
     unsigned long long* d_status = nullptr;
     size_t status_cap = 0;
@@ -1393,7 +1394,7 @@ int imm3_comm_local_handle(imm3_db* db, void* handle_out) {
     if (rc) return rc;
     if (db->world > kMaxWorld) return fail(IMM3_ERR_UNSUPPORTED, "count exchange supports at most %d ranks (world = %d)", kMaxWorld, db->world);
     if (!db->d_mailbox) {
-        CUDA_TRY(cudaMalloc(&db->d_mailbox, kMailboxBytes));
+        CUDA_TRY(cudaMalloc(&db->d_mailbox, kCommAllocBytes));  // the mailbox ring, then the exchange area of global aggregates
         CUDA_TRY(cudaMemset(db->d_mailbox, 0, kMailboxBytes));
     }
     cudaIpcMemHandle_t h;
@@ -1431,6 +1432,7 @@ int imm3_comm_connect(imm3_db* db, const void* handles, int nhandles) {
     }
     db->comm_on = db->world > 1;
     db->comm_epoch = 0;
+    db->agg_seq = 0;
     return 0;
 }
 
@@ -1765,12 +1767,22 @@ int imm3_query(imm3_db* db, const char* table, const imm3_pred* preds, int npred
     return 0;
 }
 
-int imm3_query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, const imm3_agg* aggs, int naggs,
-                   const char* const* group_cols, int ngroup, imm3_result** out) {
-    if (!db || !out || (naggs > 0 && !aggs) || (ngroup > 0 && !group_cols)) return fail(IMM3_ERR_INVALID_ARG, "imm3_query_agg: NULL argument");
-    if (naggs < 1) return fail(IMM3_ERR_INVALID_ARG, "imm3_query_agg: no aggregates");
-    if (naggs > kMaxAggs) return fail(IMM3_ERR_UNSUPPORTED, "imm3_query_agg: at most %d aggregates", kMaxAggs);
-    if (ngroup > kMaxGroupCols) return fail(IMM3_ERR_UNSUPPORTED, "imm3_query_agg: at most %d group-by columns", kMaxGroupCols);
+namespace {
+
+// imm3_query_agg (global = false) and imm3_query_agg_global: one validation, one plan, one launch sequence.  The global form
+// on a connected handle compacts this rank's partial groups into its exchange buffer instead of the result buffer and
+// queues the exchange and the merge behind them (k_comm.cuh agg_exchange_kernel, k_agg.cuh agg_merge_kernel; DESIGN §4.3).
+int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, const imm3_agg* aggs, int naggs, const char* const* group_cols,
+              int ngroup, bool global, imm3_result** out) {
+    const char* const fn = global ? "imm3_query_agg_global" : "imm3_query_agg";
+    if (!db || !out || (naggs > 0 && !aggs) || (ngroup > 0 && !group_cols)) return fail(IMM3_ERR_INVALID_ARG, "%s: NULL argument", fn);
+    // A sharded handle merges over the communicator; a single handle's partials are the global result already.
+    const bool xchg = global && db->world > 1;
+    if (xchg && !db->comm_on)
+        return fail(IMM3_ERR_STATE, "%s: a sharded handle (rank %d of %d) merges over the communicator: call imm3_comm_connect first", fn, db->rank, db->world);
+    if (naggs < 1) return fail(IMM3_ERR_INVALID_ARG, "%s: no aggregates", fn);
+    if (naggs > kMaxAggs) return fail(IMM3_ERR_UNSUPPORTED, "%s: at most %d aggregates", fn, kMaxAggs);
+    if (ngroup > kMaxGroupCols) return fail(IMM3_ERR_UNSUPPORTED, "%s: at most %d group-by columns", fn, kMaxGroupCols);
     Prepared pr;
     int rc = prepare(db, table, preds, npreds, nullptr, 0, 0, &pr);  // validation before any device work
     if (rc) return rc;
@@ -1846,13 +1858,32 @@ int imm3_query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int n
     const bool on_blocks = !pfor_cols.empty();
     if (pfor_cols.size() > (size_t)kMaxPforCols)
         return fail(IMM3_ERR_UNSUPPORTED, "aggregation decodes at most %d distinct sorted-int-codec columns, the query reads %zu", kMaxPforCols, pfor_cols.size());
-    if (on_blocks && t.max_block_rows > 1024)
-        return fail(IMM3_ERR_UNSUPPORTED, "aggregation over sorted-int-codec columns decodes blocks of at most 1024 rows, table %s has a block of %d",
-                    t.meta.name.c_str(), t.max_block_rows);
+    ap.table_slots = 1u << 16;
+    if (const char* e = getenv("IMM3_AGG_SLOTS")) {  // (tests shrink it to exercise the overflow report)
+        uint32_t v = (uint32_t)atoi(e);
+        if (v >= 64 && (v & (v - 1)) == 0) ap.table_slots = v;
+    }
+    if (xchg && ap.table_slots > kAggXchgSlots)
+        return fail(IMM3_ERR_UNSUPPORTED, "%s: IMM3_AGG_SLOTS = %u exceeds the exchange buffer of %u groups", fn, ap.table_slots, kAggXchgSlots);
+    // Refusals that depend on this rank's slice: a global aggregate posts them to the peers (every rank then returns the
+    // same status) instead of returning before the exchange.
+    std::string refusal;
+    auto refuse_slice = [&](int code) -> int {
+        if (!xchg) return code;
+        refusal = last_error();
+        return 0;
+    };
+    if (on_blocks && t.max_block_rows > 1024 &&
+        (rc = refuse_slice(fail(IMM3_ERR_UNSUPPORTED, "aggregation over sorted-int-codec columns decodes blocks of at most 1024 rows, table %s has a block of %d",
+                                t.meta.name.c_str(), t.max_block_rows))))
+        return rc;
     if ((rc = use_device(db))) return rc;
     int64_t ngroups_out = 0;
     std::vector<AggEntry> groups;
-    if (!pr.lp.always_empty && t.nrows > 0) {
+    const bool merge = xchg && !pr.lp.always_empty;          // every rank of a connected handle takes part, an empty slice too
+    bool local = !pr.lp.always_empty && t.nrows > 0 && refusal.empty();
+    ScanPlan& sp = pr.sp;
+    if (local) {
         // The filter runs in row space exactly as for a Project query without a select list (dense filter kernel: bitmap,
         // span counts, total); the aggregation kernel is queued behind it, one synchronisation for the whole query.
         const bool was_block = pr.block_mode;
@@ -1861,7 +1892,6 @@ int imm3_query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int n
         pr.for_bitmap = false;
         if ((rc = fill_scan_plan(db, &pr))) return rc;
         pr.block_mode = was_block;
-        ScanPlan& sp = pr.sp;
         sp.bitmap = nullptr;
         const int64_t ntiles = sp.ntiles, nspans = ntiles * 8;
         if ((rc = ensure_buf(&db->d_bitmap, (size_t)(ntiles * kDenseTileRowsPerWord / 32 + 64) * 4))) return rc;
@@ -1869,14 +1899,6 @@ int imm3_query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int n
         const size_t ntiles_pad = ((size_t)ntiles + 4095) / 4096 * 4096 + 16;
         if ((rc = ensure_buf(&db->d_tile_cnt, ntiles_pad * 4))) return rc;
         if ((rc = ensure_buf(&db->d_tile_off, ntiles_pad * 8))) return rc;
-        ap.table_slots = 1u << 16;
-        if (const char* e = getenv("IMM3_AGG_SLOTS")) {  // (tests shrink it to exercise the overflow report)
-            uint32_t v = (uint32_t)atoi(e);
-            if (v >= 64 && (v & (v - 1)) == 0) ap.table_slots = v;
-        }
-        if ((rc = ensure_buf(&db->d_agg_table, (size_t)ap.table_slots * sizeof(AggEntry)))) return rc;
-        if ((rc = ensure_buf(&db->d_agg_out, (size_t)ap.table_slots * sizeof(AggEntry)))) return rc;
-        if ((rc = ensure_buf(&db->d_agg_cnt, 64))) return rc;
         ap.nrows = t.nrows;
         ap.ntiles = ntiles;
         for (int g = 0; g < ngroup; g++) ap.group[g].base = t.cols[(size_t)gidx[(size_t)g]].d_arena;
@@ -1896,43 +1918,102 @@ int imm3_query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int n
             int optin = 0;
             CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, db->device));
             const size_t smem = agg_blocks_smem_bytes(naggs, ap.npfor, ap.blk_words_cap);
-            if (smem + 1024 > (size_t)optin)  // (1 KB: the kernel's static shared memory)
-                return fail(IMM3_ERR_UNSUPPORTED, "aggregation over %d sorted-int-codec columns with %d aggregates needs %zu bytes of shared memory per CTA, the device has %d",
-                            ap.npfor, naggs, smem + 1024, optin);
+            if (smem + 1024 > (size_t)optin) {  // (1 KB: the kernel's static shared memory)
+                if ((rc = refuse_slice(fail(IMM3_ERR_UNSUPPORTED, "aggregation over %d sorted-int-codec columns with %d aggregates needs %zu bytes of shared memory per CTA, the device has %d",
+                                            ap.npfor, naggs, smem + 1024, optin))))
+                    return rc;
+                local = false;
+            }
         }
         sp.scan_inline = 1;  // (only the total matters here; the last CTA's scan provides it)
+    }
+    if (local || merge) {
+        if ((rc = ensure_buf(&db->d_agg_table, (size_t)ap.table_slots * sizeof(AggEntry)))) return rc;
+        if ((rc = ensure_buf(&db->d_agg_out, (size_t)ap.table_slots * sizeof(AggEntry)))) return rc;
+        if ((rc = ensure_buf(&db->d_agg_cnt, 64 + sizeof(AggXOut)))) return rc;  // [groups, overflow] counters, then the exchange's AggXOut
+        unsigned int* const counters = (unsigned int*)db->d_agg_cnt.p;
+        AggXOut* const d_x = reinterpret_cast<AggXOut*>((uint8_t*)db->d_agg_cnt.p + 64);
+        // the local groups go to this aggregate's exchange buffer when they are merged, else straight to the result buffer
+        auto xbuf = [&](int rank) {
+            return reinterpret_cast<AggEntry*>((uint8_t*)db->comm_peer[rank] + kAggXchgOff + (size_t)(db->agg_seq & 1u) * kAggXchgSlots * sizeof(AggEntry));
+        };
+        AggEntry* const local_out = merge ? xbuf(db->rank) : (AggEntry*)db->d_agg_out.p;
+        r->route.clear();
         CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
-        CUDA_TRY(launch_agg_init((AggEntry*)db->d_agg_table.p, ap.table_slots, ap, (unsigned int*)db->d_agg_cnt.p, db->stream));
-        CUDA_TRY(launch_filter(sp, (uint32_t*)db->d_bitmap.p, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
-                               (unsigned long long*)db->d_tile_off.p, db->d_ctrl, pr.grid, pr.dyn_smem, db->stream));
-        if (on_blocks)
-            CUDA_TRY(launch_agg_blocks(ap, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, (AggEntry*)db->d_agg_table.p,
-                                       (AggEntry*)db->d_agg_out.p, (unsigned int*)db->d_agg_cnt.p, db->d_ctrl, db->num_sms, db->stream));
-        else
-            CUDA_TRY(launch_agg(ap, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, (AggEntry*)db->d_agg_table.p,
-                                (AggEntry*)db->d_agg_out.p, (unsigned int*)db->d_agg_cnt.p, db->d_ctrl, db->num_sms, db->stream));
-        CUDA_TRY(cudaEventRecord(db->ev1, db->stream));
-        r->launches = 4;
-        {
+        if (local) {
+            CUDA_TRY(launch_agg_init((AggEntry*)db->d_agg_table.p, ap.table_slots, ap, counters, db->stream));
+            CUDA_TRY(launch_filter(sp, (uint32_t*)db->d_bitmap.p, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
+                                   (unsigned long long*)db->d_tile_off.p, db->d_ctrl, pr.grid, pr.dyn_smem, db->stream));
+            if (on_blocks)
+                CUDA_TRY(launch_agg_blocks(ap, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, (AggEntry*)db->d_agg_table.p,
+                                           local_out, counters, db->d_ctrl, db->num_sms, db->stream));
+            else
+                CUDA_TRY(launch_agg(ap, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, (AggEntry*)db->d_agg_table.p,
+                                    local_out, counters, db->d_ctrl, db->num_sms, db->stream));
+            r->launches = 4;
             // the instantiation IMM3_AGG_DISPATCH (kernels.cu) picks: <= 2 group-by columns exact, else 4; 1 .. 4 aggregates exact, else 8
             const int ng = ngroup <= 2 ? ngroup : 4, na = (naggs >= 1 && naggs <= 4) ? naggs : 8;
             const std::string inst = "<" + std::to_string(ng) + "," + std::to_string(na) + ">";
             r->route = "agg_init;" + filter_route(sp) + ";" + (on_blocks ? "agg_blocks" : "agg") + inst + ";agg_compact";
         }
-        unsigned int counters[2] = {0, 0};
-        CUDA_TRY(cudaMemcpyAsync(db->h_ctrl, db->d_ctrl, sizeof(CtrlBlock), cudaMemcpyDeviceToHost, db->stream));
-        CUDA_TRY(cudaMemcpyAsync(counters, db->d_agg_cnt.p, sizeof counters, cudaMemcpyDeviceToHost, db->stream));
+        if (merge) {
+            AggXPlan xp;
+            std::memset(&xp, 0, sizeof xp);
+            for (int i = 0; i < db->world; i++) xp.peer[i] = db->comm_peer[i];
+            xp.rank = db->rank;
+            xp.world = db->world;
+            if (((++db->comm_epoch) & 0xFFFFFFu) == 0) ++db->comm_epoch;  // (the count exchange's rounds: tag 0 is an untouched mailbox)
+            xp.epoch = db->comm_epoch;
+            xp.has_local = local ? 1 : 0;
+            xp.refused = refusal.empty() ? 0 : 1;
+            xp.timeout_ns = db->comm_timeout_ns;
+            CUDA_TRY(launch_agg_exchange(xp, counters, db->d_ctrl, d_x, db->stream));
+            AggMergePlan mp;
+            std::memset(&mp, 0, sizeof mp);
+            for (int i = 0; i < db->world; i++) mp.buf[i] = xbuf(i);
+            db->agg_seq++;  // (posted: the next aggregate compacts into the other buffer)
+            mp.world = db->world;
+            mp.slots = ap.table_slots;
+            mp.naggs = naggs;
+            for (int a = 0; a < naggs; a++) mp.op[a] = ap.agg[a].op;
+            CUDA_TRY(launch_agg_init((AggEntry*)db->d_agg_table.p, ap.table_slots, ap, counters, db->stream));
+            CUDA_TRY(launch_agg_merge(mp, d_x, (AggEntry*)db->d_agg_table.p, (AggEntry*)db->d_agg_out.p, counters, db->num_sms, db->stream));
+            r->launches += 4;
+            r->route += std::string(r->route.empty() ? "" : ";") + "agg_exchange;agg_init;agg_merge;agg_compact";
+        }
+        CUDA_TRY(cudaEventRecord(db->ev1, db->stream));
+        struct {
+            unsigned int counters[16];
+            AggXOut x;
+        } hc;
+        static_assert(sizeof hc.counters == 64, "the exchange output sits 64 bytes into d_agg_cnt");
+        if (local) CUDA_TRY(cudaMemcpyAsync(db->h_ctrl, db->d_ctrl, sizeof(CtrlBlock), cudaMemcpyDeviceToHost, db->stream));
+        CUDA_TRY(cudaMemcpyAsync(&hc, db->d_agg_cnt.p, merge ? sizeof hc : sizeof hc.counters, cudaMemcpyDeviceToHost, db->stream));
         CUDA_TRY(cudaStreamSynchronize(db->stream));
-        if (db->h_ctrl->c.error) return fail(IMM3_ERR_CUDA, "kernel watchdog fired (code %u)", db->h_ctrl->c.error);
-        if (counters[1]) return fail(IMM3_ERR_UNSUPPORTED, "aggregation: more than %u groups", ap.table_slots);
+        if (local && db->h_ctrl->c.error) return fail(IMM3_ERR_CUDA, "kernel watchdog fired (code %u)", db->h_ctrl->c.error);
+        if (merge) {
+            if (hc.x.late)
+                return fail(IMM3_ERR_COMM, "aggregate exchange: a peer's groups were not announced within %llu ms (ranks must issue the same queries in the same order)",
+                            db->comm_timeout_ns / 1000000ull);
+            if (!refusal.empty()) return fail(IMM3_ERR_UNSUPPORTED, "%s", refusal.c_str());
+            if ((hc.x.err_mask >> db->rank) & 1u) return fail(IMM3_ERR_UNSUPPORTED, "aggregation: more than %u groups in the slice of rank %d", ap.table_slots, db->rank);
+            if (hc.x.err_mask)
+                return fail(IMM3_ERR_UNSUPPORTED, "%s: rank %d refused the query (more than %u groups in its slice, or a limit of its slice)", fn,
+                            __builtin_ctz(hc.x.err_mask), ap.table_slots);
+        }
+        if (hc.counters[1]) return fail(IMM3_ERR_UNSUPPORTED, "aggregation: more than %u groups", ap.table_slots);
         float f = 0;
         CUDA_TRY(cudaEventElapsedTime(&f, db->ev0, db->ev1));
         r->device_ms = f;
         r->stage_ms[0] = f;
-        ngroups_out = counters[0];
+        ngroups_out = hc.counters[0];
         groups.resize((size_t)ngroups_out);
         if (ngroups_out) CUDA_TRY(cudaMemcpy(groups.data(), db->d_agg_out.p, (size_t)ngroups_out * sizeof(AggEntry), cudaMemcpyDeviceToHost));
         std::sort(groups.begin(), groups.end(), [](const AggEntry& x, const AggEntry& y) { return x.first_row < y.first_row; });
+        if (merge)
+            for (int i = 0; i < db->world; i++) r->rank_counts[i] = (int64_t)hc.x.counts[i];
+    }
+    if (local) {
         // algorithmic bytes: filter columns once + every decoded encoded column once (its words and 4 B of word offsets per
         // block) + per selected row the cells of the dense group and aggregate columns
         int64_t bytes = 0, per_row = 0;
@@ -1972,10 +2053,22 @@ int imm3_query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int n
     r->local_count = r->fetched = ngroups_out;
     r->g_offset = 0;
     r->g_take = r->g_total = ngroups_out;
-    r->world = 1;
+    r->world = xchg ? db->world : 1;  // (a global aggregate: rank_counts = every rank's partial group count)
     db->live_results++;
     *out = r.release();
     return 0;
+}
+
+}  // namespace
+
+int imm3_query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, const imm3_agg* aggs, int naggs,
+                   const char* const* group_cols, int ngroup, imm3_result** out) {
+    return query_agg(db, table, preds, npreds, aggs, naggs, group_cols, ngroup, false, out);
+}
+
+int imm3_query_agg_global(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, const imm3_agg* aggs, int naggs,
+                          const char* const* group_cols, int ngroup, imm3_result** out) {
+    return query_agg(db, table, preds, npreds, aggs, naggs, group_cols, ngroup, true, out);
 }
 
 int imm3_query_sql(imm3_db* db, const char* sql, imm3_result** out) {

@@ -20,6 +20,8 @@
 //   agg_compact_kernel       occupied slots of the global table -> a dense array (any order; the host sorts the groups by
 //                            the canonical ordinal of their first row, the order the reference reports them in with one
 //                            worker) and clears the table for the next query
+//   agg_merge_kernel         imm3_query_agg_global only: every rank's compacted partial groups (behind k_comm.cuh's
+//                            agg_exchange_kernel) into a fresh global table, then agg_compact_kernel again
 // Exact integer arithmetic: counts are 64-bit, min / max are taken on the raw int32 / int8 values (the reference widens to
 // Double, which is exact for both types; the host formats them as Doubles).
 // =============================================================================================
@@ -96,7 +98,8 @@ __device__ __forceinline__ void agg_update(long long* v, int op, long long x) {
 __device__ __forceinline__ long long agg_identity(int op) { return op == kAggCount ? 0ll : (op == kAggMin ? LLONG_MAX : LLONG_MIN); }
 
 // One group's partial (x[a]: a count, or an extreme as int64) into the global table.  (K: agg_blocks_kernel calls its own
-// copy, K = 1, so that agg_kernel's call graph - and with it agg_kernel's register allocation - is the one it had alone.)
+// copy, K = 1, and agg_merge_kernel K = 2, so that agg_kernel's call graph - and with it agg_kernel's register allocation -
+// is the one it had alone.)
 template <int K = 0>
 __device__ __noinline__ void agg_to_global(AggEntry* table, uint32_t slots, unsigned int* overflow, unsigned long long key, unsigned long long fr,
                                            const long long* x, const AggCol* aggs, int naggs) {
@@ -571,6 +574,33 @@ __global__ void __launch_bounds__(kComputeThreads) agg_compact_kernel(const AggE
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < slots; i += gridDim.x * blockDim.x) {
         const AggEntry e = table[i];
         if (e.key != kAggEmpty) out[atomicAdd(nout, 1u)] = e;
+    }
+}
+
+// agg_merge_kernel: the global aggregate's fan-in (ProjectAggregateQueueOp, ProjectAggregateQueue.scala:21-45), behind
+// agg_exchange_kernel (k_comm.cuh).  Grid-stride over the partial groups of every rank - this rank's exchange buffer in
+// HBM, the peers' over NVLink - into the freshly initialised global table.  An entry's order key is (rank << 48) | its
+// first row in the rank's slice: sorted by it, the groups come out in first-appearance order over the global canonical
+// order (rank order, then the rank's own order) without any rank knowing another's row count.  Nothing is merged when a
+// rank posted the error bit or was late: every rank then reports the same error.
+__global__ void __launch_bounds__(kComputeThreads) agg_merge_kernel(const __grid_constant__ AggMergePlan M, const AggXOut* x, AggEntry* __restrict__ table,
+                                                                    unsigned int* __restrict__ overflow) {
+    __shared__ AggCol s_agg[kMaxAggs];
+    if (threadIdx.x < kMaxAggs) {
+        s_agg[threadIdx.x].base = nullptr;
+        s_agg[threadIdx.x].width = 0;
+        s_agg[threadIdx.x].op = M.op[threadIdx.x];
+    }
+    __syncthreads();
+    if (x->err_mask != 0u || x->late != 0u) return;
+    const unsigned long long stride = (unsigned long long)gridDim.x * blockDim.x;
+    for (int r = 0; r < M.world; r++) {
+        const unsigned long long n = x->counts[r];
+        const AggEntry* const src = M.buf[r];
+        for (unsigned long long i = (unsigned long long)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+            const AggEntry e = src[i];
+            agg_to_global<2>(table, M.slots, overflow, e.key, ((unsigned long long)r << 48) | e.first_row, e.val, s_agg, M.naggs);
+        }
     }
 }
 

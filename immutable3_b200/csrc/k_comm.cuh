@@ -92,3 +92,72 @@ __global__ void __launch_bounds__(32) count_exchange_kernel(const __grid_constan
         if (lane == 0) asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(&C.pub->pub_seq), "l"((C.pub_seq & 0x7FFFFFull) << 41) : "memory");
     }
 }
+
+// =============================================================================================
+// agg_exchange_kernel (one warp): the fan-in of a global aggregate (ProjectAggregateQueueOp, ProjectAggregateQueue.scala:
+// 9-54).  Every rank has compacted its partial groups into its own exchange buffer (plan.hpp kAggXchgOff) before this
+// kernel; what travels through the mailbox ring is one word per rank, [63:40] epoch, [32] error bit, [31:0] group count,
+// in the ring slot and epoch scheme of count_exchange_kernel (the two kernels share db->comm_epoch).
+// Unlike the count, the word announces DATA the peers then read over NVLink, so it is not self-describing: the poster
+// fences at system scope and stores with release semantics (its compacted groups are visible to any reader that sees
+// the word), the poller loads with acquire semantics at system scope before agg_merge_kernel - queued behind this kernel
+// on the same stream - reads a peer's buffer.  Error bit: this rank's local table overflowed, its filter / aggregation
+// watchdog fired, or its slice refuses the query (plan.refused); every rank sees every bit, so every rank returns the
+// same status without waiting for anything.
+// =============================================================================================
+__device__ __forceinline__ void st_release_sys_u64(unsigned long long* p, unsigned long long v) {
+    asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(p), "l"(v) : "memory");
+}
+__device__ __forceinline__ unsigned long long ld_acquire_sys_u64(const unsigned long long* p) {
+    unsigned long long v;
+    asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(p) : "memory");
+    return v;
+}
+
+__global__ void __launch_bounds__(32) agg_exchange_kernel(const __grid_constant__ AggXPlan P, const unsigned int* counters, const ScanCtrl* ctrl,
+                                                          AggXOut* out) {
+    __shared__ unsigned long long* s_peer[kMaxWorld];
+    const int lane = threadIdx.x;
+#pragma unroll
+    for (int i = 0; i < kMaxWorld; i++)
+        if (lane == i) s_peer[i] = P.peer[i];
+    __syncwarp();
+    asm volatile("griddepcontrol.wait;" ::: "memory");  // the local aggregation and its compaction are complete
+    const unsigned long long ep = (unsigned long long)(P.epoch & 0xFFFFFFu);
+    unsigned long long mine = P.refused ? kAggXchgError : 0ull;
+    if (P.has_local) {
+        mine = (unsigned long long)__ldcg(&counters[0]);
+        if (__ldcg(&counters[1]) != 0u || __ldcg(&ctrl->error) != 0u) mine = kAggXchgError;
+    }
+    const int slot = (int)(P.epoch % (unsigned)kCommRing) * kMaxWorld;
+    if (lane < P.world) {
+        __threadfence_system();  // (the compaction kernel's stores to this rank's exchange buffer, before the word)
+        st_release_sys_u64(s_peer[lane] + slot + P.rank, (ep << 40) | mine);
+    }
+    unsigned long long w = 0;
+    bool late = false;
+    if (lane < P.world) {
+        const unsigned long long* src = s_peer[P.rank] + slot + lane;
+        unsigned long long v = ld_acquire_sys_u64(src);
+        if ((v >> 40) != ep) {
+            const uint64_t t0 = globaltimer_ns();
+            unsigned spins = 0;
+            while (((v = ld_acquire_sys_u64(src)) >> 40) != ep) {
+                __nanosleep(40);
+                if ((++spins & 255u) == 0 && globaltimer_ns() - t0 > P.timeout_ns) {  // never hang the GPU: report and go on
+                    late = true;
+                    break;
+                }
+            }
+        }
+        w = late ? kAggXchgError : (v & ((1ull << 40) - 1ull));
+    }
+    const unsigned any_late = __ballot_sync(0xFFFFFFFFu, late);
+    const unsigned errs = __ballot_sync(0xFFFFFFFFu, lane < P.world && (w & kAggXchgError) != 0ull);
+    if (lane < kMaxWorld) out->counts[lane] = (w & kAggXchgError) ? 0ull : (w & 0xFFFFFFFFull);
+    if (lane == 0) {
+        out->err_mask = errs;
+        out->late = any_late ? 1u : 0u;
+    }
+    __threadfence_system();  // (every peer word this warp acquired is ordered before the merge kernel's reads of its buffer)
+}

@@ -264,6 +264,17 @@ cudaError_t launch_agg_blocks(const AggPlan& a, const uint32_t* bitmap, const ui
 #undef IMM3_AGG_DISPATCH_ROW
 #undef IMM3_AGG_DISPATCH
 
+// Global aggregate: every rank's partial groups (exchange buffers) -> the freshly initialised table -> compaction.
+cudaError_t launch_agg_merge(const AggMergePlan& m, const AggXOut* x, AggEntry* table, AggEntry* out, unsigned int* counters, int num_sms,
+                             cudaStream_t stream) {
+    cudaError_t e = configure_once();
+    if (e != cudaSuccess) return e;
+    agg_merge_kernel<<<(unsigned)std::max(1, num_sms), kComputeThreads, 0, stream>>>(m, x, table, counters + 1);
+    if ((e = cudaGetLastError()) != cudaSuccess) return e;
+    agg_compact_kernel<<<(m.slots + kComputeThreads - 1) / kComputeThreads, kComputeThreads, 0, stream>>>(table, m.slots, out, counters);
+    return cudaGetLastError();
+}
+
 long long scan_inline_max_tiles() { return kScanInlineMaxTiles; }
 cudaError_t launch_offset_scan(const uint32_t* tile_cnt, unsigned long long* tile_off, long long ntiles, long long limit, uint32_t epoch,
                                unsigned long long* partials, ScanCtrl* ctrl, unsigned int* tile_list, cudaStream_t stream) {
@@ -418,6 +429,19 @@ cudaError_t launch_count_exchange(const CommPlan& plan, const ScanCtrl* ctrl, Co
     cfg.attrs = attr;
     cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, count_exchange_kernel, plan, ctrl, out);
+}
+// ... and so does the exchange of a global aggregate (behind the compaction of the local groups).
+cudaError_t launch_agg_exchange(const AggXPlan& plan, const unsigned int* counters, const ScanCtrl* ctrl, AggXOut* out, cudaStream_t stream) {
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3(1);
+    cfg.blockDim = dim3(32);
+    cfg.stream = stream;
+    cudaLaunchAttribute attr[1];
+    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr[0].val.programmaticStreamSerializationAllowed = 1;
+    cfg.attrs = attr;
+    cfg.numAttrs = 1;
+    return cudaLaunchKernelEx(&cfg, agg_exchange_kernel, plan, counters, ctrl, out);
 }
 
 cudaError_t launch_scan_blocks(const ScanPlan& plan, ScanCtrl* ctrl, unsigned long long* status, int grid, size_t dyn_smem,

@@ -60,6 +60,9 @@ cudaError_t launch_blocks_emit(const ScanPlan& plan, const uint32_t* bitmap, con
                                long long nblocks, const ScanCtrl* ctrl, bool rowspace, bool pdl, int grid, size_t dyn_smem,
                                cudaStream_t stream);
 cudaError_t launch_count_exchange(const CommPlan& plan, const ScanCtrl* ctrl, CommOut* out, cudaStream_t stream);
+cudaError_t launch_agg_exchange(const AggXPlan& plan, const unsigned int* counters, const ScanCtrl* ctrl, AggXOut* out, cudaStream_t stream);
+cudaError_t launch_agg_merge(const AggMergePlan& m, const AggXOut* x, AggEntry* table, AggEntry* out, unsigned int* counters, int num_sms,
+                             cudaStream_t stream);
 cudaError_t launch_scan_blocks(const ScanPlan& plan, ScanCtrl* ctrl, unsigned long long* status, int grid, size_t dyn_smem,
                                cudaStream_t stream);
 

@@ -186,6 +186,39 @@ struct CommPlan {
     unsigned long long pub_seq;
 };
 
+// Global aggregation (imm3_query_agg_global, k_comm.cuh agg_exchange_kernel / k_agg.cuh agg_merge_kernel): the mailbox's
+// allocation also holds this rank's EXCHANGE AREA, two buffers of kAggXchgSlots AggEntry at kAggXchgOff bytes from the
+// mailbox base - peers reach them at the base they already mapped.  Aggregate s of a db compacts its partial groups into
+// buffer s & 1 (s = agg_seq, identical on all ranks); the ring word of the exchange round carries the group count.
+constexpr size_t kAggXchgOff = 4096;
+constexpr uint32_t kAggXchgSlots = 1u << 16;
+constexpr unsigned long long kAggXchgError = 1ull << 32;  // ring word payload: [32] this rank's partials are unusable, [31:0] its group count
+constexpr size_t kCommAllocBytes = kAggXchgOff + 2 * (size_t)kAggXchgSlots * sizeof(AggEntry);  // mailbox + exchange area (~10 MiB)
+static_assert(kMailboxBytes <= kAggXchgOff, "the exchange area starts behind the mailbox ring");
+
+struct AggXPlan {
+    unsigned long long* peer[kMaxWorld];  // mailbox of every rank as mapped in THIS process (peer[rank] = the local one)
+    int32_t rank, world;
+    uint32_t epoch;                       // exchange round (db->comm_epoch, shared with the count exchange)
+    int32_t has_local;                    // 0: no local kernels ran (empty slice, or a refusal of this slice): 0 groups
+    int32_t refused;                      // 1: this slice refuses the query (posted as the error bit)
+    int32_t pad;
+    unsigned long long timeout_ns;
+};
+// What agg_exchange_kernel leaves for agg_merge_kernel and the host.
+struct AggXOut {
+    unsigned long long counts[kMaxWorld];  // partial group count of every rank
+    unsigned int err_mask;                 // bit r: rank r posted the error bit (local overflow or a refusal of its slice)
+    unsigned int late;                     // 1: a peer's word did not arrive before the timeout
+};
+struct AggMergePlan {
+    const AggEntry* buf[kMaxWorld];  // this aggregate's exchange buffer of every rank, as mapped here
+    int32_t world;
+    uint32_t slots;                  // merged table size (power of two)
+    int32_t naggs;
+    int32_t op[kMaxAggs];            // AggOp of every aggregate
+};
+
 // What the exchange kernel leaves behind for the host (copied back together with ScanCtrl).
 struct CommOut {
     unsigned long long g_offset;  // global ordinal of this rank's first row = sum of the counts of the ranks before it

@@ -5,6 +5,8 @@ library does it itself, on the device (peer stores over NVLink behind the query'
 `SegmentManager.comm_connect`, include/imm3.h imm3_comm_*); without a connected communicator (the
 gloo CPU tests, which exercise the host arithmetic) it is a `torch.distributed.all_gather`.  Either
 way each rank then knows its global output offset and how many of its leading rows survive the LIMIT cut.
+Aggregates (`execute_agg`) exchange the partial groups themselves: merged on the GPUs on a connected handle
+(imm3_query_agg_global), otherwise all-gathered and merged on the host in rank order (`merge_partials`).
 
 The local executor is any object with `begin(query) -> handle` (handle.local_count) and
 `finish(handle, take) -> list of numpy columns`.  The product executor is `CudaExecutor`
@@ -18,7 +20,7 @@ from typing import List, Optional, Sequence
 
 import numpy as np
 
-from .engine import Engine, Query, Result
+from .engine import Count, Engine, Max, Min, Query, Result
 
 
 def shard_range(nsegments: int, rank: int, world: int):
@@ -36,6 +38,41 @@ def limit_split(counts: Sequence[int], limit: int):
         takes.append(c if limit <= 0 else max(0, min(c, limit - run)))
         run += c
     return offsets, takes
+
+
+def merge_partials(parts: Sequence[List[np.ndarray]], ngroup: int, aggs: Sequence) -> List[np.ndarray]:
+    """The fan-in of ProjectAggregateQueueOp (ProjectAggregateQueue.scala:21-45) over per-rank partial groups, in rank
+    order: `parts[r]` = rank r's columns (group columns, then one per aggregate).  A key takes the position of the first
+    rank that holds it (global first-appearance order = rank order, then the rank's own order); Count adds up, Min / Max
+    take the extreme.  The host form of what imm3_query_agg_global does on the GPUs."""
+    pos, rows, firsts = {}, [], []
+    for cols in parts:
+        n = len(cols[0]) if cols else 0
+        for i in range(n):
+            key = tuple(cols[g][i].item() for g in range(ngroup))
+            vals = [cols[ngroup + a][i].item() for a in range(len(aggs))]
+            j = pos.get(key)
+            if j is None:
+                pos[key] = len(rows)
+                rows.append(vals)
+                firsts.append((cols, i))
+                continue
+            m = rows[j]
+            for a, agg in enumerate(aggs):
+                if isinstance(agg, Count):
+                    m[a] += vals[a]
+                elif isinstance(agg, Min):
+                    m[a] = min(m[a], vals[a])
+                elif isinstance(agg, Max):
+                    m[a] = max(m[a], vals[a])
+                else:
+                    raise TypeError(f"not a mergeable aggregate: {agg!r}")
+    template = next((cols for cols in parts if cols), None)
+    if template is None:
+        return []
+    out = [np.array([c[g][i] for c, i in firsts], dtype=template[g].dtype) for g in range(ngroup)]
+    out += [np.array([m[a] for m in rows], dtype=template[ngroup + a].dtype) for a in range(len(aggs))]
+    return out
 
 
 class CudaExecutor:
@@ -92,6 +129,25 @@ class ShardedEngine:
         cols = self.executor.finish(h, takes[self.rank])
         ms = float(getattr(h, "device_ms", 0.0))
         return ShardResult(self.rank, self.world, counts, offsets[self.rank], takes[self.rank], sum(takes), cols, ms)
+
+    def execute_agg(self, query: Query) -> ShardResult:
+        """A ProjectAgg query over the whole table, the same groups on every rank: `columns` = the global groups,
+        `counts` = every rank's partial group count, offset 0, take = total = the number of global groups.  On a
+        connected handle the GPUs merge the partials themselves (imm3_query_agg_global); otherwise every rank's partial
+        columns are all-gathered through torch.distributed and merged on the host in rank order (`merge_partials`)."""
+        engine = getattr(self.executor, "engine", None)
+        if getattr(getattr(engine, "sm", None), "comm_connected", False):
+            with engine.execute_agg_global(query) as h:
+                cols = h.columns()
+                return ShardResult(self.rank, self.world, h.rank_counts, 0, h.nrows, h.nrows, cols, float(h.device_ms))
+        h = self.executor.begin(query)  # this rank's partial groups
+        mine = self.executor.finish(h, int(h.local_count))
+        everyone = [None] * self.world
+        self.dist.all_gather_object(everyone, mine, group=self.group)
+        cols = merge_partials(everyone, len(query.project.groupBy), list(query.project.aggs))
+        total = len(cols[0]) if cols else 0
+        counts = [len(p[0]) if p else 0 for p in everyone]
+        return ShardResult(self.rank, self.world, counts, 0, total, total, cols, float(getattr(h, "device_ms", 0.0)))
 
     def gather_rows(self, res: ShardResult, dst: int = 0):
         """Concatenate every rank's emitted rows on `dst` in rank order (= canonical order). Test helper."""

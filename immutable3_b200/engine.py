@@ -557,8 +557,16 @@ class Engine:
         del keep
         return Result(out, self._lib, self.sm)
 
-    def _call_agg(self, query: Query) -> Result:
+    def execute_agg_global(self, query: Query) -> Result:
+        """A ProjectAgg query over the WHOLE table on every rank of a sharded handle (imm3_query_agg_global): the ranks'
+        partial groups are merged on the GPUs over the communicator (`SegmentManager.comm_connect`).  On a single handle the
+        result is that of `execute`; an unconnected sharded handle raises (IMM3_ERR_STATE)."""
+        return self._call_agg(query, self._lib.imm3_query_agg_global)
+
+    def _call_agg(self, query: Query, fn=None) -> Result:
         """Engine.execute, ProjectAgg branch (Engine.scala:200-232): one row per group, group columns then aggregates."""
+        if not isinstance(query.project, ProjectAgg):
+            raise L.Imm3Error(L.ERR_UNSUPPORTED, "not a ProjectAgg query")
         preds, npreds, keep = _pred_array(flatten_select(query.select))
         aggs = list(query.project.aggs)
         arr = (L.Agg * max(1, len(aggs)))()
@@ -567,8 +575,8 @@ class Engine:
             arr[i].op = _AGG_OPS[type(a).__name__]
         groups = L.cstr_array(list(query.project.groupBy))
         out = C.c_void_p()
-        L.check(self._lib.imm3_query_agg(self.sm.handle, query.table.encode(), preds, npreds, arr, len(aggs),
-                                         C.cast(groups, C.POINTER(C.c_char_p)), len(query.project.groupBy), C.byref(out)))
+        L.check((fn or self._lib.imm3_query_agg)(self.sm.handle, query.table.encode(), preds, npreds, arr, len(aggs),
+                                                 C.cast(groups, C.POINTER(C.c_char_p)), len(query.project.groupBy), C.byref(out)))
         del keep
         return Result(out, self._lib, self.sm)
 

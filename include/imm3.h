@@ -207,7 +207,7 @@ int imm3_result_wait(imm3_result* r);
  * and group columns may be dense or sorted-int-codec (PFOR_INT), but one query decodes at most 4 distinct sorted-int-codec
  * columns, from blocks of at most 1024 rows; predicates on a sorted-int-codec column cannot be combined with aggregation
  * yet.  On a sharded handle the result holds
- * this rank's groups (partials); the caller merges ranks in rank order (count: sum, min / max: min / max). */
+ * this rank's groups (partials); imm3_query_agg_global below merges them on the GPUs. */
 typedef enum imm3_agg_op { IMM3_AGG_COUNT = 0, IMM3_AGG_MIN = 1, IMM3_AGG_MAX = 2, IMM3_AGG_SUM = 3, IMM3_AGG_AVG = 4 } imm3_agg_op;
 typedef struct imm3_agg {
     const char* col;
@@ -215,6 +215,19 @@ typedef struct imm3_agg {
 } imm3_agg;
 int imm3_query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, const imm3_agg* aggs, int naggs,
                    const char* const* group_cols, int ngroup, imm3_result** out);
+/* The aggregate fan-in across segment-sharded GPUs (ProjectAggregateQueueOp, ProjectAggregateQueue.scala:9-54): the same
+ * arguments, validation and result layout as imm3_query_agg, but every rank of a connected handle (imm3_comm_connect) gets
+ * the WHOLE table's groups - the same rows on every rank, in first-appearance order over the global canonical order (rank
+ * order, then the rank's own order), COUNT summed and MIN / MAX taken over the ranks.  Each rank compacts its partial
+ * groups into an exchange buffer beside its mailbox, announces their number through the mailbox ring, and merges every
+ * rank's buffer over NVLink into its own table: one stream, one synchronisation, no host round trip.  On a world == 1
+ * handle the result is exactly imm3_query_agg's; a world > 1 handle that is not connected returns IMM3_ERR_STATE.
+ * imm3_result_rank_counts reports every rank's partial group count, imm3_result_global_count the merged groups.
+ * A refusal of one rank's slice (more groups than its table holds, blocks of more than 1024 rows, shared memory) is
+ * exchanged too: every rank returns the same IMM3_ERR_UNSUPPORTED.  IMM3_AGG_SLOTS above 65536 is refused.  Every rank
+ * must issue the same queries (aggregates and Project queries alike) in the same order. */
+int imm3_query_agg_global(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, const imm3_agg* aggs, int naggs,
+                          const char* const* group_cols, int ngroup, imm3_result** out);
 
 /* Same query text the reference CLI takes (SQLParser.scala:8-129; SqlCli.scala:60). */
 int imm3_query_sql(imm3_db* db, const char* sql, imm3_result** out);
@@ -233,10 +246,11 @@ int imm3_result_kernel_launches(const imm3_result* r);      /* kernels launched 
 /* The kernels imm3_query_begin / imm3_query_agg queued, in launch order, separated by ';' ("" when none ran): kernel names
  * (select_all, filter(tma|direct), offset_scan, emit_stream, emit, emit_general, blocks_prune, blocks_filter_lane,
  * blocks_filter_quad, blocks_filter, blocks_group_emit, blocks_scan_emit, blocks_emit(rowspace|blocks), scan_blocks,
- * count_exchange, agg_init, agg<NG,NA>, agg_blocks<NG,NA>, agg_compact) with "/key=value" parameters: /s= ring stages,
+ * count_exchange, agg_init, agg<NG,NA>, agg_blocks<NG,NA>, agg_compact, agg_exchange, agg_merge) with "/key=value" parameters: /s= ring stages,
  * /w= warps per CTA of the lane kernel, /ctas= the group emit kernel's grid; "/prefix" marks the prefix pass of a small
- * LIMIT.  E.g. "blocks_prune;blocks_filter_lane/w=11/s=2;blocks_group_emit/ctas=148".  Owned by the result (valid until
- * imm3_result_free). */
+ * LIMIT.  E.g. "blocks_prune;blocks_filter_lane/w=11/s=2;blocks_group_emit/ctas=148"; a global aggregate on a connected
+ * handle: "agg_init;filter(tma)/s=4;agg<1,2>;agg_compact;agg_exchange;agg_init;agg_merge;agg_compact" (a rank with an empty
+ * slice starts at agg_exchange).  Owned by the result (valid until imm3_result_free). */
 const char* imm3_result_route(const imm3_result* r);
 /* CUDA-event time of one stage of begin: 0 = filter (+scan) kernel, 1 = emit kernel (multi-pass path);
  * the fused single-pass kernels report everything as stage 0. */
