@@ -364,6 +364,9 @@ int run_pieces(imm3_db* db, const std::vector<Piece>& pieces, bool to_device) {
     return 0;
 }
 
+// Per-warp scratch of the block decoders: the byte-swapped words of the largest encoded block, plus slack.
+int block_words_cap(int64_t max_block_words) { return (int)std::min<int64_t>(1120, ((max_block_words + 4 + 31) / 32) * 32); }
+
 int upload_all(imm3_db* db) {
     const bool otrace = getenv("IMM3_OPEN_TRACE") != nullptr;
     const double t0 = now_us();
@@ -411,8 +414,7 @@ int upload_all(imm3_db* db) {
                 PforCol pc;
                 pc.words = reinterpret_cast<const uint32_t*>(col.d_arena);
                 pc.word_off = col.d_word_off;
-                const int cap = (int)std::min<int64_t>(1120, ((col.max_block_words + 4 + 31) / 32) * 32);
-                CUDA_TRY(launch_block_stats(pc, t.d_row_start, t.nblocks, cap, db->num_sms, (BlockStat*)col.d_stats, db->stream));
+                CUDA_TRY(launch_block_stats(pc, t.d_row_start, t.nblocks, block_words_cap(col.max_block_words), db->num_sms, (BlockStat*)col.d_stats, db->stream));
             }
         }
         CUDA_TRY(cudaStreamSynchronize(db->stream));
@@ -474,19 +476,25 @@ void free_device_side(imm3_db* db) {
 }
 
 // ---- query planning on top of the logical plan --------------------------------------------------
+// The kernels of a query, chosen once per plan (choose_route); sizing (fill_scan_plan) and launching (run_scan_once) follow it.
+enum class Pipeline {
+    kDense,       // dense table: filter kernel over the row space -> offset scan -> emit kernels
+    kRowSpace,    // block table, no predicate on an encoded column: the same filter kernel over the row space (dense columns are
+                  // contiguous in HBM whatever the block framing) -> block emit kernel (decodes only blocks with surviving rows)
+    kBlocks,      // block table: [blocks_prune ->] block filter kernel -> offset scan + block emit, scan-emit or group emit
+    kSinglePass,  // block table: scan_blocks, one kernel with a look-back chain (selection bitmaps, blocks of more than 1024 rows)
+};
+
 struct Prepared {
     TableStore* table = nullptr;
     LogicalPlan lp;
-    bool block_mode = false;
-    bool multipass = false;   // dense tables: filter -> scan -> emit kernels instead of the fused single pass
-    bool blocks_multi = false;  // block mode: warp-per-block filter kernel -> offset scan -> emit kernel (no look-back chain)
-    bool for_bitmap = false;    // imm3_filter_bitmap: the canonical-row bitmap comes from the single-pass kernels
-    bool quad = false;          // block mode: the single-range-predicate filter kernel (lane = block x super-block)
-    bool lane = false;          // block mode: ... its lane-per-block successor (every warp its own TMA ring)
-    int lane_warps = 8;         // ... warps per CTA of that kernel
-    bool prune = false;         // block mode: every predicate is a range on an encoded column with block statistics: blocks_prune_kernel first
+    bool for_bitmap = false;    // imm3_filter_bitmap: the selection bitmap is the result
+    Pipeline pipeline = Pipeline::kDense;
+    BlockFilter block_filter = BlockFilter::kMini;  // kBlocks: the filter kernel
+    int lane_warps = 8;         // ... warps per CTA of the lane kernel
+    bool prune = false;         // kBlocks: every predicate is a range on an encoded column with block statistics: blocks_prune_kernel first
     PrunePlan pp;
-    bool hybrid = false;        // block mode, no predicate on an encoded column: DENSE filter kernel (row space) -> block emit kernel
+    std::vector<int> pfor_cols;  // table columns of sp.pfor, in slot order
     size_t blocks_emit_smem = 0;
     int64_t prefix_blocks = 0;  // small LIMIT on a block table: the pipeline first runs over this many leading blocks (0 = no prefix)
     int64_t prefix_rows = 0;    // small LIMIT on a dense table: ... over this many leading rows (a multiple of the tile size)
@@ -504,30 +512,67 @@ struct Prepared {
     std::vector<std::unique_ptr<Prepared>> or_terms;
 };
 
-const char* kernel_name(const imm3_db* db, const TableStore& t, const LogicalPlan& lp, bool* block_mode) {
-    bool blocks = lp.uses_pfor || (db->flags & IMM3_OPEN_FORCE_BLOCKS);  // tests: cross-check the two kernels
-    (void)t;
-    *block_mode = blocks;
-    if (lp.always_empty) return "none(always_empty)";
-    return blocks ? "blocks_filter -> blocks_emit" : ((db->flags & IMM3_OPEN_NO_TMA) ? "filter(direct) -> emit" : "filter(tma) -> emit");
+bool is_pfor(const TableStore& t, int ci) { return t.cols[(size_t)ci].meta.codec == IMM3_CODEC_PFOR_INT; }
+
+// Slot of column ci among the distinct sorted-int-codec columns a kernel decodes (`cols`, in slot order); -1: not encoded.
+int pfor_slot(const TableStore& t, std::vector<int>* cols, int ci) {
+    if (!is_pfor(t, ci)) return -1;
+    for (size_t i = 0; i < cols->size(); i++)
+        if ((*cols)[i] == ci) return (int)i;
+    cols->push_back(ci);
+    return (int)cols->size() - 1;
 }
 
-// Dense tables run the three-kernel pipeline (filter -> offset scan -> emit: no cross-CTA dependency); a small LIMIT makes it
-// run over a prefix of the table first (Prepared::prefix_rows).  (Round 1 also carried a fused single-pass kernel behind
-// IMM3_PATH=fused - 0.7x the pipeline's rate, never the default, and the home of that round's one wrong result; deleted.)
-bool choose_multipass(const LogicalPlan& lp, bool block_mode) {
-    (void)lp;
-    return !block_mode;
+// The quad kernel stages CTA tiles of 32 blocks of the one predicate's column: bytes reserved for such a tile.
+int64_t quad_tile_cap(const TableStore& t, const LogicalPlan& lp) {
+    return (t.cols[(size_t)lp.filters[0].col_idx].max_tile32_bytes + 16 + 15) & ~15ll;
+}
+constexpr size_t kLaneSmemCap = 222 * 1024;  // shared memory of one lane-kernel CTA (one CTA per SM)
+
+// Pipeline and block filter kernel of a query, from the table's codecs and block sizes, the logical plan, whether a selection
+// bitmap is wanted and the switches IMM3_PATH=fused, IMM3_NO_HYBRID, IMM3_NO_QUAD, IMM3_NO_LANE and IMM3_OPEN_FORCE_BLOCKS
+// (tests: cross-check the dense and block kernels).
+void choose_route(const imm3_db* db, Prepared* pr) {
+    const TableStore& t = *pr->table;
+    const LogicalPlan& lp = pr->lp;
+    pr->block_filter = BlockFilter::kMini;
+    if (!lp.uses_pfor && !(db->flags & IMM3_OPEN_FORCE_BLOCKS)) {
+        pr->pipeline = Pipeline::kDense;
+        return;
+    }
+    const char* path = getenv("IMM3_PATH");
+    if (pr->for_bitmap || t.max_block_rows > 1024 || (path && !strcmp(path, "fused"))) {
+        pr->pipeline = Pipeline::kSinglePass;
+        return;
+    }
+    bool filters_dense = true;
+    for (auto& f : lp.filters) filters_dense = filters_dense && !is_pfor(t, f.col_idx);
+    pr->pipeline = filters_dense && !getenv("IMM3_NO_HYBRID") ? Pipeline::kRowSpace : Pipeline::kBlocks;
+    // The only predicate is a range on one encoded column (C4): the quad kernel - lane = (block, super-block), CTA tile of
+    // 32 blocks - if such a tile of this column fits a ring slot (i.e. the column actually compresses); its lane = block
+    // successor if a CTA of 8 warps holds a two-slot ring per warp.
+    if (pr->pipeline == Pipeline::kBlocks && lp.filters.size() == 1 && !filters_dense && lp.filters[0].kind == kFilterI32Range &&
+        !getenv("IMM3_NO_QUAD")) {
+        const int qslot = blocks_filter_quad_slot_bytes((int)quad_tile_cap(t, lp));
+        if (qslot <= 40 * 1024) pr->block_filter = (2 * 8 * (size_t)qslot <= kLaneSmemCap && !getenv("IMM3_NO_LANE")) ? BlockFilter::kLane : BlockFilter::kQuad;
+    }
+}
+
+// imm3_explain's name of the kernels
+const char* explain_kernel(const imm3_db* db, const Prepared& pr) {
+    if (pr.lp.always_empty) return "none(always_empty)";
+    if (pr.pipeline != Pipeline::kDense) return "blocks_filter -> blocks_emit";
+    return (db->flags & IMM3_OPEN_NO_TMA) ? "filter(direct) -> emit" : "filter(tma) -> emit";
 }
 
 int prepare(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, const char* const* proj, int nproj,
-            int64_t limit, Prepared* pr) {
+            int64_t limit, bool for_bitmap, Prepared* pr) {
     pr->table = find_table(db, table);
     if (!pr->table) return IMM3_ERR_NOT_FOUND;
     int rc = build_logical_plan(pr->table->meta, preds, npreds, proj, nproj, limit, &pr->lp);
     if (rc) return rc;
-    kernel_name(db, *pr->table, pr->lp, &pr->block_mode);
-    pr->multipass = choose_multipass(pr->lp, pr->block_mode);
+    pr->for_bitmap = for_bitmap;
+    choose_route(db, pr);
     pr->shape_key = pr->table->meta.name + "|";
     for (auto& f : pr->lp.filters) pr->shape_key += std::to_string(f.col_idx) + ":" + std::to_string(f.kind) + ",";
     pr->shape_key += "|";
@@ -535,8 +580,23 @@ int prepare(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, 
     return 0;
 }
 
-// Fill the device plan (everything but result pointers and the bitmap).
-int fill_scan_plan(imm3_db* db, Prepared* pr) {
+// A small LIMIT is served "prefix first": the multi-pass pipelines have no early exit, so phase A scans a leading part of the
+// slice (64 rows per requested row, at least 4 M rows) and phase B the whole slice only if that did not fill the LIMIT.  (The
+// single-pass kernel does stop early, but its look-back chain costs 13 ns per block when the rows come late.)  With a
+// communicator every rank must run the same rounds, so the policy depends only on the query: phase A everywhere (a rank whose
+// slice is too small for a prefix scans all of it), then - unless RANK 0's phase A alone fills the LIMIT, in which case the
+// global result is its first `limit` rows - phase B everywhere.
+bool small_limit(const LogicalPlan& lp) { return lp.limit > 0 && lp.limit <= (1 << 20) && !getenv("IMM3_NO_PREFIX"); }
+// rows phase A wants (0: no prefix phase)
+int64_t prefix_rows_wanted(const LogicalPlan& lp) {
+    if (!small_limit(lp)) return 0;
+    const int64_t min_rows = getenv("IMM3_PREFIX_ROWS") ? std::max(1024, atoi(getenv("IMM3_PREFIX_ROWS"))) : (4 << 20);  // (tests shrink it)
+    return std::max<int64_t>(min_rows, lp.limit * 64);
+}
+
+// The part of every device plan that does not depend on the pipeline: columns, literals, encoded-column slots, the L2 hint,
+// the epoch and IMM3_DEBUG.
+int plan_columns(imm3_db* db, Prepared* pr) {
     TableStore& t = *pr->table;
     const LogicalPlan& lp = pr->lp;
     ScanPlan& sp = pr->sp;
@@ -547,14 +607,7 @@ int fill_scan_plan(imm3_db* db, Prepared* pr) {
     sp.max_block_rows = t.max_block_rows;
     sp.nfilter = (int)lp.filters.size();
     sp.nproj = (int)lp.proj.size();
-    std::vector<int> pfor_cols;
-    auto pfor_slot = [&](int ci) -> int {
-        if (t.cols[(size_t)ci].meta.codec != IMM3_CODEC_PFOR_INT) return -1;
-        for (size_t i = 0; i < pfor_cols.size(); i++)
-            if (pfor_cols[i] == ci) return (int)i;
-        pfor_cols.push_back(ci);
-        return (int)pfor_cols.size() - 1;
-    };
+    pr->pfor_cols.clear();
     int lit_at = 0;
     for (int i = 0; i < sp.nfilter; i++) {
         const LogicalFilter& lf = lp.filters[(size_t)i];
@@ -562,7 +615,7 @@ int fill_scan_plan(imm3_db* db, Prepared* pr) {
         FilterCol& f = sp.filter[i];
         f.width = c.meta.width;
         f.kind = lf.kind;
-        f.pfor_slot = pfor_slot(lf.col_idx);
+        f.pfor_slot = pfor_slot(t, &pr->pfor_cols, lf.col_idx);
         f.base = f.pfor_slot >= 0 ? nullptr : c.d_arena;
         f.smem_off = -1;
         if (lf.kind == kFilterStrMatch) {
@@ -583,7 +636,7 @@ int fill_scan_plan(imm3_db* db, Prepared* pr) {
         const ColumnStore& c = t.cols[(size_t)ci];
         ProjCol& p = sp.proj[i];
         p.width = c.meta.width;
-        p.pfor_slot = pfor_slot(ci);
+        p.pfor_slot = pfor_slot(t, &pr->pfor_cols, ci);
         p.base = p.pfor_slot >= 0 ? nullptr : c.d_arena;
         p.filter_idx = -1;
         for (int k = 0; k < sp.nfilter; k++)
@@ -598,9 +651,9 @@ int fill_scan_plan(imm3_db* db, Prepared* pr) {
         for (int i = 0; i < sp.nproj; i++)
             if (sp.proj[i].filter_idx >= 0) sp.filter[sp.proj[i].filter_idx].keep_l2 = (again > 0 && again <= (int64_t)(getenv("IMM3_KEEP_L2_MB") ? atoi(getenv("IMM3_KEEP_L2_MB")) : 84) << 20) ? 1 : 0;
     }
-    sp.npfor = (int)pfor_cols.size();
+    sp.npfor = (int)pr->pfor_cols.size();
     for (int i = 0; i < sp.npfor; i++) {
-        const ColumnStore& c = t.cols[(size_t)pfor_cols[(size_t)i]];
+        const ColumnStore& c = t.cols[(size_t)pr->pfor_cols[(size_t)i]];
         sp.pfor[i].words = reinterpret_cast<const uint32_t*>(c.d_arena);
         sp.pfor[i].word_off = c.d_word_off;
     }
@@ -610,188 +663,160 @@ int fill_scan_plan(imm3_db* db, Prepared* pr) {
     }
     sp.epoch = db->epoch;
     if (const char* e = getenv("IMM3_DEBUG")) sp.debug = (uint32_t)atoi(e);
+    return 0;
+}
 
-    int occ = 0;
-    // one 8192-row sub-tile of every (dense) filter column, and where each column sits inside a TMA stage
-    auto dense_sub_bytes = [&]() {
-        int row_bytes = 0;
-        for (int i = 0; i < sp.nfilter; i++) row_bytes += sp.filter[i].width;
-        return kDenseTileRowsPerWord * row_bytes;
-    };
-    auto dense_stage_offsets = [&](int sub_bytes) {
-        const bool can_stage = !(db->flags & IMM3_OPEN_NO_TMA) && sub_bytes > 0 && sub_bytes <= 56 * 1024;
-        int off = 0;
-        for (int i = 0; i < sp.nfilter; i++) {
-            sp.filter[i].smem_off = can_stage ? off : -1;
-            off += kDenseTileRowsPerWord * sp.filter[i].width;
-        }
-        return can_stage;
-    };
-    // Multi-pass filter kernel (K1): tile = 8192 rows; a TMA ring of ~32 KiB, so that four CTAs share an SM.
-    auto config_dense_filter = [&]() -> cudaError_t {
-        const int stage_bytes = dense_sub_bytes();
-        const bool stage_ok = dense_stage_offsets(stage_bytes);
-        sp.words_per_lane = 1;
-        sp.ntiles = (t.nrows + kDenseTileRowsPerWord - 1) / kDenseTileRowsPerWord;
-        int stages = 0;
-        if (stage_ok) stages = std::max(2, std::min(kMaxFilterStages, (32 * 1024) / stage_bytes));
-        if (const char* e = getenv("IMM3_FILTER_STAGES")) {
+// Filter kernel over the row space (kDense, kRowSpace, aggregation): tiles of 8192 rows; a TMA ring of ~32 KiB, so that four
+// CTAs share an SM.  A stage holds one 8192-row sub-tile of every filter column.
+int size_dense_filter(imm3_db* db, Prepared* pr, int* occ) {
+    ScanPlan& sp = pr->sp;
+    int stage_bytes = 0;
+    for (int i = 0; i < sp.nfilter; i++) stage_bytes += kDenseTileRowsPerWord * sp.filter[i].width;
+    const bool stage_ok = !(db->flags & IMM3_OPEN_NO_TMA) && stage_bytes > 0 && stage_bytes <= 56 * 1024;
+    for (int i = 0, off = 0; i < sp.nfilter; i++) {  // where each column sits inside a stage
+        sp.filter[i].smem_off = stage_ok ? off : -1;
+        off += kDenseTileRowsPerWord * sp.filter[i].width;
+    }
+    sp.ntiles = (pr->table->nrows + kDenseTileRowsPerWord - 1) / kDenseTileRowsPerWord;
+    int stages = 0;
+    if (stage_ok) stages = std::max(2, std::min(kMaxFilterStages, (32 * 1024) / stage_bytes));
+    if (const char* e = getenv("IMM3_FILTER_STAGES")) {
+        int v = atoi(e);
+        if (stage_ok && v >= 2 && v <= kMaxFilterStages && (size_t)v * stage_bytes <= 200 * 1024) stages = v;
+    }
+    sp.stages = stages;
+    sp.stage_bytes = stage_bytes;
+    pr->dyn_smem = (size_t)stages * (size_t)stage_bytes;
+    CUDA_TRY(filter_kernel_occupancy(pr->dyn_smem, occ));
+    return 0;
+}
+
+// kDense: the gather emit kernel (8 spans of 1024 rows per tile) and the streaming one (dense results).
+int size_dense_emit(imm3_db* db, Prepared* pr) {
+    ScanPlan& sp = pr->sp;
+    int occ_emit = 0;
+    pr->emit_general = sp.nproj > 4 || getenv("IMM3_EMIT_GENERAL");
+    for (int i = 0; i < sp.nproj; i++) pr->emit_general = pr->emit_general || !(sp.proj[i].width == 1 || sp.proj[i].width == 2 || sp.proj[i].width == 4);
+    CUDA_TRY(emit_kernel_occupancy(pr->emit_general, &occ_emit));
+    const int64_t nspans = sp.ntiles * (kDenseTileRowsPerWord / 1024);
+    pr->grid_emit = (int)std::max<int64_t>(1, std::min<int64_t>((nspans + 7) / 8, (int64_t)db->num_sms * std::max(1, occ_emit)));
+    // Streaming emit kernel: a stage = bitmap words + span counts + one 8192-row tile of every projected column, if that fits.
+    int pstage = 0;
+    for (int i = 0; i < sp.nproj; i++) {
+        sp.proj[i].stage_off = pstage;
+        pstage += 1024 * sp.proj[i].width;
+    }
+    pr->emit_stage_bytes = 0;
+    if (sp.nproj > 0 && 8 * pstage <= 64 * 1024 && !(db->flags & IMM3_OPEN_NO_TMA) && !getenv("IMM3_NO_EMIT_STREAM")) {
+        pr->emit_stage_bytes = emit_stream_header_bytes() + 8 * pstage;
+        pr->emit_ring = std::max(2, std::min(4, (80 * 1024) / pr->emit_stage_bytes));
+        if (const char* e = getenv("IMM3_EMIT_STAGES")) {
             int v = atoi(e);
-            if (stage_ok && v >= 2 && v <= kMaxFilterStages && (size_t)v * stage_bytes <= 200 * 1024) stages = v;
+            if (v >= 2 && v <= 4) pr->emit_ring = v;
         }
-        sp.stages = stages;
-        sp.stage_bytes = stage_bytes;
-        pr->dyn_smem = (size_t)stages * (size_t)stage_bytes;
-        return filter_kernel_occupancy(pr->dyn_smem, &occ);
-    };
-    if (pr->block_mode) {
-        if (t.max_block_rows > kMaxBlockRows)
-            return fail(IMM3_ERR_UNSUPPORTED, "block-mode kernel stages blocks of at most %d rows, table %s has a block of %d",
-                        kMaxBlockRows, t.meta.name.c_str(), t.max_block_rows);
-        const char* path = getenv("IMM3_PATH");
-        pr->blocks_multi = !pr->for_bitmap && t.max_block_rows <= 1024 && !(path && !strcmp(path, "fused"));
-        // Small LIMIT: the multi-pass pipeline has no early exit, so it first runs over a prefix of the table (64 rows per
-        // requested row, at least 4 M rows); only if that does not fill the LIMIT is the whole table scanned.  (The
-        // single-pass kernel does stop early, but its look-back chain costs 13 ns per block when the rows come late.)
-        if (pr->blocks_multi && lp.limit > 0 && lp.limit <= (1 << 20) && !getenv("IMM3_NO_PREFIX")) {
-            const int64_t min_rows = getenv("IMM3_PREFIX_ROWS") ? std::max(1024, atoi(getenv("IMM3_PREFIX_ROWS"))) : (4 << 20);  // (tests shrink it)
-            const int64_t want_rows = std::max<int64_t>(min_rows, lp.limit * 64);
-            const int64_t nb = (want_rows + 1023) / 1024;
-            if (nb * 2 <= t.nblocks) pr->prefix_blocks = nb;
-        }
-        if (pr->blocks_multi) {
-            bool filters_dense = true;
-            for (int i = 0; i < sp.nfilter; i++) filters_dense = filters_dense && sp.filter[i].pfor_slot < 0;
-            pr->hybrid = filters_dense && !getenv("IMM3_NO_HYBRID");
-            sp.ntiles = (t.nblocks + 7) / 8;  // the offset scan works on tiles of 8 blocks
-            int64_t cap = 0;  // per-warp scratch for the byte-swapped words of one encoded block
-            for (int ci : pfor_cols) cap = std::max<int64_t>(cap, t.cols[(size_t)ci].max_block_words);
-            sp.blk_words_cap = (int)std::min<int64_t>(1120, ((cap + 4 + 31) / 32) * 32);
-            // Filter kernel: a TMA ring of raw tiles (8 blocks of every encoded column that carries a predicate + metadata).
-            int64_t tile_cap = 0;
-            int nstaged = 0;
-            sp.pfor_filter_mask = 0;
-            for (int i = 0; i < sp.nfilter; i++)
-                if (sp.filter[i].pfor_slot >= 0) sp.pfor_filter_mask |= 1u << sp.filter[i].pfor_slot;
-            for (int s = 0; s < sp.npfor; s++)
-                if ((sp.pfor_filter_mask >> s) & 1u) {
-                    tile_cap = std::max<int64_t>(tile_cap, t.cols[(size_t)pfor_cols[(size_t)s]].max_tile_bytes);
-                    nstaged++;
-                }
-            sp.blk_tile_bytes = (int)((tile_cap + 16 + 15) & ~15ll);
-            const int slot_bytes = blocks_filter_slot_bytes(nstaged, sp.blk_tile_bytes);
-            int ring = std::max(2, std::min(kMaxFilterStages, (48 * 1024) / slot_bytes));
-            if (const char* e = getenv("IMM3_BLOCKS_STAGES")) ring = std::max(2, std::min(kMaxFilterStages, atoi(e)));
-            while (ring > 2 && (size_t)ring * slot_bytes > 200 * 1024) ring--;
-            sp.stages = ring;  // (the row-space variant below re-plans these two for the dense filter kernel)
-            sp.stage_bytes = slot_bytes;
-            pr->dyn_smem = blocks_filter_smem_bytes(nstaged, sp.blk_tile_bytes, ring);
-            // The only predicate is a range on one encoded column (C4): the quad kernel - lane = (block, super-block), CTA tile
-            // of 32 blocks - if such a tile of this column fits a ring slot (i.e. the column actually compresses).
-            pr->quad = false;
-            pr->lane = false;
-            if (sp.nfilter == 1 && sp.filter[0].pfor_slot >= 0 && sp.filter[0].kind == kFilterI32Range && !getenv("IMM3_NO_QUAD")) {
-                const int64_t cap32 = (t.cols[(size_t)pfor_cols[(size_t)sp.filter[0].pfor_slot]].max_tile32_bytes + 16 + 15) & ~15ll;
-                const int qslot = blocks_filter_quad_slot_bytes((int)cap32);
-                if (qslot <= 40 * 1024) {
-                    pr->quad = true;
-                    int qring = std::max(2, std::min(4, (40 * 1024) / qslot));
-                    if (const char* e = getenv("IMM3_BLOCKS_STAGES")) qring = std::max(2, std::min(kMaxFilterStages, atoi(e)));
-                    sp.blk_tile_bytes = (int)cap32;
-                    sp.stages = qring;
-                    sp.stage_bytes = qslot;
-                    pr->dyn_smem = (size_t)qring * (size_t)qslot;
-                }
-                // lane = block: every warp of the CTA runs its own ring of 2 .. 4 such slots; one CTA per SM with as many warps
-                // (8 .. 16) as its shared memory holds two-slot rings for
-                const size_t lane_smem_cap = 222 * 1024;
-                if (pr->quad && 2 * 8 * (size_t)qslot <= lane_smem_cap && !getenv("IMM3_NO_LANE")) {
-                    pr->lane = true;
-                    int lring = 2;
-                    if (const char* e = getenv("IMM3_LANE_STAGES")) lring = std::max(2, std::min(4, atoi(e)));
-                    while (lring > 2 && (size_t)lring * 4 * (size_t)qslot > lane_smem_cap) lring--;
-                    int lw = (int)std::min<size_t>(16, lane_smem_cap / ((size_t)lring * (size_t)qslot));
-                    if (const char* e = getenv("IMM3_LANE_WARPS")) lw = std::max(4, std::min(lw, atoi(e)));
-                    pr->lane_warps = lw;
-                    sp.stages = lring;
-                    pr->dyn_smem = (size_t)lring * (size_t)lw * (size_t)qslot;
-                }
+        pr->emit_smem = emit_stream_smem_bytes(pr->emit_stage_bytes, pr->emit_ring);
+        int occ_s = 0;
+        CUDA_TRY(emit_stream_occupancy(pr->emit_smem, &occ_s));
+        if (occ_s < 1) pr->emit_stage_bytes = 0;
+        pr->grid_emit_stream = (int)std::max<int64_t>(1, std::min<int64_t>(sp.ntiles, (int64_t)db->num_sms * std::max(1, occ_s)));
+    }
+    return 0;
+}
+
+// kBlocks: the ring of the block filter kernel.  Mini-block kernel: a TMA ring of raw tiles (8 blocks of every encoded column
+// that carries a predicate + metadata).  Quad kernel: tiles of 32 blocks of its one column.  Lane kernel: every warp of the
+// CTA runs its own ring of 2 .. 4 such slots; one CTA per SM with as many warps (8 .. 16) as its shared memory holds two-slot
+// rings for.
+void size_block_filter(Prepared* pr) {
+    const TableStore& t = *pr->table;
+    ScanPlan& sp = pr->sp;
+    const char* ring_env = getenv("IMM3_BLOCKS_STAGES");
+    sp.pfor_filter_mask = 0;
+    for (int i = 0; i < sp.nfilter; i++)
+        if (sp.filter[i].pfor_slot >= 0) sp.pfor_filter_mask |= 1u << sp.filter[i].pfor_slot;
+    if (pr->block_filter == BlockFilter::kMini) {
+        int64_t tile_cap = 0;
+        int nstaged = 0;
+        for (int s = 0; s < sp.npfor; s++)
+            if ((sp.pfor_filter_mask >> s) & 1u) {
+                tile_cap = std::max<int64_t>(tile_cap, t.cols[(size_t)pr->pfor_cols[(size_t)s]].max_tile_bytes);
+                nstaged++;
             }
-            // Pruning: every predicate is a range on an encoded column that has block statistics.
-            pr->prune = false;
-            if (sp.nfilter > 0 && !pr->hybrid && !getenv("IMM3_NO_PRUNE")) {
-                bool ok = true;
-                std::memset(&pr->pp, 0, sizeof pr->pp);
-                for (int i = 0; i < sp.nfilter && ok; i++) {
-                    const FilterCol& f = sp.filter[i];
-                    ok = f.pfor_slot >= 0 && f.kind == kFilterI32Range && t.cols[(size_t)pfor_cols[(size_t)f.pfor_slot]].d_stats != nullptr;
-                    if (ok) {
-                        pr->pp.stats[i] = (const BlockStat*)t.cols[(size_t)pfor_cols[(size_t)f.pfor_slot]].d_stats;
-                        pr->pp.lo[i] = f.lo;
-                        pr->pp.hi[i] = (int32_t)((int64_t)f.lo + (int64_t)f.span);
-                    }
-                }
-                pr->pp.nfilter = sp.nfilter;
-                pr->pp.group_shift = pr->quad ? 5 : 3;
-                pr->prune = ok;
-                // a pruned scan decides whole blocks from 8 bytes each: the whole slice costs what a prefix would - no prefix phase (with a
-                // communicator phase A then is this rank's whole slice and phase B the count exchange alone: the protocol is unchanged)
-                if (ok) pr->prefix_blocks = 0;
-            }
-            pr->blocks_emit_smem = blocks_emit_smem_bytes(sp.npfor, sp.blk_words_cap);
-            int occ_e = 0;
-            CUDA_TRY(blocks_multi_occupancy(pr->dyn_smem, pr->blocks_emit_smem, pr->hybrid ? nullptr : &occ, &occ_e, pr->lane ? (2 | (pr->lane_warps << 8)) : (pr->quad ? 1 : 0), pr->hybrid));
-            if (occ_e < 1) return fail(IMM3_ERR_CUDA, "block emit kernel does not fit on an SM (dynamic shared memory %zu bytes)", pr->blocks_emit_smem);
-            pr->grid_blocks_emit = (int)std::max<int64_t>(1, std::min<int64_t>((t.nblocks + 7) / 8, (int64_t)db->num_sms * std::max(1, occ_e)));
-            if (pr->hybrid) {
-                // No predicate touches an encoded column: the dense filter kernel runs over the table's row space (dense
-                // columns are contiguous in HBM whatever the block framing) and only the emit kernel works per block.
-                CUDA_TRY(config_dense_filter());
-            }
-        } else {
-            sp.ntiles = t.nblocks;
-            pr->dyn_smem = blocks_kernel_smem_bytes(sp.npfor, t.max_block_rows);
-            CUDA_TRY(blocks_kernel_occupancy(pr->dyn_smem, &occ));
-        }
-    } else {
-        if (pr->multipass) {
-            if (lp.limit > 0 && lp.limit <= (1 << 20) && !getenv("IMM3_NO_PREFIX")) {  // (same policy as the block tables above)
-                const int64_t min_rows = getenv("IMM3_PREFIX_ROWS") ? std::max(1024, atoi(getenv("IMM3_PREFIX_ROWS"))) : (4 << 20);
-                const int64_t want = (std::max<int64_t>(min_rows, lp.limit * 64) + kDenseTileRowsPerWord - 1) / kDenseTileRowsPerWord * kDenseTileRowsPerWord;
-                if (want * 2 <= t.nrows) pr->prefix_rows = want;
-            }
-            CUDA_TRY(config_dense_filter());
-            const int W = 1;
-            const int tile_rows = kDenseTileRowsPerWord;
-            int occ_emit = 0;
-            pr->emit_general = sp.nproj > 4 || getenv("IMM3_EMIT_GENERAL");
-            for (int i = 0; i < sp.nproj; i++) pr->emit_general = pr->emit_general || !(sp.proj[i].width == 1 || sp.proj[i].width == 2 || sp.proj[i].width == 4);
-            CUDA_TRY(emit_kernel_occupancy(pr->emit_general, &occ_emit));
-            const int64_t nspans = sp.ntiles * (tile_rows / 1024);
-            pr->grid_emit = (int)std::max<int64_t>(1, std::min<int64_t>((nspans + 7) / 8, (int64_t)db->num_sms * std::max(1, occ_emit)));
-            // Streaming emit kernel (dense results): a stage = bitmap words + span counts + one 8192-row tile of every
-            // projected column, if that fits.
-            int pstage = 0;
-            for (int i = 0; i < sp.nproj; i++) {
-                sp.proj[i].stage_off = pstage;
-                pstage += 1024 * sp.proj[i].width;
-            }
-            pr->emit_stage_bytes = 0;
-            if (sp.nproj > 0 && 8 * pstage <= 64 * 1024 && !(db->flags & IMM3_OPEN_NO_TMA) && !getenv("IMM3_NO_EMIT_STREAM")) {
-                pr->emit_stage_bytes = emit_stream_header_bytes() + 8 * pstage;
-                pr->emit_ring = std::max(2, std::min(4, (80 * 1024) / pr->emit_stage_bytes));
-                if (const char* e = getenv("IMM3_EMIT_STAGES")) {
-                    int v = atoi(e);
-                    if (v >= 2 && v <= 4) pr->emit_ring = v;
-                }
-                pr->emit_smem = emit_stream_smem_bytes(pr->emit_stage_bytes, pr->emit_ring);
-                int occ_s = 0;
-                CUDA_TRY(emit_stream_occupancy(pr->emit_smem, &occ_s));
-                if (occ_s < 1) pr->emit_stage_bytes = 0;
-                pr->grid_emit_stream = (int)std::max<int64_t>(1, std::min<int64_t>(sp.ntiles * W, (int64_t)db->num_sms * std::max(1, occ_s)));
-            }
+        sp.blk_tile_bytes = (int)((tile_cap + 16 + 15) & ~15ll);
+        const int slot_bytes = blocks_filter_slot_bytes(nstaged, sp.blk_tile_bytes);
+        int ring = std::max(2, std::min(kMaxFilterStages, (48 * 1024) / slot_bytes));
+        if (ring_env) ring = std::max(2, std::min(kMaxFilterStages, atoi(ring_env)));
+        while (ring > 2 && (size_t)ring * slot_bytes > 200 * 1024) ring--;
+        sp.stages = ring;
+        sp.stage_bytes = slot_bytes;
+        pr->dyn_smem = blocks_filter_smem_bytes(nstaged, sp.blk_tile_bytes, ring);
+        return;
+    }
+    const int64_t cap32 = quad_tile_cap(t, pr->lp);
+    const int qslot = blocks_filter_quad_slot_bytes((int)cap32);
+    sp.blk_tile_bytes = (int)cap32;
+    sp.stage_bytes = qslot;
+    if (pr->block_filter == BlockFilter::kQuad) {
+        int qring = std::max(2, std::min(4, (40 * 1024) / qslot));
+        if (ring_env) qring = std::max(2, std::min(kMaxFilterStages, atoi(ring_env)));
+        sp.stages = qring;
+        pr->dyn_smem = (size_t)qring * (size_t)qslot;
+        return;
+    }
+    int lring = 2;
+    if (const char* e = getenv("IMM3_LANE_STAGES")) lring = std::max(2, std::min(4, atoi(e)));
+    while (lring > 2 && (size_t)lring * 4 * (size_t)qslot > kLaneSmemCap) lring--;
+    int lw = (int)std::min<size_t>(16, kLaneSmemCap / ((size_t)lring * (size_t)qslot));
+    if (const char* e = getenv("IMM3_LANE_WARPS")) lw = std::max(4, std::min(lw, atoi(e)));
+    pr->lane_warps = lw;
+    sp.stages = lring;
+    pr->dyn_smem = (size_t)lring * (size_t)lw * (size_t)qslot;
+}
+
+// kBlocks: pruning, if every predicate is a range on an encoded column that has block statistics.
+void size_prune(Prepared* pr) {
+    const TableStore& t = *pr->table;
+    const ScanPlan& sp = pr->sp;
+    pr->prune = false;
+    if (sp.nfilter == 0 || getenv("IMM3_NO_PRUNE")) return;
+    bool ok = true;
+    std::memset(&pr->pp, 0, sizeof pr->pp);
+    for (int i = 0; i < sp.nfilter && ok; i++) {
+        const FilterCol& f = sp.filter[i];
+        ok = f.pfor_slot >= 0 && f.kind == kFilterI32Range && t.cols[(size_t)pr->pfor_cols[(size_t)f.pfor_slot]].d_stats != nullptr;
+        if (ok) {
+            pr->pp.stats[i] = (const BlockStat*)t.cols[(size_t)pr->pfor_cols[(size_t)f.pfor_slot]].d_stats;
+            pr->pp.lo[i] = f.lo;
+            pr->pp.hi[i] = (int32_t)((int64_t)f.lo + (int64_t)f.span);
         }
     }
+    pr->pp.nfilter = sp.nfilter;
+    pr->pp.group_shift = pr->block_filter == BlockFilter::kMini ? 3 : 5;
+    pr->prune = ok;
+    // a pruned scan decides whole blocks from 8 bytes each: the whole slice costs what a prefix would - no prefix phase (with a
+    // communicator phase A then is this rank's whole slice and phase B the count exchange alone: the protocol is unchanged)
+    if (ok) pr->prefix_blocks = 0;
+}
+
+// kRowSpace, kBlocks: the block emit kernel, and (kBlocks) the occupancy of the block filter kernel.
+int size_block_emit(imm3_db* db, Prepared* pr, int* occ) {
+    const TableStore& t = *pr->table;
+    ScanPlan& sp = pr->sp;
+    int64_t words = 0;
+    for (int ci : pr->pfor_cols) words = std::max<int64_t>(words, t.cols[(size_t)ci].max_block_words);
+    sp.blk_words_cap = block_words_cap(words);
+    pr->blocks_emit_smem = blocks_emit_smem_bytes(sp.npfor, sp.blk_words_cap);
+    const bool rowspace = pr->pipeline == Pipeline::kRowSpace;
+    int occ_e = 0;
+    CUDA_TRY(blocks_multi_occupancy(pr->dyn_smem, pr->blocks_emit_smem, rowspace ? nullptr : occ, &occ_e, pr->block_filter, pr->lane_warps, rowspace));
+    if (occ_e < 1) return fail(IMM3_ERR_CUDA, "block emit kernel does not fit on an SM (dynamic shared memory %zu bytes)", pr->blocks_emit_smem);
+    pr->grid_blocks_emit = (int)std::max<int64_t>(1, std::min<int64_t>((t.nblocks + 7) / 8, (int64_t)db->num_sms * std::max(1, occ_e)));
+    return 0;
+}
+
+// The filter kernel's persistent grid from its occupancy, and the status words of the tiles.
+int plan_grid(imm3_db* db, Prepared* pr, int occ) {
+    const ScanPlan& sp = pr->sp;
     if (sp.ntiles >= (int64_t)0x7FFFFFFF) return fail(IMM3_ERR_UNSUPPORTED, "too many tiles (%lld)", (long long)sp.ntiles);
     if (occ < 1) return fail(IMM3_ERR_CUDA, "kernel does not fit on an SM (dynamic shared memory %zu bytes)", pr->dyn_smem);
     const int64_t persistent = (int64_t)db->num_sms * occ;
@@ -808,6 +833,45 @@ int fill_scan_plan(imm3_db* db, Prepared* pr) {
     return 0;
 }
 
+// Fill the device plan of the query's pipeline (everything but result pointers and the bitmap).
+int fill_scan_plan(imm3_db* db, Prepared* pr) {
+    const TableStore& t = *pr->table;
+    int occ = 0, rc = plan_columns(db, pr);
+    if (rc) return rc;
+    const int64_t prefix = prefix_rows_wanted(pr->lp);
+    switch (pr->pipeline) {
+    case Pipeline::kDense: {
+        const int64_t want = (prefix + kDenseTileRowsPerWord - 1) / kDenseTileRowsPerWord * kDenseTileRowsPerWord;
+        if (want * 2 <= t.nrows) pr->prefix_rows = want;
+        if ((rc = size_dense_filter(db, pr, &occ)) || (rc = size_dense_emit(db, pr))) return rc;
+        break;
+    }
+    case Pipeline::kRowSpace:
+    case Pipeline::kBlocks: {
+        const int64_t nb = (prefix + 1023) / 1024;
+        if (nb * 2 <= t.nblocks) pr->prefix_blocks = nb;
+        if (pr->pipeline == Pipeline::kRowSpace) {
+            if ((rc = size_dense_filter(db, pr, &occ))) return rc;
+        } else {
+            pr->sp.ntiles = (t.nblocks + 7) / 8;  // the offset scan works on tiles of 8 blocks
+            size_block_filter(pr);
+            size_prune(pr);
+        }
+        if ((rc = size_block_emit(db, pr, &occ))) return rc;
+        break;
+    }
+    case Pipeline::kSinglePass:  // scan_blocks stages whole blocks
+        if (t.max_block_rows > kMaxBlockRows)
+            return fail(IMM3_ERR_UNSUPPORTED, "block-mode kernel stages blocks of at most %d rows, table %s has a block of %d",
+                        kMaxBlockRows, t.meta.name.c_str(), t.max_block_rows);
+        pr->sp.ntiles = t.nblocks;
+        pr->dyn_smem = blocks_kernel_smem_bytes(pr->sp.npfor, t.max_block_rows);
+        CUDA_TRY(blocks_kernel_occupancy(pr->dyn_smem, &occ));
+        break;
+    }
+    return plan_grid(db, pr, occ);
+}
+
 int ensure_buf(Buf* b, size_t bytes) {
     if (b->cap >= bytes) return 0;
     if (b->p) cudaFree(b->p);
@@ -818,7 +882,26 @@ int ensure_buf(Buf* b, size_t bytes) {
     return 0;
 }
 
-// Launch the kernels of one query and wait for the match count.
+// Tile counts and offsets, in whole rounds (4096 tiles) of the offset scan.
+int ensure_tile_scratch(imm3_db* db, int64_t ntiles) {
+    const size_t ntiles_pad = ((size_t)ntiles + 4095) / 4096 * 4096 + 16;
+    int rc = ensure_buf(&db->d_tile_cnt, ntiles_pad * 4);
+    return rc ? rc : ensure_buf(&db->d_tile_off, ntiles_pad * 8);
+}
+
+// Scratch of the filter kernel over the row space: the selection bitmap (unless the plan brings its own), span counts, tile
+// counts and offsets.  (+64 bitmap words: the row-space emit kernel reads, for every lane of a block's warp, the word holding
+// bit R0 + 32*lane and the one after it - up to 33 words past the last row's word for a 1-row tail block at the end of the slice)
+int ensure_row_space(imm3_db* db, ScanPlan& sp) {
+    int rc;
+    if (!sp.bitmap) {
+        if ((rc = ensure_buf(&db->d_bitmap, (size_t)(sp.ntiles * kDenseTileRowsPerWord / 32 + 64) * 4))) return rc;
+        sp.bitmap = (uint32_t*)db->d_bitmap.p;
+    }
+    if ((rc = ensure_buf(&db->d_span_cnt, (size_t)(sp.ntiles * (kDenseTileRowsPerWord / 1024) + 8) * 4))) return rc;
+    return ensure_tile_scratch(db, sp.ntiles);
+}
+
 // Launch the count-exchange kernel of one round (every rank of the communicator must launch the same rounds in the same
 // order).  has_count = 0: this rank ran no kernel in this query (empty slice) and contributes 0.
 int launch_exchange(imm3_db* db, int64_t limit, int has_count, unsigned long long pub_seq = 0) {
@@ -879,12 +962,8 @@ int prepare_scan_buffers(imm3_db* db, int64_t ntiles, bool want_list) {
     return 0;
 }
 int launch_scan_kernel(imm3_db* db, const ScanPlan& sp, int64_t ntiles, int* launches, bool want_list = false) {
-    {
-        int rc = prepare_scan_buffers(db, ntiles, want_list);
-        if (rc) return rc;
-    }
-    const size_t nchunks = (size_t)((ntiles + 4095) / 4096);
-    (void)nchunks;
+    int rc = prepare_scan_buffers(db, ntiles, want_list);
+    if (rc) return rc;
     CUDA_TRY(launch_offset_scan((const uint32_t*)db->d_tile_cnt.p, (unsigned long long*)db->d_tile_off.p, ntiles, sp.limit, db->scan_epoch,
                                 (unsigned long long*)db->d_scan_part.p, db->d_ctrl, want_list ? (unsigned int*)db->d_tile_list.p : nullptr, db->stream));
     note_launch(db, launches, "offset_scan");
@@ -910,246 +989,229 @@ int launch_or_terms(imm3_db* db, Prepared* pr, int scan_inline, int* launches) {
     return 0;
 }
 
+// What a pipeline's launch function tells the epilogue of run_scan_once.
+struct Queued {
+    int* launches;
+    unsigned long long pub_seq;  // publish (plan.hpp): sequence number of this launch sequence
+    bool publish;                // the pipeline's last kernel may write the pinned control block itself
+    bool published = false;      // ... and does
+    bool have_mid = false;       // ev_mid splits the device time into two stages
+};
+
+// No event may sit between a kernel and its programmatic dependent: without PDL (IMM3_NO_PDL, or nothing to emit) ev_mid
+// marks the end of the filter stage.
+int mark_mid(imm3_db* db, bool pdl, Queued* q) {
+    if (pdl) return 0;
+    CUDA_TRY(cudaEventRecord(db->ev_mid, db->stream));
+    q->have_mid = true;
+    return 0;
+}
+
+// IMM3_DEBUG bit 16 + IMM3_TRACE (debugging): phase stamps, min / max over CTAs or warps, then `extra` words
+int setup_phase_trace(imm3_db* db, ScanPlan& sp, size_t extra) {
+    if (!(sp.debug & 16u) || !getenv("IMM3_TRACE")) return 0;
+    int rc = ensure_buf(&db->d_trace, (64 + extra) * 8);
+    if (rc) return rc;
+    std::vector<unsigned long long> init(64 + extra);
+    for (int i = 0; i < 64; i++) init[(size_t)i] = (i & 1) ? 0ull : ~0ull;
+    CUDA_TRY(cudaMemcpyAsync(db->d_trace.p, init.data(), init.size() * 8, cudaMemcpyHostToDevice, db->stream));
+    CUDA_TRY(cudaStreamSynchronize(db->stream));
+    sp.trace = (unsigned long long*)db->d_trace.p;
+    return 0;
+}
+
+// The filter kernel over the row space (from ev0 on), the later terms of a real OR, and the offset scan unless the filter
+// kernel's last CTA runs it.
+int launch_row_space_filter(imm3_db* db, Prepared* pr, int* launches) {
+    ScanPlan& sp = pr->sp;
+    const int scan_inline = (sp.nfilter == 0 || scan_inline_for(sp.ntiles)) ? 1 : 0;
+    sp.scan_inline = pr->or_terms.empty() ? scan_inline : 0;
+    CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
+    CUDA_TRY(launch_filter(sp, sp.bitmap, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p, (unsigned long long*)db->d_tile_off.p,
+                           db->d_ctrl, pr->grid, pr->dyn_smem, db->stream));
+    note_launch(db, launches, filter_route(sp));
+    int rc = launch_or_terms(db, pr, scan_inline, launches);
+    if (rc) return rc;
+    sp.scan_inline = scan_inline;
+    return scan_inline ? 0 : launch_scan_kernel(db, sp, sp.ntiles, launches);
+}
+
+// kDense: filter kernel -> emit kernels.  Two emit kernels, one of which does the work: which one is decided on the device
+// from the match count, unless an earlier query of this shape said which (see emit_hint).
+int launch_dense(imm3_db* db, Prepared* pr, Queued* q) {
+    ScanPlan& sp = pr->sp;
+    int rc;
+    if ((rc = setup_phase_trace(db, sp, 0)) || (rc = ensure_row_space(db, sp))) return rc;
+    const int stream_ok = pr->emit_stage_bytes > 0 && sp.nproj > 0;
+    const char* force = getenv("IMM3_EMIT");  // experiment: "stream" / "gather" = that kernel takes every result, "both" = no feedback
+    int hint = -1;
+    if (stream_ok && !(force && !strcmp(force, "both"))) {
+        auto it = db->emit_hint.find(pr->shape_key);
+        if (it != db->emit_hint.end()) hint = it->second;
+        if (force && !strcmp(force, "stream")) hint = 1;
+        if (force && !strcmp(force, "gather")) hint = 0;
+    }
+    const bool only_stream = stream_ok && hint == 1, only_gather = stream_ok && hint == 0;
+    // The first emit kernel is launched as a programmatic dependent of the filter kernel (its prologue overlaps the filter
+    // kernel's tail); IMM3_NO_PDL=1 restores per-stage timing.
+    const bool pdl = sp.nproj > 0 && !getenv("IMM3_NO_PDL");
+    if ((rc = launch_row_space_filter(db, pr, q->launches)) || (rc = mark_mid(db, pdl, q))) return rc;
+    if (sp.nproj == 0) return 0;
+    const int64_t nspans = sp.ntiles * (kDenseTileRowsPerWord / 1024);
+    if (stream_ok && !only_gather) {
+        CUDA_TRY(launch_emit_stream(sp, sp.bitmap, (const uint32_t*)db->d_span_cnt.p, (const uint32_t*)db->d_tile_cnt.p,
+                                    (const unsigned long long*)db->d_tile_off.p, sp.ntiles, pr->emit_ring, pr->emit_stage_bytes,
+                                    only_stream ? -1 : 1, pr->grid_emit_stream, pr->emit_smem, db->d_ctrl, pdl, db->stream));
+        note_launch(db, q->launches, with_stages("emit_stream", pr->emit_ring));
+    }
+    if (!only_stream) {
+        CUDA_TRY(launch_emit(sp, sp.bitmap, (const uint32_t*)db->d_span_cnt.p, (const unsigned long long*)db->d_tile_off.p, 8,
+                             nspans, pr->grid_emit, stream_ok && !only_gather, db->d_ctrl, pr->emit_general, pdl && (only_gather || !stream_ok),
+                             db->stream));
+        note_launch(db, q->launches, pr->emit_general ? "emit_general" : "emit");
+    }
+    return 0;
+}
+
+// kRowSpace: filter kernel over the row space -> block emit kernel.
+int launch_row_space(imm3_db* db, Prepared* pr, int64_t nblocks, Queued* q) {
+    ScanPlan& sp = pr->sp;
+    const bool pdl = sp.nproj > 0 && !getenv("IMM3_NO_PDL");
+    int rc;
+    if ((rc = ensure_row_space(db, sp)) || (rc = launch_row_space_filter(db, pr, q->launches)) || (rc = mark_mid(db, pdl, q))) return rc;
+    if (sp.nproj == 0) return 0;
+    CUDA_TRY(launch_blocks_emit(sp, sp.bitmap, (const uint32_t*)db->d_span_cnt.p, nullptr, (const unsigned long long*)db->d_tile_off.p,
+                                nblocks, db->d_ctrl, true, pdl, (int)std::min<int64_t>(pr->grid_blocks_emit, (nblocks + 7) / 8),
+                                pr->blocks_emit_smem, db->stream));
+    note_launch(db, q->launches, "blocks_emit(rowspace)");
+    return 0;
+}
+
+// kBlocks: [blocks_prune ->] block filter kernel -> group emit (lane kernel, one encoded column projected: every emit warp finds
+// its rows from the group sums, no scan), scan-emit (one encoded column projected: offset scan + emit in one small-footprint
+// kernel, resident while the filter kernel runs) or offset scan + block emit kernel.
+int launch_blocks(imm3_db* db, Prepared* pr, int64_t nblocks, Queued* q) {
+    const TableStore& t = *pr->table;
+    ScanPlan& sp = pr->sp;
+    const int64_t ntiles = sp.ntiles;
+    const bool lane = pr->block_filter == BlockFilter::kLane;
+    int rc;
+    if ((rc = ensure_buf(&db->d_bitmap, (size_t)(nblocks * 32 + 2) * 4))) return rc;
+    if ((rc = ensure_buf(&db->d_span_cnt, (size_t)(nblocks + 8 + 1024) * 4))) return rc;  // (+ whole 16-byte loads of a group's counts)
+    if ((rc = ensure_tile_scratch(db, ntiles))) return rc;
+    sp.scan_inline = (scan_inline_for(ntiles) && !(lane && pr->lane_warps < 8)) ? 1 : 0;  // (the inline scan is written for 8 warps)
+    int fused_grid = 0;  // > 0: blocks_scan_emit_kernel
+    int group_grid = 0, ngroups = 0;  // > 0: blocks_group_emit_kernel
+    if (sp.nproj == 1 && sp.proj[0].pfor_slot >= 0 && !getenv("IMM3_NO_SCANEMIT")) {
+        if (lane && !getenv("IMM3_NO_GROUPEMIT")) CUDA_TRY(blocks_group_emit_grid(db->num_sms, nblocks, &group_grid, &ngroups));
+        if (group_grid > 0) {
+            if (!db->d_grp_sum.p) {
+                CUDA_TRY(cudaMalloc(&db->d_grp_sum.p, blocks_group_sum_bytes()));
+                db->d_grp_sum.cap = blocks_group_sum_bytes();
+                CUDA_TRY(cudaMemsetAsync(db->d_grp_sum.p, 0, db->d_grp_sum.cap, db->stream));
+            }
+            sp.scan_inline = 0;
+        } else {
+            CUDA_TRY(blocks_scan_emit_grid(db->num_sms, ntiles, &fused_grid));
+            if (fused_grid > 0) {
+                if ((rc = prepare_scan_buffers(db, ntiles, true))) return rc;
+                sp.scan_inline = 0;
+            }
+        }
+    }
+    uint32_t* const grp_sum = group_grid > 0 ? (uint32_t*)db->d_grp_sum.p : nullptr;
+    const unsigned int* work = nullptr;
+    if (pr->prune) {
+        if ((rc = ensure_buf(&db->d_work, (size_t)((nblocks + 7) / 8 + 2) * 4))) return rc;
+        work = (const unsigned int*)db->d_work.p;
+    }
+    if ((rc = setup_phase_trace(db, sp, 1024))) return rc;
+    CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
+    if (pr->prune) {
+        // whole blocks decided from their min / max; only the tiles a window edge cuts through reach the filter kernel
+        CUDA_TRY(cudaMemsetAsync(db->d_work.p, 0, 4, db->stream));
+        CUDA_TRY(launch_blocks_prune(pr->pp, t.d_row_start, nblocks, ntiles, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
+                                     (unsigned int*)db->d_work.p, db->num_sms, db->stream, grp_sum));
+        note_launch(db, q->launches, "blocks_prune");
+    }
+    int filter_grid = pr->grid;
+    if (pr->block_filter != BlockFilter::kMini) {  // CTA tiles of 32 blocks (quad), 32 blocks per warp (lane)
+        const int64_t per_cta = 32 * (lane ? pr->lane_warps : 1);
+        filter_grid = (int)std::max<int64_t>(1, std::min<int64_t>(pr->grid, (nblocks + per_cta - 1) / per_cta));
+    }
+    CUDA_TRY(launch_blocks_filter(sp, (uint32_t*)db->d_bitmap.p, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
+                                  (unsigned long long*)db->d_tile_off.p, db->d_ctrl, nblocks, filter_grid, pr->dyn_smem, pr->block_filter,
+                                  pr->lane_warps, work, db->stream, grp_sum));
+    note_launch(db, q->launches, lane ? "blocks_filter_lane/w=" + std::to_string(pr->lane_warps) + "/s=" + std::to_string(sp.stages)
+                                      : with_stages(pr->block_filter == BlockFilter::kQuad ? "blocks_filter_quad" : "blocks_filter", sp.stages));
+    CtrlBlock* const pub = q->publish ? db->h_ctrl : nullptr;
+    const unsigned long long pub_seq = q->publish ? q->pub_seq : 0;
+    if (group_grid > 0 || fused_grid > 0) {
+        const bool pdl = !getenv("IMM3_NO_PDL");
+        if ((rc = mark_mid(db, pdl, q))) return rc;
+        if (group_grid > 0) {
+            CUDA_TRY(launch_blocks_group_emit(sp, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, grp_sum, nblocks, ngroups,
+                                              db->d_ctrl, pdl, group_grid, db->stream, pub, pub_seq));
+            note_launch(db, q->launches, "blocks_group_emit/ctas=" + std::to_string(group_grid));
+        } else {
+            CUDA_TRY(launch_blocks_scan_emit(sp, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, (const uint32_t*)db->d_tile_cnt.p,
+                                             (unsigned long long*)db->d_tile_off.p, nblocks, db->scan_epoch, (unsigned long long*)db->d_scan_part.p,
+                                             db->d_ctrl, (unsigned int*)db->d_tile_list.p, pdl, fused_grid, db->stream, pub, pub_seq));
+            note_launch(db, q->launches, "blocks_scan_emit");
+        }
+        q->published = q->publish;
+    } else {
+        if (!sp.scan_inline && (rc = launch_scan_kernel(db, sp, ntiles, q->launches, true))) return rc;
+        const bool pdl = sp.nproj > 0 && !getenv("IMM3_NO_PDL");
+        if ((rc = mark_mid(db, pdl, q))) return rc;
+        if (sp.nproj > 0) {
+            CUDA_TRY(launch_blocks_emit(sp, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p,
+                                        sp.scan_inline ? nullptr : (const unsigned int*)db->d_tile_list.p,
+                                        (const unsigned long long*)db->d_tile_off.p, nblocks, db->d_ctrl, false, pdl,
+                                        (int)std::min<int64_t>(pr->grid_blocks_emit, (nblocks + 7) / 8), pr->blocks_emit_smem, db->stream));
+            note_launch(db, q->launches, "blocks_emit(blocks)");
+        }
+    }
+    return 0;
+}
+
+// Launch the kernels of one query and wait for the match count.
 int run_scan_once(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* launches, double* stage_ms, int64_t nblocks_use, bool exchange) {
-    bool have_mid = false;
     pr->sp.scan_inline = 1;
     *launches = 0;
     // publish (plan.hpp): the query's last kernel writes the pinned control block itself and the host polls it
     const bool publish_ok = !getenv("IMM3_NO_PUBLISH");
-    const unsigned long long pub_seq = ++db->pub_seq;
-    bool published = false;
-    if (pr->block_mode && pr->hybrid) {
-        // dense filter kernel over the row space -> block emit kernel (decodes only blocks with surviving rows)
-        TableStore& t = *pr->table;
-        const int64_t ntiles = pr->sp.ntiles, nspans = ntiles * 8;
-        int rc;
-        // (+64 words: the row-space emit kernel reads, for every lane of a block's warp, the word holding bit R0 + 32*lane
-        // and the one after it - up to 33 words past the last row's word for a 1-row tail block at the end of the slice)
-        if ((rc = ensure_buf(&db->d_bitmap, (size_t)(ntiles * kDenseTileRowsPerWord / 32 + 64) * 4))) return rc;
-        pr->sp.bitmap = (uint32_t*)db->d_bitmap.p;
-        if ((rc = ensure_buf(&db->d_span_cnt, (size_t)(nspans + 8) * 4))) return rc;
-        const size_t ntiles_pad = ((size_t)ntiles + 4095) / 4096 * 4096 + 16;  // whole rounds of the offset scan
-        if ((rc = ensure_buf(&db->d_tile_cnt, ntiles_pad * 4))) return rc;
-        if ((rc = ensure_buf(&db->d_tile_off, ntiles_pad * 8))) return rc;
-        const int scan_inline_h = (pr->sp.nfilter == 0 || scan_inline_for(ntiles)) ? 1 : 0;
-        pr->sp.scan_inline = pr->or_terms.empty() ? scan_inline_h : 0;
+    const bool sharded = exchange && db->comm_on;  // (a sharded table: the exchange kernel publishes)
+    Queued q{launches, ++db->pub_seq, publish_ok && !sharded};
+    int rc = 0;
+    switch (pr->pipeline) {
+    case Pipeline::kDense: rc = launch_dense(db, pr, &q); break;
+    case Pipeline::kRowSpace: rc = launch_row_space(db, pr, nblocks_use, &q); break;
+    case Pipeline::kBlocks: rc = launch_blocks(db, pr, nblocks_use, &q); break;
+    case Pipeline::kSinglePass:
         CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
-        CUDA_TRY(launch_filter(pr->sp, pr->sp.bitmap, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
-                               (unsigned long long*)db->d_tile_off.p, db->d_ctrl, pr->grid, pr->dyn_smem, db->stream));
-        note_launch(db, launches, filter_route(pr->sp));
-        if ((rc = launch_or_terms(db, pr, scan_inline_h, launches))) return rc;
-        pr->sp.scan_inline = scan_inline_h;
-        if (!pr->sp.scan_inline && (rc = launch_scan_kernel(db, pr->sp, ntiles, launches))) return rc;
-        const bool pdl = pr->sp.nproj > 0 && !getenv("IMM3_NO_PDL");  // (no event may sit between a kernel and its programmatic dependent)
-        if (!pdl) {
-            CUDA_TRY(cudaEventRecord(db->ev_mid, db->stream));
-            have_mid = true;
-        }
-        if (pr->sp.nproj > 0) {
-            CUDA_TRY(launch_blocks_emit(pr->sp, pr->sp.bitmap, (const uint32_t*)db->d_span_cnt.p, nullptr, (const unsigned long long*)db->d_tile_off.p,
-                                        nblocks_use, db->d_ctrl, true, pdl, (int)std::min<int64_t>(pr->grid_blocks_emit, (nblocks_use + 7) / 8),
-                                        pr->blocks_emit_smem, db->stream));
-            note_launch(db, launches, "blocks_emit(rowspace)");
-        }
-        CUDA_TRY(cudaEventRecord(db->ev1, db->stream));
-    } else if (pr->block_mode && pr->blocks_multi) {
-        TableStore& t = *pr->table;
-        const int64_t nblocks = nblocks_use, ntiles = pr->sp.ntiles;
-        int rc;
-        if ((rc = ensure_buf(&db->d_bitmap, (size_t)(nblocks * 32 + 2) * 4))) return rc;
-        if ((rc = ensure_buf(&db->d_span_cnt, (size_t)(nblocks + 8 + 1024) * 4))) return rc;  // (+ whole 16-byte loads of a group's counts)
-        const size_t ntiles_pad = ((size_t)ntiles + 4095) / 4096 * 4096 + 16;  // whole rounds of the offset scan
-        if ((rc = ensure_buf(&db->d_tile_cnt, ntiles_pad * 4))) return rc;
-        if ((rc = ensure_buf(&db->d_tile_off, ntiles_pad * 8))) return rc;
-        pr->sp.scan_inline = (scan_inline_for(ntiles) && !(pr->lane && pr->lane_warps < 8)) ? 1 : 0;  // (the inline scan is written for 8 warps)
-        const bool publish_here = publish_ok && !(exchange && db->comm_on);  // (a sharded table: the exchange kernel publishes)
-        int fused_grid = 0;  // > 0: offset scan + emit as ONE kernel behind the filter kernel (one encoded column projected)
-        int group_grid = 0, ngroups = 0;  // > 0: no offset scan at all - blocks_group_emit_kernel behind the lane kernel
-        if (pr->sp.nproj == 1 && pr->sp.proj[0].pfor_slot >= 0 && !getenv("IMM3_NO_SCANEMIT")) {
-            if (pr->lane && !getenv("IMM3_NO_GROUPEMIT")) CUDA_TRY(blocks_group_emit_grid(db->num_sms, nblocks, &group_grid, &ngroups));
-            if (group_grid > 0) {
-                if (!db->d_grp_sum.p) {
-                    CUDA_TRY(cudaMalloc(&db->d_grp_sum.p, blocks_group_sum_bytes()));
-                    db->d_grp_sum.cap = blocks_group_sum_bytes();
-                    CUDA_TRY(cudaMemsetAsync(db->d_grp_sum.p, 0, db->d_grp_sum.cap, db->stream));
-                }
-                pr->sp.scan_inline = 0;
-            } else {
-                CUDA_TRY(blocks_scan_emit_grid(db->num_sms, ntiles, &fused_grid));
-                if (fused_grid > 0) {
-                    if ((rc = prepare_scan_buffers(db, ntiles, true))) return rc;
-                    pr->sp.scan_inline = 0;
-                }
-            }
-        }
-        uint32_t* const grp_sum = group_grid > 0 ? (uint32_t*)db->d_grp_sum.p : nullptr;
-        const unsigned int* work = nullptr;
-        if (pr->prune) {
-            if ((rc = ensure_buf(&db->d_work, (size_t)((nblocks + 7) / 8 + 2) * 4))) return rc;
-            work = (const unsigned int*)db->d_work.p;
-        }
-        if ((pr->sp.debug & 16u) && getenv("IMM3_TRACE")) {  // debugging: phase stamps (min / max over warps)
-            int rc0 = ensure_buf(&db->d_trace, (64 + 1024) * 8);
-            if (rc0) return rc0;
-            std::vector<unsigned long long> init(64 + 1024);
-            for (int i = 0; i < 64; i++) init[(size_t)i] = (i & 1) ? 0ull : ~0ull;
-            CUDA_TRY(cudaMemcpyAsync(db->d_trace.p, init.data(), init.size() * 8, cudaMemcpyHostToDevice, db->stream));
-            CUDA_TRY(cudaStreamSynchronize(db->stream));
-            pr->sp.trace = (unsigned long long*)db->d_trace.p;
-        }
-        CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
-        if (pr->prune) {
-            // whole blocks decided from their min / max; only the tiles a window edge cuts through reach the filter kernel
-            CUDA_TRY(cudaMemsetAsync(db->d_work.p, 0, 4, db->stream));
-            CUDA_TRY(launch_blocks_prune(pr->pp, t.d_row_start, nblocks, ntiles, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
-                                         (unsigned int*)db->d_work.p, db->num_sms, db->stream, grp_sum));
-            note_launch(db, launches, "blocks_prune");
-        }
-        CUDA_TRY(launch_blocks_filter(pr->sp, (uint32_t*)db->d_bitmap.p, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
-                                      (unsigned long long*)db->d_tile_off.p, db->d_ctrl, nblocks,
-                                      pr->lane ? (int)std::max<int64_t>(1, std::min<int64_t>(pr->grid, (nblocks + 32 * pr->lane_warps - 1) / (32 * pr->lane_warps)))
-                                               : (pr->quad ? (int)std::max<int64_t>(1, std::min<int64_t>(pr->grid, (nblocks + 31) / 32)) : pr->grid),
-                                      pr->dyn_smem, pr->lane ? (2 | (pr->lane_warps << 8)) : (pr->quad ? 1 : 0), work, db->stream, grp_sum));
-        note_launch(db, launches, pr->lane   ? "blocks_filter_lane/w=" + std::to_string(pr->lane_warps) + "/s=" + std::to_string(pr->sp.stages)
-                                  : pr->quad ? with_stages("blocks_filter_quad", pr->sp.stages)
-                                             : with_stages("blocks_filter", pr->sp.stages));
-        if (group_grid > 0) {
-            // one encoded column projected, lane kernel in front: every emit warp finds its rows from the group sums - no scan
-            const bool pdl = !getenv("IMM3_NO_PDL");
-            if (!pdl) {
-                CUDA_TRY(cudaEventRecord(db->ev_mid, db->stream));
-                have_mid = true;
-            }
-            CUDA_TRY(launch_blocks_group_emit(pr->sp, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, grp_sum, nblocks, ngroups,
-                                              db->d_ctrl, pdl, group_grid, db->stream, publish_here ? db->h_ctrl : nullptr, publish_here ? pub_seq : 0));
-            published = publish_here;
-            note_launch(db, launches, "blocks_group_emit/ctas=" + std::to_string(group_grid));
-            CUDA_TRY(cudaEventRecord(db->ev1, db->stream));
-        } else if (fused_grid > 0) {
-            // one encoded column projected: offset scan + emit in one small-footprint kernel, resident while the filter kernel runs
-            const bool pdl = !getenv("IMM3_NO_PDL");
-            if (!pdl) {
-                CUDA_TRY(cudaEventRecord(db->ev_mid, db->stream));
-                have_mid = true;
-            }
-            CUDA_TRY(launch_blocks_scan_emit(pr->sp, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, (const uint32_t*)db->d_tile_cnt.p,
-                                             (unsigned long long*)db->d_tile_off.p, nblocks, db->scan_epoch, (unsigned long long*)db->d_scan_part.p,
-                                             db->d_ctrl, (unsigned int*)db->d_tile_list.p, pdl, fused_grid, db->stream,
-                                             publish_here ? db->h_ctrl : nullptr, publish_here ? pub_seq : 0));
-            published = publish_here;
-            note_launch(db, launches, "blocks_scan_emit");
-            CUDA_TRY(cudaEventRecord(db->ev1, db->stream));
-        } else {
-        if (!pr->sp.scan_inline && (rc = launch_scan_kernel(db, pr->sp, ntiles, launches, true))) return rc;
-        const bool pdl = pr->sp.nproj > 0 && !getenv("IMM3_NO_PDL");
-        if (!pdl) {
-            CUDA_TRY(cudaEventRecord(db->ev_mid, db->stream));
-            have_mid = true;
-        }
-        if (pr->sp.nproj > 0) {
-            CUDA_TRY(launch_blocks_emit(pr->sp, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p,
-                                        pr->sp.scan_inline ? nullptr : (const unsigned int*)db->d_tile_list.p,
-                                        (const unsigned long long*)db->d_tile_off.p, nblocks, db->d_ctrl, false, pdl,
-                                        (int)std::min<int64_t>(pr->grid_blocks_emit, (nblocks + 7) / 8), pr->blocks_emit_smem, db->stream));
-            note_launch(db, launches, "blocks_emit(blocks)");
-        }
-        CUDA_TRY(cudaEventRecord(db->ev1, db->stream));
-        }
-    } else if (pr->multipass) {
-        if ((pr->sp.debug & 16u) && getenv("IMM3_TRACE")) {  // debugging: phase stamps (min / max over CTAs)
-            int rc0 = ensure_buf(&db->d_trace, 64 * 8);
-            if (rc0) return rc0;
-            std::vector<unsigned long long> init(64);
-            for (int i = 0; i < 64; i++) init[(size_t)i] = (i & 1) ? 0ull : ~0ull;
-            CUDA_TRY(cudaMemcpyAsync(db->d_trace.p, init.data(), 64 * 8, cudaMemcpyHostToDevice, db->stream));
-            CUDA_TRY(cudaStreamSynchronize(db->stream));
-            pr->sp.trace = (unsigned long long*)db->d_trace.p;
-        }
-        const int64_t tile_rows = (int64_t)kDenseTileRowsPerWord * pr->sp.words_per_lane;
-        const int64_t ntiles = pr->sp.ntiles, nspans = ntiles * (tile_rows / 1024);
-        const int64_t nsub = ntiles * pr->sp.words_per_lane;  // 8192-row sub-tiles: the unit of the offset scan
-        int rc;
-        if (!pr->sp.bitmap) {
-            if ((rc = ensure_buf(&db->d_bitmap, (size_t)(ntiles * tile_rows / 32 + 2) * 4))) return rc;
-            pr->sp.bitmap = (uint32_t*)db->d_bitmap.p;
-        }
-        if ((rc = ensure_buf(&db->d_span_cnt, (size_t)nspans * 4))) return rc;
-        const size_t nsub_pad = ((size_t)nsub + 4095) / 4096 * 4096 + 16;  // whole rounds of the offset scan
-        if ((rc = ensure_buf(&db->d_tile_cnt, nsub_pad * 4))) return rc;
-        if ((rc = ensure_buf(&db->d_tile_off, nsub_pad * 8))) return rc;
-        // Emit-kernel choice known from an earlier query of this shape (see emit_hint).
-        const int stream_ok = pr->emit_stage_bytes > 0 && pr->sp.nproj > 0;
-        const char* force = getenv("IMM3_EMIT");  // experiment: "stream" / "gather" = that kernel takes every result, "both" = no feedback
-        int hint = -1;
-        if (stream_ok && !(force && !strcmp(force, "both"))) {
-            auto it = db->emit_hint.find(pr->shape_key);
-            if (it != db->emit_hint.end()) hint = it->second;
-            if (force && !strcmp(force, "stream")) hint = 1;
-            if (force && !strcmp(force, "gather")) hint = 0;
-        }
-        const bool only_stream = stream_ok && hint == 1, only_gather = stream_ok && hint == 0;
-        const bool pdl = pr->sp.nproj > 0 && !getenv("IMM3_NO_PDL");  // the first emit kernel launched is a programmatic dependent
-        const int scan_inline_d = (pr->sp.nfilter == 0 || scan_inline_for(nsub)) ? 1 : 0;
-        pr->sp.scan_inline = pr->or_terms.empty() ? scan_inline_d : 0;
-        CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
-        CUDA_TRY(launch_filter(pr->sp, pr->sp.bitmap, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
-                               (unsigned long long*)db->d_tile_off.p, db->d_ctrl, pr->grid, pr->dyn_smem, db->stream));
-        note_launch(db, launches, filter_route(pr->sp));
-        if ((rc = launch_or_terms(db, pr, scan_inline_d, launches))) return rc;
-        pr->sp.scan_inline = scan_inline_d;
-        if (!pr->sp.scan_inline && (rc = launch_scan_kernel(db, pr->sp, nsub, launches))) return rc;
-        // The streaming emit kernel is launched as a programmatic dependent of the filter kernel (its prologue overlaps the
-        // filter kernel's tail), so no event may sit between the two; IMM3_NO_PDL=1 restores per-stage timing.
-        if (!pdl) {
-            CUDA_TRY(cudaEventRecord(db->ev_mid, db->stream));
-            have_mid = true;
-        }
-        if (pr->sp.nproj > 0) {
-            // Two emit kernels, one of which does the work: which one is decided on the device from the match count.
-            if (stream_ok && !only_gather) {
-                CUDA_TRY(launch_emit_stream(pr->sp, pr->sp.bitmap, (const uint32_t*)db->d_span_cnt.p, (const uint32_t*)db->d_tile_cnt.p,
-                                            (const unsigned long long*)db->d_tile_off.p, nsub, pr->emit_ring, pr->emit_stage_bytes,
-                                            only_stream ? -1 : 1, pr->grid_emit_stream, pr->emit_smem, db->d_ctrl, pdl, db->stream));
-                note_launch(db, launches, with_stages("emit_stream", pr->emit_ring));
-            }
-            if (!only_stream) {
-                CUDA_TRY(launch_emit(pr->sp, pr->sp.bitmap, (const uint32_t*)db->d_span_cnt.p, (const unsigned long long*)db->d_tile_off.p, 8,
-                                     nspans, pr->grid_emit, stream_ok && !only_gather, db->d_ctrl, pr->emit_general, pdl && (only_gather || !stream_ok),
-                                     db->stream));
-                note_launch(db, launches, pr->emit_general ? "emit_general" : "emit");
-            }
-        }
-        CUDA_TRY(cudaEventRecord(db->ev1, db->stream));
-    } else {
-        if (!pr->block_mode && getenv("IMM3_TRACE")) {  // debugging: per-tile globaltimer stamps
-            int rc = ensure_buf(&db->d_trace, (size_t)pr->sp.ntiles * 64);
-            if (rc) return rc;
-            CUDA_TRY(cudaMemsetAsync(db->d_trace.p, 0, (size_t)pr->sp.ntiles * 64, db->stream));
-            pr->sp.trace = (unsigned long long*)db->d_trace.p;
-        }
-        CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
-        CUDA_TRY(launch_scan_blocks(pr->sp, db->d_ctrl, db->d_status, pr->grid, pr->dyn_smem, db->stream));  // (single-pass block kernel: blocks > 1024 rows, bitmaps)
-        CUDA_TRY(cudaEventRecord(db->ev1, db->stream));
+        CUDA_TRY(launch_scan_blocks(pr->sp, db->d_ctrl, db->d_status, pr->grid, pr->dyn_smem, db->stream));
         note_launch(db, launches, "scan_blocks");
+        break;
     }
-    if (exchange && db->comm_on) {
+    if (rc) return rc;
+    if (sharded) {
         // The per-rank counts are exchanged by the GPUs themselves (k_comm.cuh), behind the query's last kernel: no host
         // round trip between the kernels and the exchange, one synchronisation per query.
-        int rc = launch_exchange(db, pr->sp.limit, 1, publish_ok ? pub_seq : 0);
-        if (rc) return rc;
+        if ((rc = launch_exchange(db, pr->sp.limit, 1, publish_ok ? q.pub_seq : 0))) return rc;
         (*launches)++;
-        CUDA_TRY(cudaEventRecord(db->ev1, db->stream));  // (re-recorded: the timed span now ends behind the exchange)
-        published = publish_ok;
+        q.published = publish_ok;
     }
+    CUDA_TRY(cudaEventRecord(db->ev1, db->stream));
     db->ev_seq = ++db->query_seq;
-    if (published) {
+    if (q.published) {
         g_t_launched = now_us();
         const volatile unsigned long long* ps = &db->h_ctrl->pub_seq;
         bool seen = false;
         for (unsigned spins = 0;; spins++) {
             const unsigned long long word = __atomic_load_n(ps, __ATOMIC_ACQUIRE);
-            if ((word >> 41) == (pub_seq & 0x7FFFFFull)) {
-                if (!(exchange && db->comm_on)) {  // (blocks_scan_emit_kernel packs what the host needs into the word itself)
+            if ((word >> 41) == (q.pub_seq & 0x7FFFFFull)) {
+                if (!sharded) {  // (blocks_scan_emit_kernel packs what the host needs into the word itself)
                     db->h_ctrl->c.total = word & ((1ull << 40) - 1ull);
                     db->h_ctrl->c.error = (word >> 40) & 1u ? 1u : 0u;
                     db->h_ctrl->c.dense_rows = 0;
@@ -1174,33 +1236,33 @@ int run_scan_once(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* la
         g_t_synced = now_us();
     }
     if (db->h_ctrl->c.error) return fail(IMM3_ERR_CUDA, "kernel watchdog fired (code %u)", db->h_ctrl->c.error);
-    if (exchange && db->comm_on && db->h_ctrl->x.error)
+    if (sharded && db->h_ctrl->x.error)
         return fail(IMM3_ERR_COMM, "count exchange: a peer's count did not arrive within %llu ms (ranks must issue the same queries in the same order)",
                     db->comm_timeout_ns / 1000000ull);
-    float f = 0;
-    if (published && !have_mid && !g_eager_times && !getenv("IMM3_EAGER_TIMES")) {
+    if (q.published && !q.have_mid && !g_eager_times && !getenv("IMM3_EAGER_TIMES")) {
         *ms = -1.0;  // read lazily (imm3_result_device_ms): the events complete a moment after the publish, waiting for them here costs 2-3 us
         if (stage_ms) stage_ms[0] = -1.0, stage_ms[1] = 0;
     } else {
-    if (published) CUDA_TRY(cudaEventSynchronize(db->ev1));
-    CUDA_TRY(cudaEventElapsedTime(&f, db->ev0, db->ev1));
-    *ms = f;
-    if (stage_ms) {
-        stage_ms[0] = f;
-        stage_ms[1] = 0;
-        if (have_mid) {
-            float a = 0, b = 0;
-            CUDA_TRY(cudaEventElapsedTime(&a, db->ev0, db->ev_mid));
-            CUDA_TRY(cudaEventElapsedTime(&b, db->ev_mid, db->ev1));
-            stage_ms[0] = a;
-            stage_ms[1] = b;
+        float f = 0;
+        if (q.published) CUDA_TRY(cudaEventSynchronize(db->ev1));
+        CUDA_TRY(cudaEventElapsedTime(&f, db->ev0, db->ev1));
+        *ms = f;
+        if (stage_ms) {
+            stage_ms[0] = f;
+            stage_ms[1] = 0;
+            if (q.have_mid) {
+                float a = 0, b = 0;
+                CUDA_TRY(cudaEventElapsedTime(&a, db->ev0, db->ev_mid));
+                CUDA_TRY(cudaEventElapsedTime(&b, db->ev_mid, db->ev1));
+                stage_ms[0] = a;
+                stage_ms[1] = b;
+            }
         }
     }
-    }
     *total = (int64_t)db->h_ctrl->c.total;
-    if (pr->multipass && pr->sp.nproj > 0 && pr->emit_stage_bytes > 0)  // feedback for the next query of this shape
+    if (pr->pipeline == Pipeline::kDense && pr->sp.nproj > 0 && pr->emit_stage_bytes > 0)  // feedback for the next query of this shape
         db->emit_hint[pr->shape_key] = (db->h_ctrl->c.total > 0 && db->h_ctrl->c.dense_rows * 2 >= db->h_ctrl->c.total) ? 1 : 0;
-    if (pr->sp.trace && (pr->sp.debug & 16u)) {
+    if (pr->sp.trace) {
         unsigned long long h[64];
         CUDA_TRY(cudaMemcpy(h, pr->sp.trace, sizeof h, cudaMemcpyDeviceToHost));
         if (FILE* f = fopen(getenv("IMM3_TRACE"), "w")) {
@@ -1211,7 +1273,7 @@ int run_scan_once(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* la
                     fprintf(f, "%-16s min %9.2f us  max %9.2f us\n", names[i], (double)(h[2 * i] - h[0]) / 1e3, (double)(h[2 * i + 1] - h[0]) / 1e3);
             for (int i = 0; i < 8; i++)
                 if (h[32 + i] != ~0ull && h[32 + i] != 0) fprintf(f, "scan round %d after block scan: %9.2f us\n", i, (double)(h[32 + i] - h[0]) / 1e3);
-            if (pr->lane) {  // per CTA of the lane kernel: done time, SM, tiles decided
+            if (pr->block_filter == BlockFilter::kLane) {  // per CTA of the lane kernel: done time, SM, tiles decided
                 std::vector<unsigned long long> pc(1024);
                 if (cudaMemcpy(pc.data(), pr->sp.trace + 64, 1024 * 8, cudaMemcpyDeviceToHost) == cudaSuccess)
                     for (int i = 0; i < 512 && pc[2 * i]; i++)
@@ -1219,30 +1281,16 @@ int run_scan_once(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* la
             }
             fclose(f);
         }
-    } else if (pr->sp.trace) {
-        std::vector<unsigned long long> h((size_t)pr->sp.ntiles * 8);
-        CUDA_TRY(cudaMemcpy(h.data(), pr->sp.trace, h.size() * 8, cudaMemcpyDeviceToHost));
-        if (FILE* f = fopen(getenv("IMM3_TRACE"), "wb")) {
-            fwrite(h.data(), 8, h.size(), f);
-            fclose(f);
-        }
     }
     return 0;
 }
 
-// A small LIMIT is served "prefix first": phase A scans a leading part of the slice, phase B the whole slice if that did
-// not fill the LIMIT.  With a communicator every rank must run the same rounds, so the policy depends only on the query:
-// phase A everywhere (a rank whose slice is too small for a prefix scans all of it), then - unless RANK 0's phase A alone
-// fills the LIMIT, in which case the global result is its first `limit` rows - phase B everywhere.
-bool small_limit_policy(const LogicalPlan& lp) { return lp.limit > 0 && lp.limit <= (1 << 20) && !getenv("IMM3_NO_PREFIX"); }
-
-// Launch the kernels of one query and wait for the match count (see Prepared::prefix_blocks for the two-phase LIMIT).
+// Launch the kernels of one query and wait for the match count (see small_limit for the two-phase LIMIT).
 int run_scan(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* launches, double* stage_ms = nullptr) {
     TableStore& t = *pr->table;
     const bool comm = db->comm_on && !pr->for_bitmap;
-    const bool block_prefix = pr->block_mode && pr->blocks_multi && pr->prefix_blocks > 0;
-    const bool dense_prefix = !pr->block_mode && pr->multipass && pr->prefix_rows > 0;
-    const bool two_phase = comm ? small_limit_policy(pr->lp) : (block_prefix || dense_prefix);
+    const bool local_prefix = pr->prefix_blocks > 0 || pr->prefix_rows > 0;
+    const bool two_phase = comm ? small_limit(pr->lp) : local_prefix;
     db->route.clear();
     if (!two_phase) return run_scan_once(db, pr, ms, total, launches, stage_ms, t.nblocks, comm);
     struct EagerGuard {
@@ -1252,14 +1300,13 @@ int run_scan(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* launche
     // phase A: the leading blocks / rows only
     const ScanPlan full = pr->sp;
     const int grid_full = pr->grid;
-    const bool local_prefix = block_prefix || dense_prefix;
     int64_t nb = t.nblocks;
     if (local_prefix) {
         nb = pr->prefix_blocks;
-        if (dense_prefix) {
+        if (pr->prefix_rows > 0) {
             pr->sp.nrows = pr->prefix_rows;
             pr->sp.ntiles = pr->prefix_rows / kDenseTileRowsPerWord;
-        } else if (pr->hybrid) {
+        } else if (pr->pipeline == Pipeline::kRowSpace) {
             pr->sp.nrows = (int64_t)t.row_start[(size_t)nb];
             pr->sp.ntiles = (pr->sp.nrows + kDenseTileRowsPerWord - 1) / kDenseTileRowsPerWord;
         } else {
@@ -1303,6 +1350,22 @@ std::string java_double_to_string_integral(double v) {
     std::string frac = digits.substr(1);
     while (frac.size() > 1 && frac.back() == '0') frac.pop_back();
     return out + digits.substr(0, 1) + "." + frac + "E" + std::to_string(exp10);
+}
+
+// Queue the device->host copies of the first nrows rows of every column of a result on `stream`.
+int copy_columns(imm3_result* r, int64_t nrows, cudaStream_t stream) {
+    imm3_db* db = r->db;
+    for (int i = 0; i < r->ncols; i++) {
+        const size_t bytes = (size_t)nrows * (size_t)r->widths[(size_t)i];
+        if (r->h_cols[(size_t)i].cap < bytes || !r->h_cols[(size_t)i].p) {
+            db->host_pool.release(r->h_cols[(size_t)i]);
+            r->h_cols[(size_t)i] = Buf();
+            int rc = db->host_pool.acquire(bytes, &r->h_cols[(size_t)i]);
+            if (rc) return rc;
+        }
+        if (bytes) CUDA_TRY(cudaMemcpyAsync(r->h_cols[(size_t)i].p, r->d_cols[(size_t)i].p, bytes, cudaMemcpyDeviceToHost, stream));
+    }
+    return 0;
 }
 
 }  // namespace
@@ -1530,10 +1593,9 @@ int imm3_explain(imm3_db* db, const char* table, const imm3_pred* preds, int npr
                  int nproj, int64_t limit, const char** json) {
     if (!db || !json) return fail(IMM3_ERR_INVALID_ARG, "imm3_explain: NULL argument");
     Prepared pr;
-    int rc = prepare(db, table, preds, npreds, proj_cols, nproj, limit, &pr);
+    int rc = prepare(db, table, preds, npreds, proj_cols, nproj, limit, false, &pr);
     if (rc) return rc;
-    bool bm;
-    db->explain_buf = explain_json(pr.lp, kernel_name(db, *pr.table, pr.lp, &bm));
+    db->explain_buf = explain_json(pr.lp, explain_kernel(db, pr));
     *json = db->explain_buf.c_str();
     return 0;
 }
@@ -1549,7 +1611,7 @@ static int query_begin_terms(imm3_db* db, const char* table, const std::vector<s
     int rc = 0;
     for (auto& tm : terms) {
         std::unique_ptr<Prepared> p(new Prepared());
-        if ((rc = prepare(db, table, tm.first, tm.second, proj_cols, nproj, limit, p.get()))) return rc;
+        if ((rc = prepare(db, table, tm.first, tm.second, proj_cols, nproj, limit, false, p.get()))) return rc;
         prepared.push_back(std::move(p));
     }
     size_t main_i = 0;
@@ -1588,7 +1650,7 @@ static int query_begin_terms(imm3_db* db, const char* table, const std::vector<s
         if (!extra.empty()) {
             // real OR: every term's predicates are decided by the row-space filter kernel (dense columns); a disjunction over
             // an encoded column would need the block filter kernels to accumulate as well - not built
-            auto row_space = [](const Prepared& p) { return p.block_mode ? (p.blocks_multi && p.hybrid) : p.multipass; };
+            auto row_space = [](const Prepared& p) { return p.pipeline == Pipeline::kDense || p.pipeline == Pipeline::kRowSpace; };
             bool ok = row_space(pr);
             for (auto& tm : extra) {
                 if ((rc = fill_scan_plan(db, tm.get()))) { give_back(); return rc; }
@@ -1609,7 +1671,7 @@ static int query_begin_terms(imm3_db* db, const char* table, const std::vector<s
         const int64_t lim = limit > 0 ? limit : INT64_MAX;
         db->route.clear();
         if ((rc = exchange_only(db, lim, 0))) { give_back(); return rc; }
-        if (small_limit_policy(pr.lp) && (int64_t)db->h_ctrl->x.counts[0] < pr.lp.limit && (rc = exchange_only(db, lim, 0))) { give_back(); return rc; }
+        if (small_limit(pr.lp) && (int64_t)db->h_ctrl->x.counts[0] < pr.lp.limit && (rc = exchange_only(db, lim, 0))) { give_back(); return rc; }
         r->launches = 1;
     }
     r->route = r->launches > 0 ? db->route : std::string();
@@ -1704,15 +1766,7 @@ int imm3_result_fetch(imm3_result* r, int64_t nrows) {
     imm3_db* db = r->db;
     int rc = use_device(db);
     if (rc) return rc;
-    for (int i = 0; i < r->ncols; i++) {
-        const size_t bytes = (size_t)nrows * (size_t)r->widths[(size_t)i];
-        if (r->h_cols[(size_t)i].cap < bytes || !r->h_cols[(size_t)i].p) {
-            db->host_pool.release(r->h_cols[(size_t)i]);
-            r->h_cols[(size_t)i] = Buf();
-            if ((rc = db->host_pool.acquire(bytes, &r->h_cols[(size_t)i]))) return rc;
-        }
-        if (bytes) CUDA_TRY(cudaMemcpyAsync(r->h_cols[(size_t)i].p, r->d_cols[(size_t)i].p, bytes, cudaMemcpyDeviceToHost, db->stream));
-    }
+    if ((rc = copy_columns(r, nrows, db->stream))) return rc;
     CUDA_TRY(cudaStreamSynchronize(db->stream));
     r->fetched = nrows;
     return 0;
@@ -1727,15 +1781,7 @@ int imm3_result_fetch_async(imm3_result* r, int64_t nrows) {
     if (rc) return rc;
     if (!db->copy_stream) CUDA_TRY(cudaStreamCreateWithFlags(&db->copy_stream, cudaStreamNonBlocking));
     // (imm3_query_begin returned after the kernels had finished: the rows are final, the copy stream needs no event)
-    for (int i = 0; i < r->ncols; i++) {
-        const size_t bytes = (size_t)nrows * (size_t)r->widths[(size_t)i];
-        if (r->h_cols[(size_t)i].cap < bytes || !r->h_cols[(size_t)i].p) {
-            db->host_pool.release(r->h_cols[(size_t)i]);
-            r->h_cols[(size_t)i] = Buf();
-            if ((rc = db->host_pool.acquire(bytes, &r->h_cols[(size_t)i]))) return rc;
-        }
-        if (bytes) CUDA_TRY(cudaMemcpyAsync(r->h_cols[(size_t)i].p, r->d_cols[(size_t)i].p, bytes, cudaMemcpyDeviceToHost, db->copy_stream));
-    }
+    if ((rc = copy_columns(r, nrows, db->copy_stream))) return rc;
     if (!r->copied) CUDA_TRY(cudaEventCreateWithFlags(&r->copied, cudaEventDisableTiming));
     CUDA_TRY(cudaEventRecord(r->copied, db->copy_stream));
     r->pending = nrows;
@@ -1784,7 +1830,7 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
     if (naggs > kMaxAggs) return fail(IMM3_ERR_UNSUPPORTED, "%s: at most %d aggregates", fn, kMaxAggs);
     if (ngroup > kMaxGroupCols) return fail(IMM3_ERR_UNSUPPORTED, "%s: at most %d group-by columns", fn, kMaxGroupCols);
     Prepared pr;
-    int rc = prepare(db, table, preds, npreds, nullptr, 0, 0, &pr);  // validation before any device work
+    int rc = prepare(db, table, preds, npreds, nullptr, 0, 0, false, &pr);  // validation before any device work
     if (rc) return rc;
     TableStore& t = *pr.table;
     auto find_col = [&](const char* name) -> int {
@@ -1799,12 +1845,6 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
     r->db = db;
     std::vector<int> gidx, aidx;
     std::vector<int> pfor_cols;  // distinct sorted-int-codec columns decoded per block (MIN / MAX inputs, group columns)
-    auto pfor_slot = [&](int ci) -> int8_t {
-        for (size_t i = 0; i < pfor_cols.size(); i++)
-            if (pfor_cols[i] == ci) return (int8_t)i;
-        pfor_cols.push_back(ci);
-        return (int8_t)(pfor_cols.size() - 1);
-    };
     for (int i = 0; i < kMaxAggs; i++) ap.agg_pfor[i] = -1;
     for (int i = 0; i < kMaxGroupCols; i++) ap.group_pfor[i] = -1;
     int key_bits = 0;
@@ -1815,7 +1855,7 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
         if (key_bits + 8 * c.meta.width > 56) return fail(IMM3_ERR_UNSUPPORTED, "group-by cells must pack into 7 bytes");
         ap.group[g].width = c.meta.width;
         ap.group[g].key_shift = key_bits;
-        if (c.meta.codec == IMM3_CODEC_PFOR_INT) ap.group_pfor[g] = pfor_slot(ci);
+        ap.group_pfor[g] = (int8_t)pfor_slot(t, &pfor_cols, ci);
         key_bits += 8 * c.meta.width;
         gidx.push_back(ci);
         r->names.push_back(c.meta.name);
@@ -1833,7 +1873,7 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
             if (c.meta.ctype == IMM3_COL_STRING)
                 return fail(IMM3_ERR_UNSUPPORTED, "min / max on a STRING column (the reference maps both to MaxStringAggr, Engine.scala:137,147)");
             ap.agg[a].op = aggs[a].op == IMM3_AGG_MIN ? kAggMin : kAggMax;
-            if (c.meta.codec == IMM3_CODEC_PFOR_INT) ap.agg_pfor[a] = pfor_slot(ci);  // (COUNT never reads its column)
+            ap.agg_pfor[a] = (int8_t)pfor_slot(t, &pfor_cols, ci);  // (COUNT never reads its column)
             suffix = aggs[a].op == IMM3_AGG_MIN ? "_min" : "_max";
         } else {
             return fail(IMM3_ERR_UNSUPPORTED, "Unknown Aggregate type (Engine.scala:153: only Min, Max and Count are resolved)");
@@ -1849,11 +1889,9 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
     r->h_cols.resize((size_t)r->ncols);
     ap.naggs = naggs;
     ap.ngroup = ngroup;
-    if (pr.block_mode && !pr.lp.filters.empty()) {
-        for (auto& f : pr.lp.filters)
-            if (t.cols[(size_t)f.col_idx].meta.codec == IMM3_CODEC_PFOR_INT)
-                return fail(IMM3_ERR_UNSUPPORTED, "aggregation with a predicate on a sorted-int-codec column (%s) is not supported yet", t.cols[(size_t)f.col_idx].meta.name.c_str());
-    }
+    for (auto& f : pr.lp.filters)
+        if (is_pfor(t, f.col_idx))
+            return fail(IMM3_ERR_UNSUPPORTED, "aggregation with a predicate on a sorted-int-codec column (%s) is not supported yet", t.cols[(size_t)f.col_idx].meta.name.c_str());
     // A MIN / MAX input or a group column in the sorted-int codec: agg_blocks_kernel decodes them block by block.
     const bool on_blocks = !pfor_cols.empty();
     if (pfor_cols.size() > (size_t)kMaxPforCols)
@@ -1886,33 +1924,23 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
     if (local) {
         // The filter runs in row space exactly as for a Project query without a select list (dense filter kernel: bitmap,
         // span counts, total); the aggregation kernel is queued behind it, one synchronisation for the whole query.
-        const bool was_block = pr.block_mode;
-        pr.block_mode = false;
-        pr.multipass = true;
-        pr.for_bitmap = false;
-        if ((rc = fill_scan_plan(db, &pr))) return rc;
-        pr.block_mode = was_block;
-        sp.bitmap = nullptr;
-        const int64_t ntiles = sp.ntiles, nspans = ntiles * 8;
-        if ((rc = ensure_buf(&db->d_bitmap, (size_t)(ntiles * kDenseTileRowsPerWord / 32 + 64) * 4))) return rc;
-        if ((rc = ensure_buf(&db->d_span_cnt, (size_t)(nspans + 8) * 4))) return rc;
-        const size_t ntiles_pad = ((size_t)ntiles + 4095) / 4096 * 4096 + 16;
-        if ((rc = ensure_buf(&db->d_tile_cnt, ntiles_pad * 4))) return rc;
-        if ((rc = ensure_buf(&db->d_tile_off, ntiles_pad * 8))) return rc;
+        int occ = 0;
+        if ((rc = plan_columns(db, &pr)) || (rc = size_dense_filter(db, &pr, &occ)) || (rc = plan_grid(db, &pr, occ)) || (rc = ensure_row_space(db, sp)))
+            return rc;
         ap.nrows = t.nrows;
-        ap.ntiles = ntiles;
+        ap.ntiles = sp.ntiles;
         for (int g = 0; g < ngroup; g++) ap.group[g].base = t.cols[(size_t)gidx[(size_t)g]].d_arena;
         for (int a = 0; a < naggs; a++) ap.agg[a].base = t.cols[(size_t)aidx[(size_t)a]].d_arena;
         if (on_blocks) {
-            int64_t cap = 0;  // per-warp scratch for the byte-swapped words of one encoded block
+            int64_t words = 0;
             ap.npfor = (int)pfor_cols.size();
             for (int i = 0; i < ap.npfor; i++) {
                 const ColumnStore& c = t.cols[(size_t)pfor_cols[(size_t)i]];
                 ap.pfor[i].words = reinterpret_cast<const uint32_t*>(c.d_arena);
                 ap.pfor[i].word_off = c.d_word_off;
-                cap = std::max<int64_t>(cap, c.max_block_words);
+                words = std::max<int64_t>(words, c.max_block_words);
             }
-            ap.blk_words_cap = (int)std::min<int64_t>(1120, ((cap + 4 + 31) / 32) * 32);
+            ap.blk_words_cap = block_words_cap(words);
             ap.nblocks = t.nblocks;
             ap.row_start = t.d_row_start;
             int optin = 0;
@@ -2161,7 +2189,7 @@ int imm3_filter_bitmap(imm3_db* db, const char* table, const imm3_pred* preds, i
                        int64_t* nwords, int64_t* nselected) {
     if (!db || !words || !nwords || !nselected) return fail(IMM3_ERR_INVALID_ARG, "imm3_filter_bitmap: NULL argument");
     Prepared pr;
-    int rc = prepare(db, table, preds, npreds, nullptr, 0, 0, &pr);
+    int rc = prepare(db, table, preds, npreds, nullptr, 0, 0, true, &pr);
     if (rc) return rc;
     if ((rc = use_device(db))) return rc;
     TableStore& t = *pr.table;
@@ -2176,7 +2204,6 @@ int imm3_filter_bitmap(imm3_db* db, const char* table, const imm3_pred* preds, i
     CUDA_TRY(cudaMemsetAsync(db->d_bitmap.p, 0, need_words * 4, db->stream));
     int64_t total = 0;
     if (!pr.lp.always_empty && t.nrows > 0) {
-        pr.for_bitmap = true;
         if ((rc = fill_scan_plan(db, &pr))) return rc;
         pr.sp.bitmap = (uint32_t*)db->d_bitmap.p;
         pr.sp.limit = INT64_MAX;

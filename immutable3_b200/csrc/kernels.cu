@@ -376,25 +376,26 @@ size_t blocks_filter_smem_bytes(int nstaged, int tile_cap_bytes, int ring) { ret
 int blocks_filter_slot_bytes(int nstaged, int tile_cap_bytes) { return blk_filter_slot_bytes(nstaged, tile_cap_bytes); }
 size_t blocks_emit_smem_bytes(int npfor, int words_cap) { return (size_t)kComputeWarps * blk_emit_warp_words(npfor, words_cap) * 4; }
 int blocks_filter_quad_slot_bytes(int tile_cap_bytes) { return kQuadHdrBytes + tile_cap_bytes; }
-cudaError_t blocks_multi_occupancy(size_t filter_smem, size_t emit_smem, int* filter_blocks_per_sm, int* emit_blocks_per_sm, int mode, bool rowspace) {
+cudaError_t blocks_multi_occupancy(size_t filter_smem, size_t emit_smem, int* filter_blocks_per_sm, int* emit_blocks_per_sm, BlockFilter filter,
+                                   int lane_warps, bool rowspace) {
     cudaError_t e = configure_once();
     if (e != cudaSuccess) return e;
     if (filter_blocks_per_sm) {
-        e = mode >= 2   ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(filter_blocks_per_sm, blocks_filter_lane_kernel, (mode >> 8) * 32, filter_smem)
-            : mode == 1 ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(filter_blocks_per_sm, blocks_filter_quad_kernel, kComputeThreads + 32, filter_smem)
-                        : cudaOccupancyMaxActiveBlocksPerMultiprocessor(filter_blocks_per_sm, blocks_filter_kernel, kComputeThreads + 32, filter_smem);
+        e = filter == BlockFilter::kLane   ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(filter_blocks_per_sm, blocks_filter_lane_kernel, lane_warps * 32, filter_smem)
+            : filter == BlockFilter::kQuad ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(filter_blocks_per_sm, blocks_filter_quad_kernel, kComputeThreads + 32, filter_smem)
+                                           : cudaOccupancyMaxActiveBlocksPerMultiprocessor(filter_blocks_per_sm, blocks_filter_kernel, kComputeThreads + 32, filter_smem);
         if (e != cudaSuccess) return e;
     }
     if (rowspace) return cudaOccupancyMaxActiveBlocksPerMultiprocessor(emit_blocks_per_sm, blocks_emit_kernel<true>, kComputeThreads, emit_smem);
     return cudaOccupancyMaxActiveBlocksPerMultiprocessor(emit_blocks_per_sm, blocks_emit_kernel<false>, kComputeThreads, emit_smem);
 }
 cudaError_t launch_blocks_filter(const ScanPlan& plan, uint32_t* bitmapB, uint32_t* blk_cnt, uint32_t* tile_cnt, unsigned long long* tile_off,
-                                 ScanCtrl* ctrl, long long nblocks, int grid, size_t dyn_smem, int mode, const unsigned int* work,
-                                 cudaStream_t stream, uint32_t* grp_sum) {
+                                 ScanCtrl* ctrl, long long nblocks, int grid, size_t dyn_smem, BlockFilter filter, int lane_warps,
+                                 const unsigned int* work, cudaStream_t stream, uint32_t* grp_sum) {
     cudaError_t e = configure_once();
     if (e != cudaSuccess) return e;
-    if (mode >= 2) blocks_filter_lane_kernel<<<grid, (mode >> 8) * 32, dyn_smem, stream>>>(plan, bitmapB, blk_cnt, tile_cnt, tile_off, ctrl, nblocks, work, grp_sum);
-    else if (mode == 1) blocks_filter_quad_kernel<<<grid, kComputeThreads + 32, dyn_smem, stream>>>(plan, bitmapB, blk_cnt, tile_cnt, tile_off, ctrl, nblocks, work);
+    if (filter == BlockFilter::kLane) blocks_filter_lane_kernel<<<grid, lane_warps * 32, dyn_smem, stream>>>(plan, bitmapB, blk_cnt, tile_cnt, tile_off, ctrl, nblocks, work, grp_sum);
+    else if (filter == BlockFilter::kQuad) blocks_filter_quad_kernel<<<grid, kComputeThreads + 32, dyn_smem, stream>>>(plan, bitmapB, blk_cnt, tile_cnt, tile_off, ctrl, nblocks, work);
     else blocks_filter_kernel<<<grid, kComputeThreads + 32, dyn_smem, stream>>>(plan, bitmapB, blk_cnt, tile_cnt, tile_off, ctrl, nblocks, work);
     return cudaGetLastError();
 }

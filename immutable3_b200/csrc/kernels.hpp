@@ -47,10 +47,14 @@ size_t blocks_filter_smem_bytes(int nstaged, int tile_cap_bytes, int ring);
 int blocks_filter_slot_bytes(int nstaged, int tile_cap_bytes);
 size_t blocks_emit_smem_bytes(int npfor, int words_cap);
 int blocks_filter_quad_slot_bytes(int tile_cap_bytes);
-cudaError_t blocks_multi_occupancy(size_t filter_smem, size_t emit_smem, int* filter_blocks_per_sm, int* emit_blocks_per_sm, int mode, bool rowspace);  // mode 0: lane = mini-block, 1: quad, 2 | warps << 8: lane = block with that many warps per CTA
+// The block filter kernels: lane = mini-block (blocks_filter_kernel), quad (blocks_filter_quad_kernel), lane = block
+// (blocks_filter_lane_kernel, lane_warps warps per CTA).
+enum class BlockFilter { kMini, kQuad, kLane };
+cudaError_t blocks_multi_occupancy(size_t filter_smem, size_t emit_smem, int* filter_blocks_per_sm, int* emit_blocks_per_sm, BlockFilter filter,
+                                   int lane_warps, bool rowspace);
 cudaError_t launch_blocks_filter(const ScanPlan& plan, uint32_t* bitmapB, uint32_t* blk_cnt, uint32_t* tile_cnt, unsigned long long* tile_off,
-                                 ScanCtrl* ctrl, long long nblocks, int grid, size_t dyn_smem, int mode, const unsigned int* work,
-                                 cudaStream_t stream, uint32_t* grp_sum = nullptr);  // grp_sum: blocks_group_emit_kernel follows (lane mode only)
+                                 ScanCtrl* ctrl, long long nblocks, int grid, size_t dyn_smem, BlockFilter filter, int lane_warps,
+                                 const unsigned int* work, cudaStream_t stream, uint32_t* grp_sum = nullptr);  // grp_sum: blocks_group_emit_kernel follows (lane kernel only)
 cudaError_t launch_block_stats(const PforCol& pc, const uint64_t* row_start, long long nblocks, int words_cap, int num_sms, BlockStat* stats,
                                cudaStream_t stream);
 cudaError_t launch_blocks_prune(const PrunePlan& q, const uint64_t* row_start, long long nblocks, long long ntiles8, uint32_t* blk_cnt,

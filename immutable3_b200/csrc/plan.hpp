@@ -62,7 +62,7 @@ struct PforCol {
 struct ScanPlan {
     int64_t nrows;        // rows in the owned slice
     int64_t limit;        // rows wanted (INT64_MAX = unlimited)
-    int64_t ntiles;       // dense: ceil(nrows / (8192 * W)); block mode: number of reference blocks
+    int64_t ntiles;       // dense: ceil(nrows / 8192); block mode: number of reference blocks
     const uint64_t* row_start;  // block mode: nblocks+1 canonical row ordinals
     uint32_t* bitmap;     // filter-bitmap mode: selection bitmap out (else nullptr)
     unsigned long long* trace;  // debugging (IMM3_TRACE): 8 globaltimer stamps per tile, else nullptr
@@ -78,7 +78,7 @@ struct ScanPlan {
     int32_t blk_tile_bytes;  // blocks_filter_kernel: bytes reserved per staged encoded column in a ring slot (largest 8-block tile)
     int32_t scan_inline;     // 1: the filter kernel's last CTA turns the tile counts into offsets; 0: offset_scan_kernel does (large tables)
     uint32_t pfor_filter_mask;  // blocks_filter_kernel: PFOR slots that carry a predicate (their tiles are staged)
-    int32_t words_per_lane;  // multi-pass filter kernel: W (tile = 8192 * W rows)
+    int32_t pad0;            // unused: keeps the offsets of the members behind it (kernel parameter layout)
     int32_t or_accumulate;   // filter kernel: OR this conjunction's bits into the bitmap already there (second and later terms of a disjunction)
     uint32_t debug;          // IMM3_DEBUG env bits (timing experiments only; bit 0: skip the look-back -> WRONG offsets)
     FilterCol filter[kMaxFilterCols];
