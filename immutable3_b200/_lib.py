@@ -14,7 +14,8 @@ LIB_PATH = os.environ.get("IMM3_LIB") or os.path.join(HERE, "libimm3gpu.so")  # 
 OK = 0
 ERR_NOT_FOUND, ERR_UNSUPPORTED, ERR_BAD_FORMAT, ERR_CUDA, ERR_OOM, ERR_INVALID_ARG, ERR_IO, ERR_STATE, ERR_COMM = range(-1, -10, -1)
 COMM_HANDLE_BYTES = 64
-COL_INT, COL_TINYINT, COL_STRING, COL_COUNT, COL_DOUBLE = 0, 1, 2, 3, 4
+COL_INT, COL_TINYINT, COL_STRING, COL_COUNT, COL_DOUBLE, COL_INT64 = 0, 1, 2, 3, 4, 5
+AGG_FLAG_GLOBAL = 0x1  # IMM3_AGG_GLOBAL
 AGG_COUNT, AGG_MIN, AGG_MAX, AGG_SUM, AGG_AVG = 0, 1, 2, 3, 4
 CODEC_PFOR_INT, CODEC_DENSE_INT, CODEC_DENSE_TINYINT, CODEC_DENSE_STRING = 0, 1, 2, 3
 OP_GT, OP_LT, OP_EQ, OP_MATCH, OP_NOTMATCH, OP_NOOP = 1, 2, 3, 4, 5, 6
@@ -74,6 +75,7 @@ SIGNATURES = {
     "imm3_result_wait": (C.c_int, [_P]),
     "imm3_query_agg": (C.c_int, [_P, C.c_char_p, C.POINTER(Pred), C.c_int, C.POINTER(Agg), C.c_int, _STRS, C.c_int, _PP]),
     "imm3_query_agg_global": (C.c_int, [_P, C.c_char_p, C.POINTER(Pred), C.c_int, C.POINTER(Agg), C.c_int, _STRS, C.c_int, _PP]),
+    "imm3_query_agg_ext": (C.c_int, [_P, C.c_char_p, C.POINTER(Pred), C.c_int, C.POINTER(Agg), C.c_int, _STRS, C.c_int, C.c_uint32, _PP]),
     "imm3_query_sql": (C.c_int, [_P, C.c_char_p, _PP]),
     "imm3_result_nrows": (C.c_int64, [_P]),
     "imm3_result_ncols": (C.c_int, [_P]),

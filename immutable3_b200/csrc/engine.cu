@@ -26,6 +26,8 @@
 
 #include <atomic>
 #include <cerrno>
+#include <charconv>
+#include <cmath>
 #include <memory>
 #include <mutex>
 #include <string>
@@ -170,6 +172,7 @@ struct imm3_result {
     int world = 1;
     int64_t rank_counts[kMaxWorld] = {};
     int agg_first_col = -1;  // aggregate result: index of the first aggregate column (rows live in host buffers only)
+    uint32_t avg_cols = 0;   // bit a: aggregate column a is an AVG (printed with every digit, not as an integral MIN / MAX)
     int64_t fetched = 0;
     int64_t pending = -1;        // rows of an imm3_result_fetch_async still in flight (-1 = none)
     cudaEvent_t copied = nullptr;  // recorded on the copy stream after the last device->host copy
@@ -1352,6 +1355,31 @@ std::string java_double_to_string_integral(double v) {
     return out + digits.substr(0, 1) + "." + frac + "E" + std::to_string(exp10);
 }
 
+// java.lang.Double.toString for any finite or infinite double (AVG results): the shortest digits that round-trip
+// (std::to_chars), plain notation with at least one fractional digit for 10^-3 <= |v| < 10^7 ("21.5", "0.001"), else
+// computerized scientific notation ("1.0E7", "-2.5E-4").
+std::string java_double_to_string(double v) {
+    if (std::isnan(v)) return "NaN";
+    if (std::isinf(v)) return v > 0 ? "Infinity" : "-Infinity";
+    if (v == 0) return std::signbit(v) ? "-0.0" : "0.0";
+    char buf[64];
+    const std::to_chars_result tc = std::to_chars(buf, buf + sizeof buf, std::fabs(v), std::chars_format::scientific);  // d[.ddd]e[+-]xx
+    const std::string sci(buf, tc.ptr);
+    const size_t e = sci.find('e');
+    const int exp10 = std::atoi(sci.c_str() + e + 1);
+    const std::string digits = sci.substr(0, 1) + (e > 1 ? sci.substr(2, e - 2) : std::string());  // v = 0.digits x 10^(exp10 + 1)
+    const std::string sign = v < 0 ? "-" : "";
+    const double a = std::fabs(v);
+    if (a >= 1e-3 && a < 1e7) {
+        if (exp10 < 0) return sign + "0." + std::string((size_t)(-exp10 - 1), '0') + digits;
+        const size_t ni = (size_t)exp10 + 1;
+        std::string ip = digits.substr(0, std::min(ni, digits.size()));
+        ip.append(ni - ip.size(), '0');
+        return sign + ip + "." + (digits.size() > ni ? digits.substr(ni) : std::string("0"));
+    }
+    return sign + digits.substr(0, 1) + "." + (digits.size() > 1 ? digits.substr(1) : std::string("0")) + "E" + std::to_string(exp10);
+}
+
 // Queue the device->host copies of the first nrows rows of every column of a result on `stream`.
 int copy_columns(imm3_result* r, int64_t nrows, cudaStream_t stream) {
     imm3_db* db = r->db;
@@ -1815,11 +1843,12 @@ int imm3_query(imm3_db* db, const char* table, const imm3_pred* preds, int npred
 
 namespace {
 
-// imm3_query_agg (global = false) and imm3_query_agg_global: one validation, one plan, one launch sequence.  The global form
-// on a connected handle compacts this rank's partial groups into its exchange buffer instead of the result buffer and
-// queues the exchange and the merge behind them (k_comm.cuh agg_exchange_kernel, k_agg.cuh agg_merge_kernel; DESIGN §4.3).
+// imm3_query_agg (global = false), imm3_query_agg_global and imm3_query_agg_ext: one validation, one plan, one launch
+// sequence.  The global form on a connected handle compacts this rank's partial groups into its exchange buffer instead
+// of the result buffer and queues the exchange and the merge behind them (k_comm.cuh agg_exchange_kernel, k_agg.cuh
+// agg_merge_kernel; DESIGN §4.3).  allow_sum_avg (imm3_query_agg_ext only) resolves Sum / Avg (DESIGN §4.4c).
 int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, const imm3_agg* aggs, int naggs, const char* const* group_cols,
-              int ngroup, bool global, imm3_result** out) {
+              int ngroup, bool global, bool allow_sum_avg, imm3_result** out) {
     const char* const fn = global ? "imm3_query_agg_global" : "imm3_query_agg";
     if (!db || !out || (naggs > 0 && !aggs) || (ngroup > 0 && !group_cols)) return fail(IMM3_ERR_INVALID_ARG, "%s: NULL argument", fn);
     // A sharded handle merges over the communicator; a single handle's partials are the global result already.
@@ -1862,32 +1891,56 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
         r->types.push_back(c.meta.ctype);
         r->widths.push_back(c.meta.width);
     }
+    int count_slot = -1;  // the plan's first COUNT (a SUM / AVG query's group sizes)
+    bool has_sum = false;
     for (int a = 0; a < naggs; a++) {
         const int ci = find_col(aggs[a].col);
         if (ci < 0) return fail(IMM3_ERR_NOT_FOUND, "Column %s does not exist in table %s", aggs[a].col ? aggs[a].col : "(null)", t.meta.name.c_str());
         const ColumnStore& c = t.cols[(size_t)ci];
         const char* suffix = "_count";
+        int rtype = IMM3_COL_DOUBLE;
         if (aggs[a].op == IMM3_AGG_COUNT) {
             ap.agg[a].op = kAggCount;
+            rtype = IMM3_COL_COUNT;
+            if (count_slot < 0) count_slot = a;
         } else if (aggs[a].op == IMM3_AGG_MIN || aggs[a].op == IMM3_AGG_MAX) {
             if (c.meta.ctype == IMM3_COL_STRING)
                 return fail(IMM3_ERR_UNSUPPORTED, "min / max on a STRING column (the reference maps both to MaxStringAggr, Engine.scala:137,147)");
             ap.agg[a].op = aggs[a].op == IMM3_AGG_MIN ? kAggMin : kAggMax;
             ap.agg_pfor[a] = (int8_t)pfor_slot(t, &pfor_cols, ci);  // (COUNT never reads its column)
             suffix = aggs[a].op == IMM3_AGG_MIN ? "_min" : "_max";
+        } else if (allow_sum_avg && (aggs[a].op == IMM3_AGG_SUM || aggs[a].op == IMM3_AGG_AVG)) {
+            if (c.meta.ctype == IMM3_COL_STRING) return fail(IMM3_ERR_UNSUPPORTED, "sum / avg on a STRING column (%s)", c.meta.name.c_str());
+            ap.agg[a].op = kAggSum;  // (AVG = the SUM over the group's COUNT, divided on the host)
+            ap.agg_pfor[a] = (int8_t)pfor_slot(t, &pfor_cols, ci);
+            has_sum = true;
+            suffix = aggs[a].op == IMM3_AGG_SUM ? "_sum" : "_avg";
+            if (aggs[a].op == IMM3_AGG_SUM) rtype = IMM3_COL_INT64;
+            else r->avg_cols |= 1u << a;
         } else {
             return fail(IMM3_ERR_UNSUPPORTED, "Unknown Aggregate type (Engine.scala:153: only Min, Max and Count are resolved)");
         }
         ap.agg[a].width = c.meta.width;
         aidx.push_back(ci);
         r->names.push_back(c.meta.name + suffix);  // alias.getOrElse(col + "_max"), Engine.scala:136-152
-        r->types.push_back(ap.agg[a].op == kAggCount ? IMM3_COL_COUNT : IMM3_COL_DOUBLE);
+        r->types.push_back(rtype);
         r->widths.push_back(8);
+    }
+    // A SUM / AVG query carries one COUNT of the group's rows: the query's own, else a hidden one behind the visible
+    // aggregates (in the plan, never in the result).
+    int plan_naggs = naggs;
+    if (has_sum && count_slot < 0) {
+        if (naggs + 1 > kMaxAggs)
+            return fail(IMM3_ERR_UNSUPPORTED, "imm3_query_agg_ext: at most %d aggregates, including the COUNT a sum / avg query carries (the query has %d and no COUNT)",
+                        kMaxAggs, naggs);
+        count_slot = plan_naggs++;
+        ap.agg[count_slot].op = kAggCount;
+        ap.agg[count_slot].width = 4;
     }
     r->ncols = ngroup + naggs;
     r->agg_first_col = ngroup;
     r->h_cols.resize((size_t)r->ncols);
-    ap.naggs = naggs;
+    ap.naggs = plan_naggs;
     ap.ngroup = ngroup;
     for (auto& f : pr.lp.filters)
         if (is_pfor(t, f.col_idx))
@@ -1945,10 +1998,12 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
             ap.row_start = t.d_row_start;
             int optin = 0;
             CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, db->device));
-            const size_t smem = agg_blocks_smem_bytes(naggs, ap.npfor, ap.blk_words_cap);
+            int nsum = 0;
+            for (int a = 0; a < plan_naggs; a++) nsum += ap.agg[a].op == kAggSum;
+            const size_t smem = agg_blocks_smem_bytes(plan_naggs, ap.npfor, ap.blk_words_cap, nsum);
             if (smem + 1024 > (size_t)optin) {  // (1 KB: the kernel's static shared memory)
                 if ((rc = refuse_slice(fail(IMM3_ERR_UNSUPPORTED, "aggregation over %d sorted-int-codec columns with %d aggregates needs %zu bytes of shared memory per CTA, the device has %d",
-                                            ap.npfor, naggs, smem + 1024, optin))))
+                                            ap.npfor, plan_naggs, smem + 1024, optin))))
                     return rc;
                 local = false;
             }
@@ -1979,9 +2034,10 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
                 CUDA_TRY(launch_agg(ap, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, (AggEntry*)db->d_agg_table.p,
                                     local_out, counters, db->d_ctrl, db->num_sms, db->stream));
             r->launches = 4;
-            // the instantiation IMM3_AGG_DISPATCH (kernels.cu) picks: <= 2 group-by columns exact, else 4; 1 .. 4 aggregates exact, else 8
-            const int ng = ngroup <= 2 ? ngroup : 4, na = (naggs >= 1 && naggs <= 4) ? naggs : 8;
-            const std::string inst = "<" + std::to_string(ng) + "," + std::to_string(na) + ">";
+            // the instantiation IMM3_AGG_DISPATCH (kernels.cu) picks: <= 2 group-by columns exact, else 4; 1 .. 4 aggregates exact, else 8;
+            // "/sum": the SUM instantiation
+            const int ng = ngroup <= 2 ? ngroup : 4, na = (plan_naggs >= 1 && plan_naggs <= 4) ? plan_naggs : 8;
+            const std::string inst = "<" + std::to_string(ng) + "," + std::to_string(na) + ">" + (has_sum ? "/sum" : "");
             r->route = "agg_init;" + filter_route(sp) + ";" + (on_blocks ? "agg_blocks" : "agg") + inst + ";agg_compact";
         }
         if (merge) {
@@ -2002,8 +2058,8 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
             db->agg_seq++;  // (posted: the next aggregate compacts into the other buffer)
             mp.world = db->world;
             mp.slots = ap.table_slots;
-            mp.naggs = naggs;
-            for (int a = 0; a < naggs; a++) mp.op[a] = ap.agg[a].op;
+            mp.naggs = plan_naggs;
+            for (int a = 0; a < plan_naggs; a++) mp.op[a] = ap.agg[a].op == kAggSum ? kAggCount : ap.agg[a].op;  // (a SUM merges as a COUNT: a 64-bit add)
             CUDA_TRY(launch_agg_init((AggEntry*)db->d_agg_table.p, ap.table_slots, ap, counters, db->stream));
             CUDA_TRY(launch_agg_merge(mp, d_x, (AggEntry*)db->d_agg_table.p, (AggEntry*)db->d_agg_out.p, counters, db->num_sms, db->stream));
             r->launches += 4;
@@ -2043,7 +2099,7 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
     }
     if (local) {
         // algorithmic bytes: filter columns once + every decoded encoded column once (its words and 4 B of word offsets per
-        // block) + per selected row the cells of the dense group and aggregate columns
+        // block) + per selected row the cells of the dense group and aggregate columns (MIN / MAX / SUM / AVG inputs)
         int64_t bytes = 0, per_row = 0;
         for (auto& f2 : pr.lp.filters) bytes += t.cols[(size_t)f2.col_idx].encoded_bytes;
         for (int ci : pfor_cols) bytes += t.cols[(size_t)ci].encoded_bytes + 4 * (int64_t)t.nblocks;
@@ -2053,7 +2109,13 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
             if (ap.agg[a].op != kAggCount && ap.agg_pfor[a] < 0) per_row += ap.agg[a].width;
         r->alg_bytes = bytes + per_row * (int64_t)db->h_ctrl->c.total;
     }
-    // rows of the result: group cells, then the aggregates (COUNT: int64, MIN / MAX: double)
+    // SUM / AVG: every add on the way here was modulo 2^64, so a sum is exact when it fits int64 - certain for at most 2^32
+    // int32 inputs (2^32 x 2^31 <= 2^63); a larger group (on a global aggregate: the merged count) is refused, not wrapped
+    if (has_sum)
+        for (const AggEntry& e : groups)
+            if ((unsigned long long)e.val[count_slot] > (1ull << 32))
+                return fail(IMM3_ERR_UNSUPPORTED, "imm3_query_agg_ext: a group of %lld rows: sum / avg are exact for groups of at most 2^32 rows", e.val[count_slot]);
+    // rows of the result: group cells, then the aggregates (COUNT / SUM: int64, MIN / MAX / AVG: double)
     for (int c = 0; c < r->ncols; c++) {
         const size_t w = (size_t)r->widths[(size_t)c];
         if ((rc = db->host_pool.acquire(std::max<size_t>(1, (size_t)ngroups_out * w), &r->h_cols[(size_t)c]))) {
@@ -2068,8 +2130,11 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
                 for (size_t b = 0; b < w; b++) dst[(size_t)i * w + b] = (uint8_t)(cell >> (8 * b));
             } else {
                 const int a = c - ngroup;
-                if (ap.agg[a].op == kAggCount) {
+                if (ap.agg[a].op == kAggCount || (ap.agg[a].op == kAggSum && aggs[a].op == IMM3_AGG_SUM)) {
                     const int64_t v = e.val[a];
+                    std::memcpy(dst + (size_t)i * 8, &v, 8);
+                } else if (ap.agg[a].op == kAggSum) {
+                    const double v = (double)e.val[a] / (double)e.val[count_slot];  // AVG, once, in IEEE double
                     std::memcpy(dst + (size_t)i * 8, &v, 8);
                 } else {
                     const double v = (double)e.val[a];  // value.toDouble, ProjectAggregate.scala:176-178
@@ -2091,12 +2156,18 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
 
 int imm3_query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, const imm3_agg* aggs, int naggs,
                    const char* const* group_cols, int ngroup, imm3_result** out) {
-    return query_agg(db, table, preds, npreds, aggs, naggs, group_cols, ngroup, false, out);
+    return query_agg(db, table, preds, npreds, aggs, naggs, group_cols, ngroup, false, false, out);
 }
 
 int imm3_query_agg_global(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, const imm3_agg* aggs, int naggs,
                           const char* const* group_cols, int ngroup, imm3_result** out) {
-    return query_agg(db, table, preds, npreds, aggs, naggs, group_cols, ngroup, true, out);
+    return query_agg(db, table, preds, npreds, aggs, naggs, group_cols, ngroup, true, false, out);
+}
+
+int imm3_query_agg_ext(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, const imm3_agg* aggs, int naggs,
+                       const char* const* group_cols, int ngroup, uint32_t flags, imm3_result** out) {
+    if (flags & ~IMM3_AGG_GLOBAL) return fail(IMM3_ERR_INVALID_ARG, "imm3_query_agg_ext: unknown flag bits 0x%x", flags & ~IMM3_AGG_GLOBAL);
+    return query_agg(db, table, preds, npreds, aggs, naggs, group_cols, ngroup, (flags & IMM3_AGG_GLOBAL) != 0, true, out);
 }
 
 int imm3_query_sql(imm3_db* db, const char* sql, imm3_result** out) {
@@ -2150,14 +2221,14 @@ int imm3_result_format_row(const imm3_result* r, int64_t row, char* buf, size_t 
     for (int c = c0; c < r->ncols; c++) {
         if (c > c0) s += ",";
         const uint8_t* p = (const uint8_t*)r->h_cols[(size_t)c].p + (size_t)row * (size_t)r->widths[(size_t)c];
-        if (r->types[(size_t)c] == IMM3_COL_COUNT) {
+        if (r->types[(size_t)c] == IMM3_COL_COUNT || r->types[(size_t)c] == IMM3_COL_INT64) {
             int64_t v;
             std::memcpy(&v, p, 8);
             s += std::to_string(v);  // Long.toString
         } else if (r->types[(size_t)c] == IMM3_COL_DOUBLE) {
             double v;
             std::memcpy(&v, p, 8);
-            s += java_double_to_string_integral(v);
+            s += (r->avg_cols >> (c - c0)) & 1u ? java_double_to_string(v) : java_double_to_string_integral(v);
         } else if (r->types[(size_t)c] == IMM3_COL_INT) {
             int32_t v;
             std::memcpy(&v, p, 4);

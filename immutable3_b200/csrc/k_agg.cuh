@@ -24,6 +24,9 @@
 //                            agg_exchange_kernel) into a fresh global table, then agg_compact_kernel again
 // Exact integer arithmetic: counts are 64-bit, min / max are taken on the raw int32 / int8 values (the reference widens to
 // Double, which is exact for both types; the host formats them as Doubles).
+// SUM (imm3_query_agg_ext only, DESIGN §4.4c) runs its own instantiations, agg_kernel / agg_blocks_kernel<NG, NA, true>: the
+// same row loop with a 64-bit per-warp partial per SUM and slot, every add modulo 2^64.  Past the fold a SUM travels as
+// a COUNT (the global table, agg_init_kernel and agg_merge_kernel add it with the same 64-bit atomicAdd).
 // =============================================================================================
 constexpr unsigned long long kAggEmpty = ~0ull;
 
@@ -46,10 +49,37 @@ __device__ __forceinline__ uint32_t agg_hash(unsigned long long k) {
 // as the MAX of the complemented inputs (~x reverses the order of int32 without overflow) and complemented back when the
 // table leaves shared memory; after a group's first rows the atomics all but disappear.  COUNT is one native 32-bit
 // shared-memory atomic per row (a warp counts far fewer than 2^32 rows).
+// A SUM's partial is 64-bit: its low words sit in the aggregate's own plane, its high words in one more plane per SUM
+// behind the first-row plane (plane NA + 1 + j for the j-th SUM of the plan).  A 64-bit atomicAdd on shared memory is a
+// CAS loop on sm_100a (ATOMS.CAST.SPIN.64), so a row adds its value with one native 32-bit atomicAdd on the low word and
+// carries into the high word from the old value it returns: the high word moves only on a carry or a negative input.
 constexpr int kAggSlots = 256;
 constexpr int kAggDictBits = 14;
-constexpr size_t agg_smem_bytes(int na) {
-    return ((size_t)1 << kAggDictBits) + (size_t)kAggSlots * 8 + (size_t)kComputeWarps * (na + 1) * kAggSlots * 4 + (size_t)kComputeWarps * 1024 * 2;
+constexpr size_t agg_smem_bytes(int na, int nsum = 0) {
+    return ((size_t)1 << kAggDictBits) + (size_t)kAggSlots * 8 + (size_t)kComputeWarps * (na + 1 + nsum) * kAggSlots * 4 + (size_t)kComputeWarps * 1024 * 2;
+}
+// Bit a set = aggregate a is a SUM (S: a SUM instantiation; elsewhere no plan has one).
+template <int NA, bool S>
+__device__ __forceinline__ unsigned agg_sum_mask(const AggPlan& A) {
+    unsigned m = 0;
+    if constexpr (S) {
+#pragma unroll
+        for (int a = 0; a < NA; a++) m |= A.agg[a].op == kAggSum ? 1u << a : 0u;
+    }
+    return m;
+}
+// x into the 64-bit partial of aggregate a (a SUM) at slot: lo = the low word in the aggregate's plane, V = the warp's values.
+template <int NA>
+__device__ __forceinline__ void agg_sum_add(int* V, int* lo, unsigned sum_mask, int a, int slot, int x) {
+    const unsigned old = atomicAdd(reinterpret_cast<unsigned int*>(lo), (unsigned)x);
+    const int dhi = (x >> 31) + (old + (unsigned)x < old ? 1 : 0);  // sign extension + carry out of the low word
+    if (dhi != 0) atomicAdd(V + (NA + 1 + __popc(sum_mask & ((1u << a) - 1u))) * kAggSlots + slot, dhi);
+}
+// Warp partial of SUM a at slot i as a 64-bit two's-complement value (W = the warp's values).
+template <int NA>
+__device__ __forceinline__ long long agg_sum_read(const int* W, unsigned sum_mask, int a, int i) {
+    const unsigned lo = (unsigned)W[a * kAggSlots + i], hi = (unsigned)W[(NA + 1 + __popc(sum_mask & ((1u << a) - 1u))) * kAggSlots + i];
+    return (long long)(((unsigned long long)hi << 32) | lo);
 }
 __device__ __forceinline__ uint32_t agg_hash32(unsigned long long k) {
     return ((uint32_t)k * 0x9E3779B1u) ^ ((uint32_t)(k >> 32) * 0x85EBCA6Bu);
@@ -98,8 +128,8 @@ __device__ __forceinline__ void agg_update(long long* v, int op, long long x) {
 __device__ __forceinline__ long long agg_identity(int op) { return op == kAggCount ? 0ll : (op == kAggMin ? LLONG_MAX : LLONG_MIN); }
 
 // One group's partial (x[a]: a count, or an extreme as int64) into the global table.  (K: agg_blocks_kernel calls its own
-// copy, K = 1, and agg_merge_kernel K = 2, so that agg_kernel's call graph - and with it agg_kernel's register allocation -
-// is the one it had alone.)
+// copy, K = 1, agg_merge_kernel K = 2 and the SUM instantiations K = 3 and 4, so that agg_kernel's call
+// graph - and with it agg_kernel's register allocation - is the one it had alone.)
 template <int K = 0>
 __device__ __noinline__ void agg_to_global(AggEntry* table, uint32_t slots, unsigned int* overflow, unsigned long long key, unsigned long long fr,
                                            const long long* x, const AggCol* aggs, int naggs) {
@@ -111,31 +141,75 @@ __device__ __noinline__ void agg_to_global(AggEntry* table, uint32_t slots, unsi
     atomicMin(&table[gs].first_row, fr);
     for (int a = 0; a < naggs; a++) agg_update(&table[gs].val[a], aggs[a].op, x[a]);
 }
+// The fold of a SUM instantiation (agg_kernel: K = 3, agg_blocks_kernel: K = 4): thread t folds slot t over the
+// CTA's warps in 64 bits - COUNT and SUM add modulo 2^64, MIN / MAX take the extreme - and hands the group to the global
+// table, where a SUM is added as a COUNT.  nplanes = 32-bit planes per warp; first_row(w, ord) = the row of warp w's ordinal.
+template <int NA, int K, class FirstRow>
+__device__ __forceinline__ void agg_fold_sum(const AggPlan& A, int naggs, const unsigned long long* keys, const int* vals, int nplanes, unsigned sum_mask,
+                                             AggEntry* table, unsigned int* overflow, const AggCol* s_agg, int tid, FirstRow first_row) {
+    for (int i = tid; i < kAggSlots; i += kComputeThreads) {
+        const unsigned long long key = keys[i];
+        if (key == kAggEmpty) continue;
+        unsigned long long first = ~0ull;
+        unsigned long long acc[kMaxAggs];
+#pragma unroll
+        for (int a = 0; a < NA; a++) acc[a] = (A.agg[a].op == kAggMin || A.agg[a].op == kAggMax) ? (unsigned long long)(long long)INT_MIN : 0ull;
+        for (int w = 0; w < kComputeWarps; w++) {
+            const int* const W = vals + w * nplanes * kAggSlots;
+            const int fo = W[NA * kAggSlots + i];
+            if (fo == INT_MIN) continue;  // warp w never saw this group
+            const unsigned long long r = first_row(w, (unsigned)~fo);
+            first = r < first ? r : first;
+#pragma unroll
+            for (int a = 0; a < NA; a++) {
+                if (NA == 8 && a >= naggs) break;
+                const int op = A.agg[a].op, v = W[a * kAggSlots + i];
+                if (op == kAggCount) acc[a] += (unsigned)v;
+                else if (op == kAggSum) acc[a] += (unsigned long long)agg_sum_read<NA>(W, sum_mask, a, i);
+                else if ((long long)v > (long long)acc[a]) acc[a] = (unsigned long long)(long long)v;
+            }
+        }
+        if (first == ~0ull) continue;
+        long long xl[kMaxAggs];
+#pragma unroll
+        for (int a = 0; a < NA; a++) xl[a] = A.agg[a].op == kAggMin ? (long long)~(int)acc[a] : (long long)acc[a];
+        agg_to_global<K>(table, A.table_slots, overflow, key, first, xl, s_agg, naggs);
+    }
+}
+
 // NG = group-by columns (0, 1, 2 exact; 4 = A.ngroup of them, up to 4), NA = aggregates (1 .. 4 exact; 8 = A.naggs of them, up to 8):
 // the loops over the plan are unrolled with compile-time indices into the kernel's parameter block, so the per-column
 // descriptors are constant-bank operands - nothing about the query is decoded per row and nothing of it lives in registers.
-template <int NG, int NA>
+// S = true: the SUM instantiations (a plan with a SUM); with S = false the code is the one agg_kernel had before SUM existed.
+template <int NG, int NA, bool S>
 __global__ void __launch_bounds__(kComputeThreads, 3) agg_kernel(const __grid_constant__ AggPlan A, const uint32_t* __restrict__ bitmap,
                                                                   const uint32_t* __restrict__ span_cnt, AggEntry* __restrict__ table,
                                                                   unsigned int* __restrict__ overflow, const ScanCtrl* ctrl) {
     extern __shared__ __align__(128) uint8_t agg_smem[];
+    const unsigned sum_mask = agg_sum_mask<NA, S>(A);
+    const int nplanes = NA + 1 + (S ? __popc(sum_mask) : 0);  // 32-bit planes per warp
     uint8_t* const dict = agg_smem;
     unsigned long long* const keys = reinterpret_cast<unsigned long long*>(agg_smem + (1u << kAggDictBits));
     int* const vals = reinterpret_cast<int*>(agg_smem + (1u << kAggDictBits) + kAggSlots * 8);
-    unsigned short* const sel_all = reinterpret_cast<unsigned short*>(vals + kComputeWarps * (NA + 1) * kAggSlots);
+    unsigned short* const sel_all = reinterpret_cast<unsigned short*>(vals + kComputeWarps * nplanes * kAggSlots);
     __shared__ AggCol s_agg[kMaxAggs];  // (for the cold paths only: a row or a group that goes to the global table)
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
 #pragma unroll
     for (int i = 0; i < kMaxAggs; i++)
-        if (tid == i) s_agg[i] = A.agg[i];
+        if (tid == i) {
+            s_agg[i] = A.agg[i];
+            if (S && A.agg[i].op == kAggSum) s_agg[i].op = kAggCount;  // (the global table adds a SUM as a COUNT)
+        }
     const int naggs = NA == 8 ? A.naggs : NA, ngroup = NG == 4 ? A.ngroup : NG;
     for (int i = tid; i < (1 << kAggDictBits) / 4; i += kComputeThreads) reinterpret_cast<uint32_t*>(dict)[i] = 0u;
     for (int i = tid; i < kAggSlots; i += kComputeThreads) keys[i] = kAggEmpty;
-    int* const V = vals + warp * (NA + 1) * kAggSlots;  // this warp's values: V[a * kAggSlots + slot]
+    int* const V = vals + warp * nplanes * kAggSlots;  // this warp's values: V[a * kAggSlots + slot]
     for (int i = lane; i < kAggSlots; i += 32) {
 #pragma unroll
-        for (int a = 0; a < NA; a++) V[a * kAggSlots + i] = A.agg[a].op == kAggCount ? 0 : INT_MIN;
+        for (int a = 0; a < NA; a++) V[a * kAggSlots + i] = (A.agg[a].op == kAggCount || (S && A.agg[a].op == kAggSum)) ? 0 : INT_MIN;
         V[NA * kAggSlots + i] = INT_MIN;
+        if (S)
+            for (int p = NA + 1; p < nplanes; p++) V[p * kAggSlots + i] = 0;
     }
     __syncthreads();
 
@@ -198,6 +272,7 @@ __global__ void __launch_bounds__(kComputeThreads, 3) agg_kernel(const __grid_co
                 if (NA == 8 && a >= naggs) break;
                 int* const v = V + a * kAggSlots + slot;
                 if (A.agg[a].op == kAggCount) atomicAdd(reinterpret_cast<unsigned int*>(v), 1u);
+                else if (S && A.agg[a].op == kAggSum) agg_sum_add<NA>(V, v, sum_mask, a, slot, x[a]);
                 else if (x[a] > *reinterpret_cast<volatile int*>(v)) atomicMax(v, x[a]);  // (a stale read is only ever too low: at worst one atomic too many)
             }
             int* const f = V + NA * kAggSlots + slot;
@@ -207,7 +282,7 @@ __global__ void __launch_bounds__(kComputeThreads, 3) agg_kernel(const __grid_co
             long long xl[kMaxAggs];
 #pragma unroll
             for (int a = 0; a < NA; a++) xl[a] = A.agg[a].op == kAggCount ? 1ll : (long long)(A.agg[a].op == kAggMin ? ~x[a] : x[a]);
-            agg_to_global(table, A.table_slots, overflow, key, (unsigned long long)row, xl, s_agg, naggs);
+            agg_to_global<S ? 3 : 0>(table, A.table_slots, overflow, key, (unsigned long long)row, xl, s_agg, naggs);
         }
     };
 
@@ -257,46 +332,55 @@ __global__ void __launch_bounds__(kComputeThreads, 3) agg_kernel(const __grid_co
     }
     // thread t folds slot t over the CTA's warps and hands the group to the global table
     __syncthreads();
-    for (int i = tid; i < kAggSlots; i += kComputeThreads) {
-        const unsigned long long key = keys[i];
-        if (key == kAggEmpty) continue;
-        unsigned long long first = ~0ull;
-        int acc[NA];
+    if constexpr (S) {
+        agg_fold_sum<NA, 3>(A, naggs, keys, vals, nplanes, sum_mask, table, overflow, s_agg, tid, [&](int w, unsigned ord) -> unsigned long long {
+            return ((unsigned long long)((long long)blockIdx.x * kComputeWarps + w + (long long)(ord >> 10) * span_stride) << 10) | (ord & 1023u);
+        });
+    } else {
+        for (int i = tid; i < kAggSlots; i += kComputeThreads) {
+            const unsigned long long key = keys[i];
+            if (key == kAggEmpty) continue;
+            unsigned long long first = ~0ull;
+            int acc[NA];
 #pragma unroll
-        for (int a = 0; a < NA; a++) acc[a] = A.agg[a].op == kAggCount ? 0 : INT_MIN;
-        for (int w = 0; w < kComputeWarps; w++) {
-            const int* const W = vals + w * (NA + 1) * kAggSlots;
-            const int fo = W[NA * kAggSlots + i];
-            if (fo == INT_MIN) continue;  // warp w never saw this group
-            const unsigned ord = (unsigned)~fo;
-            const unsigned long long r = ((unsigned long long)((long long)blockIdx.x * kComputeWarps + w + (long long)(ord >> 10) * span_stride) << 10) | (ord & 1023u);
-            first = r < first ? r : first;
+            for (int a = 0; a < NA; a++) acc[a] = A.agg[a].op == kAggCount ? 0 : INT_MIN;
+            for (int w = 0; w < kComputeWarps; w++) {
+                const int* const W = vals + w * (NA + 1) * kAggSlots;
+                const int fo = W[NA * kAggSlots + i];
+                if (fo == INT_MIN) continue;  // warp w never saw this group
+                const unsigned ord = (unsigned)~fo;
+                const unsigned long long r = ((unsigned long long)((long long)blockIdx.x * kComputeWarps + w + (long long)(ord >> 10) * span_stride) << 10) | (ord & 1023u);
+                first = r < first ? r : first;
 #pragma unroll
-            for (int a = 0; a < NA; a++) {
-                if (NA == 8 && a >= naggs) break;
-                const int v = W[a * kAggSlots + i];
-                acc[a] = A.agg[a].op == kAggCount ? (int)((unsigned)acc[a] + (unsigned)v) : (v > acc[a] ? v : acc[a]);  // (a CTA counts < 2^32 rows)
+                for (int a = 0; a < NA; a++) {
+                    if (NA == 8 && a >= naggs) break;
+                    const int v = W[a * kAggSlots + i];
+                    acc[a] = A.agg[a].op == kAggCount ? (int)((unsigned)acc[a] + (unsigned)v) : (v > acc[a] ? v : acc[a]);  // (a CTA counts < 2^32 rows)
+                }
             }
-        }
-        if (first == ~0ull) continue;
-        long long xl[kMaxAggs];
+            if (first == ~0ull) continue;
+            long long xl[kMaxAggs];
 #pragma unroll
-        for (int a = 0; a < NA; a++) xl[a] = A.agg[a].op == kAggCount ? (long long)(unsigned int)acc[a] : (long long)(A.agg[a].op == kAggMin ? ~acc[a] : acc[a]);
-        agg_to_global(table, A.table_slots, overflow, key, first, xl, s_agg, naggs);
+            for (int a = 0; a < NA; a++) xl[a] = A.agg[a].op == kAggCount ? (long long)(unsigned int)acc[a] : (long long)(A.agg[a].op == kAggMin ? ~acc[a] : acc[a]);
+            agg_to_global(table, A.table_slots, overflow, key, first, xl, s_agg, naggs);
+        }
     }
 }
 
 // agg_blocks_kernel's per-row work, as functions of the plan: the same steps as agg_kernel's lambdas (fetch_raw / decode /
 // apply / the fold), which stay written out in agg_kernel - routed through these functions its generated code changes.
 // A CTA's empty state: no dict guesses, no keys, this warp's values at their identities (first row: "never seen").
-template <int NA>
-__device__ __forceinline__ void agg_state_init(const AggPlan& A, uint8_t* dict, unsigned long long* keys, int* V, int tid, int lane) {
+// (S: a SUM instantiation - SUM partials and the high-word planes behind the first-row plane start at 0.)
+template <int NA, bool S = false>
+__device__ __forceinline__ void agg_state_init(const AggPlan& A, uint8_t* dict, unsigned long long* keys, int* V, int tid, int lane, int nplanes = NA + 1) {
     for (int i = tid; i < (1 << kAggDictBits) / 4; i += kComputeThreads) reinterpret_cast<uint32_t*>(dict)[i] = 0u;
     for (int i = tid; i < kAggSlots; i += kComputeThreads) keys[i] = kAggEmpty;
     for (int i = lane; i < kAggSlots; i += 32) {
 #pragma unroll
-        for (int a = 0; a < NA; a++) V[a * kAggSlots + i] = A.agg[a].op == kAggCount ? 0 : INT_MIN;
+        for (int a = 0; a < NA; a++) V[a * kAggSlots + i] = (A.agg[a].op == kAggCount || (S && A.agg[a].op == kAggSum)) ? 0 : INT_MIN;
         V[NA * kAggSlots + i] = INT_MIN;
+        if (S)
+            for (int p = NA + 1; p < nplanes; p++) V[p * kAggSlots + i] = 0;
     }
 }
 // The words fetched for row `r` (gw / aw: the aligned 32-bit word holding each cell; gp = the group columns at the row
@@ -333,10 +417,10 @@ __device__ __forceinline__ void agg_decode(const AggPlan& A, int ngroup, int nag
 }
 // One row into its group: `ord` = the row's ordinal in this warp's own sequence of rows (ascending: a group's first row
 // is the one that creates its entry in the warp's values); `row` = its row ordinal (the cold path's first row).
-template <int NA>
+template <int NA, bool S = false>
 __device__ __forceinline__ void agg_apply(const AggPlan& A, int naggs, uint8_t* dict, unsigned long long* keys, int* V, AggEntry* table,
                                           unsigned int* overflow, const AggCol* s_agg, long long row, unsigned ord, unsigned long long key,
-                                          const int (&x)[NA]) {
+                                          const int (&x)[NA], unsigned sum_mask = 0u) {
     const int slot = agg_cta_slot(dict, keys, key);
     if (slot >= 0) {
 #pragma unroll
@@ -344,6 +428,7 @@ __device__ __forceinline__ void agg_apply(const AggPlan& A, int naggs, uint8_t* 
             if (NA == 8 && a >= naggs) break;
             int* const v = V + a * kAggSlots + slot;
             if (A.agg[a].op == kAggCount) atomicAdd(reinterpret_cast<unsigned int*>(v), 1u);
+            else if (S && A.agg[a].op == kAggSum) agg_sum_add<NA>(V, v, sum_mask, a, slot, x[a]);
             else if (x[a] > *reinterpret_cast<volatile int*>(v)) atomicMax(v, x[a]);  // (a stale read is only ever too low: at worst one atomic too many)
         }
         int* const f = V + NA * kAggSlots + slot;
@@ -353,7 +438,7 @@ __device__ __forceinline__ void agg_apply(const AggPlan& A, int naggs, uint8_t* 
         long long xl[kMaxAggs];
 #pragma unroll
         for (int a = 0; a < NA; a++) xl[a] = A.agg[a].op == kAggCount ? 1ll : (long long)(A.agg[a].op == kAggMin ? ~x[a] : x[a]);
-        agg_to_global<1>(table, A.table_slots, overflow, key, (unsigned long long)row, xl, s_agg, naggs);
+        agg_to_global<S ? 4 : 1>(table, A.table_slots, overflow, key, (unsigned long long)row, xl, s_agg, naggs);
     }
 }
 // Thread t folds slot t over the CTA's warps and hands the group to the global table; first_row(w, ord) = the row ordinal
@@ -403,13 +488,16 @@ __device__ __forceinline__ void agg_fold(const AggPlan& A, int naggs, const unsi
 // encoded words while a column is decoded, then the block's selection vector - and per encoded column kBlkVals decoded
 // values + 32 mini-block bases.
 __host__ __device__ constexpr int agg_blocks_warp_words(int npfor, int words_cap) { return (words_cap > 512 ? words_cap : 512) + npfor * (kBlkVals + 32); }
-constexpr size_t agg_blocks_state_bytes(int na) { return agg_smem_bytes(na) - (size_t)kComputeWarps * 1024 * 2; }
+constexpr size_t agg_blocks_state_bytes(int na, int nsum = 0) { return agg_smem_bytes(na, nsum) - (size_t)kComputeWarps * 1024 * 2; }
 
-template <int NG, int NA>
+// S = true: the SUM instantiations, as agg_kernel's.
+template <int NG, int NA, bool S>
 __global__ void __launch_bounds__(kComputeThreads, 2) agg_blocks_kernel(const __grid_constant__ AggPlan A, const uint32_t* __restrict__ bitmap,
                                                                          const uint32_t* __restrict__ span_cnt, AggEntry* __restrict__ table,
                                                                          unsigned int* __restrict__ overflow, const ScanCtrl* ctrl) {
     extern __shared__ __align__(128) uint8_t agg_smem[];
+    const unsigned sum_mask = agg_sum_mask<NA, S>(A);
+    const int nsum = S ? __popc(sum_mask) : 0, nplanes = NA + 1 + nsum;
     uint8_t* const dict = agg_smem;
     unsigned long long* const keys = reinterpret_cast<unsigned long long*>(agg_smem + (1u << kAggDictBits));
     int* const vals = reinterpret_cast<int*>(agg_smem + (1u << kAggDictBits) + kAggSlots * 8);
@@ -418,14 +506,17 @@ __global__ void __launch_bounds__(kComputeThreads, 2) agg_blocks_kernel(const __
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
 #pragma unroll
     for (int i = 0; i < kMaxAggs; i++)
-        if (tid == i) s_agg[i] = A.agg[i];
+        if (tid == i) {
+            s_agg[i] = A.agg[i];
+            if (S && A.agg[i].op == kAggSum) s_agg[i].op = kAggCount;  // (the global table adds a SUM as a COUNT)
+        }
 #pragma unroll
     for (int i = 0; i < kMaxPforCols; i++)
         if (tid == 32 + i) s_pfor[i] = A.pfor[i];
     const int naggs = NA == 8 ? A.naggs : NA, ngroup = NG == 4 ? A.ngroup : NG, npfor = A.npfor;
-    int* const V = vals + warp * (NA + 1) * kAggSlots;
-    agg_state_init<NA>(A, dict, keys, V, tid, lane);
-    uint32_t* const Wb = reinterpret_cast<uint32_t*>(agg_smem + agg_blocks_state_bytes(NA)) + warp * agg_blocks_warp_words(npfor, A.blk_words_cap);
+    int* const V = vals + warp * nplanes * kAggSlots;
+    agg_state_init<NA, S>(A, dict, keys, V, tid, lane, nplanes);
+    uint32_t* const Wb = reinterpret_cast<uint32_t*>(agg_smem + agg_blocks_state_bytes(NA, nsum)) + warp * agg_blocks_warp_words(npfor, A.blk_words_cap);
     uint32_t* const dec = Wb + (A.blk_words_cap > 512 ? A.blk_words_cap : 512);  // [slot][kBlkVals]
     uint32_t* const bases = dec + npfor * kBlkVals;                                 // [slot][mini-block]
     unsigned short* const sel_w = reinterpret_cast<unsigned short*>(Wb);
@@ -522,8 +613,8 @@ __global__ void __launch_bounds__(kComputeThreads, 2) agg_blocks_kernel(const __
                 fetch_raw(s0, g0, a0);
                 fetch_raw(s1, g1, a1);
             }
-            if (live0) agg_apply<NA>(A, naggs, dict, keys, V, table, overflow, s_agg, R0 + c0, ord0 + c0, k0, x0);
-            if (live1) agg_apply<NA>(A, naggs, dict, keys, V, table, overflow, s_agg, R0 + c1, ord0 + c1, k1, x1);
+            if (live0) agg_apply<NA, S>(A, naggs, dict, keys, V, table, overflow, s_agg, R0 + c0, ord0 + c0, k0, x0, sum_mask);
+            if (live1) agg_apply<NA, S>(A, naggs, dict, keys, V, table, overflow, s_agg, R0 + c1, ord0 + c1, k1, x1, sum_mask);
         }
     };
 
@@ -563,9 +654,11 @@ __global__ void __launch_bounds__(kComputeThreads, 2) agg_blocks_kernel(const __
         }
     }
     __syncthreads();
-    agg_fold<NA>(A, naggs, keys, vals, table, overflow, s_agg, tid, [&](int w, unsigned ord) -> unsigned long long {
+    auto first_row = [&](int w, unsigned ord) -> unsigned long long {
         return A.row_start[(long long)blockIdx.x * kComputeWarps + w + (long long)(ord >> 10) * nwarps] + (ord & 1023u);
-    });
+    };
+    if constexpr (S) agg_fold_sum<NA, 4>(A, naggs, keys, vals, nplanes, sum_mask, table, overflow, s_agg, tid, first_row);
+    else agg_fold<NA>(A, naggs, keys, vals, table, overflow, s_agg, tid, first_row);
 }
 
 // Occupied slots -> out[0 .. *nout), in any order (the host sorts the groups by first_row).

@@ -183,45 +183,64 @@ cudaError_t launch_blocks_prune(const PrunePlan& q, const uint64_t* row_start, l
     return cudaGetLastError();
 }
 
-// count / min / max ... group by: empty table -> (filter kernel, launched by the caller) -> agg_kernel -> compaction.
+// count / min / max / sum ... group by: empty table -> (filter kernel, launched by the caller) -> agg_kernel (its SUM
+// instantiation when the plan has a SUM) -> compaction.
+static int agg_nsum(const AggPlan& a) {
+    int n = 0;
+    for (int i = 0; i < a.naggs && i < kMaxAggs; i++) n += a.agg[i].op == kAggSum;
+    return n;
+}
 cudaError_t launch_agg_init(AggEntry* table, uint32_t slots, const AggPlan& a, unsigned int* counters, cudaStream_t stream) {
     cudaError_t e = configure_once();
     if (e != cudaSuccess) return e;
     AggOps ops;
-    for (int i = 0; i < kMaxAggs; i++) ops.op[i] = i < a.naggs ? a.agg[i].op : 0;
+    for (int i = 0; i < kMaxAggs; i++) ops.op[i] = i < a.naggs ? (a.agg[i].op == kAggSum ? kAggCount : a.agg[i].op) : 0;  // (a SUM starts at 0, as a COUNT)
     ops.naggs = a.naggs;
     agg_init_kernel<<<(slots + kComputeThreads - 1) / kComputeThreads, kComputeThreads, 0, stream>>>(table, slots, ops, counters);
     return cudaGetLastError();
 }
-template <int NG, int NA>
+template <int NG, int NA, bool S>
 static cudaError_t launch_agg_as(const AggPlan& a, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, unsigned int* overflow,
                                  const ScanCtrl* ctrl, int num_sms, cudaStream_t stream) {
-    const size_t smem = agg_smem_bytes(NA);
+    auto* const kern = agg_kernel<NG, NA, S>;
+    const size_t smem = agg_smem_bytes(NA, S ? agg_nsum(a) : 0);
     cudaError_t e = cudaSuccess;
     // (a per-device attribute, set per launch: one driver call per aggregation query)
-    if (smem > 48 * 1024 && (e = cudaFuncSetAttribute(agg_kernel<NG, NA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
+    if (smem > 48 * 1024 && (e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
     int occ = 0;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, agg_kernel<NG, NA>, kComputeThreads, smem);
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kComputeThreads, smem);
     if (e != cudaSuccess) return e;
     if (occ < 1) return cudaErrorInvalidConfiguration;
     const long long nspans = a.ntiles * 8;
     const long long grid = std::max<long long>(1, std::min<long long>((nspans + kComputeWarps - 1) / kComputeWarps, (long long)num_sms * occ));
-    agg_kernel<NG, NA><<<(unsigned)grid, kComputeThreads, smem, stream>>>(a, bitmap, span_cnt, table, overflow, ctrl);
+    kern<<<(unsigned)grid, kComputeThreads, smem, stream>>>(a, bitmap, span_cnt, table, overflow, ctrl);
     return cudaGetLastError();
 }
-// the instantiation for this query's shape: exact for <= 2 group-by columns and 1 .. 4 aggregates, the general forms beyond
+// the instantiation for this query's shape: exact for <= 2 group-by columns and 1 .. 4 aggregates, the general forms beyond;
+// a plan with a SUM takes the SUM instantiations (it carries a COUNT too: 2 .. 4 aggregates exact, else 8)
 #define IMM3_AGG_DISPATCH(LAUNCH)                                                                                                         \
     do {                                                                                                                                  \
         const int ng = a.ngroup <= 2 ? a.ngroup : 4, na = (a.naggs >= 1 && a.naggs <= 4) ? a.naggs : 8;                                   \
-        IMM3_AGG_DISPATCH_ROW(LAUNCH, 0) else IMM3_AGG_DISPATCH_ROW(LAUNCH, 1) else IMM3_AGG_DISPATCH_ROW(LAUNCH, 2) else IMM3_AGG_DISPATCH_ROW(LAUNCH, 4) \
+        if (agg_nsum(a) == 0) {                                                                                                           \
+            IMM3_AGG_DISPATCH_ROW(LAUNCH, 0) else IMM3_AGG_DISPATCH_ROW(LAUNCH, 1) else IMM3_AGG_DISPATCH_ROW(LAUNCH, 2) else IMM3_AGG_DISPATCH_ROW(LAUNCH, 4) \
+        } else {                                                                                                                          \
+            IMM3_AGG_SUM_ROW(LAUNCH, 0) else IMM3_AGG_SUM_ROW(LAUNCH, 1) else IMM3_AGG_SUM_ROW(LAUNCH, 2) else IMM3_AGG_SUM_ROW(LAUNCH, 4) \
+        }                                                                                                                                 \
     } while (0)
 #define IMM3_AGG_DISPATCH_ROW(LAUNCH, NG)                                                                                                  \
     if (ng == NG) {                                                                                                                       \
-        if (na == 1) e = LAUNCH<NG, 1>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                                  \
-        else if (na == 2) e = LAUNCH<NG, 2>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                             \
-        else if (na == 3) e = LAUNCH<NG, 3>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                             \
-        else if (na == 4) e = LAUNCH<NG, 4>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                             \
-        else e = LAUNCH<NG, 8>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                                          \
+        if (na == 1) e = LAUNCH<NG, 1, false>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                           \
+        else if (na == 2) e = LAUNCH<NG, 2, false>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                      \
+        else if (na == 3) e = LAUNCH<NG, 3, false>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                      \
+        else if (na == 4) e = LAUNCH<NG, 4, false>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                      \
+        else e = LAUNCH<NG, 8, false>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                                   \
+    }
+#define IMM3_AGG_SUM_ROW(LAUNCH, NG)                                                                                                       \
+    if (ng == NG) {                                                                                                                       \
+        if (na <= 2) e = LAUNCH<NG, 2, true>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                            \
+        else if (na == 3) e = LAUNCH<NG, 3, true>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                       \
+        else if (na == 4) e = LAUNCH<NG, 4, true>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                       \
+        else e = LAUNCH<NG, 8, true>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                                    \
     }
 cudaError_t launch_agg(const AggPlan& a, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, AggEntry* out, unsigned int* counters,
                        const ScanCtrl* ctrl, int num_sms, cudaStream_t stream) {
@@ -233,23 +252,24 @@ cudaError_t launch_agg(const AggPlan& a, const uint32_t* bitmap, const uint32_t*
     return cudaGetLastError();
 }
 
-// ... the same with agg_blocks_kernel (a MIN / MAX input or a group column in the sorted-int codec; blocks of <= 1024 rows)
-size_t agg_blocks_smem_bytes(int naggs, int npfor, int words_cap) {
-    const int na = (naggs >= 1 && naggs <= 4) ? naggs : 8;
-    return agg_blocks_state_bytes(na) + (size_t)kComputeWarps * (size_t)agg_blocks_warp_words(npfor, words_cap) * 4;
+// ... the same with agg_blocks_kernel (a MIN / MAX / SUM input or a group column in the sorted-int codec; blocks of <= 1024 rows)
+size_t agg_blocks_smem_bytes(int naggs, int npfor, int words_cap, int nsum) {
+    const int na = nsum > 0 ? (naggs <= 2 ? 2 : (naggs <= 4 ? naggs : 8)) : ((naggs >= 1 && naggs <= 4) ? naggs : 8);  // (IMM3_AGG_DISPATCH's NA)
+    return agg_blocks_state_bytes(na, nsum) + (size_t)kComputeWarps * (size_t)agg_blocks_warp_words(npfor, words_cap) * 4;
 }
-template <int NG, int NA>
+template <int NG, int NA, bool S>
 static cudaError_t launch_agg_blocks_as(const AggPlan& a, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, unsigned int* overflow,
                                         const ScanCtrl* ctrl, int num_sms, cudaStream_t stream) {
-    const size_t smem = agg_blocks_smem_bytes(NA, a.npfor, a.blk_words_cap);
+    auto* const kern = agg_blocks_kernel<NG, NA, S>;
+    const size_t smem = agg_blocks_smem_bytes(NA, a.npfor, a.blk_words_cap, S ? agg_nsum(a) : 0);
     cudaError_t e = cudaSuccess;
-    if (smem > 48 * 1024 && (e = cudaFuncSetAttribute(agg_blocks_kernel<NG, NA>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
+    if (smem > 48 * 1024 && (e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
     int occ = 0;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, agg_blocks_kernel<NG, NA>, kComputeThreads, smem);
+    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kComputeThreads, smem);
     if (e != cudaSuccess) return e;
     if (occ < 1) return cudaErrorInvalidConfiguration;
     const long long grid = std::max<long long>(1, std::min<long long>((a.nblocks + kComputeWarps - 1) / kComputeWarps, (long long)num_sms * occ));
-    agg_blocks_kernel<NG, NA><<<(unsigned)grid, kComputeThreads, smem, stream>>>(a, bitmap, span_cnt, table, overflow, ctrl);
+    kern<<<(unsigned)grid, kComputeThreads, smem, stream>>>(a, bitmap, span_cnt, table, overflow, ctrl);
     return cudaGetLastError();
 }
 cudaError_t launch_agg_blocks(const AggPlan& a, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, AggEntry* out, unsigned int* counters,
@@ -261,6 +281,7 @@ cudaError_t launch_agg_blocks(const AggPlan& a, const uint32_t* bitmap, const ui
     agg_compact_kernel<<<(a.table_slots + kComputeThreads - 1) / kComputeThreads, kComputeThreads, 0, stream>>>(table, a.table_slots, out, counters);
     return cudaGetLastError();
 }
+#undef IMM3_AGG_SUM_ROW
 #undef IMM3_AGG_DISPATCH_ROW
 #undef IMM3_AGG_DISPATCH
 

@@ -26,7 +26,7 @@ cudaError_t launch_emit_stream(const ScanPlan& plan, const uint32_t* bitmap, con
 cudaError_t launch_agg_init(AggEntry* table, uint32_t slots, const AggPlan& a, unsigned int* counters, cudaStream_t stream);
 cudaError_t launch_agg(const AggPlan& a, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, AggEntry* out, unsigned int* counters,
                        const ScanCtrl* ctrl, int num_sms, cudaStream_t stream);
-size_t agg_blocks_smem_bytes(int naggs, int npfor, int words_cap);  // dynamic shared memory of agg_blocks_kernel
+size_t agg_blocks_smem_bytes(int naggs, int npfor, int words_cap, int nsum = 0);  // dynamic shared memory of agg_blocks_kernel (nsum SUMs: agg_blocks_sum_kernel)
 cudaError_t launch_agg_blocks(const AggPlan& a, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, AggEntry* out, unsigned int* counters,
                               const ScanCtrl* ctrl, int num_sms, cudaStream_t stream);
 long long scan_inline_max_tiles();

@@ -117,7 +117,7 @@ struct PrunePlan {
 // a group column in the sorted-int codec is decoded per block inside agg_blocks_kernel (its slot in agg_pfor / group_pfor).
 constexpr int kMaxAggs = 8;
 constexpr int kMaxGroupCols = 4;
-enum AggOp : int32_t { kAggCount = 0, kAggMin = 1, kAggMax = 2 };
+enum AggOp : int32_t { kAggCount = 0, kAggMin = 1, kAggMax = 2, kAggSum = 3 };  // (kAggSum: imm3_query_agg_ext only)
 struct AggCol {
     const uint8_t* base;  // device arena of the aggregated column (dense INT / TINYINT; unused for COUNT)
     int32_t width;        // 4 or 1
@@ -137,7 +137,7 @@ struct AggPlan {
     AggCol agg[kMaxAggs];
     GroupCol group[kMaxGroupCols];
     // agg_blocks_kernel only (after the fields agg_kernel reads, which keep their parameter offsets):
-    int8_t agg_pfor[kMaxAggs];          // index into pfor[] of a MIN / MAX input in the sorted-int codec, -1 = dense
+    int8_t agg_pfor[kMaxAggs];          // index into pfor[] of a MIN / MAX / SUM input in the sorted-int codec, -1 = dense
     int8_t group_pfor[kMaxGroupCols];   // ... of a group column, -1 = dense
     int32_t npfor;                      // distinct encoded columns decoded per block
     int32_t blk_words_cap;              // per-warp scratch for one encoded block, in 32-bit words (from the columns' max_block_words)
@@ -145,7 +145,8 @@ struct AggPlan {
     const uint64_t* row_start;          // nblocks + 1 row ordinals of the blocks (row space of the dense arenas)
     PforCol pfor[kMaxPforCols];
 };
-// One group in the global table / in the compacted result.  val[i]: COUNT -> the count, MIN / MAX -> the extreme as int64.
+// One group in the global table / in the compacted result.  val[i]: COUNT -> the count, MIN / MAX -> the extreme as int64,
+// SUM -> the sum modulo 2^64.
 struct AggEntry {
     unsigned long long key;        // packed group cells, ~0 = empty slot
     unsigned long long first_row;  // canonical ordinal of the group's first selected row (groups are reported in that order)

@@ -20,7 +20,8 @@ from typing import List, Optional, Sequence
 
 import numpy as np
 
-from .engine import Count, Engine, Max, Min, Query, Result
+from . import _lib as L
+from .engine import Avg, Count, Engine, Max, Min, ProjectAgg, Query, Result, Sum
 
 
 def shard_range(nsegments: int, rank: int, world: int):
@@ -43,8 +44,9 @@ def limit_split(counts: Sequence[int], limit: int):
 def merge_partials(parts: Sequence[List[np.ndarray]], ngroup: int, aggs: Sequence) -> List[np.ndarray]:
     """The fan-in of ProjectAggregateQueueOp (ProjectAggregateQueue.scala:21-45) over per-rank partial groups, in rank
     order: `parts[r]` = rank r's columns (group columns, then one per aggregate).  A key takes the position of the first
-    rank that holds it (global first-appearance order = rank order, then the rank's own order); Count adds up, Min / Max
-    take the extreme.  The host form of what imm3_query_agg_global does on the GPUs."""
+    rank that holds it (global first-appearance order = rank order, then the rank's own order); Count and Sum add up
+    (exactly: Python ints), Min / Max take the extreme.  The host form of what imm3_query_agg_global does on the GPUs.
+    Avg does not merge: `sum_avg_partials` restates it as a Sum and a Count first."""
     pos, rows, firsts = {}, [], []
     for cols in parts:
         n = len(cols[0]) if cols else 0
@@ -59,7 +61,7 @@ def merge_partials(parts: Sequence[List[np.ndarray]], ngroup: int, aggs: Sequenc
                 continue
             m = rows[j]
             for a, agg in enumerate(aggs):
-                if isinstance(agg, Count):
+                if isinstance(agg, (Count, Sum)):
                     m[a] += vals[a]
                 elif isinstance(agg, Min):
                     m[a] = min(m[a], vals[a])
@@ -75,11 +77,41 @@ def merge_partials(parts: Sequence[List[np.ndarray]], ngroup: int, aggs: Sequenc
     return out
 
 
+def sum_avg_partials(aggs: Sequence):
+    """The aggregates a rank computes for a Sum / Avg query merged on the host: every Avg(c) becomes Sum(c), and one Count
+    of the group's rows is carried (the query's first Count, else one appended).  Returns (those aggregates, the index of
+    the Count)."""
+    plan = [Sum(a.col, a.alias) if isinstance(a, Avg) else a for a in aggs]
+    count = next((i for i, a in enumerate(plan) if isinstance(a, Count)), None)
+    if count is None:
+        plan.append(Count(aggs[0].col))
+        count = len(plan) - 1
+    return plan, count
+
+
+def finish_sum_avg(cols: List[np.ndarray], ngroup: int, aggs: Sequence, count: int) -> List[np.ndarray]:
+    """Merged columns of the `sum_avg_partials` plan -> the query's columns: Avg = float64(sum) / float64(count) (bitwise
+    what imm3_query_agg_ext computes), the carried Count dropped unless the query asked for it.  A group of more than 2^32
+    rows is refused as the library refuses it (its sum may not fit int64)."""
+    if not cols:
+        return []
+    n = cols[ngroup + count]
+    if len(n) and int(n.max()) > 1 << 32:
+        raise L.Imm3Error(L.ERR_UNSUPPORTED, "a group of more than 2^32 rows: sum / avg are exact for groups of at most 2^32 rows")
+    out = list(cols[:ngroup])
+    for a, agg in enumerate(aggs):
+        c = cols[ngroup + a]
+        out.append(c.astype(np.float64) / n.astype(np.float64) if isinstance(agg, Avg) else c)
+    return out
+
+
 class CudaExecutor:
     def __init__(self, engine: Engine):
         self.engine = engine
 
-    def begin(self, query: Query) -> Result:
+    def begin(self, query: Query, sum_avg: bool = False) -> Result:
+        if sum_avg:
+            return self.engine.begin(query, sum_avg=True)
         return self.engine.begin(query)
 
     def finish(self, handle: Result, take: int) -> List[np.ndarray]:
@@ -130,21 +162,31 @@ class ShardedEngine:
         ms = float(getattr(h, "device_ms", 0.0))
         return ShardResult(self.rank, self.world, counts, offsets[self.rank], takes[self.rank], sum(takes), cols, ms)
 
-    def execute_agg(self, query: Query) -> ShardResult:
+    def execute_agg(self, query: Query, sum_avg: bool = False) -> ShardResult:
         """A ProjectAgg query over the whole table, the same groups on every rank: `columns` = the global groups,
         `counts` = every rank's partial group count, offset 0, take = total = the number of global groups.  On a
         connected handle the GPUs merge the partials themselves (imm3_query_agg_global); otherwise every rank's partial
-        columns are all-gathered through torch.distributed and merged on the host in rank order (`merge_partials`)."""
+        columns are all-gathered through torch.distributed and merged on the host in rank order (`merge_partials`).
+        `sum_avg=True` resolves Sum / Avg (imm3_query_agg_ext; on the host path each rank computes Avg as a Sum and a
+        Count, `sum_avg_partials`, and the merged sums are divided once, `finish_sum_avg`)."""
         engine = getattr(self.executor, "engine", None)
         if getattr(getattr(engine, "sm", None), "comm_connected", False):
-            with engine.execute_agg_global(query) as h:
+            with engine.execute_agg_global(query, sum_avg=sum_avg) as h:
                 cols = h.columns()
                 return ShardResult(self.rank, self.world, h.rank_counts, 0, h.nrows, h.nrows, cols, float(h.device_ms))
-        h = self.executor.begin(query)  # this rank's partial groups
+        aggs, ngroup = list(query.project.aggs), len(query.project.groupBy)
+        if sum_avg:
+            plan, count = sum_avg_partials(aggs)
+            h = self.executor.begin(Query(query.table, query.select, ProjectAgg(plan, query.project.groupBy)), sum_avg=True)
+        else:
+            h = self.executor.begin(query)  # this rank's partial groups
         mine = self.executor.finish(h, int(h.local_count))
         everyone = [None] * self.world
         self.dist.all_gather_object(everyone, mine, group=self.group)
-        cols = merge_partials(everyone, len(query.project.groupBy), list(query.project.aggs))
+        if sum_avg:
+            cols = finish_sum_avg(merge_partials(everyone, ngroup, plan), ngroup, aggs, count)
+        else:
+            cols = merge_partials(everyone, ngroup, aggs)
         total = len(cols[0]) if cols else 0
         counts = [len(p[0]) if p else 0 for p in everyone]
         return ShardResult(self.rank, self.world, counts, 0, total, total, cols, float(getattr(h, "device_ms", 0.0)))

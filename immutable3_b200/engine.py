@@ -99,7 +99,9 @@ class Project:
 
 
 # Aggregates (Query.scala:17-27).  Sum / Avg exist in the ADT and the parser, but Engine.resolveProjectOp throws on them
-# (Engine.scala:153); they are accepted here only to come back as IMM3_ERR_UNSUPPORTED.
+# (Engine.scala:153): by default they come back as IMM3_ERR_UNSUPPORTED, as there.  `sum_avg=True` (Engine.execute,
+# execute_agg_global, ShardedEngine.execute_agg) resolves them through imm3_query_agg_ext: Sum = the exact int64 sum,
+# Avg = float64(sum) / float64(count).
 @dataclass(frozen=True)
 class Sum:
     col: str
@@ -215,7 +217,8 @@ class Row(tuple):
     __str__ = __repr__
 
 
-_NP = {L.COL_INT: np.dtype("<i4"), L.COL_TINYINT: np.dtype("i1"), L.COL_COUNT: np.dtype("<i8"), L.COL_DOUBLE: np.dtype("<f8")}
+_NP = {L.COL_INT: np.dtype("<i4"), L.COL_TINYINT: np.dtype("i1"), L.COL_COUNT: np.dtype("<i8"), L.COL_DOUBLE: np.dtype("<f8"),
+       L.COL_INT64: np.dtype("<i8")}
 _AGG_OPS = {"Count": L.AGG_COUNT, "Min": L.AGG_MIN, "Max": L.AGG_MAX, "Sum": L.AGG_SUM, "Avg": L.AGG_AVG}
 
 
@@ -526,20 +529,21 @@ class Engine:
         L.check(self._lib.imm3_query_begin(self.sm.handle, p[0], p[1], p[2], p[3], p[4], p[5], C.byref(out)))
         return Result(out, self._lib, self.sm)
 
-    def execute(self, query: Query, real_or: bool = False) -> Result:
+    def execute(self, query: Query, real_or: bool = False, sum_avg: bool = False) -> Result:
         """Engine.execute: the rows of the query in canonical order (iterate for Row objects).  `real_or=True` evaluates
-        Or as a disjunction (imm3_query_begin_dnf) instead of the reference's Or == And (Engine.scala:236-245)."""
+        Or as a disjunction (imm3_query_begin_dnf) instead of the reference's Or == And (Engine.scala:236-245).
+        `sum_avg=True` resolves Sum / Avg in a ProjectAgg query (imm3_query_agg_ext), which the reference refuses."""
         if isinstance(query.project, ProjectAgg):
-            return self._call_agg(query)
+            return self._call_agg(query, sum_avg=sum_avg)
         if real_or:
             r = self.begin(query, real_or=True)
             return r.fetch(r.take)
         return self._call(self._lib.imm3_query, query)
 
-    def begin(self, query: Query, real_or: bool = False) -> Result:
+    def begin(self, query: Query, real_or: bool = False, sum_avg: bool = False) -> Result:
         """First phase of a sharded query: kernels done, local match count known, nothing fetched."""
         if isinstance(query.project, ProjectAgg):
-            return self._call_agg(query)
+            return self._call_agg(query, sum_avg=sum_avg)
         if real_or:
             return self._call_dnf(query)
         return self._call(self._lib.imm3_query_begin, query)
@@ -557,13 +561,13 @@ class Engine:
         del keep
         return Result(out, self._lib, self.sm)
 
-    def execute_agg_global(self, query: Query) -> Result:
+    def execute_agg_global(self, query: Query, sum_avg: bool = False) -> Result:
         """A ProjectAgg query over the WHOLE table on every rank of a sharded handle (imm3_query_agg_global): the ranks'
         partial groups are merged on the GPUs over the communicator (`SegmentManager.comm_connect`).  On a single handle the
-        result is that of `execute`; an unconnected sharded handle raises (IMM3_ERR_STATE)."""
-        return self._call_agg(query, self._lib.imm3_query_agg_global)
+        result is that of `execute`; an unconnected sharded handle raises (IMM3_ERR_STATE).  `sum_avg` as in `execute`."""
+        return self._call_agg(query, glob=True, sum_avg=sum_avg)
 
-    def _call_agg(self, query: Query, fn=None) -> Result:
+    def _call_agg(self, query: Query, glob: bool = False, sum_avg: bool = False) -> Result:
         """Engine.execute, ProjectAgg branch (Engine.scala:200-232): one row per group, group columns then aggregates."""
         if not isinstance(query.project, ProjectAgg):
             raise L.Imm3Error(L.ERR_UNSUPPORTED, "not a ProjectAgg query")
@@ -575,8 +579,11 @@ class Engine:
             arr[i].op = _AGG_OPS[type(a).__name__]
         groups = L.cstr_array(list(query.project.groupBy))
         out = C.c_void_p()
-        L.check((fn or self._lib.imm3_query_agg)(self.sm.handle, query.table.encode(), preds, npreds, arr, len(aggs),
-                                                 C.cast(groups, C.POINTER(C.c_char_p)), len(query.project.groupBy), C.byref(out)))
+        args = (self.sm.handle, query.table.encode(), preds, npreds, arr, len(aggs), C.cast(groups, C.POINTER(C.c_char_p)), len(query.project.groupBy))
+        if sum_avg:
+            L.check(self._lib.imm3_query_agg_ext(*args, L.AGG_FLAG_GLOBAL if glob else 0, C.byref(out)))
+        else:
+            L.check((self._lib.imm3_query_agg_global if glob else self._lib.imm3_query_agg)(*args, C.byref(out)))
         del keep
         return Result(out, self._lib, self.sm)
 

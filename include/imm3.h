@@ -53,7 +53,8 @@ typedef enum imm3_status {
 typedef enum imm3_column_type {
     IMM3_COL_INT = 0, IMM3_COL_TINYINT = 1, IMM3_COL_STRING = 2,
     IMM3_COL_COUNT = 3,   /* aggregate results only: int64 (CountAggr, ProjectAggregate.scala:21-35)                 */
-    IMM3_COL_DOUBLE = 4   /* aggregate results only: IEEE double (Min/MaxDoubleAggr, ProjectAggregate.scala:37-59)    */
+    IMM3_COL_DOUBLE = 4,  /* aggregate results only: IEEE double (Min/MaxDoubleAggr, ProjectAggregate.scala:37-59)    */
+    IMM3_COL_INT64 = 5    /* aggregate results only: int64, an exact SUM (imm3_query_agg_ext)                          */
 } imm3_column_type;
 
 /* CodecType enumeration (same order), Codec.scala:20-23 */
@@ -228,6 +229,22 @@ int imm3_query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int n
  * must issue the same queries (aggregates and Project queries alike) in the same order. */
 int imm3_query_agg_global(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, const imm3_agg* aggs, int naggs,
                           const char* const* group_cols, int ngroup, imm3_result** out);
+/* Sum and Avg, which the query language has and the reference engine refuses, behind an entry point of their own (the
+ * two above keep refusing them).  flags = 0: imm3_query_agg; IMM3_AGG_GLOBAL: imm3_query_agg_global.  Without a Sum /
+ * Avg the result - rows, names, types, route, status and message - is the one that entry point returns; unknown flag
+ * bits give IMM3_ERR_INVALID_ARG.
+ *   Sum(c), c INT or TINYINT (dense or PFOR_INT): the exact sum of the group's selected values, column <c>_sum,
+ *           IMM3_COL_INT64.
+ *   Avg(c): (double)sum / (double)count, computed once on the host in IEEE double, column <c>_avg, IMM3_COL_DOUBLE;
+ *           imm3_result_format_row prints it as Double.toString does (shortest round-trip digits).
+ * Sum / Avg on a STRING column give IMM3_ERR_UNSUPPORTED.  A query with a Sum or Avg carries one Count of the group's
+ * rows: its own first Count, else a hidden one that is not in the result; visible plus hidden aggregates must be at most
+ * 8 (else IMM3_ERR_UNSUPPORTED).  Every add, on the GPU and in the merge, is a 64-bit two's-complement add, so a sum is
+ * exact whenever its group has at most 2^32 rows; a group with more rows (on a global aggregate: after the merge)
+ * returns IMM3_ERR_UNSUPPORTED, never a wrapped value. */
+#define IMM3_AGG_GLOBAL 0x1u
+int imm3_query_agg_ext(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, const imm3_agg* aggs, int naggs,
+                       const char* const* group_cols, int ngroup, uint32_t flags, imm3_result** out);
 
 /* Same query text the reference CLI takes (SQLParser.scala:8-129; SqlCli.scala:60). */
 int imm3_query_sql(imm3_db* db, const char* sql, imm3_result** out);
@@ -248,7 +265,7 @@ int imm3_result_kernel_launches(const imm3_result* r);      /* kernels launched 
  * blocks_filter_quad, blocks_filter, blocks_group_emit, blocks_scan_emit, blocks_emit(rowspace|blocks), scan_blocks,
  * count_exchange, agg_init, agg<NG,NA>, agg_blocks<NG,NA>, agg_compact, agg_exchange, agg_merge) with "/key=value" parameters: /s= ring stages,
  * /w= warps per CTA of the lane kernel, /ctas= the group emit kernel's grid; "/prefix" marks the prefix pass of a small
- * LIMIT.  E.g. "blocks_prune;blocks_filter_lane/w=11/s=2;blocks_group_emit/ctas=148"; a global aggregate on a connected
+ * LIMIT; "/sum" the SUM instantiation of agg<NG,NA> / agg_blocks<NG,NA> (imm3_query_agg_ext with a Sum or Avg).  E.g. "blocks_prune;blocks_filter_lane/w=11/s=2;blocks_group_emit/ctas=148"; a global aggregate on a connected
  * handle: "agg_init;filter(tma)/s=4;agg<1,2>;agg_compact;agg_exchange;agg_init;agg_merge;agg_compact" (a rank with an empty
  * slice starts at agg_exchange).  Owned by the result (valid until imm3_result_free). */
 const char* imm3_result_route(const imm3_result* r);
