@@ -16,6 +16,7 @@ ERR_NOT_FOUND, ERR_UNSUPPORTED, ERR_BAD_FORMAT, ERR_CUDA, ERR_OOM, ERR_INVALID_A
 COMM_HANDLE_BYTES = 64
 COL_INT, COL_TINYINT, COL_STRING, COL_COUNT, COL_DOUBLE, COL_INT64 = 0, 1, 2, 3, 4, 5
 AGG_FLAG_GLOBAL = 0x1  # IMM3_AGG_GLOBAL
+AGG_FLAG_ENCODED_FILTER = 0x4  # IMM3_AGG_ENCODED_FILTER
 AGG_COUNT, AGG_MIN, AGG_MAX, AGG_SUM, AGG_AVG = 0, 1, 2, 3, 4
 CODEC_PFOR_INT, CODEC_DENSE_INT, CODEC_DENSE_TINYINT, CODEC_DENSE_STRING = 0, 1, 2, 3
 OP_GT, OP_LT, OP_EQ, OP_MATCH, OP_NOTMATCH, OP_NOOP = 1, 2, 3, 4, 5, 6

@@ -532,6 +532,20 @@ int64_t quad_tile_cap(const TableStore& t, const LogicalPlan& lp) {
 }
 constexpr size_t kLaneSmemCap = 222 * 1024;  // shared memory of one lane-kernel CTA (one CTA per SM)
 
+// The block filter kernel of a query with a predicate on an encoded column (kBlocks, and aggregates over such predicates):
+// the only predicate is a range on one encoded column (C4): the quad kernel - lane = (block, super-block), CTA tile of 32
+// blocks - if such a tile of this column fits a ring slot (i.e. the column actually compresses); its lane = block successor
+// if a CTA of 8 warps holds a two-slot ring per warp.  Otherwise (and with IMM3_NO_QUAD) the mini-block kernel.
+void choose_block_filter(Prepared* pr) {
+    const TableStore& t = *pr->table;
+    const LogicalPlan& lp = pr->lp;
+    pr->block_filter = BlockFilter::kMini;
+    if (lp.filters.size() == 1 && is_pfor(t, lp.filters[0].col_idx) && lp.filters[0].kind == kFilterI32Range && !getenv("IMM3_NO_QUAD")) {
+        const int qslot = blocks_filter_quad_slot_bytes((int)quad_tile_cap(t, lp));
+        if (qslot <= 40 * 1024) pr->block_filter = (2 * 8 * (size_t)qslot <= kLaneSmemCap && !getenv("IMM3_NO_LANE")) ? BlockFilter::kLane : BlockFilter::kQuad;
+    }
+}
+
 // Pipeline and block filter kernel of a query, from the table's codecs and block sizes, the logical plan, whether a selection
 // bitmap is wanted and the switches IMM3_PATH=fused, IMM3_NO_HYBRID, IMM3_NO_QUAD, IMM3_NO_LANE and IMM3_OPEN_FORCE_BLOCKS
 // (tests: cross-check the dense and block kernels).
@@ -551,14 +565,7 @@ void choose_route(const imm3_db* db, Prepared* pr) {
     bool filters_dense = true;
     for (auto& f : lp.filters) filters_dense = filters_dense && !is_pfor(t, f.col_idx);
     pr->pipeline = filters_dense && !getenv("IMM3_NO_HYBRID") ? Pipeline::kRowSpace : Pipeline::kBlocks;
-    // The only predicate is a range on one encoded column (C4): the quad kernel - lane = (block, super-block), CTA tile of
-    // 32 blocks - if such a tile of this column fits a ring slot (i.e. the column actually compresses); its lane = block
-    // successor if a CTA of 8 warps holds a two-slot ring per warp.
-    if (pr->pipeline == Pipeline::kBlocks && lp.filters.size() == 1 && !filters_dense && lp.filters[0].kind == kFilterI32Range &&
-        !getenv("IMM3_NO_QUAD")) {
-        const int qslot = blocks_filter_quad_slot_bytes((int)quad_tile_cap(t, lp));
-        if (qslot <= 40 * 1024) pr->block_filter = (2 * 8 * (size_t)qslot <= kLaneSmemCap && !getenv("IMM3_NO_LANE")) ? BlockFilter::kLane : BlockFilter::kQuad;
-    }
+    if (pr->pipeline == Pipeline::kBlocks && !filters_dense) choose_block_filter(pr);
 }
 
 // imm3_explain's name of the kernels
@@ -1090,18 +1097,55 @@ int launch_row_space(imm3_db* db, Prepared* pr, int64_t nblocks, Queued* q) {
     return 0;
 }
 
-// kBlocks: [blocks_prune ->] block filter kernel -> group emit (lane kernel, one encoded column projected: every emit warp finds
-// its rows from the group sums, no scan), scan-emit (one encoded column projected: offset scan + emit in one small-footprint
-// kernel, resident while the filter kernel runs) or offset scan + block emit kernel.
-int launch_blocks(imm3_db* db, Prepared* pr, int64_t nblocks, Queued* q) {
+// Scratch of the block filter front: 32 bitmap words and one count per block, tile counts and offsets, and (pruned) the
+// work list of the tiles blocks_prune_kernel leaves to the filter kernel.
+int ensure_block_filter(imm3_db* db, const Prepared* pr, int64_t nblocks) {
+    int rc;
+    if ((rc = ensure_buf(&db->d_bitmap, (size_t)(nblocks * 32 + 2) * 4))) return rc;
+    if ((rc = ensure_buf(&db->d_span_cnt, (size_t)(nblocks + 8 + 1024) * 4))) return rc;  // (+ whole 16-byte loads of a group's counts)
+    if ((rc = ensure_tile_scratch(db, pr->sp.ntiles))) return rc;
+    return pr->prune ? ensure_buf(&db->d_work, (size_t)((nblocks + 7) / 8 + 2) * 4) : 0;
+}
+
+// The block filter front, shared by Project queries (kBlocks) and aggregates over encoded predicates: [blocks_prune ->]
+// block filter kernel [-> offset scan, when `scan` and the filter kernel's last CTA does not run it].  Per block it leaves
+// the selected row count in d_span_cnt and - only for a partially selected block - the block's 32 words in d_bitmap.
+// Buffers: ensure_block_filter first.  grp_sum: blocks_group_emit_kernel follows (lane kernel only).
+int launch_block_filter_front(imm3_db* db, Prepared* pr, int64_t nblocks, int* launches, uint32_t* grp_sum, bool scan) {
     const TableStore& t = *pr->table;
     ScanPlan& sp = pr->sp;
     const int64_t ntiles = sp.ntiles;
     const bool lane = pr->block_filter == BlockFilter::kLane;
+    const unsigned int* work = pr->prune ? (const unsigned int*)db->d_work.p : nullptr;
+    if (pr->prune) {
+        // whole blocks decided from their min / max; only the tiles a window edge cuts through reach the filter kernel
+        CUDA_TRY(cudaMemsetAsync(db->d_work.p, 0, 4, db->stream));
+        CUDA_TRY(launch_blocks_prune(pr->pp, t.d_row_start, nblocks, ntiles, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
+                                     (unsigned int*)db->d_work.p, db->num_sms, db->stream, grp_sum));
+        note_launch(db, launches, "blocks_prune");
+    }
+    int filter_grid = pr->grid;
+    if (pr->block_filter != BlockFilter::kMini) {  // CTA tiles of 32 blocks (quad), 32 blocks per warp (lane)
+        const int64_t per_cta = 32 * (lane ? pr->lane_warps : 1);
+        filter_grid = (int)std::max<int64_t>(1, std::min<int64_t>(pr->grid, (nblocks + per_cta - 1) / per_cta));
+    }
+    CUDA_TRY(launch_blocks_filter(sp, (uint32_t*)db->d_bitmap.p, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
+                                  (unsigned long long*)db->d_tile_off.p, db->d_ctrl, nblocks, filter_grid, pr->dyn_smem, pr->block_filter,
+                                  pr->lane_warps, work, db->stream, grp_sum));
+    note_launch(db, launches, lane ? "blocks_filter_lane/w=" + std::to_string(pr->lane_warps) + "/s=" + std::to_string(sp.stages)
+                                   : with_stages(pr->block_filter == BlockFilter::kQuad ? "blocks_filter_quad" : "blocks_filter", sp.stages));
+    return (scan && !sp.scan_inline) ? launch_scan_kernel(db, sp, ntiles, launches, true) : 0;
+}
+
+// kBlocks: [blocks_prune ->] block filter kernel -> group emit (lane kernel, one encoded column projected: every emit warp finds
+// its rows from the group sums, no scan), scan-emit (one encoded column projected: offset scan + emit in one small-footprint
+// kernel, resident while the filter kernel runs) or offset scan + block emit kernel.
+int launch_blocks(imm3_db* db, Prepared* pr, int64_t nblocks, Queued* q) {
+    ScanPlan& sp = pr->sp;
+    const int64_t ntiles = sp.ntiles;
+    const bool lane = pr->block_filter == BlockFilter::kLane;
     int rc;
-    if ((rc = ensure_buf(&db->d_bitmap, (size_t)(nblocks * 32 + 2) * 4))) return rc;
-    if ((rc = ensure_buf(&db->d_span_cnt, (size_t)(nblocks + 8 + 1024) * 4))) return rc;  // (+ whole 16-byte loads of a group's counts)
-    if ((rc = ensure_tile_scratch(db, ntiles))) return rc;
+    if ((rc = ensure_block_filter(db, pr, nblocks))) return rc;
     sp.scan_inline = (scan_inline_for(ntiles) && !(lane && pr->lane_warps < 8)) ? 1 : 0;  // (the inline scan is written for 8 warps)
     int fused_grid = 0;  // > 0: blocks_scan_emit_kernel
     int group_grid = 0, ngroups = 0;  // > 0: blocks_group_emit_kernel
@@ -1123,33 +1167,13 @@ int launch_blocks(imm3_db* db, Prepared* pr, int64_t nblocks, Queued* q) {
         }
     }
     uint32_t* const grp_sum = group_grid > 0 ? (uint32_t*)db->d_grp_sum.p : nullptr;
-    const unsigned int* work = nullptr;
-    if (pr->prune) {
-        if ((rc = ensure_buf(&db->d_work, (size_t)((nblocks + 7) / 8 + 2) * 4))) return rc;
-        work = (const unsigned int*)db->d_work.p;
-    }
     if ((rc = setup_phase_trace(db, sp, 1024))) return rc;
     CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
-    if (pr->prune) {
-        // whole blocks decided from their min / max; only the tiles a window edge cuts through reach the filter kernel
-        CUDA_TRY(cudaMemsetAsync(db->d_work.p, 0, 4, db->stream));
-        CUDA_TRY(launch_blocks_prune(pr->pp, t.d_row_start, nblocks, ntiles, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
-                                     (unsigned int*)db->d_work.p, db->num_sms, db->stream, grp_sum));
-        note_launch(db, q->launches, "blocks_prune");
-    }
-    int filter_grid = pr->grid;
-    if (pr->block_filter != BlockFilter::kMini) {  // CTA tiles of 32 blocks (quad), 32 blocks per warp (lane)
-        const int64_t per_cta = 32 * (lane ? pr->lane_warps : 1);
-        filter_grid = (int)std::max<int64_t>(1, std::min<int64_t>(pr->grid, (nblocks + per_cta - 1) / per_cta));
-    }
-    CUDA_TRY(launch_blocks_filter(sp, (uint32_t*)db->d_bitmap.p, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
-                                  (unsigned long long*)db->d_tile_off.p, db->d_ctrl, nblocks, filter_grid, pr->dyn_smem, pr->block_filter,
-                                  pr->lane_warps, work, db->stream, grp_sum));
-    note_launch(db, q->launches, lane ? "blocks_filter_lane/w=" + std::to_string(pr->lane_warps) + "/s=" + std::to_string(sp.stages)
-                                      : with_stages(pr->block_filter == BlockFilter::kQuad ? "blocks_filter_quad" : "blocks_filter", sp.stages));
+    const bool emit_scans = group_grid > 0 || fused_grid > 0;  // (these emit kernels find the offsets themselves)
+    if ((rc = launch_block_filter_front(db, pr, nblocks, q->launches, grp_sum, !emit_scans))) return rc;
     CtrlBlock* const pub = q->publish ? db->h_ctrl : nullptr;
     const unsigned long long pub_seq = q->publish ? q->pub_seq : 0;
-    if (group_grid > 0 || fused_grid > 0) {
+    if (emit_scans) {
         const bool pdl = !getenv("IMM3_NO_PDL");
         if ((rc = mark_mid(db, pdl, q))) return rc;
         if (group_grid > 0) {
@@ -1164,7 +1188,6 @@ int launch_blocks(imm3_db* db, Prepared* pr, int64_t nblocks, Queued* q) {
         }
         q->published = q->publish;
     } else {
-        if (!sp.scan_inline && (rc = launch_scan_kernel(db, sp, ntiles, q->launches, true))) return rc;
         const bool pdl = sp.nproj > 0 && !getenv("IMM3_NO_PDL");
         if ((rc = mark_mid(db, pdl, q))) return rc;
         if (sp.nproj > 0) {
@@ -1848,7 +1871,7 @@ namespace {
 // of the result buffer and queues the exchange and the merge behind them (k_comm.cuh agg_exchange_kernel, k_agg.cuh
 // agg_merge_kernel; DESIGN §4.3).  allow_sum_avg (imm3_query_agg_ext only) resolves Sum / Avg (DESIGN §4.4c).
 int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, const imm3_agg* aggs, int naggs, const char* const* group_cols,
-              int ngroup, bool global, bool allow_sum_avg, imm3_result** out) {
+              int ngroup, bool global, bool allow_sum_avg, bool encoded_filter, imm3_result** out) {
     const char* const fn = global ? "imm3_query_agg_global" : "imm3_query_agg";
     if (!db || !out || (naggs > 0 && !aggs) || (ngroup > 0 && !group_cols)) return fail(IMM3_ERR_INVALID_ARG, "%s: NULL argument", fn);
     // A sharded handle merges over the communicator; a single handle's partials are the global result already.
@@ -1942,11 +1965,17 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
     r->h_cols.resize((size_t)r->ncols);
     ap.naggs = plan_naggs;
     ap.ngroup = ngroup;
+    // A predicate on a sorted-int-codec column: the block filter front decides it (IMM3_AGG_ENCODED_FILTER only).
+    bool enc_filter = false;
     for (auto& f : pr.lp.filters)
-        if (is_pfor(t, f.col_idx))
-            return fail(IMM3_ERR_UNSUPPORTED, "aggregation with a predicate on a sorted-int-codec column (%s) is not supported yet", t.cols[(size_t)f.col_idx].meta.name.c_str());
-    // A MIN / MAX input or a group column in the sorted-int codec: agg_blocks_kernel decodes them block by block.
-    const bool on_blocks = !pfor_cols.empty();
+        if (is_pfor(t, f.col_idx)) {
+            if (!encoded_filter)
+                return fail(IMM3_ERR_UNSUPPORTED, "aggregation with a predicate on a sorted-int-codec column (%s) is not supported yet", t.cols[(size_t)f.col_idx].meta.name.c_str());
+            enc_filter = true;
+        }
+    // A MIN / MAX input or a group column in the sorted-int codec: agg_blocks_kernel decodes them block by block.  It also
+    // aggregates every block-space selection (blocks are not aligned to agg_kernel's 1024-row spans).
+    const bool on_blocks = !pfor_cols.empty() || enc_filter;
     if (pfor_cols.size() > (size_t)kMaxPforCols)
         return fail(IMM3_ERR_UNSUPPORTED, "aggregation decodes at most %d distinct sorted-int-codec columns, the query reads %zu", kMaxPforCols, pfor_cols.size());
     ap.table_slots = 1u << 16;
@@ -1964,8 +1993,13 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
         refusal = last_error();
         return 0;
     };
-    if (on_blocks && t.max_block_rows > 1024 &&
+    if (!pfor_cols.empty() && t.max_block_rows > 1024 &&
         (rc = refuse_slice(fail(IMM3_ERR_UNSUPPORTED, "aggregation over sorted-int-codec columns decodes blocks of at most 1024 rows, table %s has a block of %d",
+                                t.meta.name.c_str(), t.max_block_rows))))
+        return rc;
+    // (the single-pass kernel, which takes larger blocks, leaves no block-space selection behind)
+    if (enc_filter && refusal.empty() && t.max_block_rows > 1024 &&
+        (rc = refuse_slice(fail(IMM3_ERR_UNSUPPORTED, "aggregation with a predicate on a sorted-int-codec column filters blocks of at most 1024 rows, table %s has a block of %d",
                                 t.meta.name.c_str(), t.max_block_rows))))
         return rc;
     if ((rc = use_device(db))) return rc;
@@ -1974,12 +2008,28 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
     const bool merge = xchg && !pr.lp.always_empty;          // every rank of a connected handle takes part, an empty slice too
     bool local = !pr.lp.always_empty && t.nrows > 0 && refusal.empty();
     ScanPlan& sp = pr.sp;
-    if (local) {
+    if (local && enc_filter) {
+        // The block pipeline's filter front (DESIGN §4.4d): [blocks_prune ->] lane / quad / mini-block filter kernel [-> offset
+        // scan]; per block a count and - partially selected blocks only - 32 bitmap words, which agg_blocks_kernel<.., BS> reads.
+        int occ = 0;
+        if ((rc = plan_columns(db, &pr))) return rc;
+        pr.pipeline = Pipeline::kBlocks;  // (IMM3_PATH=fused and IMM3_NO_HYBRID choose Project pipelines only)
+        choose_block_filter(&pr);
+        sp.ntiles = (t.nblocks + 7) / 8;  // the offset scan works on tiles of 8 blocks
+        size_block_filter(&pr);
+        size_prune(&pr);
+        CUDA_TRY(blocks_filter_occupancy(pr.dyn_smem, pr.block_filter, pr.lane_warps, &occ));
+        if ((rc = plan_grid(db, &pr, occ)) || (rc = ensure_block_filter(db, &pr, t.nblocks))) return rc;
+        sp.scan_inline = (scan_inline_for(sp.ntiles) && !(pr.block_filter == BlockFilter::kLane && pr.lane_warps < 8)) ? 1 : 0;  // (as launch_blocks)
+    } else if (local) {
         // The filter runs in row space exactly as for a Project query without a select list (dense filter kernel: bitmap,
         // span counts, total); the aggregation kernel is queued behind it, one synchronisation for the whole query.
         int occ = 0;
         if ((rc = plan_columns(db, &pr)) || (rc = size_dense_filter(db, &pr, &occ)) || (rc = plan_grid(db, &pr, occ)) || (rc = ensure_row_space(db, sp)))
             return rc;
+        sp.scan_inline = 1;  // (only the total matters here; the last CTA's scan provides it)
+    }
+    if (local) {
         ap.nrows = t.nrows;
         ap.ntiles = sp.ntiles;
         for (int g = 0; g < ngroup; g++) ap.group[g].base = t.cols[(size_t)gidx[(size_t)g]].d_arena;
@@ -2008,7 +2058,6 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
                 local = false;
             }
         }
-        sp.scan_inline = 1;  // (only the total matters here; the last CTA's scan provides it)
     }
     if (local || merge) {
         if ((rc = ensure_buf(&db->d_agg_table, (size_t)ap.table_slots * sizeof(AggEntry)))) return rc;
@@ -2025,20 +2074,31 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
         CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
         if (local) {
             CUDA_TRY(launch_agg_init((AggEntry*)db->d_agg_table.p, ap.table_slots, ap, counters, db->stream));
-            CUDA_TRY(launch_filter(sp, (uint32_t*)db->d_bitmap.p, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
-                                   (unsigned long long*)db->d_tile_off.p, db->d_ctrl, pr.grid, pr.dyn_smem, db->stream));
+            std::string front;  // the filter's part of the route
+            int front_launches = 1;
+            if (enc_filter) {
+                db->route.clear();
+                db->route_tag = "";
+                front_launches = 0;
+                if ((rc = launch_block_filter_front(db, &pr, t.nblocks, &front_launches, nullptr, true))) return rc;
+                front = db->route;
+            } else {
+                CUDA_TRY(launch_filter(sp, (uint32_t*)db->d_bitmap.p, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
+                                       (unsigned long long*)db->d_tile_off.p, db->d_ctrl, pr.grid, pr.dyn_smem, db->stream));
+                front = filter_route(sp);
+            }
             if (on_blocks)
                 CUDA_TRY(launch_agg_blocks(ap, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, (AggEntry*)db->d_agg_table.p,
-                                           local_out, counters, db->d_ctrl, db->num_sms, db->stream));
+                                           local_out, counters, db->d_ctrl, db->num_sms, db->stream, enc_filter));
             else
                 CUDA_TRY(launch_agg(ap, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, (AggEntry*)db->d_agg_table.p,
                                     local_out, counters, db->d_ctrl, db->num_sms, db->stream));
-            r->launches = 4;
+            r->launches = 3 + front_launches;
             // the instantiation IMM3_AGG_DISPATCH (kernels.cu) picks: <= 2 group-by columns exact, else 4; 1 .. 4 aggregates exact, else 8;
-            // "/sum": the SUM instantiation
+            // "/sum": the SUM instantiation; "/bsel": agg_blocks_kernel over the block filter's selection
             const int ng = ngroup <= 2 ? ngroup : 4, na = (plan_naggs >= 1 && plan_naggs <= 4) ? plan_naggs : 8;
-            const std::string inst = "<" + std::to_string(ng) + "," + std::to_string(na) + ">" + (has_sum ? "/sum" : "");
-            r->route = "agg_init;" + filter_route(sp) + ";" + (on_blocks ? "agg_blocks" : "agg") + inst + ";agg_compact";
+            const std::string inst = "<" + std::to_string(ng) + "," + std::to_string(na) + ">" + (has_sum ? "/sum" : "") + (enc_filter ? "/bsel" : "");
+            r->route = "agg_init;" + front + ";" + (on_blocks ? "agg_blocks" : "agg") + inst + ";agg_compact";
         }
         if (merge) {
             AggXPlan xp;
@@ -2100,9 +2160,17 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
     if (local) {
         // algorithmic bytes: filter columns once + every decoded encoded column once (its words and 4 B of word offsets per
         // block) + per selected row the cells of the dense group and aggregate columns (MIN / MAX / SUM / AVG inputs)
+        // (with a predicate on an encoded column: every filter column once, and an encoded column that is filtered and
+        // decoded once - its words once, plus the word offsets the decode reads)
         int64_t bytes = 0, per_row = 0;
-        for (auto& f2 : pr.lp.filters) bytes += t.cols[(size_t)f2.col_idx].encoded_bytes;
-        for (int ci : pfor_cols) bytes += t.cols[(size_t)ci].encoded_bytes + 4 * (int64_t)t.nblocks;
+        std::vector<int> counted;
+        auto seen = [&](int ci) { return std::find(counted.begin(), counted.end(), ci) != counted.end(); };
+        for (auto& f2 : pr.lp.filters) {
+            if (enc_filter && seen(f2.col_idx)) continue;
+            counted.push_back(f2.col_idx);
+            bytes += t.cols[(size_t)f2.col_idx].encoded_bytes;
+        }
+        for (int ci : pfor_cols) bytes += (seen(ci) ? 0 : t.cols[(size_t)ci].encoded_bytes) + 4 * (int64_t)t.nblocks;
         for (int g = 0; g < ngroup; g++)
             if (ap.group_pfor[g] < 0) per_row += t.cols[(size_t)gidx[(size_t)g]].meta.width;
         for (int a = 0; a < naggs; a++)
@@ -2156,18 +2224,19 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
 
 int imm3_query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, const imm3_agg* aggs, int naggs,
                    const char* const* group_cols, int ngroup, imm3_result** out) {
-    return query_agg(db, table, preds, npreds, aggs, naggs, group_cols, ngroup, false, false, out);
+    return query_agg(db, table, preds, npreds, aggs, naggs, group_cols, ngroup, false, false, false, out);
 }
 
 int imm3_query_agg_global(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, const imm3_agg* aggs, int naggs,
                           const char* const* group_cols, int ngroup, imm3_result** out) {
-    return query_agg(db, table, preds, npreds, aggs, naggs, group_cols, ngroup, true, false, out);
+    return query_agg(db, table, preds, npreds, aggs, naggs, group_cols, ngroup, true, false, false, out);
 }
 
 int imm3_query_agg_ext(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, const imm3_agg* aggs, int naggs,
                        const char* const* group_cols, int ngroup, uint32_t flags, imm3_result** out) {
-    if (flags & ~IMM3_AGG_GLOBAL) return fail(IMM3_ERR_INVALID_ARG, "imm3_query_agg_ext: unknown flag bits 0x%x", flags & ~IMM3_AGG_GLOBAL);
-    return query_agg(db, table, preds, npreds, aggs, naggs, group_cols, ngroup, (flags & IMM3_AGG_GLOBAL) != 0, true, out);
+    const uint32_t known = IMM3_AGG_GLOBAL | IMM3_AGG_ENCODED_FILTER;
+    if (flags & ~known) return fail(IMM3_ERR_INVALID_ARG, "imm3_query_agg_ext: unknown flag bits 0x%x", flags & ~known);
+    return query_agg(db, table, preds, npreds, aggs, naggs, group_cols, ngroup, (flags & IMM3_AGG_GLOBAL) != 0, true, (flags & IMM3_AGG_ENCODED_FILTER) != 0, out);
 }
 
 int imm3_query_sql(imm3_db* db, const char* sql, imm3_result** out) {

@@ -491,7 +491,11 @@ __host__ __device__ constexpr int agg_blocks_warp_words(int npfor, int words_cap
 constexpr size_t agg_blocks_state_bytes(int na, int nsum = 0) { return agg_smem_bytes(na, nsum) - (size_t)kComputeWarps * 1024 * 2; }
 
 // S = true: the SUM instantiations, as agg_kernel's.
-template <int NG, int NA, bool S>
+// BS = true: the selection is the BLOCK filter's output (imm3_query_agg_ext with IMM3_AGG_ENCODED_FILTER, DESIGN §4.4d):
+// `bitmap` = 32 words per block (bit r of block b = row R0 + r), `span_cnt` = the selected rows per block (blk_cnt).  A block
+// is a candidate iff its count is not 0; its words are read only if 0 < count < rows (blocks_prune_kernel and the filter
+// kernels write no words for an empty or a fully selected block: those words are stale from earlier queries).
+template <int NG, int NA, bool S, bool BS>
 __global__ void __launch_bounds__(kComputeThreads, 2) agg_blocks_kernel(const __grid_constant__ AggPlan A, const uint32_t* __restrict__ bitmap,
                                                                          const uint32_t* __restrict__ span_cnt, AggEntry* __restrict__ table,
                                                                          unsigned int* __restrict__ overflow, const ScanCtrl* ctrl) {
@@ -529,6 +533,7 @@ __global__ void __launch_bounds__(kComputeThreads, 2) agg_blocks_kernel(const __
         if (b < nblocks) {
             if (lane < 2) m = A.row_start[b + lane];
             else if (lane < 2 + 2 * npfor) m = s_pfor[(lane - 2) >> 1].word_off[b + (lane & 1)];
+            else if (BS && lane == 31) m = __ldcg(span_cnt + b);  // (BS: the block's count; 2 + 2 * kMaxPforCols < 31)
         }
         return m;
     };
@@ -538,9 +543,17 @@ __global__ void __launch_bounds__(kComputeThreads, 2) agg_blocks_kernel(const __
     auto handle = [&](long long blk, unsigned long long meta) {
         const long long R0 = (long long)__shfl_sync(0xFFFFFFFFu, meta, 0);
         const int n = (int)((long long)__shfl_sync(0xFFFFFFFFu, meta, 1) - R0);
-        const long long bit0 = R0 + 32 * lane;
-        const uint32_t lo = __ldg(bitmap + (bit0 >> 5)), hi = __ldg(bitmap + (bit0 >> 5) + 1);
-        uint32_t myword = __funnelshift_r(lo, hi, (uint32_t)(bit0 & 31));
+        uint32_t myword;
+        if constexpr (BS) {
+            // the block's count (lane 31 of the metadata): all rows, or its own 32 words
+            const unsigned bc = (unsigned)__shfl_sync(0xFFFFFFFFu, meta, 31);
+            IMM3_CHECK(ctrl, bc <= (unsigned)n, 10);
+            myword = bc == (unsigned)n ? 0xFFFFFFFFu : __ldg(bitmap + blk * 32 + lane);
+        } else {
+            const long long bit0 = R0 + 32 * lane;
+            const uint32_t lo = __ldg(bitmap + (bit0 >> 5)), hi = __ldg(bitmap + (bit0 >> 5) + 1);
+            myword = __funnelshift_r(lo, hi, (uint32_t)(bit0 & 31));
+        }
         const int left = n - lane * 32;
         myword &= left >= 32 ? 0xFFFFFFFFu : (left <= 0 ? 0u : ((1u << left) - 1u));
         if (__ballot_sync(0xFFFFFFFFu, myword != 0u) == 0u) return;
@@ -620,16 +633,19 @@ __global__ void __launch_bounds__(kComputeThreads, 2) agg_blocks_kernel(const __
 
     asm volatile("griddepcontrol.wait;" ::: "memory");  // (a no-op unless launched as a programmatic dependent)
     // 32 of the warp's blocks at a time, a lane each.  Fewer selected rows than blocks (most blocks empty): a lane tests its
-    // block through the counts of the (at most two) 1024-row spans it overlaps; otherwise every block is a candidate.  The
-    // warp then handles the candidates in order, the next one's metadata in flight.  (One call site of `handle`: with two,
-    // the compiler keeps it as a called function and the row loop's arrays in local memory.)
+    // block through the counts of the (at most two) 1024-row spans it overlaps; otherwise every block is a candidate.  (BS:
+    // a block is a candidate iff its own count is not 0 - one coalesced load per lane.)  The warp then handles the
+    // candidates in order, the next one's metadata in flight.  (One call site of `handle`: with two, the compiler keeps it
+    // as a called function and the row loop's arrays in local memory.)
     const unsigned long long total = __ldcg(&ctrl->total);
     const bool sparse = total < (unsigned long long)nblocks;
 #pragma unroll 1
     for (long long b0 = warp0; total != 0ull && b0 < nblocks; b0 += 32 * nwarps) {
         const long long b = b0 + lane * nwarps;
         bool cand = b < nblocks;
-        if (cand && sparse) {
+        if (BS) {
+            if (cand) cand = __ldcg(span_cnt + b) != 0u;
+        } else if (cand && sparse) {
             const unsigned long long r0 = A.row_start[b], r1 = A.row_start[b + 1];
             const long long q0 = (long long)(r0 >> 10), q1 = (long long)((r1 - 1) >> 10);
             const unsigned c = __ldg(span_cnt + q0) + (q1 != q0 ? __ldg(span_cnt + q1) : 0u);

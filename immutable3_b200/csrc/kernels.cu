@@ -201,7 +201,7 @@ cudaError_t launch_agg_init(AggEntry* table, uint32_t slots, const AggPlan& a, u
 }
 template <int NG, int NA, bool S>
 static cudaError_t launch_agg_as(const AggPlan& a, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, unsigned int* overflow,
-                                 const ScanCtrl* ctrl, int num_sms, cudaStream_t stream) {
+                                 const ScanCtrl* ctrl, int num_sms, cudaStream_t stream, bool /*bsel: agg_blocks_kernel only*/) {
     auto* const kern = agg_kernel<NG, NA, S>;
     const size_t smem = agg_smem_bytes(NA, S ? agg_nsum(a) : 0);
     cudaError_t e = cudaSuccess;
@@ -217,7 +217,8 @@ static cudaError_t launch_agg_as(const AggPlan& a, const uint32_t* bitmap, const
     return cudaGetLastError();
 }
 // the instantiation for this query's shape: exact for <= 2 group-by columns and 1 .. 4 aggregates, the general forms beyond;
-// a plan with a SUM takes the SUM instantiations (it carries a COUNT too: 2 .. 4 aggregates exact, else 8)
+// a plan with a SUM takes the SUM instantiations (it carries a COUNT too: 2 .. 4 aggregates exact, else 8); `bsel` picks
+// agg_blocks_kernel's block-space-selection instantiations
 #define IMM3_AGG_DISPATCH(LAUNCH)                                                                                                         \
     do {                                                                                                                                  \
         const int ng = a.ngroup <= 2 ? a.ngroup : 4, na = (a.naggs >= 1 && a.naggs <= 4) ? a.naggs : 8;                                   \
@@ -229,23 +230,24 @@ static cudaError_t launch_agg_as(const AggPlan& a, const uint32_t* bitmap, const
     } while (0)
 #define IMM3_AGG_DISPATCH_ROW(LAUNCH, NG)                                                                                                  \
     if (ng == NG) {                                                                                                                       \
-        if (na == 1) e = LAUNCH<NG, 1, false>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                           \
-        else if (na == 2) e = LAUNCH<NG, 2, false>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                      \
-        else if (na == 3) e = LAUNCH<NG, 3, false>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                      \
-        else if (na == 4) e = LAUNCH<NG, 4, false>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                      \
-        else e = LAUNCH<NG, 8, false>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                                   \
+        if (na == 1) e = LAUNCH<NG, 1, false>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream, bsel);                     \
+        else if (na == 2) e = LAUNCH<NG, 2, false>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream, bsel);                \
+        else if (na == 3) e = LAUNCH<NG, 3, false>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream, bsel);                \
+        else if (na == 4) e = LAUNCH<NG, 4, false>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream, bsel);                \
+        else e = LAUNCH<NG, 8, false>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream, bsel);                             \
     }
 #define IMM3_AGG_SUM_ROW(LAUNCH, NG)                                                                                                       \
     if (ng == NG) {                                                                                                                       \
-        if (na <= 2) e = LAUNCH<NG, 2, true>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                            \
-        else if (na == 3) e = LAUNCH<NG, 3, true>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                       \
-        else if (na == 4) e = LAUNCH<NG, 4, true>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                       \
-        else e = LAUNCH<NG, 8, true>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream);                                    \
+        if (na <= 2) e = LAUNCH<NG, 2, true>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream, bsel);                      \
+        else if (na == 3) e = LAUNCH<NG, 3, true>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream, bsel);                 \
+        else if (na == 4) e = LAUNCH<NG, 4, true>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream, bsel);                 \
+        else e = LAUNCH<NG, 8, true>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream, bsel);                              \
     }
 cudaError_t launch_agg(const AggPlan& a, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, AggEntry* out, unsigned int* counters,
                        const ScanCtrl* ctrl, int num_sms, cudaStream_t stream) {
     cudaError_t e = configure_once();
     if (e != cudaSuccess) return e;
+    const bool bsel = false;
     IMM3_AGG_DISPATCH(launch_agg_as);
     if (e != cudaSuccess) return e;
     agg_compact_kernel<<<(a.table_slots + kComputeThreads - 1) / kComputeThreads, kComputeThreads, 0, stream>>>(table, a.table_slots, out, counters);
@@ -259,8 +261,8 @@ size_t agg_blocks_smem_bytes(int naggs, int npfor, int words_cap, int nsum) {
 }
 template <int NG, int NA, bool S>
 static cudaError_t launch_agg_blocks_as(const AggPlan& a, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, unsigned int* overflow,
-                                        const ScanCtrl* ctrl, int num_sms, cudaStream_t stream) {
-    auto* const kern = agg_blocks_kernel<NG, NA, S>;
+                                        const ScanCtrl* ctrl, int num_sms, cudaStream_t stream, bool bsel) {
+    auto* const kern = bsel ? agg_blocks_kernel<NG, NA, S, true> : agg_blocks_kernel<NG, NA, S, false>;
     const size_t smem = agg_blocks_smem_bytes(NA, a.npfor, a.blk_words_cap, S ? agg_nsum(a) : 0);
     cudaError_t e = cudaSuccess;
     if (smem > 48 * 1024 && (e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
@@ -273,7 +275,7 @@ static cudaError_t launch_agg_blocks_as(const AggPlan& a, const uint32_t* bitmap
     return cudaGetLastError();
 }
 cudaError_t launch_agg_blocks(const AggPlan& a, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, AggEntry* out, unsigned int* counters,
-                              const ScanCtrl* ctrl, int num_sms, cudaStream_t stream) {
+                              const ScanCtrl* ctrl, int num_sms, cudaStream_t stream, bool bsel) {
     cudaError_t e = configure_once();
     if (e != cudaSuccess) return e;
     IMM3_AGG_DISPATCH(launch_agg_blocks_as);
@@ -397,16 +399,18 @@ size_t blocks_filter_smem_bytes(int nstaged, int tile_cap_bytes, int ring) { ret
 int blocks_filter_slot_bytes(int nstaged, int tile_cap_bytes) { return blk_filter_slot_bytes(nstaged, tile_cap_bytes); }
 size_t blocks_emit_smem_bytes(int npfor, int words_cap) { return (size_t)kComputeWarps * blk_emit_warp_words(npfor, words_cap) * 4; }
 int blocks_filter_quad_slot_bytes(int tile_cap_bytes) { return kQuadHdrBytes + tile_cap_bytes; }
+cudaError_t blocks_filter_occupancy(size_t filter_smem, BlockFilter filter, int lane_warps, int* blocks_per_sm) {
+    cudaError_t e = configure_once();
+    if (e != cudaSuccess) return e;
+    return filter == BlockFilter::kLane   ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, blocks_filter_lane_kernel, lane_warps * 32, filter_smem)
+           : filter == BlockFilter::kQuad ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, blocks_filter_quad_kernel, kComputeThreads + 32, filter_smem)
+                                          : cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, blocks_filter_kernel, kComputeThreads + 32, filter_smem);
+}
 cudaError_t blocks_multi_occupancy(size_t filter_smem, size_t emit_smem, int* filter_blocks_per_sm, int* emit_blocks_per_sm, BlockFilter filter,
                                    int lane_warps, bool rowspace) {
     cudaError_t e = configure_once();
     if (e != cudaSuccess) return e;
-    if (filter_blocks_per_sm) {
-        e = filter == BlockFilter::kLane   ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(filter_blocks_per_sm, blocks_filter_lane_kernel, lane_warps * 32, filter_smem)
-            : filter == BlockFilter::kQuad ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(filter_blocks_per_sm, blocks_filter_quad_kernel, kComputeThreads + 32, filter_smem)
-                                           : cudaOccupancyMaxActiveBlocksPerMultiprocessor(filter_blocks_per_sm, blocks_filter_kernel, kComputeThreads + 32, filter_smem);
-        if (e != cudaSuccess) return e;
-    }
+    if (filter_blocks_per_sm && (e = blocks_filter_occupancy(filter_smem, filter, lane_warps, filter_blocks_per_sm)) != cudaSuccess) return e;
     if (rowspace) return cudaOccupancyMaxActiveBlocksPerMultiprocessor(emit_blocks_per_sm, blocks_emit_kernel<true>, kComputeThreads, emit_smem);
     return cudaOccupancyMaxActiveBlocksPerMultiprocessor(emit_blocks_per_sm, blocks_emit_kernel<false>, kComputeThreads, emit_smem);
 }

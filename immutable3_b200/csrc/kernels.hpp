@@ -27,8 +27,9 @@ cudaError_t launch_agg_init(AggEntry* table, uint32_t slots, const AggPlan& a, u
 cudaError_t launch_agg(const AggPlan& a, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, AggEntry* out, unsigned int* counters,
                        const ScanCtrl* ctrl, int num_sms, cudaStream_t stream);
 size_t agg_blocks_smem_bytes(int naggs, int npfor, int words_cap, int nsum = 0);  // dynamic shared memory of agg_blocks_kernel (nsum SUMs: agg_blocks_sum_kernel)
+// bsel: bitmap / span_cnt are the block filter's output (32 words and one count per block), not the row-space filter's
 cudaError_t launch_agg_blocks(const AggPlan& a, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, AggEntry* out, unsigned int* counters,
-                              const ScanCtrl* ctrl, int num_sms, cudaStream_t stream);
+                              const ScanCtrl* ctrl, int num_sms, cudaStream_t stream, bool bsel = false);
 long long scan_inline_max_tiles();
 cudaError_t launch_offset_scan(const uint32_t* tile_cnt, unsigned long long* tile_off, long long ntiles, long long limit, uint32_t epoch,
                                unsigned long long* partials, ScanCtrl* ctrl, unsigned int* tile_list, cudaStream_t stream);
@@ -50,6 +51,7 @@ int blocks_filter_quad_slot_bytes(int tile_cap_bytes);
 // The block filter kernels: lane = mini-block (blocks_filter_kernel), quad (blocks_filter_quad_kernel), lane = block
 // (blocks_filter_lane_kernel, lane_warps warps per CTA).
 enum class BlockFilter { kMini, kQuad, kLane };
+cudaError_t blocks_filter_occupancy(size_t filter_smem, BlockFilter filter, int lane_warps, int* blocks_per_sm);
 cudaError_t blocks_multi_occupancy(size_t filter_smem, size_t emit_smem, int* filter_blocks_per_sm, int* emit_blocks_per_sm, BlockFilter filter,
                                    int lane_warps, bool rowspace);
 cudaError_t launch_blocks_filter(const ScanPlan& plan, uint32_t* bitmapB, uint32_t* blk_cnt, uint32_t* tile_cnt, unsigned long long* tile_off,

@@ -109,9 +109,9 @@ class CudaExecutor:
     def __init__(self, engine: Engine):
         self.engine = engine
 
-    def begin(self, query: Query, sum_avg: bool = False) -> Result:
-        if sum_avg:
-            return self.engine.begin(query, sum_avg=True)
+    def begin(self, query: Query, sum_avg: bool = False, encoded_filter: bool = False) -> Result:
+        if sum_avg or encoded_filter:
+            return self.engine.begin(query, sum_avg=sum_avg, encoded_filter=encoded_filter)
         return self.engine.begin(query)
 
     def finish(self, handle: Result, take: int) -> List[np.ndarray]:
@@ -162,24 +162,27 @@ class ShardedEngine:
         ms = float(getattr(h, "device_ms", 0.0))
         return ShardResult(self.rank, self.world, counts, offsets[self.rank], takes[self.rank], sum(takes), cols, ms)
 
-    def execute_agg(self, query: Query, sum_avg: bool = False) -> ShardResult:
+    def execute_agg(self, query: Query, sum_avg: bool = False, encoded_filter: bool = False) -> ShardResult:
         """A ProjectAgg query over the whole table, the same groups on every rank: `columns` = the global groups,
         `counts` = every rank's partial group count, offset 0, take = total = the number of global groups.  On a
         connected handle the GPUs merge the partials themselves (imm3_query_agg_global); otherwise every rank's partial
         columns are all-gathered through torch.distributed and merged on the host in rank order (`merge_partials`).
         `sum_avg=True` resolves Sum / Avg (imm3_query_agg_ext; on the host path each rank computes Avg as a Sum and a
-        Count, `sum_avg_partials`, and the merged sums are divided once, `finish_sum_avg`)."""
+        Count, `sum_avg_partials`, and the merged sums are divided once, `finish_sum_avg`).  `encoded_filter=True` accepts
+        predicates on sorted-int-codec columns (IMM3_AGG_ENCODED_FILTER, on the GPU merge and on every rank's partial query of
+        the host merge alike)."""
         engine = getattr(self.executor, "engine", None)
         if getattr(getattr(engine, "sm", None), "comm_connected", False):
-            with engine.execute_agg_global(query, sum_avg=sum_avg) as h:
+            with engine.execute_agg_global(query, sum_avg=sum_avg, encoded_filter=encoded_filter) as h:
                 cols = h.columns()
                 return ShardResult(self.rank, self.world, h.rank_counts, 0, h.nrows, h.nrows, cols, float(h.device_ms))
         aggs, ngroup = list(query.project.aggs), len(query.project.groupBy)
+        kw = {"encoded_filter": True} if encoded_filter else {}
         if sum_avg:
             plan, count = sum_avg_partials(aggs)
-            h = self.executor.begin(Query(query.table, query.select, ProjectAgg(plan, query.project.groupBy)), sum_avg=True)
+            h = self.executor.begin(Query(query.table, query.select, ProjectAgg(plan, query.project.groupBy)), sum_avg=True, **kw)
         else:
-            h = self.executor.begin(query)  # this rank's partial groups
+            h = self.executor.begin(query, **kw)  # this rank's partial groups
         mine = self.executor.finish(h, int(h.local_count))
         everyone = [None] * self.world
         self.dist.all_gather_object(everyone, mine, group=self.group)

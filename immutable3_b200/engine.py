@@ -102,6 +102,10 @@ class Project:
 # (Engine.scala:153): by default they come back as IMM3_ERR_UNSUPPORTED, as there.  `sum_avg=True` (Engine.execute,
 # execute_agg_global, ShardedEngine.execute_agg) resolves them through imm3_query_agg_ext: Sum = the exact int64 sum,
 # Avg = float64(sum) / float64(count).
+# A predicate on a sorted-int-codec column in a ProjectAgg query is refused (IMM3_ERR_UNSUPPORTED) unless
+# `encoded_filter=True` (the same methods), which sets IMM3_AGG_ENCODED_FILTER on imm3_query_agg_ext: the block filter
+# kernels decide such predicates and the aggregation reads their per-block selection.  The two keywords are independent:
+# `encoded_filter=True` alone still refuses Sum / Avg as the parity path does.
 @dataclass(frozen=True)
 class Sum:
     col: str
@@ -529,21 +533,22 @@ class Engine:
         L.check(self._lib.imm3_query_begin(self.sm.handle, p[0], p[1], p[2], p[3], p[4], p[5], C.byref(out)))
         return Result(out, self._lib, self.sm)
 
-    def execute(self, query: Query, real_or: bool = False, sum_avg: bool = False) -> Result:
+    def execute(self, query: Query, real_or: bool = False, sum_avg: bool = False, encoded_filter: bool = False) -> Result:
         """Engine.execute: the rows of the query in canonical order (iterate for Row objects).  `real_or=True` evaluates
         Or as a disjunction (imm3_query_begin_dnf) instead of the reference's Or == And (Engine.scala:236-245).
-        `sum_avg=True` resolves Sum / Avg in a ProjectAgg query (imm3_query_agg_ext), which the reference refuses."""
+        `sum_avg=True` resolves Sum / Avg in a ProjectAgg query (imm3_query_agg_ext), which the reference refuses.
+        `encoded_filter=True` accepts predicates on sorted-int-codec columns in a ProjectAgg query (IMM3_AGG_ENCODED_FILTER)."""
         if isinstance(query.project, ProjectAgg):
-            return self._call_agg(query, sum_avg=sum_avg)
+            return self._call_agg(query, sum_avg=sum_avg, encoded_filter=encoded_filter)
         if real_or:
             r = self.begin(query, real_or=True)
             return r.fetch(r.take)
         return self._call(self._lib.imm3_query, query)
 
-    def begin(self, query: Query, real_or: bool = False, sum_avg: bool = False) -> Result:
+    def begin(self, query: Query, real_or: bool = False, sum_avg: bool = False, encoded_filter: bool = False) -> Result:
         """First phase of a sharded query: kernels done, local match count known, nothing fetched."""
         if isinstance(query.project, ProjectAgg):
-            return self._call_agg(query, sum_avg=sum_avg)
+            return self._call_agg(query, sum_avg=sum_avg, encoded_filter=encoded_filter)
         if real_or:
             return self._call_dnf(query)
         return self._call(self._lib.imm3_query_begin, query)
@@ -561,13 +566,14 @@ class Engine:
         del keep
         return Result(out, self._lib, self.sm)
 
-    def execute_agg_global(self, query: Query, sum_avg: bool = False) -> Result:
+    def execute_agg_global(self, query: Query, sum_avg: bool = False, encoded_filter: bool = False) -> Result:
         """A ProjectAgg query over the WHOLE table on every rank of a sharded handle (imm3_query_agg_global): the ranks'
         partial groups are merged on the GPUs over the communicator (`SegmentManager.comm_connect`).  On a single handle the
-        result is that of `execute`; an unconnected sharded handle raises (IMM3_ERR_STATE).  `sum_avg` as in `execute`."""
-        return self._call_agg(query, glob=True, sum_avg=sum_avg)
+        result is that of `execute`; an unconnected sharded handle raises (IMM3_ERR_STATE).  `sum_avg` and
+        `encoded_filter` as in `execute`."""
+        return self._call_agg(query, glob=True, sum_avg=sum_avg, encoded_filter=encoded_filter)
 
-    def _call_agg(self, query: Query, glob: bool = False, sum_avg: bool = False) -> Result:
+    def _call_agg(self, query: Query, glob: bool = False, sum_avg: bool = False, encoded_filter: bool = False) -> Result:
         """Engine.execute, ProjectAgg branch (Engine.scala:200-232): one row per group, group columns then aggregates."""
         if not isinstance(query.project, ProjectAgg):
             raise L.Imm3Error(L.ERR_UNSUPPORTED, "not a ProjectAgg query")
@@ -580,8 +586,12 @@ class Engine:
         groups = L.cstr_array(list(query.project.groupBy))
         out = C.c_void_p()
         args = (self.sm.handle, query.table.encode(), preds, npreds, arr, len(aggs), C.cast(groups, C.POINTER(C.c_char_p)), len(query.project.groupBy))
-        if sum_avg:
-            L.check(self._lib.imm3_query_agg_ext(*args, L.AGG_FLAG_GLOBAL if glob else 0, C.byref(out)))
+        if encoded_filter and not sum_avg and any(isinstance(a, (Sum, Avg)) for a in aggs):
+            # (imm3_query_agg_ext would resolve them: refuse them as the parity path does, so that the keywords stay independent)
+            raise L.Imm3Error(L.ERR_UNSUPPORTED, "Unknown Aggregate type (Engine.scala:153: only Min, Max and Count are resolved)")
+        if sum_avg or encoded_filter:
+            flags = (L.AGG_FLAG_GLOBAL if glob else 0) | (L.AGG_FLAG_ENCODED_FILTER if encoded_filter else 0)
+            L.check(self._lib.imm3_query_agg_ext(*args, flags, C.byref(out)))
         else:
             L.check((self._lib.imm3_query_agg_global if glob else self._lib.imm3_query_agg)(*args, C.byref(out)))
         del keep

@@ -207,7 +207,7 @@ int imm3_result_wait(imm3_result* r);
  * Library limits (IMM3_ERR_UNSUPPORTED): group cells must pack into 7 bytes (a sorted-int-codec INT cell takes 4); aggregate
  * and group columns may be dense or sorted-int-codec (PFOR_INT), but one query decodes at most 4 distinct sorted-int-codec
  * columns, from blocks of at most 1024 rows; predicates on a sorted-int-codec column cannot be combined with aggregation
- * yet.  On a sharded handle the result holds
+ * here (imm3_query_agg_ext with IMM3_AGG_ENCODED_FILTER accepts them).  On a sharded handle the result holds
  * this rank's groups (partials); imm3_query_agg_global below merges them on the GPUs. */
 typedef enum imm3_agg_op { IMM3_AGG_COUNT = 0, IMM3_AGG_MIN = 1, IMM3_AGG_MAX = 2, IMM3_AGG_SUM = 3, IMM3_AGG_AVG = 4 } imm3_agg_op;
 typedef struct imm3_agg {
@@ -241,8 +241,16 @@ int imm3_query_agg_global(imm3_db* db, const char* table, const imm3_pred* preds
  * rows: its own first Count, else a hidden one that is not in the result; visible plus hidden aggregates must be at most
  * 8 (else IMM3_ERR_UNSUPPORTED).  Every add, on the GPU and in the merge, is a 64-bit two's-complement add, so a sum is
  * exact whenever its group has at most 2^32 rows; a group with more rows (on a global aggregate: after the merge)
- * returns IMM3_ERR_UNSUPPORTED, never a wrapped value. */
+ * returns IMM3_ERR_UNSUPPORTED, never a wrapped value.
+ * IMM3_AGG_ENCODED_FILTER: predicates on sorted-int-codec (PFOR_INT) columns are accepted - ranges (GT / LT / EQ), alone or
+ * mixed with predicates on dense columns - and decided by the block pipeline's filter kernels (blocks pruned from their
+ * min / max statistics where every predicate is such a range), whose per-block selection the aggregation kernel reads;
+ * the route then ends in agg_blocks<NG,NA>/bsel.  The table's blocks must hold at most 1024 rows (else
+ * IMM3_ERR_UNSUPPORTED).  A query with no predicate on an encoded column is unaffected by the flag: the same rows, names,
+ * types, route, status and message.  Combines with IMM3_AGG_GLOBAL and with Sum / Avg.  Without the flag (and in the two
+ * entry points above) such predicates keep giving IMM3_ERR_UNSUPPORTED. */
 #define IMM3_AGG_GLOBAL 0x1u
+#define IMM3_AGG_ENCODED_FILTER 0x4u
 int imm3_query_agg_ext(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, const imm3_agg* aggs, int naggs,
                        const char* const* group_cols, int ngroup, uint32_t flags, imm3_result** out);
 
@@ -265,7 +273,10 @@ int imm3_result_kernel_launches(const imm3_result* r);      /* kernels launched 
  * blocks_filter_quad, blocks_filter, blocks_group_emit, blocks_scan_emit, blocks_emit(rowspace|blocks), scan_blocks,
  * count_exchange, agg_init, agg<NG,NA>, agg_blocks<NG,NA>, agg_compact, agg_exchange, agg_merge) with "/key=value" parameters: /s= ring stages,
  * /w= warps per CTA of the lane kernel, /ctas= the group emit kernel's grid; "/prefix" marks the prefix pass of a small
- * LIMIT; "/sum" the SUM instantiation of agg<NG,NA> / agg_blocks<NG,NA> (imm3_query_agg_ext with a Sum or Avg).  E.g. "blocks_prune;blocks_filter_lane/w=11/s=2;blocks_group_emit/ctas=148"; a global aggregate on a connected
+ * LIMIT; "/sum" the SUM instantiation of agg<NG,NA> / agg_blocks<NG,NA> (imm3_query_agg_ext with a Sum or Avg); "/bsel" (after
+ * "/sum" when both) agg_blocks<NG,NA> over the block filter's selection (IMM3_AGG_ENCODED_FILTER with a predicate on an encoded
+ * column, whose filter kernels - blocks_prune, blocks_filter*, offset_scan - are recorded as for a Project query), e.g.
+ * "agg_init;blocks_prune;blocks_filter_lane/w=11/s=2;agg_blocks<1,3>/bsel;agg_compact".  E.g. "blocks_prune;blocks_filter_lane/w=11/s=2;blocks_group_emit/ctas=148"; a global aggregate on a connected
  * handle: "agg_init;filter(tma)/s=4;agg<1,2>;agg_compact;agg_exchange;agg_init;agg_merge;agg_compact" (a rank with an empty
  * slice starts at agg_exchange).  Owned by the result (valid until imm3_result_free). */
 const char* imm3_result_route(const imm3_result* r);
