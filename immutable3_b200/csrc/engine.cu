@@ -808,17 +808,26 @@ void size_prune(Prepared* pr) {
     if (ok) pr->prefix_blocks = 0;
 }
 
-// kRowSpace, kBlocks: the block emit kernel, and (kBlocks) the occupancy of the block filter kernel.
-int size_block_emit(imm3_db* db, Prepared* pr, int* occ) {
+// kBlocks, and aggregates over encoded predicates: the block filter front on tiles of 8 blocks (the offset scan's), its
+// filter kernel's ring and occupancy, and pruning.
+int size_block_front(Prepared* pr, int* occ) {
+    pr->sp.ntiles = (pr->table->nblocks + 7) / 8;
+    size_block_filter(pr);
+    size_prune(pr);
+    CUDA_TRY(blocks_filter_occupancy(pr->dyn_smem, pr->block_filter, pr->lane_warps, occ));
+    return 0;
+}
+
+// kRowSpace, kBlocks: the block emit kernel.
+int size_block_emit(imm3_db* db, Prepared* pr) {
     const TableStore& t = *pr->table;
     ScanPlan& sp = pr->sp;
     int64_t words = 0;
     for (int ci : pr->pfor_cols) words = std::max<int64_t>(words, t.cols[(size_t)ci].max_block_words);
     sp.blk_words_cap = block_words_cap(words);
     pr->blocks_emit_smem = blocks_emit_smem_bytes(sp.npfor, sp.blk_words_cap);
-    const bool rowspace = pr->pipeline == Pipeline::kRowSpace;
     int occ_e = 0;
-    CUDA_TRY(blocks_multi_occupancy(pr->dyn_smem, pr->blocks_emit_smem, rowspace ? nullptr : occ, &occ_e, pr->block_filter, pr->lane_warps, rowspace));
+    CUDA_TRY(blocks_emit_occupancy(pr->blocks_emit_smem, pr->pipeline == Pipeline::kRowSpace, &occ_e));
     if (occ_e < 1) return fail(IMM3_ERR_CUDA, "block emit kernel does not fit on an SM (dynamic shared memory %zu bytes)", pr->blocks_emit_smem);
     pr->grid_blocks_emit = (int)std::max<int64_t>(1, std::min<int64_t>((t.nblocks + 7) / 8, (int64_t)db->num_sms * std::max(1, occ_e)));
     return 0;
@@ -860,14 +869,8 @@ int fill_scan_plan(imm3_db* db, Prepared* pr) {
     case Pipeline::kBlocks: {
         const int64_t nb = (prefix + 1023) / 1024;
         if (nb * 2 <= t.nblocks) pr->prefix_blocks = nb;
-        if (pr->pipeline == Pipeline::kRowSpace) {
-            if ((rc = size_dense_filter(db, pr, &occ))) return rc;
-        } else {
-            pr->sp.ntiles = (t.nblocks + 7) / 8;  // the offset scan works on tiles of 8 blocks
-            size_block_filter(pr);
-            size_prune(pr);
-        }
-        if ((rc = size_block_emit(db, pr, &occ))) return rc;
+        rc = pr->pipeline == Pipeline::kRowSpace ? size_dense_filter(db, pr, &occ) : size_block_front(pr, &occ);
+        if (rc || (rc = size_block_emit(db, pr))) return rc;
         break;
     }
     case Pipeline::kSinglePass:  // scan_blocks stages whole blocks
@@ -954,6 +957,8 @@ bool scan_inline_for(int64_t ntiles) {
     }
     return ntiles <= scan_inline_max_tiles();
 }
+// ... for the block filter front (the lane kernel's inline scan is written for 8 warps)
+int block_scan_inline(const Prepared& pr) { return scan_inline_for(pr.sp.ntiles) && !(pr.block_filter == BlockFilter::kLane && pr.lane_warps < 8); }
 int prepare_scan_buffers(imm3_db* db, int64_t ntiles, bool want_list) {
     if (want_list) {
         int rc = ensure_buf(&db->d_tile_list, (size_t)(ntiles + 16) * 4);
@@ -1146,7 +1151,7 @@ int launch_blocks(imm3_db* db, Prepared* pr, int64_t nblocks, Queued* q) {
     const bool lane = pr->block_filter == BlockFilter::kLane;
     int rc;
     if ((rc = ensure_block_filter(db, pr, nblocks))) return rc;
-    sp.scan_inline = (scan_inline_for(ntiles) && !(lane && pr->lane_warps < 8)) ? 1 : 0;  // (the inline scan is written for 8 warps)
+    sp.scan_inline = block_scan_inline(*pr);
     int fused_grid = 0;  // > 0: blocks_scan_emit_kernel
     int group_grid = 0, ngroups = 0;  // > 0: blocks_group_emit_kernel
     if (sp.nproj == 1 && sp.proj[0].pfor_slot >= 0 && !getenv("IMM3_NO_SCANEMIT")) {
@@ -1866,58 +1871,62 @@ int imm3_query(imm3_db* db, const char* table, const imm3_pred* preds, int npred
 
 namespace {
 
-// imm3_query_agg (global = false), imm3_query_agg_global and imm3_query_agg_ext: one validation, one plan, one launch
-// sequence.  The global form on a connected handle compacts this rank's partial groups into its exchange buffer instead
-// of the result buffer and queues the exchange and the merge behind them (k_comm.cuh agg_exchange_kernel, k_agg.cuh
-// agg_merge_kernel; DESIGN §4.3).  allow_sum_avg (imm3_query_agg_ext only) resolves Sum / Avg (DESIGN §4.4c).
-int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, const imm3_agg* aggs, int naggs, const char* const* group_cols,
-              int ngroup, bool global, bool allow_sum_avg, bool encoded_filter, imm3_result** out) {
-    const char* const fn = global ? "imm3_query_agg_global" : "imm3_query_agg";
-    if (!db || !out || (naggs > 0 && !aggs) || (ngroup > 0 && !group_cols)) return fail(IMM3_ERR_INVALID_ARG, "%s: NULL argument", fn);
+// An aggregate between the steps of query_agg.
+struct AggQuery {
+    const char* fn = nullptr;        // the entry point, in messages
+    bool xchg = false;               // a global aggregate of a sharded handle: the ranks' groups are merged over the communicator
+    Prepared pr;                     // the validated logical plan; the filter front's device plan after plan_agg_slice
+    AggPlan ap;                      // naggs: the visible aggregates and a hidden COUNT
+    AggShape shape{};                // the aggregation kernel's instantiation
+    std::unique_ptr<imm3_result> r;  // schema from plan_agg, rows from agg_rows
+    std::vector<int> pfor_cols;      // distinct sorted-int-codec columns decoded per block (MIN / MAX / SUM inputs, group columns)
+    int count_slot = -1;             // the plan's first COUNT (a SUM / AVG query's group sizes)
+    bool has_sum = false;
+    bool enc_filter = false;         // a predicate on a sorted-int-codec column: the block filter front decides it
+    int smem_optin = 0;              // agg_blocks_kernel: the device's shared memory per CTA (cudaDevAttrMaxSharedMemoryPerBlockOptin)
+};
+
+// Validation and plan of an aggregate, before any device work: group and aggregate columns, the result schema, the COUNT a
+// SUM / AVG query carries, the encoded predicates and the hash table's size.
+int plan_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, const imm3_agg* aggs, int naggs, const char* const* group_cols,
+             int ngroup, bool global, bool allow_sum_avg, bool encoded_filter, bool have_out, AggQuery* q) {
+    const char* const fn = q->fn = global ? "imm3_query_agg_global" : "imm3_query_agg";
+    if (!db || !have_out || (naggs > 0 && !aggs) || (ngroup > 0 && !group_cols)) return fail(IMM3_ERR_INVALID_ARG, "%s: NULL argument", fn);
     // A sharded handle merges over the communicator; a single handle's partials are the global result already.
-    const bool xchg = global && db->world > 1;
-    if (xchg && !db->comm_on)
+    q->xchg = global && db->world > 1;
+    if (q->xchg && !db->comm_on)
         return fail(IMM3_ERR_STATE, "%s: a sharded handle (rank %d of %d) merges over the communicator: call imm3_comm_connect first", fn, db->rank, db->world);
     if (naggs < 1) return fail(IMM3_ERR_INVALID_ARG, "%s: no aggregates", fn);
     if (naggs > kMaxAggs) return fail(IMM3_ERR_UNSUPPORTED, "%s: at most %d aggregates", fn, kMaxAggs);
     if (ngroup > kMaxGroupCols) return fail(IMM3_ERR_UNSUPPORTED, "%s: at most %d group-by columns", fn, kMaxGroupCols);
-    Prepared pr;
-    int rc = prepare(db, table, preds, npreds, nullptr, 0, 0, false, &pr);  // validation before any device work
+    Prepared& pr = q->pr;
+    int rc = prepare(db, table, preds, npreds, nullptr, 0, 0, false, &pr);
     if (rc) return rc;
-    TableStore& t = *pr.table;
-    auto find_col = [&](const char* name) -> int {
-        if (!name) return -1;
-        for (size_t i = 0; i < t.cols.size(); i++)
-            if (t.cols[i].meta.name == name) return (int)i;
-        return -1;
-    };
-    AggPlan ap;
+    const TableStore& t = *pr.table;
+    AggPlan& ap = q->ap;
     std::memset(&ap, 0, sizeof ap);
-    std::unique_ptr<imm3_result> r(new imm3_result());
+    q->r.reset(new imm3_result());
+    imm3_result* const r = q->r.get();
     r->db = db;
-    std::vector<int> gidx, aidx;
-    std::vector<int> pfor_cols;  // distinct sorted-int-codec columns decoded per block (MIN / MAX inputs, group columns)
     for (int i = 0; i < kMaxAggs; i++) ap.agg_pfor[i] = -1;
     for (int i = 0; i < kMaxGroupCols; i++) ap.group_pfor[i] = -1;
     int key_bits = 0;
     for (int g = 0; g < ngroup; g++) {
-        const int ci = find_col(group_cols[g]);
+        const int ci = find_col(t.meta, group_cols[g]);
         if (ci < 0) return fail(IMM3_ERR_NOT_FOUND, "Column %s does not exist in table %s", group_cols[g] ? group_cols[g] : "(null)", t.meta.name.c_str());
         const ColumnStore& c = t.cols[(size_t)ci];
         if (key_bits + 8 * c.meta.width > 56) return fail(IMM3_ERR_UNSUPPORTED, "group-by cells must pack into 7 bytes");
+        ap.group[g].base = c.d_arena;
         ap.group[g].width = c.meta.width;
         ap.group[g].key_shift = key_bits;
-        ap.group_pfor[g] = (int8_t)pfor_slot(t, &pfor_cols, ci);
+        ap.group_pfor[g] = (int8_t)pfor_slot(t, &q->pfor_cols, ci);
         key_bits += 8 * c.meta.width;
-        gidx.push_back(ci);
         r->names.push_back(c.meta.name);
         r->types.push_back(c.meta.ctype);
         r->widths.push_back(c.meta.width);
     }
-    int count_slot = -1;  // the plan's first COUNT (a SUM / AVG query's group sizes)
-    bool has_sum = false;
     for (int a = 0; a < naggs; a++) {
-        const int ci = find_col(aggs[a].col);
+        const int ci = find_col(t.meta, aggs[a].col);
         if (ci < 0) return fail(IMM3_ERR_NOT_FOUND, "Column %s does not exist in table %s", aggs[a].col ? aggs[a].col : "(null)", t.meta.name.c_str());
         const ColumnStore& c = t.cols[(size_t)ci];
         const char* suffix = "_count";
@@ -1925,298 +1934,328 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
         if (aggs[a].op == IMM3_AGG_COUNT) {
             ap.agg[a].op = kAggCount;
             rtype = IMM3_COL_COUNT;
-            if (count_slot < 0) count_slot = a;
+            if (q->count_slot < 0) q->count_slot = a;
         } else if (aggs[a].op == IMM3_AGG_MIN || aggs[a].op == IMM3_AGG_MAX) {
             if (c.meta.ctype == IMM3_COL_STRING)
                 return fail(IMM3_ERR_UNSUPPORTED, "min / max on a STRING column (the reference maps both to MaxStringAggr, Engine.scala:137,147)");
             ap.agg[a].op = aggs[a].op == IMM3_AGG_MIN ? kAggMin : kAggMax;
-            ap.agg_pfor[a] = (int8_t)pfor_slot(t, &pfor_cols, ci);  // (COUNT never reads its column)
+            ap.agg_pfor[a] = (int8_t)pfor_slot(t, &q->pfor_cols, ci);  // (COUNT never reads its column)
             suffix = aggs[a].op == IMM3_AGG_MIN ? "_min" : "_max";
         } else if (allow_sum_avg && (aggs[a].op == IMM3_AGG_SUM || aggs[a].op == IMM3_AGG_AVG)) {
             if (c.meta.ctype == IMM3_COL_STRING) return fail(IMM3_ERR_UNSUPPORTED, "sum / avg on a STRING column (%s)", c.meta.name.c_str());
             ap.agg[a].op = kAggSum;  // (AVG = the SUM over the group's COUNT, divided on the host)
-            ap.agg_pfor[a] = (int8_t)pfor_slot(t, &pfor_cols, ci);
-            has_sum = true;
+            ap.agg_pfor[a] = (int8_t)pfor_slot(t, &q->pfor_cols, ci);
+            q->has_sum = true;
             suffix = aggs[a].op == IMM3_AGG_SUM ? "_sum" : "_avg";
             if (aggs[a].op == IMM3_AGG_SUM) rtype = IMM3_COL_INT64;
             else r->avg_cols |= 1u << a;
         } else {
             return fail(IMM3_ERR_UNSUPPORTED, "Unknown Aggregate type (Engine.scala:153: only Min, Max and Count are resolved)");
         }
+        ap.agg[a].base = c.d_arena;
         ap.agg[a].width = c.meta.width;
-        aidx.push_back(ci);
         r->names.push_back(c.meta.name + suffix);  // alias.getOrElse(col + "_max"), Engine.scala:136-152
         r->types.push_back(rtype);
         r->widths.push_back(8);
     }
     // A SUM / AVG query carries one COUNT of the group's rows: the query's own, else a hidden one behind the visible
     // aggregates (in the plan, never in the result).
-    int plan_naggs = naggs;
-    if (has_sum && count_slot < 0) {
+    ap.naggs = naggs;
+    if (q->has_sum && q->count_slot < 0) {
         if (naggs + 1 > kMaxAggs)
             return fail(IMM3_ERR_UNSUPPORTED, "imm3_query_agg_ext: at most %d aggregates, including the COUNT a sum / avg query carries (the query has %d and no COUNT)",
                         kMaxAggs, naggs);
-        count_slot = plan_naggs++;
-        ap.agg[count_slot].op = kAggCount;
-        ap.agg[count_slot].width = 4;
+        q->count_slot = ap.naggs++;
+        ap.agg[q->count_slot].op = kAggCount;
+        ap.agg[q->count_slot].width = 4;
     }
     r->ncols = ngroup + naggs;
     r->agg_first_col = ngroup;
     r->h_cols.resize((size_t)r->ncols);
-    ap.naggs = plan_naggs;
     ap.ngroup = ngroup;
     // A predicate on a sorted-int-codec column: the block filter front decides it (IMM3_AGG_ENCODED_FILTER only).
-    bool enc_filter = false;
     for (auto& f : pr.lp.filters)
         if (is_pfor(t, f.col_idx)) {
             if (!encoded_filter)
                 return fail(IMM3_ERR_UNSUPPORTED, "aggregation with a predicate on a sorted-int-codec column (%s) is not supported yet", t.cols[(size_t)f.col_idx].meta.name.c_str());
-            enc_filter = true;
+            q->enc_filter = true;
         }
     // A MIN / MAX input or a group column in the sorted-int codec: agg_blocks_kernel decodes them block by block.  It also
     // aggregates every block-space selection (blocks are not aligned to agg_kernel's 1024-row spans).
-    const bool on_blocks = !pfor_cols.empty() || enc_filter;
-    if (pfor_cols.size() > (size_t)kMaxPforCols)
-        return fail(IMM3_ERR_UNSUPPORTED, "aggregation decodes at most %d distinct sorted-int-codec columns, the query reads %zu", kMaxPforCols, pfor_cols.size());
+    q->shape = agg_shape(ap, !q->pfor_cols.empty() || q->enc_filter, q->enc_filter);
+    if (q->pfor_cols.size() > (size_t)kMaxPforCols)
+        return fail(IMM3_ERR_UNSUPPORTED, "aggregation decodes at most %d distinct sorted-int-codec columns, the query reads %zu", kMaxPforCols, q->pfor_cols.size());
     ap.table_slots = 1u << 16;
     if (const char* e = getenv("IMM3_AGG_SLOTS")) {  // (tests shrink it to exercise the overflow report)
         uint32_t v = (uint32_t)atoi(e);
         if (v >= 64 && (v & (v - 1)) == 0) ap.table_slots = v;
     }
-    if (xchg && ap.table_slots > kAggXchgSlots)
+    if (q->xchg && ap.table_slots > kAggXchgSlots)
         return fail(IMM3_ERR_UNSUPPORTED, "%s: IMM3_AGG_SLOTS = %u exceeds the exchange buffer of %u groups", fn, ap.table_slots, kAggXchgSlots);
-    // Refusals that depend on this rank's slice: a global aggregate posts them to the peers (every rank then returns the
-    // same status) instead of returning before the exchange.
-    std::string refusal;
-    auto refuse_slice = [&](int code) -> int {
-        if (!xchg) return code;
-        refusal = last_error();
-        return 0;
-    };
-    if (!pfor_cols.empty() && t.max_block_rows > 1024 &&
-        (rc = refuse_slice(fail(IMM3_ERR_UNSUPPORTED, "aggregation over sorted-int-codec columns decodes blocks of at most 1024 rows, table %s has a block of %d",
-                                t.meta.name.c_str(), t.max_block_rows))))
-        return rc;
-    // (the single-pass kernel, which takes larger blocks, leaves no block-space selection behind)
-    if (enc_filter && refusal.empty() && t.max_block_rows > 1024 &&
-        (rc = refuse_slice(fail(IMM3_ERR_UNSUPPORTED, "aggregation with a predicate on a sorted-int-codec column filters blocks of at most 1024 rows, table %s has a block of %d",
-                                t.meta.name.c_str(), t.max_block_rows))))
-        return rc;
-    if ((rc = use_device(db))) return rc;
-    int64_t ngroups_out = 0;
-    std::vector<AggEntry> groups;
-    const bool merge = xchg && !pr.lp.always_empty;          // every rank of a connected handle takes part, an empty slice too
-    bool local = !pr.lp.always_empty && t.nrows > 0 && refusal.empty();
+    return 0;
+}
+
+// Limits of this rank's slice (query_agg's refuse_slice applies them).  Blocks of more than 1024 rows, before any device
+// work: agg_blocks_kernel decodes, and the block filter front filters, no larger ones (the single-pass kernel, which takes
+// larger blocks, leaves no block-space selection behind).
+int check_agg_block_rows(const AggQuery& q) {
+    const TableStore& t = *q.pr.table;
+    if (t.max_block_rows <= 1024) return 0;
+    if (!q.pfor_cols.empty())
+        return fail(IMM3_ERR_UNSUPPORTED, "aggregation over sorted-int-codec columns decodes blocks of at most 1024 rows, table %s has a block of %d",
+                    t.meta.name.c_str(), t.max_block_rows);
+    if (q.enc_filter)
+        return fail(IMM3_ERR_UNSUPPORTED, "aggregation with a predicate on a sorted-int-codec column filters blocks of at most 1024 rows, table %s has a block of %d",
+                    t.meta.name.c_str(), t.max_block_rows);
+    return 0;
+}
+// ... and, once the slice is planned, agg_blocks_kernel's shared memory against the device's opt-in limit.
+int check_agg_smem(const AggQuery& q) {
+    const size_t smem = agg_blocks_smem_bytes(q.shape, q.ap.npfor, q.ap.blk_words_cap) + 1024;  // (1 KB: the kernel's static shared memory)
+    if (!q.shape.blocks || smem <= (size_t)q.smem_optin) return 0;
+    return fail(IMM3_ERR_UNSUPPORTED, "aggregation over %d sorted-int-codec columns with %d aggregates needs %zu bytes of shared memory per CTA, the device has %d",
+                q.ap.npfor, q.ap.naggs, smem, q.smem_optin);
+}
+
+// The device plans of this rank's slice: the filter front, then the AggPlan's columns.  An encoded predicate: the block
+// pipeline's front (DESIGN §4.4d) leaves per block a count and - partially selected blocks only - 32 bitmap words, which
+// agg_blocks_kernel<.., BS> reads.  Otherwise the dense filter kernel in row space, as for a Project query without a select list.
+int plan_agg_slice(imm3_db* db, AggQuery* q) {
+    Prepared& pr = q->pr;
     ScanPlan& sp = pr.sp;
-    if (local && enc_filter) {
-        // The block pipeline's filter front (DESIGN §4.4d): [blocks_prune ->] lane / quad / mini-block filter kernel [-> offset
-        // scan]; per block a count and - partially selected blocks only - 32 bitmap words, which agg_blocks_kernel<.., BS> reads.
-        int occ = 0;
-        if ((rc = plan_columns(db, &pr))) return rc;
+    const TableStore& t = *pr.table;
+    int occ = 0, rc = plan_columns(db, &pr);
+    if (rc) return rc;
+    if (q->enc_filter) {
         pr.pipeline = Pipeline::kBlocks;  // (IMM3_PATH=fused and IMM3_NO_HYBRID choose Project pipelines only)
         choose_block_filter(&pr);
-        sp.ntiles = (t.nblocks + 7) / 8;  // the offset scan works on tiles of 8 blocks
-        size_block_filter(&pr);
-        size_prune(&pr);
-        CUDA_TRY(blocks_filter_occupancy(pr.dyn_smem, pr.block_filter, pr.lane_warps, &occ));
-        if ((rc = plan_grid(db, &pr, occ)) || (rc = ensure_block_filter(db, &pr, t.nblocks))) return rc;
-        sp.scan_inline = (scan_inline_for(sp.ntiles) && !(pr.block_filter == BlockFilter::kLane && pr.lane_warps < 8)) ? 1 : 0;  // (as launch_blocks)
-    } else if (local) {
-        // The filter runs in row space exactly as for a Project query without a select list (dense filter kernel: bitmap,
-        // span counts, total); the aggregation kernel is queued behind it, one synchronisation for the whole query.
-        int occ = 0;
-        if ((rc = plan_columns(db, &pr)) || (rc = size_dense_filter(db, &pr, &occ)) || (rc = plan_grid(db, &pr, occ)) || (rc = ensure_row_space(db, sp)))
-            return rc;
-        sp.scan_inline = 1;  // (only the total matters here; the last CTA's scan provides it)
     }
-    if (local) {
-        ap.nrows = t.nrows;
-        ap.ntiles = sp.ntiles;
-        for (int g = 0; g < ngroup; g++) ap.group[g].base = t.cols[(size_t)gidx[(size_t)g]].d_arena;
-        for (int a = 0; a < naggs; a++) ap.agg[a].base = t.cols[(size_t)aidx[(size_t)a]].d_arena;
-        if (on_blocks) {
-            int64_t words = 0;
-            ap.npfor = (int)pfor_cols.size();
-            for (int i = 0; i < ap.npfor; i++) {
-                const ColumnStore& c = t.cols[(size_t)pfor_cols[(size_t)i]];
-                ap.pfor[i].words = reinterpret_cast<const uint32_t*>(c.d_arena);
-                ap.pfor[i].word_off = c.d_word_off;
-                words = std::max<int64_t>(words, c.max_block_words);
-            }
-            ap.blk_words_cap = block_words_cap(words);
-            ap.nblocks = t.nblocks;
-            ap.row_start = t.d_row_start;
-            int optin = 0;
-            CUDA_TRY(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, db->device));
-            int nsum = 0;
-            for (int a = 0; a < plan_naggs; a++) nsum += ap.agg[a].op == kAggSum;
-            const size_t smem = agg_blocks_smem_bytes(plan_naggs, ap.npfor, ap.blk_words_cap, nsum);
-            if (smem + 1024 > (size_t)optin) {  // (1 KB: the kernel's static shared memory)
-                if ((rc = refuse_slice(fail(IMM3_ERR_UNSUPPORTED, "aggregation over %d sorted-int-codec columns with %d aggregates needs %zu bytes of shared memory per CTA, the device has %d",
-                                            ap.npfor, plan_naggs, smem + 1024, optin))))
-                    return rc;
-                local = false;
-            }
+    rc = q->enc_filter ? size_block_front(&pr, &occ) : size_dense_filter(db, &pr, &occ);
+    if (rc || (rc = plan_grid(db, &pr, occ)) || (rc = q->enc_filter ? ensure_block_filter(db, &pr, t.nblocks) : ensure_row_space(db, sp))) return rc;
+    sp.scan_inline = q->enc_filter ? block_scan_inline(pr) : 1;  // (row space: only the total matters here, the last CTA's scan provides it)
+    AggPlan& ap = q->ap;
+    ap.nrows = t.nrows;
+    ap.ntiles = sp.ntiles;
+    if (q->shape.blocks) {
+        int64_t words = 0;
+        ap.npfor = (int)q->pfor_cols.size();
+        for (int i = 0; i < ap.npfor; i++) {
+            const ColumnStore& c = t.cols[(size_t)q->pfor_cols[(size_t)i]];
+            ap.pfor[i].words = reinterpret_cast<const uint32_t*>(c.d_arena);
+            ap.pfor[i].word_off = c.d_word_off;
+            words = std::max<int64_t>(words, c.max_block_words);
         }
+        ap.blk_words_cap = block_words_cap(words);
+        ap.nblocks = t.nblocks;
+        ap.row_start = t.d_row_start;
+        CUDA_TRY(cudaDeviceGetAttribute(&q->smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, db->device));
     }
-    if (local || merge) {
-        if ((rc = ensure_buf(&db->d_agg_table, (size_t)ap.table_slots * sizeof(AggEntry)))) return rc;
-        if ((rc = ensure_buf(&db->d_agg_out, (size_t)ap.table_slots * sizeof(AggEntry)))) return rc;
-        if ((rc = ensure_buf(&db->d_agg_cnt, 64 + sizeof(AggXOut)))) return rc;  // [groups, overflow] counters, then the exchange's AggXOut
-        unsigned int* const counters = (unsigned int*)db->d_agg_cnt.p;
-        AggXOut* const d_x = reinterpret_cast<AggXOut*>((uint8_t*)db->d_agg_cnt.p + 64);
-        // the local groups go to this aggregate's exchange buffer when they are merged, else straight to the result buffer
-        auto xbuf = [&](int rank) {
-            return reinterpret_cast<AggEntry*>((uint8_t*)db->comm_peer[rank] + kAggXchgOff + (size_t)(db->agg_seq & 1u) * kAggXchgSlots * sizeof(AggEntry));
-        };
-        AggEntry* const local_out = merge ? xbuf(db->rank) : (AggEntry*)db->d_agg_out.p;
-        r->route.clear();
-        CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
-        if (local) {
-            CUDA_TRY(launch_agg_init((AggEntry*)db->d_agg_table.p, ap.table_slots, ap, counters, db->stream));
-            std::string front;  // the filter's part of the route
-            int front_launches = 1;
-            if (enc_filter) {
-                db->route.clear();
-                db->route_tag = "";
-                front_launches = 0;
-                if ((rc = launch_block_filter_front(db, &pr, t.nblocks, &front_launches, nullptr, true))) return rc;
-                front = db->route;
-            } else {
-                CUDA_TRY(launch_filter(sp, (uint32_t*)db->d_bitmap.p, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
-                                       (unsigned long long*)db->d_tile_off.p, db->d_ctrl, pr.grid, pr.dyn_smem, db->stream));
-                front = filter_route(sp);
-            }
-            if (on_blocks)
-                CUDA_TRY(launch_agg_blocks(ap, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, (AggEntry*)db->d_agg_table.p,
-                                           local_out, counters, db->d_ctrl, db->num_sms, db->stream, enc_filter));
-            else
-                CUDA_TRY(launch_agg(ap, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, (AggEntry*)db->d_agg_table.p,
-                                    local_out, counters, db->d_ctrl, db->num_sms, db->stream));
-            r->launches = 3 + front_launches;
-            // the instantiation IMM3_AGG_DISPATCH (kernels.cu) picks: <= 2 group-by columns exact, else 4; 1 .. 4 aggregates exact, else 8;
-            // "/sum": the SUM instantiation; "/bsel": agg_blocks_kernel over the block filter's selection
-            const int ng = ngroup <= 2 ? ngroup : 4, na = (plan_naggs >= 1 && plan_naggs <= 4) ? plan_naggs : 8;
-            const std::string inst = "<" + std::to_string(ng) + "," + std::to_string(na) + ">" + (has_sum ? "/sum" : "") + (enc_filter ? "/bsel" : "");
-            r->route = "agg_init;" + front + ";" + (on_blocks ? "agg_blocks" : "agg") + inst + ";agg_compact";
-        }
-        if (merge) {
-            AggXPlan xp;
-            std::memset(&xp, 0, sizeof xp);
-            for (int i = 0; i < db->world; i++) xp.peer[i] = db->comm_peer[i];
-            xp.rank = db->rank;
-            xp.world = db->world;
-            if (((++db->comm_epoch) & 0xFFFFFFu) == 0) ++db->comm_epoch;  // (the count exchange's rounds: tag 0 is an untouched mailbox)
-            xp.epoch = db->comm_epoch;
-            xp.has_local = local ? 1 : 0;
-            xp.refused = refusal.empty() ? 0 : 1;
-            xp.timeout_ns = db->comm_timeout_ns;
-            CUDA_TRY(launch_agg_exchange(xp, counters, db->d_ctrl, d_x, db->stream));
-            AggMergePlan mp;
-            std::memset(&mp, 0, sizeof mp);
-            for (int i = 0; i < db->world; i++) mp.buf[i] = xbuf(i);
-            db->agg_seq++;  // (posted: the next aggregate compacts into the other buffer)
-            mp.world = db->world;
-            mp.slots = ap.table_slots;
-            mp.naggs = plan_naggs;
-            for (int a = 0; a < plan_naggs; a++) mp.op[a] = ap.agg[a].op == kAggSum ? kAggCount : ap.agg[a].op;  // (a SUM merges as a COUNT: a 64-bit add)
-            CUDA_TRY(launch_agg_init((AggEntry*)db->d_agg_table.p, ap.table_slots, ap, counters, db->stream));
-            CUDA_TRY(launch_agg_merge(mp, d_x, (AggEntry*)db->d_agg_table.p, (AggEntry*)db->d_agg_out.p, counters, db->num_sms, db->stream));
-            r->launches += 4;
-            r->route += std::string(r->route.empty() ? "" : ";") + "agg_exchange;agg_init;agg_merge;agg_compact";
-        }
-        CUDA_TRY(cudaEventRecord(db->ev1, db->stream));
-        struct {
-            unsigned int counters[16];
-            AggXOut x;
-        } hc;
-        static_assert(sizeof hc.counters == 64, "the exchange output sits 64 bytes into d_agg_cnt");
-        if (local) CUDA_TRY(cudaMemcpyAsync(db->h_ctrl, db->d_ctrl, sizeof(CtrlBlock), cudaMemcpyDeviceToHost, db->stream));
-        CUDA_TRY(cudaMemcpyAsync(&hc, db->d_agg_cnt.p, merge ? sizeof hc : sizeof hc.counters, cudaMemcpyDeviceToHost, db->stream));
-        CUDA_TRY(cudaStreamSynchronize(db->stream));
-        if (local && db->h_ctrl->c.error) return fail(IMM3_ERR_CUDA, "kernel watchdog fired (code %u)", db->h_ctrl->c.error);
-        if (merge) {
-            if (hc.x.late)
-                return fail(IMM3_ERR_COMM, "aggregate exchange: a peer's groups were not announced within %llu ms (ranks must issue the same queries in the same order)",
-                            db->comm_timeout_ns / 1000000ull);
-            if (!refusal.empty()) return fail(IMM3_ERR_UNSUPPORTED, "%s", refusal.c_str());
-            if ((hc.x.err_mask >> db->rank) & 1u) return fail(IMM3_ERR_UNSUPPORTED, "aggregation: more than %u groups in the slice of rank %d", ap.table_slots, db->rank);
-            if (hc.x.err_mask)
-                return fail(IMM3_ERR_UNSUPPORTED, "%s: rank %d refused the query (more than %u groups in its slice, or a limit of its slice)", fn,
-                            __builtin_ctz(hc.x.err_mask), ap.table_slots);
-        }
-        if (hc.counters[1]) return fail(IMM3_ERR_UNSUPPORTED, "aggregation: more than %u groups", ap.table_slots);
-        float f = 0;
-        CUDA_TRY(cudaEventElapsedTime(&f, db->ev0, db->ev1));
-        r->device_ms = f;
-        r->stage_ms[0] = f;
-        ngroups_out = hc.counters[0];
-        groups.resize((size_t)ngroups_out);
-        if (ngroups_out) CUDA_TRY(cudaMemcpy(groups.data(), db->d_agg_out.p, (size_t)ngroups_out * sizeof(AggEntry), cudaMemcpyDeviceToHost));
-        std::sort(groups.begin(), groups.end(), [](const AggEntry& x, const AggEntry& y) { return x.first_row < y.first_row; });
-        if (merge)
-            for (int i = 0; i < db->world; i++) r->rank_counts[i] = (int64_t)hc.x.counts[i];
+    return 0;
+}
+
+// Local step: empty table -> filter front -> aggregation kernel -> compaction of this rank's groups into `out`.
+int launch_agg_local(imm3_db* db, AggQuery* q, AggEntry* out, int* launches) {
+    Prepared& pr = q->pr;
+    const ScanPlan& sp = pr.sp;
+    AggEntry* const table = (AggEntry*)db->d_agg_table.p;
+    unsigned int* const counters = (unsigned int*)db->d_agg_cnt.p;
+    CUDA_TRY(launch_agg_init(table, q->ap.table_slots, q->ap, counters, db->stream));
+    note_launch(db, launches, "agg_init");
+    if (q->enc_filter) {
+        const int rc = launch_block_filter_front(db, &pr, pr.table->nblocks, launches, nullptr, true);
+        if (rc) return rc;
+    } else {
+        CUDA_TRY(launch_filter(sp, (uint32_t*)db->d_bitmap.p, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
+                               (unsigned long long*)db->d_tile_off.p, db->d_ctrl, pr.grid, pr.dyn_smem, db->stream));
+        note_launch(db, launches, filter_route(sp));
     }
-    if (local) {
-        // algorithmic bytes: filter columns once + every decoded encoded column once (its words and 4 B of word offsets per
-        // block) + per selected row the cells of the dense group and aggregate columns (MIN / MAX / SUM / AVG inputs)
-        // (with a predicate on an encoded column: every filter column once, and an encoded column that is filtered and
-        // decoded once - its words once, plus the word offsets the decode reads)
-        int64_t bytes = 0, per_row = 0;
-        std::vector<int> counted;
-        auto seen = [&](int ci) { return std::find(counted.begin(), counted.end(), ci) != counted.end(); };
-        for (auto& f2 : pr.lp.filters) {
-            if (enc_filter && seen(f2.col_idx)) continue;
-            counted.push_back(f2.col_idx);
-            bytes += t.cols[(size_t)f2.col_idx].encoded_bytes;
-        }
-        for (int ci : pfor_cols) bytes += (seen(ci) ? 0 : t.cols[(size_t)ci].encoded_bytes) + 4 * (int64_t)t.nblocks;
-        for (int g = 0; g < ngroup; g++)
-            if (ap.group_pfor[g] < 0) per_row += t.cols[(size_t)gidx[(size_t)g]].meta.width;
-        for (int a = 0; a < naggs; a++)
-            if (ap.agg[a].op != kAggCount && ap.agg_pfor[a] < 0) per_row += ap.agg[a].width;
-        r->alg_bytes = bytes + per_row * (int64_t)db->h_ctrl->c.total;
+    CUDA_TRY(launch_agg(q->ap, q->shape, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, table, counters, db->d_ctrl,
+                        db->num_sms, db->stream));
+    note_launch(db, launches, agg_route(q->shape));
+    CUDA_TRY(launch_agg_compact(table, q->ap.table_slots, out, counters, db->stream));
+    note_launch(db, launches, "agg_compact");
+    return 0;
+}
+
+// This aggregate's exchange buffer of `rank`, as mapped here (DESIGN §4.3a: two per rank, used in turn).
+AggEntry* agg_xbuf(const imm3_db* db, int rank) {
+    return reinterpret_cast<AggEntry*>((uint8_t*)db->comm_peer[rank] + kAggXchgOff + (size_t)(db->agg_seq & 1u) * kAggXchgSlots * sizeof(AggEntry));
+}
+
+// Merge step of a global aggregate (DESIGN §4.3): this rank's group count - or that its slice ran nothing, or refused the
+// query - posted to the peers -> a fresh table -> every rank's groups merged into it -> compaction into the result buffer.
+int launch_agg_merge_step(imm3_db* db, const AggQuery& q, bool has_local, bool refused, int* launches) {
+    const AggPlan& ap = q.ap;
+    AggEntry* const table = (AggEntry*)db->d_agg_table.p;
+    unsigned int* const counters = (unsigned int*)db->d_agg_cnt.p;
+    AggXOut* const d_x = reinterpret_cast<AggXOut*>((uint8_t*)db->d_agg_cnt.p + 64);
+    AggXPlan xp;
+    std::memset(&xp, 0, sizeof xp);
+    for (int i = 0; i < db->world; i++) xp.peer[i] = db->comm_peer[i];
+    xp.rank = db->rank;
+    xp.world = db->world;
+    if (((++db->comm_epoch) & 0xFFFFFFu) == 0) ++db->comm_epoch;  // (the count exchange's rounds: tag 0 is an untouched mailbox)
+    xp.epoch = db->comm_epoch;
+    xp.has_local = has_local ? 1 : 0;
+    xp.refused = refused ? 1 : 0;
+    xp.timeout_ns = db->comm_timeout_ns;
+    CUDA_TRY(launch_agg_exchange(xp, counters, db->d_ctrl, d_x, db->stream));
+    note_launch(db, launches, "agg_exchange");
+    AggMergePlan mp;
+    std::memset(&mp, 0, sizeof mp);
+    for (int i = 0; i < db->world; i++) mp.buf[i] = agg_xbuf(db, i);
+    db->agg_seq++;  // (posted: the next aggregate compacts into the other buffer)
+    mp.world = db->world;
+    mp.slots = ap.table_slots;
+    mp.naggs = ap.naggs;
+    for (int a = 0; a < ap.naggs; a++) mp.op[a] = ap.agg[a].op == kAggSum ? kAggCount : ap.agg[a].op;  // (a SUM merges as a COUNT: a 64-bit add)
+    CUDA_TRY(launch_agg_init(table, ap.table_slots, ap, counters, db->stream));
+    note_launch(db, launches, "agg_init");
+    CUDA_TRY(launch_agg_merge(mp, d_x, table, counters, db->num_sms, db->stream));
+    note_launch(db, launches, "agg_merge");
+    CUDA_TRY(launch_agg_compact(table, ap.table_slots, (AggEntry*)db->d_agg_out.p, counters, db->stream));
+    note_launch(db, launches, "agg_compact");
+    return 0;
+}
+
+// Read-back: the counters, the exchange's output and (local step) the control block, one synchronisation, the errors, the
+// device time, the groups in first-row order and every rank's partial group count.
+int read_agg_groups(imm3_db* db, const AggQuery& q, bool local, bool merge, const std::string& refusal, std::vector<AggEntry>* groups) {
+    imm3_result* const r = q.r.get();
+    const uint32_t slots = q.ap.table_slots;
+    struct { unsigned int counters[16]; AggXOut x; } hc;
+    static_assert(sizeof hc.counters == 64, "the exchange output sits 64 bytes into d_agg_cnt");
+    if (local) CUDA_TRY(cudaMemcpyAsync(db->h_ctrl, db->d_ctrl, sizeof(CtrlBlock), cudaMemcpyDeviceToHost, db->stream));
+    CUDA_TRY(cudaMemcpyAsync(&hc, db->d_agg_cnt.p, merge ? sizeof hc : sizeof hc.counters, cudaMemcpyDeviceToHost, db->stream));
+    CUDA_TRY(cudaStreamSynchronize(db->stream));
+    if (local && db->h_ctrl->c.error) return fail(IMM3_ERR_CUDA, "kernel watchdog fired (code %u)", db->h_ctrl->c.error);
+    if (merge) {
+        if (hc.x.late)
+            return fail(IMM3_ERR_COMM, "aggregate exchange: a peer's groups were not announced within %llu ms (ranks must issue the same queries in the same order)",
+                        db->comm_timeout_ns / 1000000ull);
+        if (!refusal.empty()) return fail(IMM3_ERR_UNSUPPORTED, "%s", refusal.c_str());
+        if ((hc.x.err_mask >> db->rank) & 1u) return fail(IMM3_ERR_UNSUPPORTED, "aggregation: more than %u groups in the slice of rank %d", slots, db->rank);
+        if (hc.x.err_mask)
+            return fail(IMM3_ERR_UNSUPPORTED, "%s: rank %d refused the query (more than %u groups in its slice, or a limit of its slice)", q.fn,
+                        __builtin_ctz(hc.x.err_mask), slots);
     }
-    // SUM / AVG: every add on the way here was modulo 2^64, so a sum is exact when it fits int64 - certain for at most 2^32
-    // int32 inputs (2^32 x 2^31 <= 2^63); a larger group (on a global aggregate: the merged count) is refused, not wrapped
-    if (has_sum)
+    if (hc.counters[1]) return fail(IMM3_ERR_UNSUPPORTED, "aggregation: more than %u groups", slots);
+    float f = 0;
+    CUDA_TRY(cudaEventElapsedTime(&f, db->ev0, db->ev1));
+    r->device_ms = f;
+    r->stage_ms[0] = f;
+    groups->resize((size_t)hc.counters[0]);
+    if (!groups->empty()) CUDA_TRY(cudaMemcpy(groups->data(), db->d_agg_out.p, groups->size() * sizeof(AggEntry), cudaMemcpyDeviceToHost));
+    std::sort(groups->begin(), groups->end(), [](const AggEntry& x, const AggEntry& y) { return x.first_row < y.first_row; });
+    if (merge)
+        for (int i = 0; i < db->world; i++) r->rank_counts[i] = (int64_t)hc.x.counts[i];
+    return 0;
+}
+
+// Algorithmic bytes of the local step: filter columns once + every decoded encoded column once (its words and 4 B of word
+// offsets per block) + per selected row the cells of the dense group and aggregate columns (MIN / MAX / SUM / AVG inputs).
+// (With a predicate on an encoded column: every filter column once, and an encoded column that is filtered and decoded once
+// - its words once, plus the word offsets the decode reads.)
+int64_t agg_alg_bytes(const AggQuery& q, int64_t selected_rows) {
+    const TableStore& t = *q.pr.table;
+    const AggPlan& ap = q.ap;
+    int64_t bytes = 0, per_row = 0;
+    std::vector<int> counted;
+    auto seen = [&](int ci) { return std::find(counted.begin(), counted.end(), ci) != counted.end(); };
+    for (auto& f : q.pr.lp.filters) {
+        if (q.enc_filter && seen(f.col_idx)) continue;
+        counted.push_back(f.col_idx);
+        bytes += t.cols[(size_t)f.col_idx].encoded_bytes;
+    }
+    for (int ci : q.pfor_cols) bytes += (seen(ci) ? 0 : t.cols[(size_t)ci].encoded_bytes) + 4 * (int64_t)t.nblocks;
+    for (int g = 0; g < ap.ngroup; g++)
+        if (ap.group_pfor[g] < 0) per_row += ap.group[g].width;
+    for (int a = 0; a < ap.naggs; a++)
+        if (ap.agg[a].op != kAggCount && ap.agg_pfor[a] < 0) per_row += ap.agg[a].width;
+    return bytes + per_row * selected_rows;
+}
+
+// The result's rows - group cells, then the aggregates (COUNT / SUM: int64, MIN / MAX / AVG: double) - and counts.
+// SUM / AVG: every add on the way here was modulo 2^64, so a sum is exact when it fits int64 - certain for at most 2^32
+// int32 inputs (2^32 x 2^31 <= 2^63); a larger group (on a global aggregate: the merged count) is refused, not wrapped.
+int agg_rows(imm3_db* db, const AggQuery& q, const std::vector<AggEntry>& groups) {
+    imm3_result* const r = q.r.get();
+    const AggPlan& ap = q.ap;
+    const int64_t n = (int64_t)groups.size();
+    if (q.has_sum)
         for (const AggEntry& e : groups)
-            if ((unsigned long long)e.val[count_slot] > (1ull << 32))
-                return fail(IMM3_ERR_UNSUPPORTED, "imm3_query_agg_ext: a group of %lld rows: sum / avg are exact for groups of at most 2^32 rows", e.val[count_slot]);
-    // rows of the result: group cells, then the aggregates (COUNT / SUM: int64, MIN / MAX / AVG: double)
+            if ((unsigned long long)e.val[q.count_slot] > (1ull << 32))
+                return fail(IMM3_ERR_UNSUPPORTED, "imm3_query_agg_ext: a group of %lld rows: sum / avg are exact for groups of at most 2^32 rows", e.val[q.count_slot]);
     for (int c = 0; c < r->ncols; c++) {
         const size_t w = (size_t)r->widths[(size_t)c];
-        if ((rc = db->host_pool.acquire(std::max<size_t>(1, (size_t)ngroups_out * w), &r->h_cols[(size_t)c]))) {
+        if (const int rc = db->host_pool.acquire(std::max<size_t>(1, (size_t)n * w), &r->h_cols[(size_t)c])) {
             for (auto& b : r->h_cols) db->host_pool.release(b);
             return rc;
         }
         uint8_t* dst = (uint8_t*)r->h_cols[(size_t)c].p;
-        for (int64_t i = 0; i < ngroups_out; i++) {
+        for (int64_t i = 0; i < n; i++) {
             const AggEntry& e = groups[(size_t)i];
-            if (c < ngroup) {
+            if (c < ap.ngroup) {
                 const unsigned long long cell = e.key >> ap.group[c].key_shift;
                 for (size_t b = 0; b < w; b++) dst[(size_t)i * w + b] = (uint8_t)(cell >> (8 * b));
             } else {
-                const int a = c - ngroup;
-                if (ap.agg[a].op == kAggCount || (ap.agg[a].op == kAggSum && aggs[a].op == IMM3_AGG_SUM)) {
-                    const int64_t v = e.val[a];
-                    std::memcpy(dst + (size_t)i * 8, &v, 8);
-                } else if (ap.agg[a].op == kAggSum) {
-                    const double v = (double)e.val[a] / (double)e.val[count_slot];  // AVG, once, in IEEE double
-                    std::memcpy(dst + (size_t)i * 8, &v, 8);
-                } else {
-                    const double v = (double)e.val[a];  // value.toDouble, ProjectAggregate.scala:176-178
-                    std::memcpy(dst + (size_t)i * 8, &v, 8);
-                }
+                const int a = c - ap.ngroup;
+                const bool avg = (r->avg_cols >> a) & 1u;
+                double v = (double)e.val[a];  // MIN / MAX: value.toDouble, ProjectAggregate.scala:176-178
+                if (avg) v /= (double)e.val[q.count_slot];  // AVG, once, in IEEE double
+                if (ap.agg[a].op == kAggCount || (ap.agg[a].op == kAggSum && !avg)) std::memcpy(dst + (size_t)i * 8, &e.val[a], 8);
+                else std::memcpy(dst + (size_t)i * 8, &v, 8);
             }
         }
     }
-    r->local_count = r->fetched = ngroups_out;
-    r->g_offset = 0;
-    r->g_take = r->g_total = ngroups_out;
-    r->world = xchg ? db->world : 1;  // (a global aggregate: rank_counts = every rank's partial group count)
+    r->local_count = r->fetched = r->g_take = r->g_total = n;  // (g_offset 0)
+    r->world = q.xchg ? db->world : 1;  // (a global aggregate: rank_counts = every rank's partial group count)
+    return 0;
+}
+
+// imm3_query_agg (global = false), imm3_query_agg_global and imm3_query_agg_ext, step by step.  The global form on a
+// connected handle compacts this rank's partial groups into its exchange buffer instead of the result buffer and queues the
+// exchange and the merge behind them (k_comm.cuh agg_exchange_kernel, k_agg.cuh agg_merge_kernel; DESIGN §4.3).
+// allow_sum_avg (imm3_query_agg_ext only) resolves Sum / Avg (DESIGN §4.4c).
+int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds, const imm3_agg* aggs, int naggs, const char* const* group_cols,
+              int ngroup, bool global, bool allow_sum_avg, bool encoded_filter, imm3_result** out) {
+    AggQuery q;
+    int rc = plan_agg(db, table, preds, npreds, aggs, naggs, group_cols, ngroup, global, allow_sum_avg, encoded_filter, out != nullptr, &q);
+    if (rc) return rc;
+    // Refusals that depend on this rank's slice: a global aggregate posts them to the peers (every rank then returns the
+    // same status) instead of returning before the exchange.
+    std::string refusal;
+    auto refuse_slice = [&](int code) -> int {
+        if (!code || !q.xchg) return code;
+        refusal = last_error();
+        return 0;
+    };
+    if ((rc = refuse_slice(check_agg_block_rows(q))) || (rc = use_device(db))) return rc;
+    const bool merge = q.xchg && !q.pr.lp.always_empty;  // every rank of a connected handle takes part, an empty slice too
+    bool local = !q.pr.lp.always_empty && q.pr.table->nrows > 0 && refusal.empty();
+    if (local && ((rc = plan_agg_slice(db, &q)) || (rc = refuse_slice(check_agg_smem(q))))) return rc;
+    local = local && refusal.empty();
+    std::vector<AggEntry> groups;
+    if (local || merge) {
+        const size_t table_bytes = (size_t)q.ap.table_slots * sizeof(AggEntry);
+        if ((rc = ensure_buf(&db->d_agg_table, table_bytes)) || (rc = ensure_buf(&db->d_agg_out, table_bytes)) ||
+            (rc = ensure_buf(&db->d_agg_cnt, 64 + sizeof(AggXOut))))  // [groups, overflow] counters, then the exchange's AggXOut
+            return rc;
+        // every kernel noted (note_launch) between ev0 and ev1: the result's route and launch count; the local groups go to this
+        // aggregate's exchange buffer when they are merged, else straight to the result buffer
+        db->route.clear();
+        db->route_tag = "";
+        CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
+        if (local && (rc = launch_agg_local(db, &q, merge ? agg_xbuf(db, db->rank) : (AggEntry*)db->d_agg_out.p, &q.r->launches))) return rc;
+        if (merge && (rc = launch_agg_merge_step(db, q, local, !refusal.empty(), &q.r->launches))) return rc;
+        CUDA_TRY(cudaEventRecord(db->ev1, db->stream));
+        q.r->route = db->route;
+        if ((rc = read_agg_groups(db, q, local, merge, refusal, &groups))) return rc;
+    }
+    if (local) q.r->alg_bytes = agg_alg_bytes(q, (int64_t)db->h_ctrl->c.total);
+    if ((rc = agg_rows(db, q, groups))) return rc;
     db->live_results++;
-    *out = r.release();
+    *out = q.r.release();
     return 0;
 }
 

@@ -183,12 +183,23 @@ cudaError_t launch_blocks_prune(const PrunePlan& q, const uint64_t* row_start, l
     return cudaGetLastError();
 }
 
-// count / min / max / sum ... group by: empty table -> (filter kernel, launched by the caller) -> agg_kernel (its SUM
-// instantiation when the plan has a SUM) -> compaction.
-static int agg_nsum(const AggPlan& a) {
-    int n = 0;
-    for (int i = 0; i < a.naggs && i < kMaxAggs; i++) n += a.agg[i].op == kAggSum;
-    return n;
+// count / min / max / sum ... group by: empty table -> (filter front, launched by the caller) -> agg_kernel or
+// agg_blocks_kernel -> compaction.  The instantiation: exact for <= 2 group-by columns and 1 .. 4 aggregates, the general
+// forms beyond; a plan with a SUM takes the SUM instantiations (it carries a COUNT too: 2 .. 4 aggregates exact, else 8).
+AggShape agg_shape(const AggPlan& a, bool blocks, bool bsel) {
+    AggShape s;
+    s.ng = a.ngroup <= 2 ? a.ngroup : 4;
+    s.na = (a.naggs >= 1 && a.naggs <= 4) ? a.naggs : 8;
+    s.nsum = 0;
+    for (int i = 0; i < a.naggs && i < kMaxAggs; i++) s.nsum += a.agg[i].op == kAggSum;
+    if (s.nsum > 0 && s.na < 2) s.na = 2;
+    s.blocks = blocks;
+    s.bsel = blocks && bsel;
+    return s;
+}
+std::string agg_route(const AggShape& s) {
+    return std::string(s.blocks ? "agg_blocks<" : "agg<") + std::to_string(s.ng) + "," + std::to_string(s.na) + ">" + (s.nsum > 0 ? "/sum" : "") +
+           (s.bsel ? "/bsel" : "");
 }
 cudaError_t launch_agg_init(AggEntry* table, uint32_t slots, const AggPlan& a, unsigned int* counters, cudaStream_t stream) {
     cudaError_t e = configure_once();
@@ -199,102 +210,50 @@ cudaError_t launch_agg_init(AggEntry* table, uint32_t slots, const AggPlan& a, u
     agg_init_kernel<<<(slots + kComputeThreads - 1) / kComputeThreads, kComputeThreads, 0, stream>>>(table, slots, ops, counters);
     return cudaGetLastError();
 }
+size_t agg_blocks_smem_bytes(const AggShape& s, int npfor, int words_cap) {
+    return agg_blocks_state_bytes(s.na, s.nsum) + (size_t)kComputeWarps * (size_t)agg_blocks_warp_words(npfor, words_cap) * 4;
+}
+// The kernel of a shape.  These switches instantiate every aggregation kernel of the library: agg_kernel<NG, NA, S> and
+// agg_blocks_kernel<NG, NA, S, BS> for NG in {0, 1, 2, 4}, NA in {1, 2, 3, 4, 8} (S = false) or {2, 3, 4, 8} (S = true).
+using AggKernel = void (*)(AggPlan, const uint32_t*, const uint32_t*, AggEntry*, unsigned int*, const ScanCtrl*);
 template <int NG, int NA, bool S>
-static cudaError_t launch_agg_as(const AggPlan& a, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, unsigned int* overflow,
-                                 const ScanCtrl* ctrl, int num_sms, cudaStream_t stream, bool /*bsel: agg_blocks_kernel only*/) {
-    auto* const kern = agg_kernel<NG, NA, S>;
-    const size_t smem = agg_smem_bytes(NA, S ? agg_nsum(a) : 0);
-    cudaError_t e = cudaSuccess;
+static AggKernel agg_kernel_of(const AggShape& s) {
+    if (!s.blocks) return agg_kernel<NG, NA, S>;
+    return s.bsel ? agg_blocks_kernel<NG, NA, S, true> : agg_blocks_kernel<NG, NA, S, false>;
+}
+template <int NG>
+static AggKernel agg_kernel_of(const AggShape& s) {
+    if (s.nsum > 0) return s.na == 2 ? agg_kernel_of<NG, 2, true>(s) : s.na == 3 ? agg_kernel_of<NG, 3, true>(s) : s.na == 4 ? agg_kernel_of<NG, 4, true>(s) : agg_kernel_of<NG, 8, true>(s);
+    return s.na == 1 ? agg_kernel_of<NG, 1, false>(s) : s.na == 2 ? agg_kernel_of<NG, 2, false>(s) : s.na == 3 ? agg_kernel_of<NG, 3, false>(s)
+         : s.na == 4 ? agg_kernel_of<NG, 4, false>(s) : agg_kernel_of<NG, 8, false>(s);
+}
+cudaError_t launch_agg(const AggPlan& a, const AggShape& s, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, unsigned int* counters,
+                       const ScanCtrl* ctrl, int num_sms, cudaStream_t stream) {
+    cudaError_t e = configure_once();
+    if (e != cudaSuccess) return e;
+    const AggKernel kern = s.ng == 0 ? agg_kernel_of<0>(s) : s.ng == 1 ? agg_kernel_of<1>(s) : s.ng == 2 ? agg_kernel_of<2>(s) : agg_kernel_of<4>(s);
+    const size_t smem = s.blocks ? agg_blocks_smem_bytes(s, a.npfor, a.blk_words_cap) : agg_smem_bytes(s.na, s.nsum);
     // (a per-device attribute, set per launch: one driver call per aggregation query)
     if (smem > 48 * 1024 && (e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
     int occ = 0;
     e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kComputeThreads, smem);
     if (e != cudaSuccess) return e;
     if (occ < 1) return cudaErrorInvalidConfiguration;
-    const long long nspans = a.ntiles * 8;
-    const long long grid = std::max<long long>(1, std::min<long long>((nspans + kComputeWarps - 1) / kComputeWarps, (long long)num_sms * occ));
-    kern<<<(unsigned)grid, kComputeThreads, smem, stream>>>(a, bitmap, span_cnt, table, overflow, ctrl);
+    const long long units = s.blocks ? a.nblocks : a.ntiles * 8;  // one warp per block, or per 1024-row span
+    const long long grid = std::max<long long>(1, std::min<long long>((units + kComputeWarps - 1) / kComputeWarps, (long long)num_sms * occ));
+    kern<<<(unsigned)grid, kComputeThreads, smem, stream>>>(a, bitmap, span_cnt, table, counters + 1, ctrl);
     return cudaGetLastError();
 }
-// the instantiation for this query's shape: exact for <= 2 group-by columns and 1 .. 4 aggregates, the general forms beyond;
-// a plan with a SUM takes the SUM instantiations (it carries a COUNT too: 2 .. 4 aggregates exact, else 8); `bsel` picks
-// agg_blocks_kernel's block-space-selection instantiations
-#define IMM3_AGG_DISPATCH(LAUNCH)                                                                                                         \
-    do {                                                                                                                                  \
-        const int ng = a.ngroup <= 2 ? a.ngroup : 4, na = (a.naggs >= 1 && a.naggs <= 4) ? a.naggs : 8;                                   \
-        if (agg_nsum(a) == 0) {                                                                                                           \
-            IMM3_AGG_DISPATCH_ROW(LAUNCH, 0) else IMM3_AGG_DISPATCH_ROW(LAUNCH, 1) else IMM3_AGG_DISPATCH_ROW(LAUNCH, 2) else IMM3_AGG_DISPATCH_ROW(LAUNCH, 4) \
-        } else {                                                                                                                          \
-            IMM3_AGG_SUM_ROW(LAUNCH, 0) else IMM3_AGG_SUM_ROW(LAUNCH, 1) else IMM3_AGG_SUM_ROW(LAUNCH, 2) else IMM3_AGG_SUM_ROW(LAUNCH, 4) \
-        }                                                                                                                                 \
-    } while (0)
-#define IMM3_AGG_DISPATCH_ROW(LAUNCH, NG)                                                                                                  \
-    if (ng == NG) {                                                                                                                       \
-        if (na == 1) e = LAUNCH<NG, 1, false>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream, bsel);                     \
-        else if (na == 2) e = LAUNCH<NG, 2, false>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream, bsel);                \
-        else if (na == 3) e = LAUNCH<NG, 3, false>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream, bsel);                \
-        else if (na == 4) e = LAUNCH<NG, 4, false>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream, bsel);                \
-        else e = LAUNCH<NG, 8, false>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream, bsel);                             \
-    }
-#define IMM3_AGG_SUM_ROW(LAUNCH, NG)                                                                                                       \
-    if (ng == NG) {                                                                                                                       \
-        if (na <= 2) e = LAUNCH<NG, 2, true>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream, bsel);                      \
-        else if (na == 3) e = LAUNCH<NG, 3, true>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream, bsel);                 \
-        else if (na == 4) e = LAUNCH<NG, 4, true>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream, bsel);                 \
-        else e = LAUNCH<NG, 8, true>(a, bitmap, span_cnt, table, counters + 1, ctrl, num_sms, stream, bsel);                              \
-    }
-cudaError_t launch_agg(const AggPlan& a, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, AggEntry* out, unsigned int* counters,
-                       const ScanCtrl* ctrl, int num_sms, cudaStream_t stream) {
-    cudaError_t e = configure_once();
-    if (e != cudaSuccess) return e;
-    const bool bsel = false;
-    IMM3_AGG_DISPATCH(launch_agg_as);
-    if (e != cudaSuccess) return e;
-    agg_compact_kernel<<<(a.table_slots + kComputeThreads - 1) / kComputeThreads, kComputeThreads, 0, stream>>>(table, a.table_slots, out, counters);
+cudaError_t launch_agg_compact(const AggEntry* table, uint32_t slots, AggEntry* out, unsigned int* counters, cudaStream_t stream) {
+    agg_compact_kernel<<<(slots + kComputeThreads - 1) / kComputeThreads, kComputeThreads, 0, stream>>>(table, slots, out, counters);
     return cudaGetLastError();
 }
 
-// ... the same with agg_blocks_kernel (a MIN / MAX / SUM input or a group column in the sorted-int codec; blocks of <= 1024 rows)
-size_t agg_blocks_smem_bytes(int naggs, int npfor, int words_cap, int nsum) {
-    const int na = nsum > 0 ? (naggs <= 2 ? 2 : (naggs <= 4 ? naggs : 8)) : ((naggs >= 1 && naggs <= 4) ? naggs : 8);  // (IMM3_AGG_DISPATCH's NA)
-    return agg_blocks_state_bytes(na, nsum) + (size_t)kComputeWarps * (size_t)agg_blocks_warp_words(npfor, words_cap) * 4;
-}
-template <int NG, int NA, bool S>
-static cudaError_t launch_agg_blocks_as(const AggPlan& a, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, unsigned int* overflow,
-                                        const ScanCtrl* ctrl, int num_sms, cudaStream_t stream, bool bsel) {
-    auto* const kern = bsel ? agg_blocks_kernel<NG, NA, S, true> : agg_blocks_kernel<NG, NA, S, false>;
-    const size_t smem = agg_blocks_smem_bytes(NA, a.npfor, a.blk_words_cap, S ? agg_nsum(a) : 0);
-    cudaError_t e = cudaSuccess;
-    if (smem > 48 * 1024 && (e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) return e;
-    int occ = 0;
-    e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kComputeThreads, smem);
-    if (e != cudaSuccess) return e;
-    if (occ < 1) return cudaErrorInvalidConfiguration;
-    const long long grid = std::max<long long>(1, std::min<long long>((a.nblocks + kComputeWarps - 1) / kComputeWarps, (long long)num_sms * occ));
-    kern<<<(unsigned)grid, kComputeThreads, smem, stream>>>(a, bitmap, span_cnt, table, overflow, ctrl);
-    return cudaGetLastError();
-}
-cudaError_t launch_agg_blocks(const AggPlan& a, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, AggEntry* out, unsigned int* counters,
-                              const ScanCtrl* ctrl, int num_sms, cudaStream_t stream, bool bsel) {
-    cudaError_t e = configure_once();
-    if (e != cudaSuccess) return e;
-    IMM3_AGG_DISPATCH(launch_agg_blocks_as);
-    if (e != cudaSuccess) return e;
-    agg_compact_kernel<<<(a.table_slots + kComputeThreads - 1) / kComputeThreads, kComputeThreads, 0, stream>>>(table, a.table_slots, out, counters);
-    return cudaGetLastError();
-}
-#undef IMM3_AGG_SUM_ROW
-#undef IMM3_AGG_DISPATCH_ROW
-#undef IMM3_AGG_DISPATCH
-
-// Global aggregate: every rank's partial groups (exchange buffers) -> the freshly initialised table -> compaction.
-cudaError_t launch_agg_merge(const AggMergePlan& m, const AggXOut* x, AggEntry* table, AggEntry* out, unsigned int* counters, int num_sms,
-                             cudaStream_t stream) {
+// Global aggregate: every rank's partial groups (exchange buffers) -> the freshly initialised table (compaction follows).
+cudaError_t launch_agg_merge(const AggMergePlan& m, const AggXOut* x, AggEntry* table, unsigned int* counters, int num_sms, cudaStream_t stream) {
     cudaError_t e = configure_once();
     if (e != cudaSuccess) return e;
     agg_merge_kernel<<<(unsigned)std::max(1, num_sms), kComputeThreads, 0, stream>>>(m, x, table, counters + 1);
-    if ((e = cudaGetLastError()) != cudaSuccess) return e;
-    agg_compact_kernel<<<(m.slots + kComputeThreads - 1) / kComputeThreads, kComputeThreads, 0, stream>>>(table, m.slots, out, counters);
     return cudaGetLastError();
 }
 
@@ -406,13 +365,11 @@ cudaError_t blocks_filter_occupancy(size_t filter_smem, BlockFilter filter, int 
            : filter == BlockFilter::kQuad ? cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, blocks_filter_quad_kernel, kComputeThreads + 32, filter_smem)
                                           : cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, blocks_filter_kernel, kComputeThreads + 32, filter_smem);
 }
-cudaError_t blocks_multi_occupancy(size_t filter_smem, size_t emit_smem, int* filter_blocks_per_sm, int* emit_blocks_per_sm, BlockFilter filter,
-                                   int lane_warps, bool rowspace) {
+cudaError_t blocks_emit_occupancy(size_t emit_smem, bool rowspace, int* blocks_per_sm) {
     cudaError_t e = configure_once();
     if (e != cudaSuccess) return e;
-    if (filter_blocks_per_sm && (e = blocks_filter_occupancy(filter_smem, filter, lane_warps, filter_blocks_per_sm)) != cudaSuccess) return e;
-    if (rowspace) return cudaOccupancyMaxActiveBlocksPerMultiprocessor(emit_blocks_per_sm, blocks_emit_kernel<true>, kComputeThreads, emit_smem);
-    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(emit_blocks_per_sm, blocks_emit_kernel<false>, kComputeThreads, emit_smem);
+    if (rowspace) return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, blocks_emit_kernel<true>, kComputeThreads, emit_smem);
+    return cudaOccupancyMaxActiveBlocksPerMultiprocessor(blocks_per_sm, blocks_emit_kernel<false>, kComputeThreads, emit_smem);
 }
 cudaError_t launch_blocks_filter(const ScanPlan& plan, uint32_t* bitmapB, uint32_t* blk_cnt, uint32_t* tile_cnt, unsigned long long* tile_off,
                                  ScanCtrl* ctrl, long long nblocks, int grid, size_t dyn_smem, BlockFilter filter, int lane_warps,

@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 
 #include <cstddef>
+#include <string>
 
 #include "plan.hpp"
 
@@ -23,13 +24,17 @@ cudaError_t emit_stream_occupancy(size_t dyn_smem, int* blocks_per_sm);
 cudaError_t launch_emit_stream(const ScanPlan& plan, const uint32_t* bitmap, const uint32_t* span_cnt, const uint32_t* tile_cnt,
                                const unsigned long long* tile_off, long long nsub, int ring, int stage_bytes, int dense_mode, int grid,
                                size_t dyn_smem, ScanCtrl* ctrl, bool pdl, cudaStream_t stream);
+// The aggregation kernel's instantiation (agg_shape is the one place that chooses it): NG group-by columns, NA aggregates,
+// nsum SUMs; blocks: agg_blocks_kernel, else agg_kernel; bsel: agg_blocks_kernel reads the block filter's selection (32
+// words and one count per block), not the row-space filter's.
+struct AggShape { int ng, na, nsum; bool blocks, bsel; };
+AggShape agg_shape(const AggPlan& a, bool blocks, bool bsel);
+std::string agg_route(const AggShape& s);  // its name in Result.route, e.g. "agg<1,2>", "agg_blocks<0,3>/sum/bsel"
+size_t agg_blocks_smem_bytes(const AggShape& s, int npfor, int words_cap);  // dynamic shared memory of agg_blocks_kernel
 cudaError_t launch_agg_init(AggEntry* table, uint32_t slots, const AggPlan& a, unsigned int* counters, cudaStream_t stream);
-cudaError_t launch_agg(const AggPlan& a, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, AggEntry* out, unsigned int* counters,
+cudaError_t launch_agg(const AggPlan& a, const AggShape& s, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, unsigned int* counters,
                        const ScanCtrl* ctrl, int num_sms, cudaStream_t stream);
-size_t agg_blocks_smem_bytes(int naggs, int npfor, int words_cap, int nsum = 0);  // dynamic shared memory of agg_blocks_kernel (nsum SUMs: agg_blocks_sum_kernel)
-// bsel: bitmap / span_cnt are the block filter's output (32 words and one count per block), not the row-space filter's
-cudaError_t launch_agg_blocks(const AggPlan& a, const uint32_t* bitmap, const uint32_t* span_cnt, AggEntry* table, AggEntry* out, unsigned int* counters,
-                              const ScanCtrl* ctrl, int num_sms, cudaStream_t stream, bool bsel = false);
+cudaError_t launch_agg_compact(const AggEntry* table, uint32_t slots, AggEntry* out, unsigned int* counters, cudaStream_t stream);
 long long scan_inline_max_tiles();
 cudaError_t launch_offset_scan(const uint32_t* tile_cnt, unsigned long long* tile_off, long long ntiles, long long limit, uint32_t epoch,
                                unsigned long long* partials, ScanCtrl* ctrl, unsigned int* tile_list, cudaStream_t stream);
@@ -52,8 +57,7 @@ int blocks_filter_quad_slot_bytes(int tile_cap_bytes);
 // (blocks_filter_lane_kernel, lane_warps warps per CTA).
 enum class BlockFilter { kMini, kQuad, kLane };
 cudaError_t blocks_filter_occupancy(size_t filter_smem, BlockFilter filter, int lane_warps, int* blocks_per_sm);
-cudaError_t blocks_multi_occupancy(size_t filter_smem, size_t emit_smem, int* filter_blocks_per_sm, int* emit_blocks_per_sm, BlockFilter filter,
-                                   int lane_warps, bool rowspace);
+cudaError_t blocks_emit_occupancy(size_t emit_smem, bool rowspace, int* blocks_per_sm);
 cudaError_t launch_blocks_filter(const ScanPlan& plan, uint32_t* bitmapB, uint32_t* blk_cnt, uint32_t* tile_cnt, unsigned long long* tile_off,
                                  ScanCtrl* ctrl, long long nblocks, int grid, size_t dyn_smem, BlockFilter filter, int lane_warps,
                                  const unsigned int* work, cudaStream_t stream, uint32_t* grp_sum = nullptr);  // grp_sum: blocks_group_emit_kernel follows (lane kernel only)
@@ -67,8 +71,7 @@ cudaError_t launch_blocks_emit(const ScanPlan& plan, const uint32_t* bitmap, con
                                cudaStream_t stream);
 cudaError_t launch_count_exchange(const CommPlan& plan, const ScanCtrl* ctrl, CommOut* out, cudaStream_t stream);
 cudaError_t launch_agg_exchange(const AggXPlan& plan, const unsigned int* counters, const ScanCtrl* ctrl, AggXOut* out, cudaStream_t stream);
-cudaError_t launch_agg_merge(const AggMergePlan& m, const AggXOut* x, AggEntry* table, AggEntry* out, unsigned int* counters, int num_sms,
-                             cudaStream_t stream);
+cudaError_t launch_agg_merge(const AggMergePlan& m, const AggXOut* x, AggEntry* table, unsigned int* counters, int num_sms, cudaStream_t stream);
 cudaError_t launch_scan_blocks(const ScanPlan& plan, ScanCtrl* ctrl, unsigned long long* status, int grid, size_t dyn_smem,
                                cudaStream_t stream);
 

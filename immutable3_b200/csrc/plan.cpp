@@ -22,7 +22,8 @@
 
 namespace imm3 {
 
-static int find_col(const TableMeta& t, const char* name) {
+int find_col(const TableMeta& t, const char* name) {
+    if (!name) return -1;
     for (size_t i = 0; i < t.cols.size(); i++)
         if (t.cols[i].name == name) return (int)i;
     return -1;

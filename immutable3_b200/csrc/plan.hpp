@@ -262,6 +262,7 @@ struct LogicalPlan {
     std::vector<Narrowed> narrowed;
 };
 
+int find_col(const TableMeta& t, const char* name);  // column index by name, -1: none (or NULL)
 int build_logical_plan(const TableMeta& table, const imm3_pred* preds, int npreds, const char* const* proj_cols,
                        int nproj, int64_t limit, LogicalPlan* out);
 std::string explain_json(const LogicalPlan& lp, const char* kernel);

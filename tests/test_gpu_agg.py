@@ -40,6 +40,7 @@ def check_agg(orc, eng, table, sel, aggs, group_by):
             assert got.format_row(i) == want
         names = [got.col_name(c) for c in range(got.ncols)]
         assert names == list(group_by) + [f"{a.col}_{type(a).__name__.lower()}" for a in aggs]
+        assert got.kernel_launches == (len(got.route.split(";")) if got.route else 0), (got.kernel_launches, got.route)
         return got.nrows
 
 

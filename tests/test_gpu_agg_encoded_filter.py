@@ -407,6 +407,7 @@ def _worker(rank, world, data_dir, port, out_dir, mode):
                         assert r.global_count == n
                         assert r.route.endswith("agg_exchange;agg_init;agg_merge;agg_compact"), r.route
                         assert "/bsel;agg_compact;agg_exchange" in r.route or r.route.startswith("agg_exchange"), r.route
+                        assert r.kernel_launches == len(r.route.split(";")), (r.kernel_launches, r.route)
         open(os.path.join(out_dir, f"ok{rank}"), "w").write("ok")
     finally:
         dist.destroy_process_group()

@@ -100,6 +100,7 @@ def _worker(rank, world, data_dir, port, out_dir, mode):
                         _same(r.columns(), exp, (rank, table, sel, aggs, gb))
                         assert r.global_count == exp.nrows and r.rank_counts == res.counts
                         assert r.route.endswith("agg_exchange;agg_init;agg_merge;agg_compact"), r.route
+                        assert r.kernel_launches == len(r.route.split(";")), (r.kernel_launches, r.route)
                 return res
 
             for table, sel, aggs, gb in _cases():

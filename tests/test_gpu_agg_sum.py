@@ -29,6 +29,7 @@ def check_ext(orc, eng, table, sel, aggs, group_by, route=None):
         assert got.nrows == n, (table, sel, aggs, group_by, got.nrows, n)
         if route:
             assert route in got.route, (route, got.route)
+        assert got.kernel_launches == (len(got.route.split(";")) if got.route else 0), (got.kernel_launches, got.route)
         names = [got.col_name(c) for c in range(got.ncols)]
         assert names == list(group_by) + [f"{a.col}_{type(a).__name__.lower()}" for a in aggs]
         for a, agg in enumerate(aggs):
@@ -245,6 +246,7 @@ def _worker(rank, world, data_dir, port, out_dir, mode):
                     with eng.execute_agg_global(q, sum_avg=True) as r:
                         assert r.global_count == n
                         assert r.route.endswith("agg_exchange;agg_init;agg_merge;agg_compact"), r.route
+                        assert r.kernel_launches == len(r.route.split(";")), (r.kernel_launches, r.route)
         open(os.path.join(out_dir, f"ok{rank}"), "w").write("ok")
     finally:
         dist.destroy_process_group()
