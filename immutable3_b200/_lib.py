@@ -17,6 +17,7 @@ COMM_HANDLE_BYTES = 64
 COL_INT, COL_TINYINT, COL_STRING, COL_COUNT, COL_DOUBLE, COL_INT64 = 0, 1, 2, 3, 4, 5
 AGG_FLAG_GLOBAL = 0x1  # IMM3_AGG_GLOBAL
 AGG_FLAG_ENCODED_FILTER = 0x4  # IMM3_AGG_ENCODED_FILTER
+DNF_FLAG_ENCODED_FILTER = 0x4  # IMM3_DNF_ENCODED_FILTER
 AGG_COUNT, AGG_MIN, AGG_MAX, AGG_SUM, AGG_AVG = 0, 1, 2, 3, 4
 CODEC_PFOR_INT, CODEC_DENSE_INT, CODEC_DENSE_TINYINT, CODEC_DENSE_STRING = 0, 1, 2, 3
 OP_GT, OP_LT, OP_EQ, OP_MATCH, OP_NOTMATCH, OP_NOOP = 1, 2, 3, 4, 5, 6
@@ -64,6 +65,7 @@ SIGNATURES = {
     "imm3_query": (C.c_int, [_P, C.c_char_p, C.POINTER(Pred), C.c_int, _STRS, C.c_int, C.c_int64, _PP]),
     "imm3_query_begin": (C.c_int, [_P, C.c_char_p, C.POINTER(Pred), C.c_int, _STRS, C.c_int, C.c_int64, _PP]),
     "imm3_query_begin_dnf": (C.c_int, [_P, C.c_char_p, C.POINTER(Pred), C.POINTER(C.c_int32), C.c_int, _STRS, C.c_int, C.c_int64, _PP]),
+    "imm3_query_begin_dnf_ext": (C.c_int, [_P, C.c_char_p, C.POINTER(Pred), C.POINTER(C.c_int32), C.c_int, _STRS, C.c_int, C.c_int64, C.c_uint32, _PP]),
     "imm3_result_local_count": (C.c_int64, [_P]),
     "imm3_comm_local_handle": (C.c_int, [_P, _P]),
     "imm3_comm_connect": (C.c_int, [_P, _P, C.c_int]),

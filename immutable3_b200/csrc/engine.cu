@@ -150,6 +150,7 @@ struct imm3_db {
     Buf d_scan_part;                         // offset_scan_kernel: epoch-tagged chunk sums (zeroed when (re)allocated)
     Buf d_tile_list;                         // offset_scan_kernel (block pipeline): the non-empty tiles, for the emit kernel
     Buf d_grp_sum;                           // blocks_group_emit_kernel: match counts per group of 1024 blocks (zero between queries)
+    Buf d_or_bitmap, d_or_cnt;               // real OR over encoded columns: a later term's block selection (words, counts)
     uint32_t scan_epoch = 0;
     Buf d_trace;                             // IMM3_TRACE debugging buffer
     // Emit-kernel feedback: result density class (1 dense, 0 sparse) last seen for a query shape (table, filter
@@ -458,6 +459,8 @@ void free_device_side(imm3_db* db) {
     if (db->d_scan_part.p) cudaFree(db->d_scan_part.p);
     if (db->d_tile_list.p) cudaFree(db->d_tile_list.p);
     if (db->d_grp_sum.p) cudaFree(db->d_grp_sum.p);
+    if (db->d_or_bitmap.p) cudaFree(db->d_or_bitmap.p);
+    if (db->d_or_cnt.p) cudaFree(db->d_or_cnt.p);
     if (db->d_work.p) cudaFree(db->d_work.p);
     if (db->d_agg_table.p) cudaFree(db->d_agg_table.p);
     if (db->d_agg_out.p) cudaFree(db->d_agg_out.p);
@@ -511,7 +514,9 @@ struct Prepared {
     size_t dyn_smem = 0;
     int grid = 0;
     // real OR (imm3_query_begin_dnf): the second and later conjunctions of the disjunction - their filter kernels run behind this
-    // plan's and OR their rows into its bitmap; counts, offsets and the emit kernels then see the union
+    // plan's and OR their rows into its bitmap; counts, offsets and the emit kernels then see the union.  On kBlocks (a term
+    // with a predicate on an encoded column, IMM3_DNF_ENCODED_FILTER) each term's block filter front runs into the term
+    // buffers and blocks_or_merge_kernel ORs that selection into this plan's.
     std::vector<std::unique_ptr<Prepared>> or_terms;
 };
 
@@ -602,6 +607,11 @@ int64_t prefix_rows_wanted(const LogicalPlan& lp) {
     if (!small_limit(lp)) return 0;
     const int64_t min_rows = getenv("IMM3_PREFIX_ROWS") ? std::max(1024, atoi(getenv("IMM3_PREFIX_ROWS"))) : (4 << 20);  // (tests shrink it)
     return std::max<int64_t>(min_rows, lp.limit * 64);
+}
+// ... as leading blocks of a block table (0: no prefix phase - the prefix would be half the table or more)
+int64_t prefix_blocks_wanted(const Prepared& pr) {
+    const int64_t nb = (prefix_rows_wanted(pr.lp) + 1023) / 1024;
+    return nb * 2 <= pr.table->nblocks ? nb : 0;
 }
 
 // The part of every device plan that does not depend on the pipeline: columns, literals, encoded-column slots, the L2 hint,
@@ -867,8 +877,7 @@ int fill_scan_plan(imm3_db* db, Prepared* pr) {
     }
     case Pipeline::kRowSpace:
     case Pipeline::kBlocks: {
-        const int64_t nb = (prefix + 1023) / 1024;
-        if (nb * 2 <= t.nblocks) pr->prefix_blocks = nb;
+        pr->prefix_blocks = prefix_blocks_wanted(*pr);
         rc = pr->pipeline == Pipeline::kRowSpace ? size_dense_filter(db, pr, &occ) : size_block_front(pr, &occ);
         if (rc || (rc = size_block_emit(db, pr))) return rc;
         break;
@@ -883,6 +892,32 @@ int fill_scan_plan(imm3_db* db, Prepared* pr) {
         break;
     }
     return plan_grid(db, pr, occ);
+}
+
+bool has_encoded_filter(const Prepared& pr) {
+    for (auto& f : pr.lp.filters)
+        if (is_pfor(*pr.table, f.col_idx)) return true;
+    return false;
+}
+
+// Real OR over encoded columns (IMM3_DNF_ENCODED_FILTER): every term on kBlocks - a term of dense predicates alone takes the
+// mini-block kernel, which decides them per block (what IMM3_NO_HYBRID runs for a conjunction).
+void force_blocks(Prepared* pr) {
+    pr->pipeline = Pipeline::kBlocks;
+    choose_block_filter(pr);
+}
+
+// ... the plan of every term but the first (which carries the projection and the emit plan, fill_scan_plan): its own filter
+// kernel, ring and pruning over the table's tiles of 8 blocks.  A prefix phase runs unless every term is pruned.
+int fill_or_terms_plan(imm3_db* db, Prepared* pr) {
+    bool pruned = pr->prune;
+    for (auto& tm : pr->or_terms) {
+        int occ = 0, rc = plan_columns(db, tm.get());
+        if (rc || (rc = size_block_front(tm.get(), &occ)) || (rc = plan_grid(db, tm.get(), occ))) return rc;
+        pruned = pruned && tm->prune;
+    }
+    pr->prefix_blocks = pruned ? 0 : prefix_blocks_wanted(*pr);
+    return 0;
 }
 
 int ensure_buf(Buf* b, size_t bytes) {
@@ -1115,8 +1150,9 @@ int ensure_block_filter(imm3_db* db, const Prepared* pr, int64_t nblocks) {
 // The block filter front, shared by Project queries (kBlocks) and aggregates over encoded predicates: [blocks_prune ->]
 // block filter kernel [-> offset scan, when `scan` and the filter kernel's last CTA does not run it].  Per block it leaves
 // the selected row count in d_span_cnt and - only for a partially selected block - the block's 32 words in d_bitmap.
-// Buffers: ensure_block_filter first.  grp_sum: blocks_group_emit_kernel follows (lane kernel only).
-int launch_block_filter_front(imm3_db* db, Prepared* pr, int64_t nblocks, int* launches, uint32_t* grp_sum, bool scan) {
+// Buffers: ensure_block_filter first.  grp_sum: blocks_group_emit_kernel follows (lane kernel only).  The selection goes to
+// (words, cnts): db->d_bitmap / d_span_cnt, or a later term's buffers of a real OR.
+int launch_block_filter_front(imm3_db* db, Prepared* pr, int64_t nblocks, int* launches, uint32_t* grp_sum, bool scan, uint32_t* words, uint32_t* cnts) {
     const TableStore& t = *pr->table;
     ScanPlan& sp = pr->sp;
     const int64_t ntiles = sp.ntiles;
@@ -1125,7 +1161,7 @@ int launch_block_filter_front(imm3_db* db, Prepared* pr, int64_t nblocks, int* l
     if (pr->prune) {
         // whole blocks decided from their min / max; only the tiles a window edge cuts through reach the filter kernel
         CUDA_TRY(cudaMemsetAsync(db->d_work.p, 0, 4, db->stream));
-        CUDA_TRY(launch_blocks_prune(pr->pp, t.d_row_start, nblocks, ntiles, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
+        CUDA_TRY(launch_blocks_prune(pr->pp, t.d_row_start, nblocks, ntiles, cnts, (uint32_t*)db->d_tile_cnt.p,
                                      (unsigned int*)db->d_work.p, db->num_sms, db->stream, grp_sum));
         note_launch(db, launches, "blocks_prune");
     }
@@ -1134,7 +1170,7 @@ int launch_block_filter_front(imm3_db* db, Prepared* pr, int64_t nblocks, int* l
         const int64_t per_cta = 32 * (lane ? pr->lane_warps : 1);
         filter_grid = (int)std::max<int64_t>(1, std::min<int64_t>(pr->grid, (nblocks + per_cta - 1) / per_cta));
     }
-    CUDA_TRY(launch_blocks_filter(sp, (uint32_t*)db->d_bitmap.p, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
+    CUDA_TRY(launch_blocks_filter(sp, words, cnts, (uint32_t*)db->d_tile_cnt.p,
                                   (unsigned long long*)db->d_tile_off.p, db->d_ctrl, nblocks, filter_grid, pr->dyn_smem, pr->block_filter,
                                   pr->lane_warps, work, db->stream, grp_sum));
     note_launch(db, launches, lane ? "blocks_filter_lane/w=" + std::to_string(pr->lane_warps) + "/s=" + std::to_string(sp.stages)
@@ -1142,20 +1178,54 @@ int launch_block_filter_front(imm3_db* db, Prepared* pr, int64_t nblocks, int* l
     return (scan && !sp.scan_inline) ? launch_scan_kernel(db, sp, ntiles, launches, true) : 0;
 }
 
+// Real OR over encoded columns: the scratch of every term's front, and the term buffers (grow-only).
+int ensure_or_terms(imm3_db* db, const Prepared* pr, int64_t nblocks) {
+    int rc;
+    for (auto& tm : pr->or_terms)
+        if ((rc = ensure_block_filter(db, tm.get(), nblocks))) return rc;
+    if ((rc = ensure_buf(&db->d_or_bitmap, (size_t)(nblocks * 32 + 2) * 4))) return rc;
+    return ensure_buf(&db->d_or_cnt, (size_t)(nblocks + 8 + 1024) * 4);
+}
+
+// ... behind the first term's front: each later term's front into the term buffers (no scan: the tile counts it leaves are
+// rewritten by the merge), then blocks_or_merge_kernel into d_bitmap / d_span_cnt.  Every term runs over the first term's
+// blocks and tiles - in a prefix phase too.
+int launch_or_merges(imm3_db* db, Prepared* pr, int64_t nblocks, int* launches) {
+    for (auto& up : pr->or_terms) {
+        Prepared* tm = up.get();
+        const int64_t ntiles = tm->sp.ntiles;
+        const int grid = tm->grid;
+        tm->sp.ntiles = pr->sp.ntiles;
+        tm->sp.scan_inline = 0;
+        tm->grid = (int)std::max<int64_t>(1, std::min<int64_t>(pr->sp.ntiles, grid));
+        const int rc = launch_block_filter_front(db, tm, nblocks, launches, nullptr, false, (uint32_t*)db->d_or_bitmap.p, (uint32_t*)db->d_or_cnt.p);
+        tm->sp.ntiles = ntiles;
+        tm->grid = grid;
+        if (rc) return rc;
+        CUDA_TRY(launch_blocks_or_merge(pr->table->d_row_start, nblocks, pr->sp.ntiles, (uint32_t*)db->d_bitmap.p, (uint32_t*)db->d_span_cnt.p,
+                                        (const uint32_t*)db->d_or_bitmap.p, (const uint32_t*)db->d_or_cnt.p, (uint32_t*)db->d_tile_cnt.p,
+                                        db->d_ctrl, db->num_sms, db->stream));
+        note_launch(db, launches, "blocks_or_merge");
+    }
+    return 0;
+}
+
 // kBlocks: [blocks_prune ->] block filter kernel -> group emit (lane kernel, one encoded column projected: every emit warp finds
 // its rows from the group sums, no scan), scan-emit (one encoded column projected: offset scan + emit in one small-footprint
-// kernel, resident while the filter kernel runs) or offset scan + block emit kernel.
+// kernel, resident while the filter kernel runs) or offset scan + block emit kernel.  A real OR over encoded columns merges
+// its later terms' fronts (launch_or_merges) before the emit; group emit needs a single term's group sums and is not used.
 int launch_blocks(imm3_db* db, Prepared* pr, int64_t nblocks, Queued* q) {
     ScanPlan& sp = pr->sp;
     const int64_t ntiles = sp.ntiles;
     const bool lane = pr->block_filter == BlockFilter::kLane;
+    const bool merge = !pr->or_terms.empty();
     int rc;
-    if ((rc = ensure_block_filter(db, pr, nblocks))) return rc;
-    sp.scan_inline = block_scan_inline(*pr);
+    if ((rc = ensure_block_filter(db, pr, nblocks)) || (merge && (rc = ensure_or_terms(db, pr, nblocks)))) return rc;
+    sp.scan_inline = merge ? 0 : block_scan_inline(*pr);
     int fused_grid = 0;  // > 0: blocks_scan_emit_kernel
     int group_grid = 0, ngroups = 0;  // > 0: blocks_group_emit_kernel
     if (sp.nproj == 1 && sp.proj[0].pfor_slot >= 0 && !getenv("IMM3_NO_SCANEMIT")) {
-        if (lane && !getenv("IMM3_NO_GROUPEMIT")) CUDA_TRY(blocks_group_emit_grid(db->num_sms, nblocks, &group_grid, &ngroups));
+        if (lane && !merge && !getenv("IMM3_NO_GROUPEMIT")) CUDA_TRY(blocks_group_emit_grid(db->num_sms, nblocks, &group_grid, &ngroups));
         if (group_grid > 0) {
             if (!db->d_grp_sum.p) {
                 CUDA_TRY(cudaMalloc(&db->d_grp_sum.p, blocks_group_sum_bytes()));
@@ -1175,7 +1245,11 @@ int launch_blocks(imm3_db* db, Prepared* pr, int64_t nblocks, Queued* q) {
     if ((rc = setup_phase_trace(db, sp, 1024))) return rc;
     CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
     const bool emit_scans = group_grid > 0 || fused_grid > 0;  // (these emit kernels find the offsets themselves)
-    if ((rc = launch_block_filter_front(db, pr, nblocks, q->launches, grp_sum, !emit_scans))) return rc;
+    if ((rc = launch_block_filter_front(db, pr, nblocks, q->launches, grp_sum, !emit_scans && !merge, (uint32_t*)db->d_bitmap.p,
+                                        (uint32_t*)db->d_span_cnt.p)))
+        return rc;
+    if (merge && ((rc = launch_or_merges(db, pr, nblocks, q->launches)) || (!emit_scans && (rc = launch_scan_kernel(db, sp, ntiles, q->launches, true)))))
+        return rc;
     CtrlBlock* const pub = q->publish ? db->h_ctrl : nullptr;
     const unsigned long long pub_seq = q->publish ? q->pub_seq : 0;
     if (emit_scans) {
@@ -1657,8 +1731,9 @@ int imm3_explain(imm3_db* db, const char* table, const imm3_pred* preds, int npr
 }
 
 // One conjunction (imm3_query_begin) or a disjunction of conjunctions (imm3_query_begin_dnf): terms[i] = (predicates, count).
+// encoded_or (IMM3_DNF_ENCODED_FILTER): a disjunction whose terms test an encoded column runs on the block pipeline.
 static int query_begin_terms(imm3_db* db, const char* table, const std::vector<std::pair<const imm3_pred*, int>>& terms,
-                             const char* const* proj_cols, int nproj, int64_t limit, imm3_result** out) {
+                             const char* const* proj_cols, int nproj, int64_t limit, imm3_result** out, bool encoded_or = false) {
     if (!db || !out) return fail(IMM3_ERR_INVALID_ARG, "imm3_query_begin: NULL argument");
     const double t_in = now_us();
     // validation before any device work; a term that can never hold (a wrong-length literal, an empty range) drops out of a
@@ -1676,6 +1751,15 @@ static int query_begin_terms(imm3_db* db, const char* table, const std::vector<s
     std::vector<std::unique_ptr<Prepared>> extra;
     for (size_t i = main_i + 1; i < prepared.size(); i++)
         if (!prepared[i]->lp.always_empty) extra.push_back(std::move(prepared[i]));
+    bool block_or = false;  // every term's block filter front, merged in block space (launch_or_merges)
+    if (encoded_or && !extra.empty()) {
+        block_or = has_encoded_filter(pr);
+        for (auto& tm : extra) block_or = block_or || has_encoded_filter(*tm);
+        const TableStore& t = *pr.table;
+        if (block_or && std::max(t.max_block_rows, t.meta.block_size) > 1024)
+            return fail(IMM3_ERR_UNSUPPORTED, "imm3_query_begin_dnf_ext: a disjunction over a sorted-int-codec column filters blocks of at most 1024 rows, table %s has blocks of %d",
+                        t.meta.name.c_str(), std::max(t.max_block_rows, t.meta.block_size));
+    }
     if ((rc = use_device(db))) return rc;
     const double t_plan = now_us();
     double t_dev = t_plan;
@@ -1700,10 +1784,17 @@ static int query_begin_terms(imm3_db* db, const char* table, const std::vector<s
         r->h_cols.emplace_back();
     }
     if (!pr.lp.always_empty && t.nrows > 0) {
+        if (block_or) {
+            force_blocks(&pr);
+            for (auto& tm : extra) force_blocks(tm.get());
+        }
         if ((rc = fill_scan_plan(db, &pr))) { give_back(); return rc; }
         for (int i = 0; i < r->ncols; i++) pr.sp.proj[i].out = (uint8_t*)r->d_cols[(size_t)i].p;
         pr.sp.bitmap = nullptr;
-        if (!extra.empty()) {
+        if (block_or) {
+            pr.or_terms = std::move(extra);
+            if ((rc = fill_or_terms_plan(db, &pr))) { give_back(); return rc; }
+        } else if (!extra.empty()) {
             // real OR: every term's predicates are decided by the row-space filter kernel (dense columns); a disjunction over
             // an encoded column would need the block filter kernels to accumulate as well - not built
             auto row_space = [](const Prepared& p) { return p.pipeline == Pipeline::kDense || p.pipeline == Pipeline::kRowSpace; };
@@ -1791,8 +1882,8 @@ int imm3_query_begin(imm3_db* db, const char* table, const imm3_pred* preds, int
     return query_begin_terms(db, table, {{preds, npreds}}, proj_cols, nproj, limit, out);
 }
 
-int imm3_query_begin_dnf(imm3_db* db, const char* table, const imm3_pred* preds, const int32_t* term_sizes, int nterms,
-                         const char* const* proj_cols, int nproj, int64_t limit, imm3_result** out) {
+static int query_begin_dnf(imm3_db* db, const char* table, const imm3_pred* preds, const int32_t* term_sizes, int nterms,
+                           const char* const* proj_cols, int nproj, int64_t limit, bool encoded_or, imm3_result** out) {
     if (!term_sizes || nterms < 1 || nterms > IMM3_MAX_OR_TERMS) return fail(IMM3_ERR_INVALID_ARG, "imm3_query_begin_dnf: 1 .. %d terms", IMM3_MAX_OR_TERMS);
     std::vector<std::pair<const imm3_pred*, int>> terms;
     int at = 0;
@@ -1802,7 +1893,19 @@ int imm3_query_begin_dnf(imm3_db* db, const char* table, const imm3_pred* preds,
         terms.push_back({preds + at, term_sizes[i]});
         at += term_sizes[i];
     }
-    return query_begin_terms(db, table, terms, proj_cols, nproj, limit, out);
+    return query_begin_terms(db, table, terms, proj_cols, nproj, limit, out, encoded_or);
+}
+
+int imm3_query_begin_dnf(imm3_db* db, const char* table, const imm3_pred* preds, const int32_t* term_sizes, int nterms,
+                         const char* const* proj_cols, int nproj, int64_t limit, imm3_result** out) {
+    return query_begin_dnf(db, table, preds, term_sizes, nterms, proj_cols, nproj, limit, false, out);
+}
+
+int imm3_query_begin_dnf_ext(imm3_db* db, const char* table, const imm3_pred* preds, const int32_t* term_sizes, int nterms,
+                             const char* const* proj_cols, int nproj, int64_t limit, uint32_t flags, imm3_result** out) {
+    const uint32_t known = IMM3_DNF_ENCODED_FILTER;
+    if (flags & ~known) return fail(IMM3_ERR_INVALID_ARG, "imm3_query_begin_dnf_ext: unknown flag bits 0x%x", flags & ~known);
+    return query_begin_dnf(db, table, preds, term_sizes, nterms, proj_cols, nproj, limit, (flags & IMM3_DNF_ENCODED_FILTER) != 0, out);
 }
 
 int64_t imm3_result_local_count(const imm3_result* r) { return r ? r->local_count : IMM3_ERR_INVALID_ARG; }
@@ -2062,7 +2165,8 @@ int launch_agg_local(imm3_db* db, AggQuery* q, AggEntry* out, int* launches) {
     CUDA_TRY(launch_agg_init(table, q->ap.table_slots, q->ap, counters, db->stream));
     note_launch(db, launches, "agg_init");
     if (q->enc_filter) {
-        const int rc = launch_block_filter_front(db, &pr, pr.table->nblocks, launches, nullptr, true);
+        const int rc = launch_block_filter_front(db, &pr, pr.table->nblocks, launches, nullptr, true, (uint32_t*)db->d_bitmap.p,
+                                                 (uint32_t*)db->d_span_cnt.p);
         if (rc) return rc;
     } else {
         CUDA_TRY(launch_filter(sp, (uint32_t*)db->d_bitmap.p, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,

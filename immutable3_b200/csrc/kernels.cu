@@ -9,6 +9,7 @@
 //                        results, TMA-streamed) or emit_kernel / emit_general_kernel (sparse results, gathers)
 //   k_blocks_multi.cuh   any query touching a sorted-int-codec column: blocks_filter_kernel (or the dense filter kernel in
 //                        row space when no predicate touches an encoded column) -> blocks_emit_kernel, one warp per block
+//   k_blocks_or.cuh      blocks_or_merge_kernel: real OR over encoded columns, the union of two block filter selections
 //   k_blocks_single.cuh  scan_blocks_kernel: single-pass block kernel with decoupled look-back (blocks > 1024 rows, bitmaps)
 //   k_rowspace.cuh       predicates (SIMD within a register), selection vectors, gathers, plan tables in shared memory
 //   k_ptx.cuh            mbarrier / TMA / L2-policy / relaxed-load helpers
@@ -38,6 +39,7 @@ namespace imm3 {
 #include "k_blocks_filter.cuh"
 #include "k_blocks_lane.cuh"
 #include "k_blocks_prune.cuh"
+#include "k_blocks_or.cuh"
 #include "k_comm.cuh"
 #include "k_agg.cuh"
 
@@ -180,6 +182,16 @@ cudaError_t launch_blocks_prune(const PrunePlan& q, const uint64_t* row_start, l
     const long long groups = (nblocks + 31) / 32;
     const long long grid = std::max<long long>(1, std::min<long long>((groups + kComputeWarps - 1) / kComputeWarps, (long long)num_sms * 8));
     blocks_prune_kernel<<<(unsigned)grid, kComputeThreads, 0, stream>>>(q, row_start, nblocks, ntiles8, blk_cnt, tile_cnt, work, grp_sum);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_blocks_or_merge(const uint64_t* row_start, long long nblocks, long long ntiles8, uint32_t* acc_words, uint32_t* acc_cnt,
+                                   const uint32_t* term_words, const uint32_t* term_cnt, uint32_t* tile_cnt, ScanCtrl* ctrl, int num_sms,
+                                   cudaStream_t stream) {
+    const long long groups = (nblocks + 31) / 32;
+    const long long grid = std::max<long long>(1, std::min<long long>((groups + kComputeWarps - 1) / kComputeWarps, (long long)num_sms * 8));
+    blocks_or_merge_kernel<<<(unsigned)grid, kComputeThreads, 0, stream>>>(row_start, nblocks, ntiles8, acc_words, acc_cnt, term_words, term_cnt,
+                                                                           tile_cnt, ctrl);
     return cudaGetLastError();
 }
 

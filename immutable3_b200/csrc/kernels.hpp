@@ -65,6 +65,11 @@ cudaError_t launch_block_stats(const PforCol& pc, const uint64_t* row_start, lon
                                cudaStream_t stream);
 cudaError_t launch_blocks_prune(const PrunePlan& q, const uint64_t* row_start, long long nblocks, long long ntiles8, uint32_t* blk_cnt,
                                 uint32_t* tile_cnt, unsigned int* work, int num_sms, cudaStream_t stream, uint32_t* grp_sum = nullptr);
+// Real OR over encoded columns: acc_* (the block filter's selection of the terms so far) |= term_* (the next term's), in the
+// same contract - every block's count, the words of partial blocks only - and every 8-block tile count rewritten.
+cudaError_t launch_blocks_or_merge(const uint64_t* row_start, long long nblocks, long long ntiles8, uint32_t* acc_words, uint32_t* acc_cnt,
+                                   const uint32_t* term_words, const uint32_t* term_cnt, uint32_t* tile_cnt, ScanCtrl* ctrl, int num_sms,
+                                   cudaStream_t stream);
 // rowspace: the bitmap / counts come from the dense filter kernel (row space), not from blocks_filter_kernel (block-local)
 cudaError_t launch_blocks_emit(const ScanPlan& plan, const uint32_t* bitmap, const uint32_t* cnts, const unsigned int* tile_list, const unsigned long long* tile_off,
                                long long nblocks, const ScanCtrl* ctrl, bool rowspace, bool pdl, int grid, size_t dyn_smem,

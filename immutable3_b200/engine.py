@@ -537,11 +537,12 @@ class Engine:
         """Engine.execute: the rows of the query in canonical order (iterate for Row objects).  `real_or=True` evaluates
         Or as a disjunction (imm3_query_begin_dnf) instead of the reference's Or == And (Engine.scala:236-245).
         `sum_avg=True` resolves Sum / Avg in a ProjectAgg query (imm3_query_agg_ext), which the reference refuses.
-        `encoded_filter=True` accepts predicates on sorted-int-codec columns in a ProjectAgg query (IMM3_AGG_ENCODED_FILTER)."""
+        `encoded_filter=True` accepts predicates on sorted-int-codec columns in a ProjectAgg query (IMM3_AGG_ENCODED_FILTER),
+        and with `real_or=True` in the terms of a disjunction (imm3_query_begin_dnf_ext, IMM3_DNF_ENCODED_FILTER)."""
         if isinstance(query.project, ProjectAgg):
             return self._call_agg(query, sum_avg=sum_avg, encoded_filter=encoded_filter)
         if real_or:
-            r = self.begin(query, real_or=True)
+            r = self.begin(query, real_or=True, encoded_filter=encoded_filter)
             return r.fetch(r.take)
         return self._call(self._lib.imm3_query, query)
 
@@ -550,10 +551,10 @@ class Engine:
         if isinstance(query.project, ProjectAgg):
             return self._call_agg(query, sum_avg=sum_avg, encoded_filter=encoded_filter)
         if real_or:
-            return self._call_dnf(query)
+            return self._call_dnf(query, encoded_filter)
         return self._call(self._lib.imm3_query_begin, query)
 
-    def _call_dnf(self, query: Query) -> Result:
+    def _call_dnf(self, query: Query, encoded_filter: bool = False) -> Result:
         if not isinstance(query.project, Project):
             raise L.Imm3Error(L.ERR_UNSUPPORTED, "only Project queries are on the scan/filter/project path")
         terms = select_dnf(query.select)
@@ -561,8 +562,12 @@ class Engine:
         sizes = (C.c_int32 * len(terms))(*[len(t) for t in terms])
         proj = L.cstr_array(list(query.project.cols))
         out = C.c_void_p()
-        L.check(self._lib.imm3_query_begin_dnf(self.sm.handle, query.table.encode(), preds, sizes, len(terms),
-                                               C.cast(proj, C.POINTER(C.c_char_p)), len(query.project.cols), int(query.project.limit), C.byref(out)))
+        args = (self.sm.handle, query.table.encode(), preds, sizes, len(terms), C.cast(proj, C.POINTER(C.c_char_p)), len(query.project.cols),
+                int(query.project.limit))
+        if encoded_filter:
+            L.check(self._lib.imm3_query_begin_dnf_ext(*args, L.DNF_FLAG_ENCODED_FILTER, C.byref(out)))
+        else:
+            L.check(self._lib.imm3_query_begin_dnf(*args, C.byref(out)))
         del keep
         return Result(out, self._lib, self.sm)
 

@@ -164,6 +164,19 @@ int64_t imm3_result_local_count(const imm3_result* r);
 #define IMM3_MAX_OR_TERMS 16
 int imm3_query_begin_dnf(imm3_db* db, const char* table, const imm3_pred* preds, const int32_t* term_sizes, int nterms,
                          const char* const* proj_cols, int nproj, int64_t limit, imm3_result** out);
+/* The same disjunction with options.  flags = 0: imm3_query_begin_dnf, word for word (rows, route, launches, status and
+ * message); unknown flag bits give IMM3_ERR_INVALID_ARG.
+ * IMM3_DNF_ENCODED_FILTER: a term may also hold ranges (GT / LT / EQ) on sorted-int-codec (PFOR_INT) columns, alone or beside
+ * dense predicates.  When at least two terms remain and one of them tests an encoded column, every term runs the block
+ * pipeline's filter front (blocks pruned from their min / max where the term's predicates allow it; a term of dense
+ * predicates alone takes the mini-block kernel) and blocks_or_merge ORs its per-block selection into the first term's, which
+ * the emit kernels then read: e.g. "blocks_prune;blocks_filter_lane/w=11/s=2;blocks_prune;blocks_filter_lane/w=11/s=2;
+ * blocks_or_merge;blocks_scan_emit".  Rows, order, LIMIT and the sharded count exchange are those of imm3_query_begin.
+ * The table's blocks must hold at most 1024 rows (else IMM3_ERR_UNSUPPORTED).  Terms that touch no encoded column take
+ * imm3_query_begin_dnf's row-space path; a single remaining term is the plain conjunction of imm3_query_begin. */
+#define IMM3_DNF_ENCODED_FILTER 0x4u /* the bit of IMM3_AGG_ENCODED_FILTER */
+int imm3_query_begin_dnf_ext(imm3_db* db, const char* table, const imm3_pred* preds, const int32_t* term_sizes, int nterms,
+                             const char* const* proj_cols, int nproj, int64_t limit, uint32_t flags, imm3_result** out);
 
 /* ---- The fan-in across GPUs: ResultQueueOp (ResultQueue.scala:7-56) + the queue of Engine.scala:166,190-196 ----
  * The reference funnels every worker's batches through one queue; across segment-sharded GPUs the ordered
@@ -270,7 +283,7 @@ double imm3_result_device_ms(const imm3_result* r);         /* CUDA-event time o
 int imm3_result_kernel_launches(const imm3_result* r);      /* kernels launched by begin                */
 /* The kernels imm3_query_begin / imm3_query_agg queued, in launch order, separated by ';' ("" when none ran): kernel names
  * (select_all, filter(tma|direct), offset_scan, emit_stream, emit, emit_general, blocks_prune, blocks_filter_lane,
- * blocks_filter_quad, blocks_filter, blocks_group_emit, blocks_scan_emit, blocks_emit(rowspace|blocks), scan_blocks,
+ * blocks_filter_quad, blocks_filter, blocks_or_merge, blocks_group_emit, blocks_scan_emit, blocks_emit(rowspace|blocks), scan_blocks,
  * count_exchange, agg_init, agg<NG,NA>, agg_blocks<NG,NA>, agg_compact, agg_exchange, agg_merge) with "/key=value" parameters: /s= ring stages,
  * /w= warps per CTA of the lane kernel, /ctas= the group emit kernel's grid; "/prefix" marks the prefix pass of a small
  * LIMIT; "/sum" the SUM instantiation of agg<NG,NA> / agg_blocks<NG,NA> (imm3_query_agg_ext with a Sum or Avg); "/bsel" (after
