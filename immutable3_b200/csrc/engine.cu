@@ -61,8 +61,6 @@ inline double now_us() {
     clock_gettime(CLOCK_MONOTONIC, &ts);
     return (double)ts.tv_sec * 1e6 + (double)ts.tv_nsec * 1e-3;
 }
-thread_local double g_t_launched = 0, g_t_synced = 0;  // stamps taken inside run_scan_once (last launch queued / GPU done)
-thread_local bool g_eager_times = false;               // two-phase LIMIT queries add their phases' device times up: no lazy reading
 
 // Grow-only cache of device / pinned-host buffers: result columns are handed back on
 // imm3_result_free and reused by the next query (cudaMalloc / cudaMallocHost cost milliseconds).
@@ -158,8 +156,6 @@ struct imm3_db {
     // for any result, so a stale hint costs time, never rows.
     std::unordered_map<std::string, int> emit_hint;
     std::string explain_buf;
-    std::string route;         // kernels queued by the query in progress (imm3_result_route), in launch order
-    const char* route_tag = "";  // appended to every name: "/prefix" while the prefix pass of a small LIMIT is queued
 };
 
 struct imm3_result {
@@ -181,8 +177,7 @@ struct imm3_result {
     unsigned long long timing_seq = 0;
     double stage_ms[2] = {0, 0};
     double host_us[5] = {0, 0, 0, 0, 0};  // wall clock inside imm3_query_begin: plan, buffers + device plan, launches, wait for the GPU, epilogue
-    int launches = 0;
-    std::string route;  // imm3_result_route: "kernel[/key=value...];kernel..." in launch order
+    std::string route;  // imm3_result_route: "kernel[/key=value...];kernel..." in launch order, an entry per kernel launch
     int64_t alg_bytes = 0;
 };
 
@@ -203,13 +198,19 @@ int use_device(imm3_db* db) {
     return 0;
 }
 
-// Route of the query in progress (imm3_result_route): one entry per queued kernel, recorded on the host only.
-void note_launch(imm3_db* db, int* launches, const std::string& name) {
-    if (launches) (*launches)++;
-    if (!db->route.empty()) db->route += ';';
-    db->route += name;
-    db->route += db->route_tag;
-}
+// What one query reports about its launches, created by the entry point and passed down.
+struct Run {
+    std::string route;     // imm3_result_route: one entry per queued kernel, in launch order, recorded on the host only
+    const char* tag = "";  // appended to every entry: "/prefix" while phase A of a small LIMIT is queued
+    double t_launched = 0, t_synced = 0;  // host stamps of the last phase: last launch queued, GPU done
+    bool eager_times = false;             // a two-phase LIMIT query adds its phases' device times up: no lazy reading
+    double device_ms = 0, stage_ms[2] = {0, 0};
+    void note(const std::string& name) {
+        if (!route.empty()) route += ';';
+        route += name;
+        route += tag;
+    }
+};
 std::string with_stages(const char* name, int stages) { return std::string(name) + "/s=" + std::to_string(stages); }
 // the kernel launch_filter picks for this plan
 std::string filter_route(const ScanPlan& sp) {
@@ -952,7 +953,7 @@ int ensure_row_space(imm3_db* db, ScanPlan& sp) {
 
 // Launch the count-exchange kernel of one round (every rank of the communicator must launch the same rounds in the same
 // order).  has_count = 0: this rank ran no kernel in this query (empty slice) and contributes 0.
-int launch_exchange(imm3_db* db, int64_t limit, int has_count, unsigned long long pub_seq = 0) {
+int launch_exchange(imm3_db* db, Run* run, int64_t limit, int has_count, unsigned long long pub_seq = 0) {
     CommPlan cp;
     std::memset(&cp, 0, sizeof cp);
     cp.pub = pub_seq ? db->h_ctrl : nullptr;
@@ -966,14 +967,14 @@ int launch_exchange(imm3_db* db, int64_t limit, int has_count, unsigned long lon
     cp.limit = limit;
     cp.timeout_ns = db->comm_timeout_ns;
     CUDA_TRY(launch_count_exchange(cp, db->d_ctrl, &reinterpret_cast<CtrlBlock*>(db->d_ctrl)->x, db->stream));
-    note_launch(db, nullptr, "count_exchange");  // (the caller counts the launch where it has a count)
+    run->note("count_exchange");
     return 0;
 }
 
 // A round of the exchange without a scan of this rank's own: its slice is empty (has_count = 0) or its previous phase
 // already covered the whole slice (has_count = 1: ctrl->total still holds that count).
-int exchange_only(imm3_db* db, int64_t limit, int has_count) {
-    int rc = launch_exchange(db, limit, has_count);
+int exchange_only(imm3_db* db, Run* run, int64_t limit, int has_count) {
+    int rc = launch_exchange(db, run, limit, has_count);
     if (rc) return rc;
     CUDA_TRY(cudaMemcpyAsync(db->h_ctrl, db->d_ctrl, sizeof(CtrlBlock), cudaMemcpyDeviceToHost, db->stream));
     CUDA_TRY(cudaStreamSynchronize(db->stream));
@@ -992,8 +993,8 @@ bool scan_inline_for(int64_t ntiles) {
     }
     return ntiles <= scan_inline_max_tiles();
 }
-// ... for the block filter front (the lane kernel's inline scan is written for 8 warps)
-int block_scan_inline(const Prepared& pr) { return scan_inline_for(pr.sp.ntiles) && !(pr.block_filter == BlockFilter::kLane && pr.lane_warps < 8); }
+// ... for the block filter front over `ntiles` tiles (the lane kernel's inline scan is written for 8 warps)
+int block_scan_inline(const Prepared& pr, int64_t ntiles) { return scan_inline_for(ntiles) && !(pr.block_filter == BlockFilter::kLane && pr.lane_warps < 8); }
 int prepare_scan_buffers(imm3_db* db, int64_t ntiles, bool want_list) {
     if (want_list) {
         int rc = ensure_buf(&db->d_tile_list, (size_t)(ntiles + 16) * 4);
@@ -1011,37 +1012,42 @@ int prepare_scan_buffers(imm3_db* db, int64_t ntiles, bool want_list) {
     if (((++db->scan_epoch) & 0xFFFFFFu) == 0) ++db->scan_epoch;  // (tag 0 = never written)
     return 0;
 }
-int launch_scan_kernel(imm3_db* db, const ScanPlan& sp, int64_t ntiles, int* launches, bool want_list = false) {
+int launch_scan_kernel(imm3_db* db, const ScanPlan& sp, int64_t ntiles, Run* run, bool want_list = false) {
     int rc = prepare_scan_buffers(db, ntiles, want_list);
     if (rc) return rc;
     CUDA_TRY(launch_offset_scan((const uint32_t*)db->d_tile_cnt.p, (unsigned long long*)db->d_tile_off.p, ntiles, sp.limit, db->scan_epoch,
                                 (unsigned long long*)db->d_scan_part.p, db->d_ctrl, want_list ? (unsigned int*)db->d_tile_list.p : nullptr, db->stream));
-    note_launch(db, launches, "offset_scan");
+    run->note("offset_scan");
     return 0;
 }
 
-// Real OR: the filter kernels of the later terms, behind the first term's (same bitmap, same span / tile counts: every pass
-// rewrites the counts of the union so far; only the last pass may run the inline offset scan).
-int launch_or_terms(imm3_db* db, Prepared* pr, int scan_inline, int* launches) {
-    for (size_t i = 0; i < pr->or_terms.size(); i++) {
-        Prepared* tm = pr->or_terms[i].get();
-        tm->sp.bitmap = pr->sp.bitmap;
-        tm->sp.or_accumulate = 1;
-        tm->sp.nrows = pr->sp.nrows;
-        tm->sp.ntiles = pr->sp.ntiles;
-        tm->sp.limit = pr->sp.limit;
-        tm->sp.debug = pr->sp.debug;
-        tm->sp.scan_inline = (i + 1 == pr->or_terms.size()) ? scan_inline : 0;
-        CUDA_TRY(launch_filter(tm->sp, tm->sp.bitmap, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p, (unsigned long long*)db->d_tile_off.p,
-                               db->d_ctrl, (int)std::max<int64_t>(1, std::min<int64_t>(tm->grid, tm->sp.ntiles)), tm->dyn_smem, db->stream));
-        note_launch(db, launches, filter_route(tm->sp));
-    }
-    return 0;
+// The part of the slice one phase scans (see small_limit): all of it, or phase A's leading prefix_rows rows or prefix_blocks
+// blocks.
+struct Extent {
+    int64_t nrows, ntiles, nblocks;
+};
+Extent phase_extent(const Prepared& pr, bool prefix) {
+    const TableStore& t = *pr.table;
+    const int64_t nb = pr.prefix_blocks;
+    if (!prefix) return {pr.sp.nrows, pr.sp.ntiles, t.nblocks};
+    if (pr.prefix_rows > 0) return {pr.prefix_rows, pr.prefix_rows / kDenseTileRowsPerWord, nb};
+    if (pr.pipeline != Pipeline::kRowSpace) return {pr.sp.nrows, (nb + 7) / 8, nb};
+    const int64_t rows = (int64_t)t.row_start[(size_t)nb];
+    return {rows, (rows + kDenseTileRowsPerWord - 1) / kDenseTileRowsPerWord, nb};
+}
+// A filter kernel's grid over a phase's tiles: its plan's persistent grid, fewer CTAs for a shorter phase.
+int phase_grid(const Prepared& p, int64_t ntiles) { return (int)std::max<int64_t>(1, std::min<int64_t>(p.grid, ntiles)); }
+// A later term's device plan of a real OR in one phase: its own, over the first term's rows, tiles and bitmap.
+ScanPlan term_plan(const Prepared& tm, const ScanPlan& first) {
+    ScanPlan sp = tm.sp;
+    sp.nrows = first.nrows;
+    sp.ntiles = first.ntiles;
+    sp.bitmap = first.bitmap;
+    return sp;
 }
 
 // What a pipeline's launch function tells the epilogue of run_scan_once.
 struct Queued {
-    int* launches;
     unsigned long long pub_seq;  // publish (plan.hpp): sequence number of this launch sequence
     bool publish;                // the pipeline's last kernel may write the pinned control block itself
     bool published = false;      // ... and does
@@ -1070,33 +1076,38 @@ int setup_phase_trace(imm3_db* db, ScanPlan& sp, size_t extra) {
     return 0;
 }
 
-// The filter kernel over the row space (from ev0 on), the later terms of a real OR, and the offset scan unless the filter
-// kernel's last CTA runs it.
-int launch_row_space_filter(imm3_db* db, Prepared* pr, int* launches) {
-    ScanPlan& sp = pr->sp;
-    const int scan_inline = (sp.nfilter == 0 || scan_inline_for(sp.ntiles)) ? 1 : 0;
-    sp.scan_inline = pr->or_terms.empty() ? scan_inline : 0;
+// The filter kernel over the row space (from ev0 on) - for a real OR the first term's, then each later term's, ORing its rows
+// into the same bitmap (same span / tile counts: every pass rewrites the counts of the union so far) - and the offset scan
+// unless the last pass's last CTA runs it.
+int launch_row_space_filter(imm3_db* db, const Prepared& pr, ScanPlan& sp, Run* run) {
+    const bool scan_inline = sp.nfilter == 0 || scan_inline_for(sp.ntiles);
+    auto filter = [&](const Prepared& p, ScanPlan& f, bool last) {
+        f.scan_inline = last && scan_inline;
+        CUDA_TRY(launch_filter(f, sp.bitmap, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p, (unsigned long long*)db->d_tile_off.p,
+                               db->d_ctrl, phase_grid(p, f.ntiles), p.dyn_smem, db->stream));
+        run->note(filter_route(f));
+        return 0;
+    };
     CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
-    CUDA_TRY(launch_filter(sp, sp.bitmap, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p, (unsigned long long*)db->d_tile_off.p,
-                           db->d_ctrl, pr->grid, pr->dyn_smem, db->stream));
-    note_launch(db, launches, filter_route(sp));
-    int rc = launch_or_terms(db, pr, scan_inline, launches);
+    int rc = filter(pr, sp, pr.or_terms.empty());
+    for (size_t i = 0; !rc && i < pr.or_terms.size(); i++) {
+        ScanPlan term = term_plan(*pr.or_terms[i], sp);
+        rc = filter(*pr.or_terms[i], term, i + 1 == pr.or_terms.size());
+    }
     if (rc) return rc;
-    sp.scan_inline = scan_inline;
-    return scan_inline ? 0 : launch_scan_kernel(db, sp, sp.ntiles, launches);
+    return scan_inline ? 0 : launch_scan_kernel(db, sp, sp.ntiles, run);
 }
 
 // kDense: filter kernel -> emit kernels.  Two emit kernels, one of which does the work: which one is decided on the device
 // from the match count, unless an earlier query of this shape said which (see emit_hint).
-int launch_dense(imm3_db* db, Prepared* pr, Queued* q) {
-    ScanPlan& sp = pr->sp;
+int launch_dense(imm3_db* db, const Prepared& pr, ScanPlan& sp, Run* run, Queued* q) {
     int rc;
     if ((rc = setup_phase_trace(db, sp, 0)) || (rc = ensure_row_space(db, sp))) return rc;
-    const int stream_ok = pr->emit_stage_bytes > 0 && sp.nproj > 0;
+    const int stream_ok = pr.emit_stage_bytes > 0 && sp.nproj > 0;
     const char* force = getenv("IMM3_EMIT");  // experiment: "stream" / "gather" = that kernel takes every result, "both" = no feedback
     int hint = -1;
     if (stream_ok && !(force && !strcmp(force, "both"))) {
-        auto it = db->emit_hint.find(pr->shape_key);
+        auto it = db->emit_hint.find(pr.shape_key);
         if (it != db->emit_hint.end()) hint = it->second;
         if (force && !strcmp(force, "stream")) hint = 1;
         if (force && !strcmp(force, "gather")) hint = 0;
@@ -1105,46 +1116,45 @@ int launch_dense(imm3_db* db, Prepared* pr, Queued* q) {
     // The first emit kernel is launched as a programmatic dependent of the filter kernel (its prologue overlaps the filter
     // kernel's tail); IMM3_NO_PDL=1 restores per-stage timing.
     const bool pdl = sp.nproj > 0 && !getenv("IMM3_NO_PDL");
-    if ((rc = launch_row_space_filter(db, pr, q->launches)) || (rc = mark_mid(db, pdl, q))) return rc;
+    if ((rc = launch_row_space_filter(db, pr, sp, run)) || (rc = mark_mid(db, pdl, q))) return rc;
     if (sp.nproj == 0) return 0;
     const int64_t nspans = sp.ntiles * (kDenseTileRowsPerWord / 1024);
     if (stream_ok && !only_gather) {
         CUDA_TRY(launch_emit_stream(sp, sp.bitmap, (const uint32_t*)db->d_span_cnt.p, (const uint32_t*)db->d_tile_cnt.p,
-                                    (const unsigned long long*)db->d_tile_off.p, sp.ntiles, pr->emit_ring, pr->emit_stage_bytes,
-                                    only_stream ? -1 : 1, pr->grid_emit_stream, pr->emit_smem, db->d_ctrl, pdl, db->stream));
-        note_launch(db, q->launches, with_stages("emit_stream", pr->emit_ring));
+                                    (const unsigned long long*)db->d_tile_off.p, sp.ntiles, pr.emit_ring, pr.emit_stage_bytes,
+                                    only_stream ? -1 : 1, pr.grid_emit_stream, pr.emit_smem, db->d_ctrl, pdl, db->stream));
+        run->note(with_stages("emit_stream", pr.emit_ring));
     }
     if (!only_stream) {
         CUDA_TRY(launch_emit(sp, sp.bitmap, (const uint32_t*)db->d_span_cnt.p, (const unsigned long long*)db->d_tile_off.p, 8,
-                             nspans, pr->grid_emit, stream_ok && !only_gather, db->d_ctrl, pr->emit_general, pdl && (only_gather || !stream_ok),
+                             nspans, pr.grid_emit, stream_ok && !only_gather, db->d_ctrl, pr.emit_general, pdl && (only_gather || !stream_ok),
                              db->stream));
-        note_launch(db, q->launches, pr->emit_general ? "emit_general" : "emit");
+        run->note(pr.emit_general ? "emit_general" : "emit");
     }
     return 0;
 }
 
 // kRowSpace: filter kernel over the row space -> block emit kernel.
-int launch_row_space(imm3_db* db, Prepared* pr, int64_t nblocks, Queued* q) {
-    ScanPlan& sp = pr->sp;
+int launch_row_space(imm3_db* db, const Prepared& pr, ScanPlan& sp, int64_t nblocks, Run* run, Queued* q) {
     const bool pdl = sp.nproj > 0 && !getenv("IMM3_NO_PDL");
     int rc;
-    if ((rc = ensure_row_space(db, sp)) || (rc = launch_row_space_filter(db, pr, q->launches)) || (rc = mark_mid(db, pdl, q))) return rc;
+    if ((rc = ensure_row_space(db, sp)) || (rc = launch_row_space_filter(db, pr, sp, run)) || (rc = mark_mid(db, pdl, q))) return rc;
     if (sp.nproj == 0) return 0;
     CUDA_TRY(launch_blocks_emit(sp, sp.bitmap, (const uint32_t*)db->d_span_cnt.p, nullptr, (const unsigned long long*)db->d_tile_off.p,
-                                nblocks, db->d_ctrl, true, pdl, (int)std::min<int64_t>(pr->grid_blocks_emit, (nblocks + 7) / 8),
-                                pr->blocks_emit_smem, db->stream));
-    note_launch(db, q->launches, "blocks_emit(rowspace)");
+                                nblocks, db->d_ctrl, true, pdl, (int)std::min<int64_t>(pr.grid_blocks_emit, (nblocks + 7) / 8),
+                                pr.blocks_emit_smem, db->stream));
+    run->note("blocks_emit(rowspace)");
     return 0;
 }
 
-// Scratch of the block filter front: 32 bitmap words and one count per block, tile counts and offsets, and (pruned) the
-// work list of the tiles blocks_prune_kernel leaves to the filter kernel.
-int ensure_block_filter(imm3_db* db, const Prepared* pr, int64_t nblocks) {
+// Scratch of the block filter front over `ntiles` tiles: 32 bitmap words and one count per block, tile counts and offsets,
+// and (pruned) the work list of the tiles blocks_prune_kernel leaves to the filter kernel.
+int ensure_block_filter(imm3_db* db, const Prepared& pr, int64_t ntiles, int64_t nblocks) {
     int rc;
     if ((rc = ensure_buf(&db->d_bitmap, (size_t)(nblocks * 32 + 2) * 4))) return rc;
     if ((rc = ensure_buf(&db->d_span_cnt, (size_t)(nblocks + 8 + 1024) * 4))) return rc;  // (+ whole 16-byte loads of a group's counts)
-    if ((rc = ensure_tile_scratch(db, pr->sp.ntiles))) return rc;
-    return pr->prune ? ensure_buf(&db->d_work, (size_t)((nblocks + 7) / 8 + 2) * 4) : 0;
+    if ((rc = ensure_tile_scratch(db, ntiles))) return rc;
+    return pr.prune ? ensure_buf(&db->d_work, (size_t)((nblocks + 7) / 8 + 2) * 4) : 0;
 }
 
 // The block filter front, shared by Project queries (kBlocks) and aggregates over encoded predicates: [blocks_prune ->]
@@ -1152,60 +1162,53 @@ int ensure_block_filter(imm3_db* db, const Prepared* pr, int64_t nblocks) {
 // the selected row count in d_span_cnt and - only for a partially selected block - the block's 32 words in d_bitmap.
 // Buffers: ensure_block_filter first.  grp_sum: blocks_group_emit_kernel follows (lane kernel only).  The selection goes to
 // (words, cnts): db->d_bitmap / d_span_cnt, or a later term's buffers of a real OR.
-int launch_block_filter_front(imm3_db* db, Prepared* pr, int64_t nblocks, int* launches, uint32_t* grp_sum, bool scan, uint32_t* words, uint32_t* cnts) {
-    const TableStore& t = *pr->table;
-    ScanPlan& sp = pr->sp;
+int launch_block_filter_front(imm3_db* db, const Prepared& pr, const ScanPlan& sp, int64_t nblocks, Run* run, uint32_t* grp_sum, bool scan,
+                              uint32_t* words, uint32_t* cnts) {
+    const TableStore& t = *pr.table;
     const int64_t ntiles = sp.ntiles;
-    const bool lane = pr->block_filter == BlockFilter::kLane;
-    const unsigned int* work = pr->prune ? (const unsigned int*)db->d_work.p : nullptr;
-    if (pr->prune) {
+    const bool lane = pr.block_filter == BlockFilter::kLane;
+    const unsigned int* work = pr.prune ? (const unsigned int*)db->d_work.p : nullptr;
+    if (pr.prune) {
         // whole blocks decided from their min / max; only the tiles a window edge cuts through reach the filter kernel
         CUDA_TRY(cudaMemsetAsync(db->d_work.p, 0, 4, db->stream));
-        CUDA_TRY(launch_blocks_prune(pr->pp, t.d_row_start, nblocks, ntiles, cnts, (uint32_t*)db->d_tile_cnt.p,
+        CUDA_TRY(launch_blocks_prune(pr.pp, t.d_row_start, nblocks, ntiles, cnts, (uint32_t*)db->d_tile_cnt.p,
                                      (unsigned int*)db->d_work.p, db->num_sms, db->stream, grp_sum));
-        note_launch(db, launches, "blocks_prune");
+        run->note("blocks_prune");
     }
-    int filter_grid = pr->grid;
-    if (pr->block_filter != BlockFilter::kMini) {  // CTA tiles of 32 blocks (quad), 32 blocks per warp (lane)
-        const int64_t per_cta = 32 * (lane ? pr->lane_warps : 1);
-        filter_grid = (int)std::max<int64_t>(1, std::min<int64_t>(pr->grid, (nblocks + per_cta - 1) / per_cta));
+    int filter_grid = phase_grid(pr, ntiles);
+    if (pr.block_filter != BlockFilter::kMini) {  // CTA tiles of 32 blocks (quad), 32 blocks per warp (lane)
+        const int64_t per_cta = 32 * (lane ? pr.lane_warps : 1);
+        filter_grid = (int)std::max<int64_t>(1, std::min<int64_t>(filter_grid, (nblocks + per_cta - 1) / per_cta));
     }
     CUDA_TRY(launch_blocks_filter(sp, words, cnts, (uint32_t*)db->d_tile_cnt.p,
-                                  (unsigned long long*)db->d_tile_off.p, db->d_ctrl, nblocks, filter_grid, pr->dyn_smem, pr->block_filter,
-                                  pr->lane_warps, work, db->stream, grp_sum));
-    note_launch(db, launches, lane ? "blocks_filter_lane/w=" + std::to_string(pr->lane_warps) + "/s=" + std::to_string(sp.stages)
-                                   : with_stages(pr->block_filter == BlockFilter::kQuad ? "blocks_filter_quad" : "blocks_filter", sp.stages));
-    return (scan && !sp.scan_inline) ? launch_scan_kernel(db, sp, ntiles, launches, true) : 0;
+                                  (unsigned long long*)db->d_tile_off.p, db->d_ctrl, nblocks, filter_grid, pr.dyn_smem, pr.block_filter,
+                                  pr.lane_warps, work, db->stream, grp_sum));
+    run->note(lane ? "blocks_filter_lane/w=" + std::to_string(pr.lane_warps) + "/s=" + std::to_string(sp.stages)
+                   : with_stages(pr.block_filter == BlockFilter::kQuad ? "blocks_filter_quad" : "blocks_filter", sp.stages));
+    return (scan && !sp.scan_inline) ? launch_scan_kernel(db, sp, ntiles, run, true) : 0;
 }
 
 // Real OR over encoded columns: the scratch of every term's front, and the term buffers (grow-only).
-int ensure_or_terms(imm3_db* db, const Prepared* pr, int64_t nblocks) {
+int ensure_or_terms(imm3_db* db, const Prepared& pr, int64_t nblocks) {
     int rc;
-    for (auto& tm : pr->or_terms)
-        if ((rc = ensure_block_filter(db, tm.get(), nblocks))) return rc;
+    for (auto& tm : pr.or_terms)
+        if ((rc = ensure_block_filter(db, *tm, tm->sp.ntiles, nblocks))) return rc;
     if ((rc = ensure_buf(&db->d_or_bitmap, (size_t)(nblocks * 32 + 2) * 4))) return rc;
     return ensure_buf(&db->d_or_cnt, (size_t)(nblocks + 8 + 1024) * 4);
 }
 
-// ... behind the first term's front: each later term's front into the term buffers (no scan: the tile counts it leaves are
-// rewritten by the merge), then blocks_or_merge_kernel into d_bitmap / d_span_cnt.  Every term runs over the first term's
-// blocks and tiles - in a prefix phase too.
-int launch_or_merges(imm3_db* db, Prepared* pr, int64_t nblocks, int* launches) {
-    for (auto& up : pr->or_terms) {
-        Prepared* tm = up.get();
-        const int64_t ntiles = tm->sp.ntiles;
-        const int grid = tm->grid;
-        tm->sp.ntiles = pr->sp.ntiles;
-        tm->sp.scan_inline = 0;
-        tm->grid = (int)std::max<int64_t>(1, std::min<int64_t>(pr->sp.ntiles, grid));
-        const int rc = launch_block_filter_front(db, tm, nblocks, launches, nullptr, false, (uint32_t*)db->d_or_bitmap.p, (uint32_t*)db->d_or_cnt.p);
-        tm->sp.ntiles = ntiles;
-        tm->grid = grid;
+// ... behind the first term's front: each later term's front into the term buffers, then blocks_or_merge_kernel into
+// d_bitmap / d_span_cnt.  Every term runs over the first term's blocks and tiles - in a prefix phase too - and runs no scan:
+// the tile counts it leaves are rewritten by the merge (a term's plan keeps the scan_inline = 0 of plan_columns).
+int launch_or_merges(imm3_db* db, const Prepared& pr, const ScanPlan& sp, int64_t nblocks, Run* run) {
+    for (auto& tm : pr.or_terms) {
+        const int rc = launch_block_filter_front(db, *tm, term_plan(*tm, sp), nblocks, run, nullptr, false, (uint32_t*)db->d_or_bitmap.p,
+                                                 (uint32_t*)db->d_or_cnt.p);
         if (rc) return rc;
-        CUDA_TRY(launch_blocks_or_merge(pr->table->d_row_start, nblocks, pr->sp.ntiles, (uint32_t*)db->d_bitmap.p, (uint32_t*)db->d_span_cnt.p,
+        CUDA_TRY(launch_blocks_or_merge(pr.table->d_row_start, nblocks, sp.ntiles, (uint32_t*)db->d_bitmap.p, (uint32_t*)db->d_span_cnt.p,
                                         (const uint32_t*)db->d_or_bitmap.p, (const uint32_t*)db->d_or_cnt.p, (uint32_t*)db->d_tile_cnt.p,
                                         db->d_ctrl, db->num_sms, db->stream));
-        note_launch(db, launches, "blocks_or_merge");
+        run->note("blocks_or_merge");
     }
     return 0;
 }
@@ -1214,14 +1217,12 @@ int launch_or_merges(imm3_db* db, Prepared* pr, int64_t nblocks, int* launches) 
 // its rows from the group sums, no scan), scan-emit (one encoded column projected: offset scan + emit in one small-footprint
 // kernel, resident while the filter kernel runs) or offset scan + block emit kernel.  A real OR over encoded columns merges
 // its later terms' fronts (launch_or_merges) before the emit; group emit needs a single term's group sums and is not used.
-int launch_blocks(imm3_db* db, Prepared* pr, int64_t nblocks, Queued* q) {
-    ScanPlan& sp = pr->sp;
+int launch_blocks(imm3_db* db, const Prepared& pr, ScanPlan& sp, int64_t nblocks, Run* run, Queued* q) {
     const int64_t ntiles = sp.ntiles;
-    const bool lane = pr->block_filter == BlockFilter::kLane;
-    const bool merge = !pr->or_terms.empty();
+    const bool lane = pr.block_filter == BlockFilter::kLane;
+    const bool merge = !pr.or_terms.empty();
     int rc;
-    if ((rc = ensure_block_filter(db, pr, nblocks)) || (merge && (rc = ensure_or_terms(db, pr, nblocks)))) return rc;
-    sp.scan_inline = merge ? 0 : block_scan_inline(*pr);
+    if ((rc = ensure_block_filter(db, pr, ntiles, nblocks)) || (merge && (rc = ensure_or_terms(db, pr, nblocks)))) return rc;
     int fused_grid = 0;  // > 0: blocks_scan_emit_kernel
     int group_grid = 0, ngroups = 0;  // > 0: blocks_group_emit_kernel
     if (sp.nproj == 1 && sp.proj[0].pfor_slot >= 0 && !getenv("IMM3_NO_SCANEMIT")) {
@@ -1232,23 +1233,20 @@ int launch_blocks(imm3_db* db, Prepared* pr, int64_t nblocks, Queued* q) {
                 db->d_grp_sum.cap = blocks_group_sum_bytes();
                 CUDA_TRY(cudaMemsetAsync(db->d_grp_sum.p, 0, db->d_grp_sum.cap, db->stream));
             }
-            sp.scan_inline = 0;
         } else {
             CUDA_TRY(blocks_scan_emit_grid(db->num_sms, ntiles, &fused_grid));
-            if (fused_grid > 0) {
-                if ((rc = prepare_scan_buffers(db, ntiles, true))) return rc;
-                sp.scan_inline = 0;
-            }
+            if (fused_grid > 0 && (rc = prepare_scan_buffers(db, ntiles, true))) return rc;
         }
     }
+    const bool emit_scans = group_grid > 0 || fused_grid > 0;  // (these emit kernels find the offsets themselves)
+    sp.scan_inline = !merge && !emit_scans && block_scan_inline(pr, ntiles);
     uint32_t* const grp_sum = group_grid > 0 ? (uint32_t*)db->d_grp_sum.p : nullptr;
     if ((rc = setup_phase_trace(db, sp, 1024))) return rc;
     CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
-    const bool emit_scans = group_grid > 0 || fused_grid > 0;  // (these emit kernels find the offsets themselves)
-    if ((rc = launch_block_filter_front(db, pr, nblocks, q->launches, grp_sum, !emit_scans && !merge, (uint32_t*)db->d_bitmap.p,
+    if ((rc = launch_block_filter_front(db, pr, sp, nblocks, run, grp_sum, !emit_scans && !merge, (uint32_t*)db->d_bitmap.p,
                                         (uint32_t*)db->d_span_cnt.p)))
         return rc;
-    if (merge && ((rc = launch_or_merges(db, pr, nblocks, q->launches)) || (!emit_scans && (rc = launch_scan_kernel(db, sp, ntiles, q->launches, true)))))
+    if (merge && ((rc = launch_or_merges(db, pr, sp, nblocks, run)) || (!emit_scans && (rc = launch_scan_kernel(db, sp, ntiles, run, true)))))
         return rc;
     CtrlBlock* const pub = q->publish ? db->h_ctrl : nullptr;
     const unsigned long long pub_seq = q->publish ? q->pub_seq : 0;
@@ -1258,12 +1256,12 @@ int launch_blocks(imm3_db* db, Prepared* pr, int64_t nblocks, Queued* q) {
         if (group_grid > 0) {
             CUDA_TRY(launch_blocks_group_emit(sp, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, grp_sum, nblocks, ngroups,
                                               db->d_ctrl, pdl, group_grid, db->stream, pub, pub_seq));
-            note_launch(db, q->launches, "blocks_group_emit/ctas=" + std::to_string(group_grid));
+            run->note("blocks_group_emit/ctas=" + std::to_string(group_grid));
         } else {
             CUDA_TRY(launch_blocks_scan_emit(sp, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, (const uint32_t*)db->d_tile_cnt.p,
                                              (unsigned long long*)db->d_tile_off.p, nblocks, db->scan_epoch, (unsigned long long*)db->d_scan_part.p,
                                              db->d_ctrl, (unsigned int*)db->d_tile_list.p, pdl, fused_grid, db->stream, pub, pub_seq));
-            note_launch(db, q->launches, "blocks_scan_emit");
+            run->note("blocks_scan_emit");
         }
         q->published = q->publish;
     } else {
@@ -1273,44 +1271,44 @@ int launch_blocks(imm3_db* db, Prepared* pr, int64_t nblocks, Queued* q) {
             CUDA_TRY(launch_blocks_emit(sp, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p,
                                         sp.scan_inline ? nullptr : (const unsigned int*)db->d_tile_list.p,
                                         (const unsigned long long*)db->d_tile_off.p, nblocks, db->d_ctrl, false, pdl,
-                                        (int)std::min<int64_t>(pr->grid_blocks_emit, (nblocks + 7) / 8), pr->blocks_emit_smem, db->stream));
-            note_launch(db, q->launches, "blocks_emit(blocks)");
+                                        (int)std::min<int64_t>(pr.grid_blocks_emit, (nblocks + 7) / 8), pr.blocks_emit_smem, db->stream));
+            run->note("blocks_emit(blocks)");
         }
     }
     return 0;
 }
 
-// Launch the kernels of one query and wait for the match count.
-int run_scan_once(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* launches, double* stage_ms, int64_t nblocks_use, bool exchange) {
-    pr->sp.scan_inline = 1;
-    *launches = 0;
+// Launch the kernels of one phase over `ex` and wait for the match count.
+int run_scan_once(imm3_db* db, const Prepared& pr, const Extent& ex, Run* run, int64_t* total, bool exchange) {
+    ScanPlan sp = pr.sp;  // this phase's device plan: the pipeline binds its bitmap and decides scan_inline
+    sp.nrows = ex.nrows;
+    sp.ntiles = ex.ntiles;
     // publish (plan.hpp): the query's last kernel writes the pinned control block itself and the host polls it
     const bool publish_ok = !getenv("IMM3_NO_PUBLISH");
     const bool sharded = exchange && db->comm_on;  // (a sharded table: the exchange kernel publishes)
-    Queued q{launches, ++db->pub_seq, publish_ok && !sharded};
+    Queued q{++db->pub_seq, publish_ok && !sharded};
     int rc = 0;
-    switch (pr->pipeline) {
-    case Pipeline::kDense: rc = launch_dense(db, pr, &q); break;
-    case Pipeline::kRowSpace: rc = launch_row_space(db, pr, nblocks_use, &q); break;
-    case Pipeline::kBlocks: rc = launch_blocks(db, pr, nblocks_use, &q); break;
+    switch (pr.pipeline) {
+    case Pipeline::kDense: rc = launch_dense(db, pr, sp, run, &q); break;
+    case Pipeline::kRowSpace: rc = launch_row_space(db, pr, sp, ex.nblocks, run, &q); break;
+    case Pipeline::kBlocks: rc = launch_blocks(db, pr, sp, ex.nblocks, run, &q); break;
     case Pipeline::kSinglePass:
         CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
-        CUDA_TRY(launch_scan_blocks(pr->sp, db->d_ctrl, db->d_status, pr->grid, pr->dyn_smem, db->stream));
-        note_launch(db, launches, "scan_blocks");
+        CUDA_TRY(launch_scan_blocks(sp, db->d_ctrl, db->d_status, pr.grid, pr.dyn_smem, db->stream));
+        run->note("scan_blocks");
         break;
     }
     if (rc) return rc;
     if (sharded) {
         // The per-rank counts are exchanged by the GPUs themselves (k_comm.cuh), behind the query's last kernel: no host
         // round trip between the kernels and the exchange, one synchronisation per query.
-        if ((rc = launch_exchange(db, pr->sp.limit, 1, publish_ok ? q.pub_seq : 0))) return rc;
-        (*launches)++;
+        if ((rc = launch_exchange(db, run, sp.limit, 1, publish_ok ? q.pub_seq : 0))) return rc;
         q.published = publish_ok;
     }
     CUDA_TRY(cudaEventRecord(db->ev1, db->stream));
     db->ev_seq = ++db->query_seq;
     if (q.published) {
-        g_t_launched = now_us();
+        run->t_launched = now_us();
         const volatile unsigned long long* ps = &db->h_ctrl->pub_seq;
         bool seen = false;
         for (unsigned spins = 0;; spins++) {
@@ -1324,7 +1322,7 @@ int run_scan_once(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* la
                 seen = true;
                 break;
             }
-            if ((spins & 0xFFFu) == 0xFFFu && now_us() - g_t_launched > 2e5) break;  // 0.2 s: something is wrong - ask the runtime
+            if ((spins & 0xFFFu) == 0xFFFu && now_us() - run->t_launched > 2e5) break;  // 0.2 s: something is wrong - ask the runtime
 #if defined(__x86_64__)
             __builtin_ia32_pause();
 #endif
@@ -1333,43 +1331,39 @@ int run_scan_once(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* la
             CUDA_TRY(cudaMemcpyAsync(db->h_ctrl, db->d_ctrl, sizeof(CtrlBlock) - sizeof(unsigned long long), cudaMemcpyDeviceToHost, db->stream));
             CUDA_TRY(cudaStreamSynchronize(db->stream));
         }
-        g_t_synced = now_us();
+        run->t_synced = now_us();
     } else {
         CUDA_TRY(cudaMemcpyAsync(db->h_ctrl, db->d_ctrl, sizeof(CtrlBlock) - sizeof(unsigned long long), cudaMemcpyDeviceToHost, db->stream));
-        g_t_launched = now_us();
+        run->t_launched = now_us();
         CUDA_TRY(cudaStreamSynchronize(db->stream));
-        g_t_synced = now_us();
+        run->t_synced = now_us();
     }
     if (db->h_ctrl->c.error) return fail(IMM3_ERR_CUDA, "kernel watchdog fired (code %u)", db->h_ctrl->c.error);
     if (sharded && db->h_ctrl->x.error)
         return fail(IMM3_ERR_COMM, "count exchange: a peer's count did not arrive within %llu ms (ranks must issue the same queries in the same order)",
                     db->comm_timeout_ns / 1000000ull);
-    if (q.published && !q.have_mid && !g_eager_times && !getenv("IMM3_EAGER_TIMES")) {
-        *ms = -1.0;  // read lazily (imm3_result_device_ms): the events complete a moment after the publish, waiting for them here costs 2-3 us
-        if (stage_ms) stage_ms[0] = -1.0, stage_ms[1] = 0;
+    if (q.published && !q.have_mid && !run->eager_times && !getenv("IMM3_EAGER_TIMES")) {
+        run->device_ms = -1.0;  // read lazily (imm3_result_device_ms): the events complete a moment after the publish, waiting for them here costs 2-3 us
+        run->stage_ms[0] = -1.0, run->stage_ms[1] = 0;
     } else {
-        float f = 0;
+        float f = 0, a = 0, b = 0;
         if (q.published) CUDA_TRY(cudaEventSynchronize(db->ev1));
         CUDA_TRY(cudaEventElapsedTime(&f, db->ev0, db->ev1));
-        *ms = f;
-        if (stage_ms) {
-            stage_ms[0] = f;
-            stage_ms[1] = 0;
-            if (q.have_mid) {
-                float a = 0, b = 0;
-                CUDA_TRY(cudaEventElapsedTime(&a, db->ev0, db->ev_mid));
-                CUDA_TRY(cudaEventElapsedTime(&b, db->ev_mid, db->ev1));
-                stage_ms[0] = a;
-                stage_ms[1] = b;
-            }
+        a = f;
+        if (q.have_mid) {
+            CUDA_TRY(cudaEventElapsedTime(&a, db->ev0, db->ev_mid));
+            CUDA_TRY(cudaEventElapsedTime(&b, db->ev_mid, db->ev1));
         }
+        run->device_ms += f;  // (two-phase LIMIT queries: the phases' times add up)
+        run->stage_ms[0] += a;
+        run->stage_ms[1] += b;
     }
     *total = (int64_t)db->h_ctrl->c.total;
-    if (pr->pipeline == Pipeline::kDense && pr->sp.nproj > 0 && pr->emit_stage_bytes > 0)  // feedback for the next query of this shape
-        db->emit_hint[pr->shape_key] = (db->h_ctrl->c.total > 0 && db->h_ctrl->c.dense_rows * 2 >= db->h_ctrl->c.total) ? 1 : 0;
-    if (pr->sp.trace) {
+    if (pr.pipeline == Pipeline::kDense && sp.nproj > 0 && pr.emit_stage_bytes > 0)  // feedback for the next query of this shape
+        db->emit_hint[pr.shape_key] = (db->h_ctrl->c.total > 0 && db->h_ctrl->c.dense_rows * 2 >= db->h_ctrl->c.total) ? 1 : 0;
+    if (sp.trace) {
         unsigned long long h[64];
-        CUDA_TRY(cudaMemcpy(h, pr->sp.trace, sizeof h, cudaMemcpyDeviceToHost));
+        CUDA_TRY(cudaMemcpy(h, sp.trace, sizeof h, cudaMemcpyDeviceToHost));
         if (FILE* f = fopen(getenv("IMM3_TRACE"), "w")) {
             const char* names[] = {"K1 entry", "K1 cta done", "K1 scan start", "K1 scan end", "K3s entry", "K3s first tile", "K3s cta done", "-",
                                    "K3b entry", "K3b dep ready", "K3b tiles seen", "K3b tile meta", "K3b block start", "K3b block done", "K3b warp done", "K3b words here", "K3b store start", "K3b store done"};
@@ -1378,9 +1372,9 @@ int run_scan_once(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* la
                     fprintf(f, "%-16s min %9.2f us  max %9.2f us\n", names[i], (double)(h[2 * i] - h[0]) / 1e3, (double)(h[2 * i + 1] - h[0]) / 1e3);
             for (int i = 0; i < 8; i++)
                 if (h[32 + i] != ~0ull && h[32 + i] != 0) fprintf(f, "scan round %d after block scan: %9.2f us\n", i, (double)(h[32 + i] - h[0]) / 1e3);
-            if (pr->block_filter == BlockFilter::kLane) {  // per CTA of the lane kernel: done time, SM, tiles decided
+            if (pr.block_filter == BlockFilter::kLane) {  // per CTA of the lane kernel: done time, SM, tiles decided
                 std::vector<unsigned long long> pc(1024);
-                if (cudaMemcpy(pc.data(), pr->sp.trace + 64, 1024 * 8, cudaMemcpyDeviceToHost) == cudaSuccess)
+                if (cudaMemcpy(pc.data(), sp.trace + 64, 1024 * 8, cudaMemcpyDeviceToHost) == cudaSuccess)
                     for (int i = 0; i < 512 && pc[2 * i]; i++)
                         fprintf(f, "cta %3d done %9.2f us  sm %3llu  tiles %llu\n", i, (double)(pc[2 * i] - h[0]) / 1e3, pc[2 * i + 1] >> 32, pc[2 * i + 1] & 0xFFFFFFFFull);
             }
@@ -1391,55 +1385,19 @@ int run_scan_once(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* la
 }
 
 // Launch the kernels of one query and wait for the match count (see small_limit for the two-phase LIMIT).
-int run_scan(imm3_db* db, Prepared* pr, double* ms, int64_t* total, int* launches, double* stage_ms = nullptr) {
-    TableStore& t = *pr->table;
-    const bool comm = db->comm_on && !pr->for_bitmap;
-    const bool local_prefix = pr->prefix_blocks > 0 || pr->prefix_rows > 0;
-    const bool two_phase = comm ? small_limit(pr->lp) : local_prefix;
-    db->route.clear();
-    if (!two_phase) return run_scan_once(db, pr, ms, total, launches, stage_ms, t.nblocks, comm);
-    struct EagerGuard {
-        EagerGuard() { g_eager_times = true; }
-        ~EagerGuard() { g_eager_times = false; }
-    } eager_guard;
+int run_scan(imm3_db* db, const Prepared& pr, Run* run, int64_t* total) {
+    const bool comm = db->comm_on && !pr.for_bitmap;
+    const bool local_prefix = pr.prefix_blocks > 0 || pr.prefix_rows > 0;
+    if (!(comm ? small_limit(pr.lp) : local_prefix)) return run_scan_once(db, pr, phase_extent(pr, false), run, total, comm);
     // phase A: the leading blocks / rows only
-    const ScanPlan full = pr->sp;
-    const int grid_full = pr->grid;
-    int64_t nb = t.nblocks;
-    if (local_prefix) {
-        nb = pr->prefix_blocks;
-        if (pr->prefix_rows > 0) {
-            pr->sp.nrows = pr->prefix_rows;
-            pr->sp.ntiles = pr->prefix_rows / kDenseTileRowsPerWord;
-        } else if (pr->pipeline == Pipeline::kRowSpace) {
-            pr->sp.nrows = (int64_t)t.row_start[(size_t)nb];
-            pr->sp.ntiles = (pr->sp.nrows + kDenseTileRowsPerWord - 1) / kDenseTileRowsPerWord;
-        } else {
-            pr->sp.ntiles = (nb + 7) / 8;
-        }
-        pr->grid = (int)std::max<int64_t>(1, std::min<int64_t>(pr->sp.ntiles, grid_full));
-    }
-    double ms_a = 0, st_a[2] = {0, 0};
-    int launches_a = 0;
-    if (local_prefix) db->route_tag = "/prefix";
-    int rc = run_scan_once(db, pr, &ms_a, total, &launches_a, st_a, nb, comm);
-    db->route_tag = "";
-    pr->sp = full;
-    pr->grid = grid_full;
-    if (rc) return rc;
-    *ms = ms_a;
-    *launches = launches_a;
-    if (stage_ms) stage_ms[0] = st_a[0], stage_ms[1] = st_a[1];
-    if (comm ? (int64_t)db->h_ctrl->x.counts[0] >= pr->lp.limit : *total >= pr->lp.limit) return 0;
+    run->eager_times = true;
+    if (local_prefix) run->tag = "/prefix";
+    int rc = run_scan_once(db, pr, phase_extent(pr, local_prefix), run, total, comm);
+    run->tag = "";
+    if (rc || (comm ? (int64_t)db->h_ctrl->x.counts[0] >= pr.lp.limit : *total >= pr.lp.limit)) return rc;
     // phase B: the prefix did not fill the LIMIT - the whole table
-    if (!local_prefix) return exchange_only(db, pr->sp.limit, 1);  // (comm only: phase A was this rank's whole slice already)
-    double ms_b = 0, st_b[2] = {0, 0};
-    int launches_b = 0;
-    if ((rc = run_scan_once(db, pr, &ms_b, total, &launches_b, st_b, t.nblocks, comm))) return rc;
-    *ms += ms_b;
-    *launches += launches_b;
-    if (stage_ms) stage_ms[0] += st_b[0], stage_ms[1] += st_b[1];
-    return 0;
+    if (!local_prefix) return exchange_only(db, run, pr.sp.limit, 1);  // (comm only: phase A was this rank's whole slice already)
+    return run_scan_once(db, pr, phase_extent(pr, false), run, total, comm);
 }
 
 // java.lang.Double.toString for an integral value of int32 magnitude (all Min/MaxDoubleAggr ever hold here): "18.0",
@@ -1730,148 +1688,184 @@ int imm3_explain(imm3_db* db, const char* table, const imm3_pred* preds, int npr
     return 0;
 }
 
-// One conjunction (imm3_query_begin) or a disjunction of conjunctions (imm3_query_begin_dnf): terms[i] = (predicates, count).
-// encoded_or (IMM3_DNF_ENCODED_FILTER): a disjunction whose terms test an encoded column runs on the block pipeline.
-static int query_begin_terms(imm3_db* db, const char* table, const std::vector<std::pair<const imm3_pred*, int>>& terms,
-                             const char* const* proj_cols, int nproj, int64_t limit, imm3_result** out, bool encoded_or = false) {
-    if (!db || !out) return fail(IMM3_ERR_INVALID_ARG, "imm3_query_begin: NULL argument");
-    const double t_in = now_us();
-    // validation before any device work; a term that can never hold (a wrong-length literal, an empty range) drops out of a
-    // disjunction; the first term that can hold carries the query, the others only add their filter kernels
+namespace {
+
+// Validation and logical plan of every term, before any device work.  A term that can never hold (a wrong-length literal, an
+// empty range) drops out of a disjunction; the first term that can hold carries the query, the others only add their filter
+// kernels.
+int plan_terms(imm3_db* db, const char* table, const std::vector<std::pair<const imm3_pred*, int>>& terms, const char* const* proj_cols,
+               int nproj, int64_t limit, std::unique_ptr<Prepared>* main, std::vector<std::unique_ptr<Prepared>>* extra) {
     std::vector<std::unique_ptr<Prepared>> prepared;
-    int rc = 0;
     for (auto& tm : terms) {
-        std::unique_ptr<Prepared> p(new Prepared());
-        if ((rc = prepare(db, table, tm.first, tm.second, proj_cols, nproj, limit, false, p.get()))) return rc;
-        prepared.push_back(std::move(p));
+        prepared.emplace_back(new Prepared());
+        if (int rc = prepare(db, table, tm.first, tm.second, proj_cols, nproj, limit, false, prepared.back().get())) return rc;
     }
     size_t main_i = 0;
     while (main_i + 1 < prepared.size() && prepared[main_i]->lp.always_empty) main_i++;
-    Prepared& pr = *prepared[main_i];
-    std::vector<std::unique_ptr<Prepared>> extra;
+    *main = std::move(prepared[main_i]);
     for (size_t i = main_i + 1; i < prepared.size(); i++)
-        if (!prepared[i]->lp.always_empty) extra.push_back(std::move(prepared[i]));
-    bool block_or = false;  // every term's block filter front, merged in block space (launch_or_merges)
-    if (encoded_or && !extra.empty()) {
-        block_or = has_encoded_filter(pr);
-        for (auto& tm : extra) block_or = block_or || has_encoded_filter(*tm);
-        const TableStore& t = *pr.table;
-        if (block_or && std::max(t.max_block_rows, t.meta.block_size) > 1024)
-            return fail(IMM3_ERR_UNSUPPORTED, "imm3_query_begin_dnf_ext: a disjunction over a sorted-int-codec column filters blocks of at most 1024 rows, table %s has blocks of %d",
-                        t.meta.name.c_str(), std::max(t.max_block_rows, t.meta.block_size));
-    }
-    if ((rc = use_device(db))) return rc;
-    const double t_plan = now_us();
-    double t_dev = t_plan;
-    g_t_launched = g_t_synced = 0;
-    TableStore& t = *pr.table;
-    std::unique_ptr<imm3_result> r(new imm3_result());
-    r->db = db;
-    r->ncols = (int)pr.lp.proj.size();
+        if (!prepared[i]->lp.always_empty) extra->push_back(std::move(prepared[i]));
+    return 0;
+}
+
+// How a disjunction runs: every term's filter kernel over the row space, ORing into one bitmap (launch_row_space_filter), or -
+// block_or: encoded_or and a term tests an encoded column - every term's block filter front, merged in block space
+// (launch_or_merges).
+int choose_or(const Prepared& pr, const std::vector<std::unique_ptr<Prepared>>& extra, bool encoded_or, bool* block_or) {
+    if (!encoded_or || extra.empty()) return 0;
+    *block_or = has_encoded_filter(pr);
+    for (auto& tm : extra) *block_or = *block_or || has_encoded_filter(*tm);
+    const TableStore& t = *pr.table;
+    if (*block_or && std::max(t.max_block_rows, t.meta.block_size) > 1024)
+        return fail(IMM3_ERR_UNSUPPORTED, "imm3_query_begin_dnf_ext: a disjunction over a sorted-int-codec column filters blocks of at most 1024 rows, table %s has blocks of %d",
+                    t.meta.name.c_str(), std::max(t.max_block_rows, t.meta.block_size));
+    return 0;
+}
+
+// The result's schema, and a device column of up to `limit` rows per projected column.
+int result_columns(imm3_db* db, const Prepared& pr, int64_t limit, imm3_result* r) {
+    const TableStore& t = *pr.table;
     const int64_t capacity = limit > 0 ? std::min<int64_t>(limit, t.nrows) : t.nrows;
-    auto give_back = [&]() {
-        for (auto& b : r->d_cols) db->dev_pool.release(b);
-        r->d_cols.clear();
-    };
+    r->ncols = (int)pr.lp.proj.size();
     for (int i = 0; i < r->ncols; i++) {
         const ColumnMeta& c = t.meta.cols[(size_t)pr.lp.proj[(size_t)i]];
         r->names.push_back(c.name);
         r->types.push_back(c.ctype);
         r->widths.push_back(c.width);
         Buf b;
-        if ((rc = db->dev_pool.acquire((size_t)capacity * (size_t)c.width, &b))) { give_back(); return rc; }
+        if (int rc = db->dev_pool.acquire((size_t)capacity * (size_t)c.width, &b)) return rc;
         r->d_cols.push_back(b);
         r->h_cols.emplace_back();
     }
-    if (!pr.lp.always_empty && t.nrows > 0) {
-        if (block_or) {
-            force_blocks(&pr);
-            for (auto& tm : extra) force_blocks(tm.get());
-        }
-        if ((rc = fill_scan_plan(db, &pr))) { give_back(); return rc; }
-        for (int i = 0; i < r->ncols; i++) pr.sp.proj[i].out = (uint8_t*)r->d_cols[(size_t)i].p;
-        pr.sp.bitmap = nullptr;
-        if (block_or) {
-            pr.or_terms = std::move(extra);
-            if ((rc = fill_or_terms_plan(db, &pr))) { give_back(); return rc; }
-        } else if (!extra.empty()) {
-            // real OR: every term's predicates are decided by the row-space filter kernel (dense columns); a disjunction over
-            // an encoded column would need the block filter kernels to accumulate as well - not built
-            auto row_space = [](const Prepared& p) { return p.pipeline == Pipeline::kDense || p.pipeline == Pipeline::kRowSpace; };
-            bool ok = row_space(pr);
-            for (auto& tm : extra) {
-                if ((rc = fill_scan_plan(db, tm.get()))) { give_back(); return rc; }
-                ok = ok && row_space(*tm);
-            }
-            if (!ok) {
-                give_back();
-                return fail(IMM3_ERR_UNSUPPORTED, "imm3_query_begin_dnf: a disjunction needs every predicate on a dense (DENSE_INT / DENSE_TINYINT / DENSE_STRING) column");
-            }
-            pr.or_terms = std::move(extra);
-        }
-        t_dev = now_us();
-        if ((rc = run_scan(db, &pr, &r->device_ms, &r->local_count, &r->launches, r->stage_ms))) { give_back(); return rc; }
-        r->timing_seq = db->ev_seq;
-    } else if (db->comm_on && !pr.lp.always_empty) {
-        // Empty slice (more ranks than segments): this rank still takes part in every round of the exchange.  (A predicate
-        // that can never hold is a property of the query, known to every rank: nobody exchanges anything.)
-        const int64_t lim = limit > 0 ? limit : INT64_MAX;
-        db->route.clear();
-        if ((rc = exchange_only(db, lim, 0))) { give_back(); return rc; }
-        if (small_limit(pr.lp) && (int64_t)db->h_ctrl->x.counts[0] < pr.lp.limit && (rc = exchange_only(db, lim, 0))) { give_back(); return rc; }
-        r->launches = 1;
+    return 0;
+}
+
+// The device plans of the main term, which writes the result's columns, and of the OR terms.
+int plan_device(imm3_db* db, Prepared* pr, std::vector<std::unique_ptr<Prepared>> extra, bool block_or, const imm3_result& r) {
+    if (block_or) {
+        force_blocks(pr);
+        for (auto& tm : extra) force_blocks(tm.get());
     }
-    r->route = r->launches > 0 ? db->route : std::string();
-    // Global placement of this rank's rows (SURVEY.md 8e): from the on-device exchange, or trivially for a single handle.
-    r->world = 1;
+    int rc = fill_scan_plan(db, pr);
+    if (rc) return rc;
+    for (int i = 0; i < r.ncols; i++) pr->sp.proj[i].out = (uint8_t*)r.d_cols[(size_t)i].p;
+    if (block_or) {
+        pr->or_terms = std::move(extra);
+        return fill_or_terms_plan(db, pr);
+    }
+    if (extra.empty()) return 0;
+    // real OR: every term's predicates are decided by the row-space filter kernel (dense columns); a disjunction over
+    // an encoded column would need the block filter kernels to accumulate as well - not built
+    auto row_space = [](const Prepared& p) { return p.pipeline == Pipeline::kDense || p.pipeline == Pipeline::kRowSpace; };
+    bool ok = row_space(*pr);
+    for (auto& tm : extra) {
+        if ((rc = fill_scan_plan(db, tm.get()))) return rc;
+        ok = ok && row_space(*tm);
+        tm->sp.or_accumulate = 1;
+    }
+    if (!ok) return fail(IMM3_ERR_UNSUPPORTED, "imm3_query_begin_dnf: a disjunction needs every predicate on a dense (DENSE_INT / DENSE_TINYINT / DENSE_STRING) column");
+    pr->or_terms = std::move(extra);
+    return 0;
+}
+
+// This rank's scan, or - its slice is empty (more ranks than segments) - its part in every round of the exchange.  (A
+// predicate that can never hold is a property of the query, known to every rank: nobody exchanges anything.)
+int run_query(imm3_db* db, const Prepared& pr, bool local, Run* run, imm3_result* r) {
+    if (local) {
+        const int rc = run_scan(db, pr, run, &r->local_count);
+        r->timing_seq = db->ev_seq;
+        return rc;
+    }
+    if (!db->comm_on || pr.lp.always_empty) return 0;
+    const int64_t lim = pr.lp.limit > 0 ? pr.lp.limit : INT64_MAX;
+    int rc = exchange_only(db, run, lim, 0);
+    if (!rc && small_limit(pr.lp) && (int64_t)db->h_ctrl->x.counts[0] < pr.lp.limit) rc = exchange_only(db, run, lim, 0);
+    return rc;
+}
+
+// Global placement of this rank's rows (SURVEY.md 8e): from the on-device exchange, or trivially for a single handle.
+void place_rows(const imm3_db* db, const LogicalPlan& lp, imm3_result* r) {
+    r->world = db->comm_on ? db->world : 1;
     r->g_offset = 0;
     r->g_take = r->g_total = r->local_count;
     r->rank_counts[0] = r->local_count;
-    if (db->comm_on && !pr.lp.always_empty) {
-        const CommOut& x = db->h_ctrl->x;
-        r->world = db->world;
-        r->g_offset = (int64_t)x.g_offset;
-        r->g_take = (int64_t)x.g_take;
-        r->g_total = (int64_t)x.g_total;
-        for (int i = 0; i < db->world; i++) r->rank_counts[i] = (int64_t)x.counts[i];
-    } else if (db->comm_on) {
-        r->world = db->world;
-    }
-    // Algorithmic bytes (SURVEY.md §8d): filter columns' encoded bytes once + per surviving row the
-    // project-only widths read and every projected width written (+ 4 B/block for PFOR offsets).
-    {
-        int64_t a = 0, per_row = 0;
-        std::vector<int> seen;
-        auto count_filters = [&](const LogicalPlan& lp) {
-            for (auto& f : lp.filters) {
-                if (std::find(seen.begin(), seen.end(), f.col_idx) != seen.end()) continue;  // (a column several terms of a disjunction test: once)
-                const ColumnStore& c = t.cols[(size_t)f.col_idx];
-                a += c.encoded_bytes + (c.meta.codec == IMM3_CODEC_PFOR_INT ? 4 * t.nblocks : 0);
-                seen.push_back(f.col_idx);
-            }
-        };
-        count_filters(pr.lp);
-        for (auto& tm : pr.or_terms) count_filters(tm->lp);
-        for (int ci : pr.lp.proj) {
+    if (!db->comm_on || lp.always_empty) return;
+    const CommOut& x = db->h_ctrl->x;
+    r->g_offset = (int64_t)x.g_offset;
+    r->g_take = (int64_t)x.g_take;
+    r->g_total = (int64_t)x.g_total;
+    for (int i = 0; i < db->world; i++) r->rank_counts[i] = (int64_t)x.counts[i];
+}
+
+// Algorithmic bytes (SURVEY.md §8d): filter columns' encoded bytes once + per surviving row the
+// project-only widths read and every projected width written (+ 4 B/block for PFOR offsets).
+int64_t query_alg_bytes(const Prepared& pr, int64_t rows) {
+    const TableStore& t = *pr.table;
+    int64_t a = 0, per_row = 0;
+    std::vector<int> seen;
+    auto count_filters = [&](const LogicalPlan& lp) {
+        for (auto& f : lp.filters) {
+            if (std::find(seen.begin(), seen.end(), f.col_idx) != seen.end()) continue;  // (a column several terms of a disjunction test: once)
+            const ColumnStore& c = t.cols[(size_t)f.col_idx];
+            a += c.encoded_bytes + (c.meta.codec == IMM3_CODEC_PFOR_INT ? 4 * t.nblocks : 0);
+            seen.push_back(f.col_idx);
+        }
+    };
+    count_filters(pr.lp);
+    for (auto& tm : pr.or_terms) count_filters(tm->lp);
+    for (int ci : pr.lp.proj) {
+        per_row += t.cols[(size_t)ci].meta.width;
+        if (std::find(seen.begin(), seen.end(), ci) == seen.end()) {
             per_row += t.cols[(size_t)ci].meta.width;
-            if (std::find(seen.begin(), seen.end(), ci) == seen.end()) {
-                per_row += t.cols[(size_t)ci].meta.width;
-                seen.push_back(ci);
-            }
+            seen.push_back(ci);
         }
-        r->alg_bytes = a + per_row * r->local_count;
     }
+    return a + per_row * rows;
+}
+
+// The launch record and the times: device and stage times, and the wall clock inside imm3_query_begin by phase - plan,
+// buffers + device plan, launches, wait for the GPU, epilogue (two-phase LIMIT queries: the last phase's stamps).
+void report_run(imm3_result* r, const Run& run, double t_in, double t_plan, double t_dev) {
+    const double t_out = now_us();
+    r->route = run.route;
+    r->device_ms = run.device_ms;
+    r->stage_ms[0] = run.stage_ms[0], r->stage_ms[1] = run.stage_ms[1];
+    r->host_us[0] = t_plan - t_in;
+    r->host_us[1] = t_dev - t_plan;
+    if (run.t_launched > 0) {
+        r->host_us[2] = run.t_launched - t_dev;
+        r->host_us[3] = run.t_synced - run.t_launched;
+        r->host_us[4] = t_out - run.t_synced;
+    }
+}
+
+}  // namespace
+
+// One conjunction (imm3_query_begin) or a disjunction of conjunctions (imm3_query_begin_dnf): terms[i] = (predicates, count).
+// encoded_or (IMM3_DNF_ENCODED_FILTER): a disjunction whose terms test an encoded column runs on the block pipeline.
+static int query_begin_terms(imm3_db* db, const char* table, const std::vector<std::pair<const imm3_pred*, int>>& terms,
+                             const char* const* proj_cols, int nproj, int64_t limit, imm3_result** out, bool encoded_or = false) {
+    if (!db || !out) return fail(IMM3_ERR_INVALID_ARG, "imm3_query_begin: NULL argument");
+    const double t_in = now_us();
+    std::unique_ptr<Prepared> pr;
+    std::vector<std::unique_ptr<Prepared>> extra;
+    bool block_or = false;
+    int rc;
+    if ((rc = plan_terms(db, table, terms, proj_cols, nproj, limit, &pr, &extra)) || (rc = choose_or(*pr, extra, encoded_or, &block_or)) ||
+        (rc = use_device(db)))
+        return rc;
+    const double t_plan = now_us();
+    std::unique_ptr<imm3_result, int (*)(imm3_result*)> r(new imm3_result(), imm3_result_free);  // (every error path: buffers back to the pools)
+    r->db = db;
     db->live_results++;
-    {
-        const double t_out = now_us();
-        r->host_us[0] = t_plan - t_in;
-        r->host_us[1] = t_dev - t_plan;
-        if (g_t_launched > 0) {
-            r->host_us[2] = g_t_launched - t_dev;     // (two-phase LIMIT queries: the last phase's stamps)
-            r->host_us[3] = g_t_synced - g_t_launched;
-            r->host_us[4] = t_out - g_t_synced;
-        }
-    }
+    const bool local = !pr->lp.always_empty && pr->table->nrows > 0;
+    if ((rc = result_columns(db, *pr, limit, r.get())) || (local && (rc = plan_device(db, pr.get(), std::move(extra), block_or, *r)))) return rc;
+    const double t_dev = local ? now_us() : t_plan;
+    Run run;
+    if ((rc = run_query(db, *pr, local, &run, r.get()))) return rc;
+    place_rows(db, pr->lp, r.get());
+    r->alg_bytes = query_alg_bytes(*pr, r->local_count);
+    report_run(r.get(), run, t_in, t_plan, t_dev);
     *out = r.release();
     return 0;
 }
@@ -2134,8 +2128,8 @@ int plan_agg_slice(imm3_db* db, AggQuery* q) {
         choose_block_filter(&pr);
     }
     rc = q->enc_filter ? size_block_front(&pr, &occ) : size_dense_filter(db, &pr, &occ);
-    if (rc || (rc = plan_grid(db, &pr, occ)) || (rc = q->enc_filter ? ensure_block_filter(db, &pr, t.nblocks) : ensure_row_space(db, sp))) return rc;
-    sp.scan_inline = q->enc_filter ? block_scan_inline(pr) : 1;  // (row space: only the total matters here, the last CTA's scan provides it)
+    if (rc || (rc = plan_grid(db, &pr, occ)) || (rc = q->enc_filter ? ensure_block_filter(db, pr, sp.ntiles, t.nblocks) : ensure_row_space(db, sp))) return rc;
+    sp.scan_inline = q->enc_filter ? block_scan_inline(pr, sp.ntiles) : 1;  // (row space: only the total matters here, the last CTA's scan provides it)
     AggPlan& ap = q->ap;
     ap.nrows = t.nrows;
     ap.ntiles = sp.ntiles;
@@ -2157,27 +2151,27 @@ int plan_agg_slice(imm3_db* db, AggQuery* q) {
 }
 
 // Local step: empty table -> filter front -> aggregation kernel -> compaction of this rank's groups into `out`.
-int launch_agg_local(imm3_db* db, AggQuery* q, AggEntry* out, int* launches) {
-    Prepared& pr = q->pr;
+int launch_agg_local(imm3_db* db, const AggQuery* q, AggEntry* out, Run* run) {
+    const Prepared& pr = q->pr;
     const ScanPlan& sp = pr.sp;
     AggEntry* const table = (AggEntry*)db->d_agg_table.p;
     unsigned int* const counters = (unsigned int*)db->d_agg_cnt.p;
     CUDA_TRY(launch_agg_init(table, q->ap.table_slots, q->ap, counters, db->stream));
-    note_launch(db, launches, "agg_init");
+    run->note("agg_init");
     if (q->enc_filter) {
-        const int rc = launch_block_filter_front(db, &pr, pr.table->nblocks, launches, nullptr, true, (uint32_t*)db->d_bitmap.p,
+        const int rc = launch_block_filter_front(db, pr, sp, pr.table->nblocks, run, nullptr, true, (uint32_t*)db->d_bitmap.p,
                                                  (uint32_t*)db->d_span_cnt.p);
         if (rc) return rc;
     } else {
         CUDA_TRY(launch_filter(sp, (uint32_t*)db->d_bitmap.p, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
                                (unsigned long long*)db->d_tile_off.p, db->d_ctrl, pr.grid, pr.dyn_smem, db->stream));
-        note_launch(db, launches, filter_route(sp));
+        run->note(filter_route(sp));
     }
     CUDA_TRY(launch_agg(q->ap, q->shape, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, table, counters, db->d_ctrl,
                         db->num_sms, db->stream));
-    note_launch(db, launches, agg_route(q->shape));
+    run->note(agg_route(q->shape));
     CUDA_TRY(launch_agg_compact(table, q->ap.table_slots, out, counters, db->stream));
-    note_launch(db, launches, "agg_compact");
+    run->note("agg_compact");
     return 0;
 }
 
@@ -2188,7 +2182,7 @@ AggEntry* agg_xbuf(const imm3_db* db, int rank) {
 
 // Merge step of a global aggregate (DESIGN §4.3): this rank's group count - or that its slice ran nothing, or refused the
 // query - posted to the peers -> a fresh table -> every rank's groups merged into it -> compaction into the result buffer.
-int launch_agg_merge_step(imm3_db* db, const AggQuery& q, bool has_local, bool refused, int* launches) {
+int launch_agg_merge_step(imm3_db* db, const AggQuery& q, bool has_local, bool refused, Run* run) {
     const AggPlan& ap = q.ap;
     AggEntry* const table = (AggEntry*)db->d_agg_table.p;
     unsigned int* const counters = (unsigned int*)db->d_agg_cnt.p;
@@ -2204,7 +2198,7 @@ int launch_agg_merge_step(imm3_db* db, const AggQuery& q, bool has_local, bool r
     xp.refused = refused ? 1 : 0;
     xp.timeout_ns = db->comm_timeout_ns;
     CUDA_TRY(launch_agg_exchange(xp, counters, db->d_ctrl, d_x, db->stream));
-    note_launch(db, launches, "agg_exchange");
+    run->note("agg_exchange");
     AggMergePlan mp;
     std::memset(&mp, 0, sizeof mp);
     for (int i = 0; i < db->world; i++) mp.buf[i] = agg_xbuf(db, i);
@@ -2214,11 +2208,11 @@ int launch_agg_merge_step(imm3_db* db, const AggQuery& q, bool has_local, bool r
     mp.naggs = ap.naggs;
     for (int a = 0; a < ap.naggs; a++) mp.op[a] = ap.agg[a].op == kAggSum ? kAggCount : ap.agg[a].op;  // (a SUM merges as a COUNT: a 64-bit add)
     CUDA_TRY(launch_agg_init(table, ap.table_slots, ap, counters, db->stream));
-    note_launch(db, launches, "agg_init");
+    run->note("agg_init");
     CUDA_TRY(launch_agg_merge(mp, d_x, table, counters, db->num_sms, db->stream));
-    note_launch(db, launches, "agg_merge");
+    run->note("agg_merge");
     CUDA_TRY(launch_agg_compact(table, ap.table_slots, (AggEntry*)db->d_agg_out.p, counters, db->stream));
-    note_launch(db, launches, "agg_compact");
+    run->note("agg_compact");
     return 0;
 }
 
@@ -2345,15 +2339,14 @@ int query_agg(imm3_db* db, const char* table, const imm3_pred* preds, int npreds
         if ((rc = ensure_buf(&db->d_agg_table, table_bytes)) || (rc = ensure_buf(&db->d_agg_out, table_bytes)) ||
             (rc = ensure_buf(&db->d_agg_cnt, 64 + sizeof(AggXOut))))  // [groups, overflow] counters, then the exchange's AggXOut
             return rc;
-        // every kernel noted (note_launch) between ev0 and ev1: the result's route and launch count; the local groups go to this
+        // every kernel noted (Run::note) between ev0 and ev1: the result's route and launch count; the local groups go to this
         // aggregate's exchange buffer when they are merged, else straight to the result buffer
-        db->route.clear();
-        db->route_tag = "";
+        Run run;
         CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
-        if (local && (rc = launch_agg_local(db, &q, merge ? agg_xbuf(db, db->rank) : (AggEntry*)db->d_agg_out.p, &q.r->launches))) return rc;
-        if (merge && (rc = launch_agg_merge_step(db, q, local, !refusal.empty(), &q.r->launches))) return rc;
+        if (local && (rc = launch_agg_local(db, &q, merge ? agg_xbuf(db, db->rank) : (AggEntry*)db->d_agg_out.p, &run))) return rc;
+        if (merge && (rc = launch_agg_merge_step(db, q, local, !refusal.empty(), &run))) return rc;
         CUDA_TRY(cudaEventRecord(db->ev1, db->stream));
-        q.r->route = db->route;
+        q.r->route = run.route;
         if ((rc = read_agg_groups(db, q, local, merge, refusal, &groups))) return rc;
     }
     if (local) q.r->alg_bytes = agg_alg_bytes(q, (int64_t)db->h_ctrl->c.total);
@@ -2415,7 +2408,7 @@ double imm3_result_device_ms(const imm3_result* r) {
     resolve_times(const_cast<imm3_result*>(r));
     return r->device_ms;
 }
-int imm3_result_kernel_launches(const imm3_result* r) { return r ? r->launches : IMM3_ERR_INVALID_ARG; }
+int imm3_result_kernel_launches(const imm3_result* r) { return r ? (r->route.empty() ? 0 : 1 + (int)std::count(r->route.begin(), r->route.end(), ';')) : IMM3_ERR_INVALID_ARG; }
 const char* imm3_result_route(const imm3_result* r) { return r ? r->route.c_str() : nullptr; }
 double imm3_result_host_us(const imm3_result* r, int phase) { return (r && phase >= 0 && phase < 5) ? r->host_us[phase] : -1.0; }
 double imm3_result_stage_ms(const imm3_result* r, int stage) {
@@ -2490,9 +2483,8 @@ int imm3_filter_bitmap(imm3_db* db, const char* table, const imm3_pred* preds, i
         if ((rc = fill_scan_plan(db, &pr))) return rc;
         pr.sp.bitmap = (uint32_t*)db->d_bitmap.p;
         pr.sp.limit = INT64_MAX;
-        double ms;
-        int launches;
-        if ((rc = run_scan(db, &pr, &ms, &total, &launches))) return rc;
+        Run run;
+        if ((rc = run_scan(db, pr, &run, &total))) return rc;
     }
     const size_t out_words = (size_t)((t.nrows + 31) / 32);
     if (out_words) CUDA_TRY(cudaMemcpyAsync(db->h_bitmap.p, db->d_bitmap.p, out_words * 4, cudaMemcpyDeviceToHost, db->stream));

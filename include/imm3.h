@@ -280,7 +280,9 @@ const void* imm3_result_col_device(const imm3_result* r, int col); /* device cop
 /* Row.toString (Record.scala:13): writes "Row(v1,v2,...)" for row i; returns length or <0. */
 int imm3_result_format_row(const imm3_result* r, int64_t row, char* buf, size_t buflen);
 double imm3_result_device_ms(const imm3_result* r);         /* CUDA-event time of the kernels of begin  */
-int imm3_result_kernel_launches(const imm3_result* r);      /* kernels launched by begin                */
+/* Kernels launched by begin / imm3_query_agg, count exchanges included: the number of entries in imm3_result_route (0 when
+ * it is ""). */
+int imm3_result_kernel_launches(const imm3_result* r);
 /* The kernels imm3_query_begin / imm3_query_agg queued, in launch order, separated by ';' ("" when none ran): kernel names
  * (select_all, filter(tma|direct), offset_scan, emit_stream, emit, emit_general, blocks_prune, blocks_filter_lane,
  * blocks_filter_quad, blocks_filter, blocks_or_merge, blocks_group_emit, blocks_scan_emit, blocks_emit(rowspace|blocks), scan_blocks,

@@ -115,6 +115,49 @@ def test_more_ranks_than_segments_device_exchange(tmp_path):
     assert all(os.path.exists(tmp_path / f"ok{r}") for r in range(4))
 
 
+def _launches_worker(rank, world, data_dir, port, out_dir):
+    sys.path.insert(0, HERE)
+    sys.path.insert(0, os.path.dirname(HERE))
+    import torch.distributed as dist
+
+    import oracle_lib as O
+    from helpers import conj, oracle_preds
+    from immutable3_b200 import GT, LT, Engine, Project, Query, SegmentManager, Select
+
+    dist.init_process_group("gloo", init_method=f"tcp://127.0.0.1:{port}", rank=rank, world_size=world)
+    os.environ["IMM3_COMM_TIMEOUT_MS"] = "10000"
+    try:
+        with SegmentManager(data_dir, device=0, rank=rank, world=world) as sm, O.Oracle(data_dir) as whole:
+            sm.comm_connect()
+            eng = Engine(sm)
+            for table, sel, proj in [("t", Select("age", LT(50)), ["id", "age"]), ("p", conj(Select("id", GT(2000)), Select("id", LT(900000))), ["id"])]:
+                empty = sm.getTable(table).nrows == 0
+                for limit in (0, 1, 10, 5000):
+                    exp = whole.query(table, oracle_preds(sel), proj, limit=limit)
+                    with eng.begin(Query(table, sel, Project(proj, limit))) as h:
+                        r = h.route
+                        assert h.kernel_launches == (len(r.split(";")) if r else 0), (rank, table, limit, r, h.kernel_launches)
+                        assert h.global_count == exp.nrows, (rank, table, limit, h.global_count, exp.nrows, r)
+                        if limit:  # rank 0's empty slice fills no LIMIT: every rank runs phase B's exchange round
+                            assert r == "count_exchange;count_exchange" if empty else r.endswith(";count_exchange;count_exchange"), (rank, table, limit, r)
+        open(os.path.join(out_dir, f"ok{rank}"), "w").write("ok")
+    finally:
+        dist.destroy_process_group()
+
+
+def test_launch_count_matches_the_route_on_small_limits(tmp_path):
+    """kernel_launches counts every exchange round of a small LIMIT: rank 0's slice is empty, so its two rounds are all it
+    launches, and a rank whose slice is too small for a prefix scans it in phase A and runs phase B's round alone."""
+    from helpers import make_table
+
+    data = tmp_path / "data"
+    make_table(data, "t", 600, 64, 5, seed=2)    # 2 segments: ranks 1 and 2 own one each
+    make_table(data, "p", 2000, 1024, 3, seed=4, id_codec="PFOR_INT", id_mode="steps")  # 1 segment: rank 2's
+    port = 35700 + (os.getpid() % 2000)
+    mp.spawn(_launches_worker, args=(3, str(data), port, str(tmp_path)), nprocs=3, join=True)
+    assert all(os.path.exists(tmp_path / f"ok{r}") for r in range(3))
+
+
 def test_two_handles_on_two_devices_in_one_process(tmp_path):
     """Kernel attributes (dynamic shared memory limit) are per device: a second handle on another GPU must work."""
     import torch

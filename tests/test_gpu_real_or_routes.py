@@ -3,7 +3,7 @@ switches, the two-phase LIMIT, ranks and a 40 M-row table, against select_tree_r
 
 Every term of such a disjunction runs filter_kernel over the same selection bitmap: the second and later terms OR their rows
 into it (ScanPlan::or_accumulate), each pass rewrites the span and tile counts of the union so far, and only the last pass
-may turn the tile counts into offsets (launch_or_terms).  The expected rows here come from walking the select tree itself
+may turn the tile counts into offsets (launch_row_space_filter).  The expected rows here come from walking the select tree itself
 with numpy, not from select_dnf's expansion, so a wrong expansion cannot move the expected and the actual rows together.
 
 As in test_gpu_routes.py, a route's first query must show in Result.route that the route's switch applied, and every query
@@ -474,6 +474,8 @@ def _worker(rank, world, data_dir, port, out_dir):
                     for limit in limits:
                         want = [c[:limit] for c in full] if limit else full
                         with eng.begin(Query("t", sel, Project(proj, limit)), real_or=True) as h:
+                            r = h.route
+                            assert h.kernel_launches == (len(r.split(";")) if r else 0), (rank, sel, limit, r, h.kernel_launches)
                             assert h.global_count == len(want[0]), (rank, sel, limit, h.global_count, len(want[0]), h.route)
                             h.fetch(h.take)
                             for c in range(len(proj)):

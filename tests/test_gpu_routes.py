@@ -228,9 +228,16 @@ def _limits(count):
     return sorted({0, 1, 33, count // 2 + 17, count, count + 1})
 
 
+def _check_launches(got, what):
+    """kernel_launches counts the route's entries."""
+    r = got.route
+    assert got.kernel_launches == (len(r.split(";")) if r else 0), (what, r, got.kernel_launches)
+
+
 def _run(eng, expect, table, sel, proj, limit, what):
     exp = expect(table, sel, proj, limit)
     with eng.execute(Query(table, sel, Project(proj, limit))) as got:
+        _check_launches(got, what)
         assert got.nrows == exp.nrows, (what, table, sel, proj, limit, got.route, got.nrows, exp.nrows)
         for c in range(len(proj)):
             a, b = got.column(c), exp.columns[c]
@@ -292,6 +299,7 @@ def test_aggregate_routes(world):
             assert r.kernel_launches == 4 and int(r.column(0)[0]) == expect("twin", Select("age", LT(50)), ["id"], 0).nrows
         with eng.execute(Query("b4", NoSelect, ProjectAgg([Max("id"), Count("age")], ["age"]))) as r:
             assert re.search(r"^agg_init;select_all;agg_blocks<1,2>;agg_compact$", r.route), r.route
+            _check_launches(r, "agg_blocks")
 
 
 def test_block_routes_at_40m_rows(tmp_path_factory, monkeypatch):
