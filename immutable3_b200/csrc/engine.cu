@@ -211,12 +211,6 @@ struct Run {
         route += tag;
     }
 };
-std::string with_stages(const char* name, int stages) { return std::string(name) + "/s=" + std::to_string(stages); }
-// the kernel launch_filter picks for this plan
-std::string filter_route(const ScanPlan& sp) {
-    if (sp.nfilter == 0) return "select_all";
-    return sp.stages > 0 ? with_stages("filter(tma)", sp.stages) : std::string("filter(direct)");
-}
 
 // ---- SegmentManager upload path: files -> pinned staging -> HBM --------------------------------
 // The owned slice of every column is one contiguous byte range in canonical order (its segments' block bytes back to
@@ -369,9 +363,6 @@ int run_pieces(imm3_db* db, const std::vector<Piece>& pieces, bool to_device) {
     return 0;
 }
 
-// Per-warp scratch of the block decoders: the byte-swapped words of the largest encoded block, plus slack.
-int block_words_cap(int64_t max_block_words) { return (int)std::min<int64_t>(1120, ((max_block_words + 4 + 31) / 32) * 32); }
-
 int upload_all(imm3_db* db) {
     const bool otrace = getenv("IMM3_OPEN_TRACE") != nullptr;
     const double t0 = now_us();
@@ -419,7 +410,7 @@ int upload_all(imm3_db* db) {
                 PforCol pc;
                 pc.words = reinterpret_cast<const uint32_t*>(col.d_arena);
                 pc.word_off = col.d_word_off;
-                CUDA_TRY(launch_block_stats(pc, t.d_row_start, t.nblocks, block_words_cap(col.max_block_words), db->num_sms, (BlockStat*)col.d_stats, db->stream));
+                CUDA_TRY(launch_block_stats(pc, t.d_row_start, t.nblocks, col.max_block_words, db->num_sms, (BlockStat*)col.d_stats, db->stream));
             }
         }
         CUDA_TRY(cudaStreamSynchronize(db->stream));
@@ -498,22 +489,16 @@ struct Prepared {
     bool for_bitmap = false;    // imm3_filter_bitmap: the selection bitmap is the result
     Pipeline pipeline = Pipeline::kDense;
     BlockFilter block_filter = BlockFilter::kMini;  // kBlocks: the filter kernel
-    int lane_warps = 8;         // ... warps per CTA of the lane kernel
     bool prune = false;         // kBlocks: every predicate is a range on an encoded column with block statistics: blocks_prune_kernel first
     PrunePlan pp;
     std::vector<int> pfor_cols;  // table columns of sp.pfor, in slot order
-    size_t blocks_emit_smem = 0;
     int64_t prefix_blocks = 0;  // small LIMIT on a block table: the pipeline first runs over this many leading blocks (0 = no prefix)
     int64_t prefix_rows = 0;    // small LIMIT on a dense table: ... over this many leading rows (a multiple of the tile size)
-    int grid_blocks_emit = 0;
-    int grid_emit = 0;
-    bool emit_general = false;  // select list needs the general gather kernel (> 4 columns or a width other than 1/2/4)
-    int grid_emit_stream = 0, emit_stage_bytes = 0, emit_ring = 0;  // streaming emit kernel (dense results); 0 = not usable
     std::string shape_key;    // key of imm3_db::emit_hint
-    size_t emit_smem = 0;
     ScanPlan sp;
-    size_t dyn_smem = 0;
-    int grid = 0;
+    KernelShape front;        // the filter kernel (row space or block), or scan_blocks; grid: its persistent grid (plan_grid)
+    EmitShape emit;           // kDense: the gather and streaming emit kernels
+    KernelShape blocks_emit;  // kRowSpace, kBlocks: the block emit kernel
     // real OR (imm3_query_begin_dnf): the second and later conjunctions of the disjunction - their filter kernels run behind this
     // plan's and OR their rows into its bitmap; counts, offsets and the emit kernels then see the union.  On kBlocks (a term
     // with a predicate on an encoded column, IMM3_DNF_ENCODED_FILTER) each term's block filter front runs into the term
@@ -532,24 +517,15 @@ int pfor_slot(const TableStore& t, std::vector<int>* cols, int ci) {
     return (int)cols->size() - 1;
 }
 
-// The quad kernel stages CTA tiles of 32 blocks of the one predicate's column: bytes reserved for such a tile.
-int64_t quad_tile_cap(const TableStore& t, const LogicalPlan& lp) {
-    return (t.cols[(size_t)lp.filters[0].col_idx].max_tile32_bytes + 16 + 15) & ~15ll;
-}
-constexpr size_t kLaneSmemCap = 222 * 1024;  // shared memory of one lane-kernel CTA (one CTA per SM)
-
 // The block filter kernel of a query with a predicate on an encoded column (kBlocks, and aggregates over such predicates):
-// the only predicate is a range on one encoded column (C4): the quad kernel - lane = (block, super-block), CTA tile of 32
-// blocks - if such a tile of this column fits a ring slot (i.e. the column actually compresses); its lane = block successor
-// if a CTA of 8 warps holds a two-slot ring per warp.  Otherwise (and with IMM3_NO_QUAD) the mini-block kernel.
+// the only predicate is a range on one encoded column (C4): the quad or lane kernel if that column's tiles fit them
+// (single_range_block_filter).  Otherwise (and with IMM3_NO_QUAD) the mini-block kernel.
 void choose_block_filter(Prepared* pr) {
     const TableStore& t = *pr->table;
     const LogicalPlan& lp = pr->lp;
     pr->block_filter = BlockFilter::kMini;
-    if (lp.filters.size() == 1 && is_pfor(t, lp.filters[0].col_idx) && lp.filters[0].kind == kFilterI32Range && !getenv("IMM3_NO_QUAD")) {
-        const int qslot = blocks_filter_quad_slot_bytes((int)quad_tile_cap(t, lp));
-        if (qslot <= 40 * 1024) pr->block_filter = (2 * 8 * (size_t)qslot <= kLaneSmemCap && !getenv("IMM3_NO_LANE")) ? BlockFilter::kLane : BlockFilter::kQuad;
-    }
+    if (lp.filters.size() == 1 && is_pfor(t, lp.filters[0].col_idx) && lp.filters[0].kind == kFilterI32Range && !getenv("IMM3_NO_QUAD"))
+        pr->block_filter = single_range_block_filter(t.cols[(size_t)lp.filters[0].col_idx].max_tile32_bytes);
 }
 
 // Pipeline and block filter kernel of a query, from the table's codecs and block sizes, the logical plan, whether a selection
@@ -687,111 +663,11 @@ int plan_columns(imm3_db* db, Prepared* pr) {
     return 0;
 }
 
-// Filter kernel over the row space (kDense, kRowSpace, aggregation): tiles of 8192 rows; a TMA ring of ~32 KiB, so that four
-// CTAs share an SM.  A stage holds one 8192-row sub-tile of every filter column.
-int size_dense_filter(imm3_db* db, Prepared* pr, int* occ) {
-    ScanPlan& sp = pr->sp;
-    int stage_bytes = 0;
-    for (int i = 0; i < sp.nfilter; i++) stage_bytes += kDenseTileRowsPerWord * sp.filter[i].width;
-    const bool stage_ok = !(db->flags & IMM3_OPEN_NO_TMA) && stage_bytes > 0 && stage_bytes <= 56 * 1024;
-    for (int i = 0, off = 0; i < sp.nfilter; i++) {  // where each column sits inside a stage
-        sp.filter[i].smem_off = stage_ok ? off : -1;
-        off += kDenseTileRowsPerWord * sp.filter[i].width;
-    }
-    sp.ntiles = (pr->table->nrows + kDenseTileRowsPerWord - 1) / kDenseTileRowsPerWord;
-    int stages = 0;
-    if (stage_ok) stages = std::max(2, std::min(kMaxFilterStages, (32 * 1024) / stage_bytes));
-    if (const char* e = getenv("IMM3_FILTER_STAGES")) {
-        int v = atoi(e);
-        if (stage_ok && v >= 2 && v <= kMaxFilterStages && (size_t)v * stage_bytes <= 200 * 1024) stages = v;
-    }
-    sp.stages = stages;
-    sp.stage_bytes = stage_bytes;
-    pr->dyn_smem = (size_t)stages * (size_t)stage_bytes;
-    CUDA_TRY(filter_kernel_occupancy(pr->dyn_smem, occ));
+// Filter kernel over the row space (kDense, kRowSpace, aggregation): tiles of 8192 rows, its ring from size_filter.
+int size_dense_filter(imm3_db* db, Prepared* pr) {
+    pr->sp.ntiles = (pr->table->nrows + kDenseTileRowsPerWord - 1) / kDenseTileRowsPerWord;
+    CUDA_TRY(size_filter(&pr->sp, db->flags & IMM3_OPEN_NO_TMA, &pr->front));
     return 0;
-}
-
-// kDense: the gather emit kernel (8 spans of 1024 rows per tile) and the streaming one (dense results).
-int size_dense_emit(imm3_db* db, Prepared* pr) {
-    ScanPlan& sp = pr->sp;
-    int occ_emit = 0;
-    pr->emit_general = sp.nproj > 4 || getenv("IMM3_EMIT_GENERAL");
-    for (int i = 0; i < sp.nproj; i++) pr->emit_general = pr->emit_general || !(sp.proj[i].width == 1 || sp.proj[i].width == 2 || sp.proj[i].width == 4);
-    CUDA_TRY(emit_kernel_occupancy(pr->emit_general, &occ_emit));
-    const int64_t nspans = sp.ntiles * (kDenseTileRowsPerWord / 1024);
-    pr->grid_emit = (int)std::max<int64_t>(1, std::min<int64_t>((nspans + 7) / 8, (int64_t)db->num_sms * std::max(1, occ_emit)));
-    // Streaming emit kernel: a stage = bitmap words + span counts + one 8192-row tile of every projected column, if that fits.
-    int pstage = 0;
-    for (int i = 0; i < sp.nproj; i++) {
-        sp.proj[i].stage_off = pstage;
-        pstage += 1024 * sp.proj[i].width;
-    }
-    pr->emit_stage_bytes = 0;
-    if (sp.nproj > 0 && 8 * pstage <= 64 * 1024 && !(db->flags & IMM3_OPEN_NO_TMA) && !getenv("IMM3_NO_EMIT_STREAM")) {
-        pr->emit_stage_bytes = emit_stream_header_bytes() + 8 * pstage;
-        pr->emit_ring = std::max(2, std::min(4, (80 * 1024) / pr->emit_stage_bytes));
-        if (const char* e = getenv("IMM3_EMIT_STAGES")) {
-            int v = atoi(e);
-            if (v >= 2 && v <= 4) pr->emit_ring = v;
-        }
-        pr->emit_smem = emit_stream_smem_bytes(pr->emit_stage_bytes, pr->emit_ring);
-        int occ_s = 0;
-        CUDA_TRY(emit_stream_occupancy(pr->emit_smem, &occ_s));
-        if (occ_s < 1) pr->emit_stage_bytes = 0;
-        pr->grid_emit_stream = (int)std::max<int64_t>(1, std::min<int64_t>(sp.ntiles, (int64_t)db->num_sms * std::max(1, occ_s)));
-    }
-    return 0;
-}
-
-// kBlocks: the ring of the block filter kernel.  Mini-block kernel: a TMA ring of raw tiles (8 blocks of every encoded column
-// that carries a predicate + metadata).  Quad kernel: tiles of 32 blocks of its one column.  Lane kernel: every warp of the
-// CTA runs its own ring of 2 .. 4 such slots; one CTA per SM with as many warps (8 .. 16) as its shared memory holds two-slot
-// rings for.
-void size_block_filter(Prepared* pr) {
-    const TableStore& t = *pr->table;
-    ScanPlan& sp = pr->sp;
-    const char* ring_env = getenv("IMM3_BLOCKS_STAGES");
-    sp.pfor_filter_mask = 0;
-    for (int i = 0; i < sp.nfilter; i++)
-        if (sp.filter[i].pfor_slot >= 0) sp.pfor_filter_mask |= 1u << sp.filter[i].pfor_slot;
-    if (pr->block_filter == BlockFilter::kMini) {
-        int64_t tile_cap = 0;
-        int nstaged = 0;
-        for (int s = 0; s < sp.npfor; s++)
-            if ((sp.pfor_filter_mask >> s) & 1u) {
-                tile_cap = std::max<int64_t>(tile_cap, t.cols[(size_t)pr->pfor_cols[(size_t)s]].max_tile_bytes);
-                nstaged++;
-            }
-        sp.blk_tile_bytes = (int)((tile_cap + 16 + 15) & ~15ll);
-        const int slot_bytes = blocks_filter_slot_bytes(nstaged, sp.blk_tile_bytes);
-        int ring = std::max(2, std::min(kMaxFilterStages, (48 * 1024) / slot_bytes));
-        if (ring_env) ring = std::max(2, std::min(kMaxFilterStages, atoi(ring_env)));
-        while (ring > 2 && (size_t)ring * slot_bytes > 200 * 1024) ring--;
-        sp.stages = ring;
-        sp.stage_bytes = slot_bytes;
-        pr->dyn_smem = blocks_filter_smem_bytes(nstaged, sp.blk_tile_bytes, ring);
-        return;
-    }
-    const int64_t cap32 = quad_tile_cap(t, pr->lp);
-    const int qslot = blocks_filter_quad_slot_bytes((int)cap32);
-    sp.blk_tile_bytes = (int)cap32;
-    sp.stage_bytes = qslot;
-    if (pr->block_filter == BlockFilter::kQuad) {
-        int qring = std::max(2, std::min(4, (40 * 1024) / qslot));
-        if (ring_env) qring = std::max(2, std::min(kMaxFilterStages, atoi(ring_env)));
-        sp.stages = qring;
-        pr->dyn_smem = (size_t)qring * (size_t)qslot;
-        return;
-    }
-    int lring = 2;
-    if (const char* e = getenv("IMM3_LANE_STAGES")) lring = std::max(2, std::min(4, atoi(e)));
-    while (lring > 2 && (size_t)lring * 4 * (size_t)qslot > kLaneSmemCap) lring--;
-    int lw = (int)std::min<size_t>(16, kLaneSmemCap / ((size_t)lring * (size_t)qslot));
-    if (const char* e = getenv("IMM3_LANE_WARPS")) lw = std::max(4, std::min(lw, atoi(e)));
-    pr->lane_warps = lw;
-    sp.stages = lring;
-    pr->dyn_smem = (size_t)lring * (size_t)lw * (size_t)qslot;
 }
 
 // kBlocks: pruning, if every predicate is a range on an encoded column that has block statistics.
@@ -820,37 +696,44 @@ void size_prune(Prepared* pr) {
 }
 
 // kBlocks, and aggregates over encoded predicates: the block filter front on tiles of 8 blocks (the offset scan's), its
-// filter kernel's ring and occupancy, and pruning.
-int size_block_front(Prepared* pr, int* occ) {
-    pr->sp.ntiles = (pr->table->nblocks + 7) / 8;
-    size_block_filter(pr);
+// filter kernel's ring over the encoded predicate columns' tiles (size_block_filter), and pruning.
+int size_block_front(Prepared* pr) {
+    const TableStore& t = *pr->table;
+    ScanPlan& sp = pr->sp;
+    sp.ntiles = (t.nblocks + 7) / 8;
+    sp.pfor_filter_mask = 0;
+    int64_t tile8 = 0, tile32 = 0;
+    for (int i = 0; i < sp.nfilter; i++)
+        if (sp.filter[i].pfor_slot >= 0) {
+            const ColumnStore& c = t.cols[(size_t)pr->pfor_cols[(size_t)sp.filter[i].pfor_slot]];
+            sp.pfor_filter_mask |= 1u << sp.filter[i].pfor_slot;
+            tile8 = std::max<int64_t>(tile8, c.max_tile_bytes);
+            tile32 = std::max<int64_t>(tile32, c.max_tile32_bytes);
+        }
+    CUDA_TRY(size_block_filter(pr->block_filter, &sp, tile8, tile32, &pr->front));
     size_prune(pr);
-    CUDA_TRY(blocks_filter_occupancy(pr->dyn_smem, pr->block_filter, pr->lane_warps, occ));
     return 0;
 }
 
 // kRowSpace, kBlocks: the block emit kernel.
 int size_block_emit(imm3_db* db, Prepared* pr) {
     const TableStore& t = *pr->table;
-    ScanPlan& sp = pr->sp;
     int64_t words = 0;
     for (int ci : pr->pfor_cols) words = std::max<int64_t>(words, t.cols[(size_t)ci].max_block_words);
-    sp.blk_words_cap = block_words_cap(words);
-    pr->blocks_emit_smem = blocks_emit_smem_bytes(sp.npfor, sp.blk_words_cap);
-    int occ_e = 0;
-    CUDA_TRY(blocks_emit_occupancy(pr->blocks_emit_smem, pr->pipeline == Pipeline::kRowSpace, &occ_e));
-    if (occ_e < 1) return fail(IMM3_ERR_CUDA, "block emit kernel does not fit on an SM (dynamic shared memory %zu bytes)", pr->blocks_emit_smem);
-    pr->grid_blocks_emit = (int)std::max<int64_t>(1, std::min<int64_t>((t.nblocks + 7) / 8, (int64_t)db->num_sms * std::max(1, occ_e)));
+    CUDA_TRY(size_blocks_emit(&pr->sp, pr->pipeline == Pipeline::kRowSpace, words, t.nblocks, db->num_sms, &pr->blocks_emit));
+    if (pr->blocks_emit.occupancy < 1)
+        return fail(IMM3_ERR_CUDA, "block emit kernel does not fit on an SM (dynamic shared memory %zu bytes)", pr->blocks_emit.smem);
     return 0;
 }
 
 // The filter kernel's persistent grid from its occupancy, and the status words of the tiles.
-int plan_grid(imm3_db* db, Prepared* pr, int occ) {
+int plan_grid(imm3_db* db, Prepared* pr) {
     const ScanPlan& sp = pr->sp;
+    KernelShape& ks = pr->front;
     if (sp.ntiles >= (int64_t)0x7FFFFFFF) return fail(IMM3_ERR_UNSUPPORTED, "too many tiles (%lld)", (long long)sp.ntiles);
-    if (occ < 1) return fail(IMM3_ERR_CUDA, "kernel does not fit on an SM (dynamic shared memory %zu bytes)", pr->dyn_smem);
-    const int64_t persistent = (int64_t)db->num_sms * occ;
-    pr->grid = (int)std::max<int64_t>(1, std::min<int64_t>(sp.ntiles, persistent));
+    if (ks.occupancy < 1) return fail(IMM3_ERR_CUDA, "kernel does not fit on an SM (dynamic shared memory %zu bytes)", ks.smem);
+    const int64_t persistent = (int64_t)db->num_sms * ks.occupancy;
+    ks.grid = (int)std::max<int64_t>(1, std::min<int64_t>(sp.ntiles, persistent));
     const size_t status_need = 2 * (size_t)status_round_up(sp.ntiles);  // tile counts + (dense kernel) tile offsets
     if (status_need > db->status_cap) {
         if (db->d_status) CUDA_TRY(cudaFree(db->d_status));
@@ -866,33 +749,33 @@ int plan_grid(imm3_db* db, Prepared* pr, int occ) {
 // Fill the device plan of the query's pipeline (everything but result pointers and the bitmap).
 int fill_scan_plan(imm3_db* db, Prepared* pr) {
     const TableStore& t = *pr->table;
-    int occ = 0, rc = plan_columns(db, pr);
+    int rc = plan_columns(db, pr);
     if (rc) return rc;
     const int64_t prefix = prefix_rows_wanted(pr->lp);
     switch (pr->pipeline) {
     case Pipeline::kDense: {
         const int64_t want = (prefix + kDenseTileRowsPerWord - 1) / kDenseTileRowsPerWord * kDenseTileRowsPerWord;
         if (want * 2 <= t.nrows) pr->prefix_rows = want;
-        if ((rc = size_dense_filter(db, pr, &occ)) || (rc = size_dense_emit(db, pr))) return rc;
+        if ((rc = size_dense_filter(db, pr))) return rc;
+        CUDA_TRY(size_emit(&pr->sp, db->flags & IMM3_OPEN_NO_TMA, db->num_sms, &pr->emit));
         break;
     }
     case Pipeline::kRowSpace:
     case Pipeline::kBlocks: {
         pr->prefix_blocks = prefix_blocks_wanted(*pr);
-        rc = pr->pipeline == Pipeline::kRowSpace ? size_dense_filter(db, pr, &occ) : size_block_front(pr, &occ);
+        rc = pr->pipeline == Pipeline::kRowSpace ? size_dense_filter(db, pr) : size_block_front(pr);
         if (rc || (rc = size_block_emit(db, pr))) return rc;
         break;
     }
-    case Pipeline::kSinglePass:  // scan_blocks stages whole blocks
+    case Pipeline::kSinglePass:
         if (t.max_block_rows > kMaxBlockRows)
             return fail(IMM3_ERR_UNSUPPORTED, "block-mode kernel stages blocks of at most %d rows, table %s has a block of %d",
                         kMaxBlockRows, t.meta.name.c_str(), t.max_block_rows);
         pr->sp.ntiles = t.nblocks;
-        pr->dyn_smem = blocks_kernel_smem_bytes(pr->sp.npfor, t.max_block_rows);
-        CUDA_TRY(blocks_kernel_occupancy(pr->dyn_smem, &occ));
+        CUDA_TRY(size_scan_blocks(pr->sp, t.max_block_rows, &pr->front));
         break;
     }
-    return plan_grid(db, pr, occ);
+    return plan_grid(db, pr);
 }
 
 bool has_encoded_filter(const Prepared& pr) {
@@ -913,8 +796,8 @@ void force_blocks(Prepared* pr) {
 int fill_or_terms_plan(imm3_db* db, Prepared* pr) {
     bool pruned = pr->prune;
     for (auto& tm : pr->or_terms) {
-        int occ = 0, rc = plan_columns(db, tm.get());
-        if (rc || (rc = size_block_front(tm.get(), &occ)) || (rc = plan_grid(db, tm.get(), occ))) return rc;
+        int rc = plan_columns(db, tm.get());
+        if (rc || (rc = size_block_front(tm.get())) || (rc = plan_grid(db, tm.get()))) return rc;
         pruned = pruned && tm->prune;
     }
     pr->prefix_blocks = pruned ? 0 : prefix_blocks_wanted(*pr);
@@ -984,17 +867,9 @@ int exchange_only(imm3_db* db, Run* run, int64_t limit, int has_count) {
     return 0;
 }
 
-// Who turns the tile counts into offsets: the filter kernel's last CTA (small tables), or offset_scan_kernel - one CTA per
-// 4096 counts, launched behind the filter kernel (large tables: 122 K counts at 1 B rows take one SM ~50 us).
-bool scan_inline_for(int64_t ntiles) {
-    if (const char* e = getenv("IMM3_SCAN")) {
-        if (!strcmp(e, "inline")) return true;
-        if (!strcmp(e, "kernel")) return false;
-    }
-    return ntiles <= scan_inline_max_tiles();
-}
-// ... for the block filter front over `ntiles` tiles (the lane kernel's inline scan is written for 8 warps)
-int block_scan_inline(const Prepared& pr, int64_t ntiles) { return scan_inline_for(ntiles) && !(pr.block_filter == BlockFilter::kLane && pr.lane_warps < 8); }
+// Whether the block filter front's last CTA runs the offset scan over `ntiles` tiles (scan_inline_for; the lane kernel's
+// inline scan is written for 8 warps)
+int block_scan_inline(const Prepared& pr, int64_t ntiles) { return scan_inline_for(ntiles) && !(pr.block_filter == BlockFilter::kLane && pr.front.lane_warps < 8); }
 int prepare_scan_buffers(imm3_db* db, int64_t ntiles, bool want_list) {
     if (want_list) {
         int rc = ensure_buf(&db->d_tile_list, (size_t)(ntiles + 16) * 4);
@@ -1036,7 +911,7 @@ Extent phase_extent(const Prepared& pr, bool prefix) {
     return {rows, (rows + kDenseTileRowsPerWord - 1) / kDenseTileRowsPerWord, nb};
 }
 // A filter kernel's grid over a phase's tiles: its plan's persistent grid, fewer CTAs for a shorter phase.
-int phase_grid(const Prepared& p, int64_t ntiles) { return (int)std::max<int64_t>(1, std::min<int64_t>(p.grid, ntiles)); }
+int phase_grid(const Prepared& p, int64_t ntiles) { return (int)std::max<int64_t>(1, std::min<int64_t>(p.front.grid, ntiles)); }
 // A later term's device plan of a real OR in one phase: its own, over the first term's rows, tiles and bitmap.
 ScanPlan term_plan(const Prepared& tm, const ScanPlan& first) {
     ScanPlan sp = tm.sp;
@@ -1083,9 +958,10 @@ int launch_row_space_filter(imm3_db* db, const Prepared& pr, ScanPlan& sp, Run* 
     const bool scan_inline = sp.nfilter == 0 || scan_inline_for(sp.ntiles);
     auto filter = [&](const Prepared& p, ScanPlan& f, bool last) {
         f.scan_inline = last && scan_inline;
+        std::string route;
         CUDA_TRY(launch_filter(f, sp.bitmap, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p, (unsigned long long*)db->d_tile_off.p,
-                               db->d_ctrl, phase_grid(p, f.ntiles), p.dyn_smem, db->stream));
-        run->note(filter_route(f));
+                               db->d_ctrl, phase_grid(p, f.ntiles), p.front.smem, db->stream, &route));
+        run->note(route);
         return 0;
     };
     CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
@@ -1103,7 +979,7 @@ int launch_row_space_filter(imm3_db* db, const Prepared& pr, ScanPlan& sp, Run* 
 int launch_dense(imm3_db* db, const Prepared& pr, ScanPlan& sp, Run* run, Queued* q) {
     int rc;
     if ((rc = setup_phase_trace(db, sp, 0)) || (rc = ensure_row_space(db, sp))) return rc;
-    const int stream_ok = pr.emit_stage_bytes > 0 && sp.nproj > 0;
+    const int stream_ok = pr.emit.stream.stage_bytes > 0 && sp.nproj > 0;
     const char* force = getenv("IMM3_EMIT");  // experiment: "stream" / "gather" = that kernel takes every result, "both" = no feedback
     int hint = -1;
     if (stream_ok && !(force && !strcmp(force, "both"))) {
@@ -1121,15 +997,14 @@ int launch_dense(imm3_db* db, const Prepared& pr, ScanPlan& sp, Run* run, Queued
     const int64_t nspans = sp.ntiles * (kDenseTileRowsPerWord / 1024);
     if (stream_ok && !only_gather) {
         CUDA_TRY(launch_emit_stream(sp, sp.bitmap, (const uint32_t*)db->d_span_cnt.p, (const uint32_t*)db->d_tile_cnt.p,
-                                    (const unsigned long long*)db->d_tile_off.p, sp.ntiles, pr.emit_ring, pr.emit_stage_bytes,
-                                    only_stream ? -1 : 1, pr.grid_emit_stream, pr.emit_smem, db->d_ctrl, pdl, db->stream));
-        run->note(with_stages("emit_stream", pr.emit_ring));
+                                    (const unsigned long long*)db->d_tile_off.p, sp.ntiles, pr.emit.stream, only_stream ? -1 : 1, db->d_ctrl,
+                                    pdl, db->stream));
+        run->note("emit_stream/s=" + std::to_string(pr.emit.stream.stages));
     }
     if (!only_stream) {
         CUDA_TRY(launch_emit(sp, sp.bitmap, (const uint32_t*)db->d_span_cnt.p, (const unsigned long long*)db->d_tile_off.p, 8,
-                             nspans, pr.grid_emit, stream_ok && !only_gather, db->d_ctrl, pr.emit_general, pdl && (only_gather || !stream_ok),
-                             db->stream));
-        run->note(pr.emit_general ? "emit_general" : "emit");
+                             nspans, pr.emit, stream_ok && !only_gather, db->d_ctrl, pdl && (only_gather || !stream_ok), db->stream));
+        run->note(pr.emit.general ? "emit_general" : "emit");
     }
     return 0;
 }
@@ -1141,8 +1016,7 @@ int launch_row_space(imm3_db* db, const Prepared& pr, ScanPlan& sp, int64_t nblo
     if ((rc = ensure_row_space(db, sp)) || (rc = launch_row_space_filter(db, pr, sp, run)) || (rc = mark_mid(db, pdl, q))) return rc;
     if (sp.nproj == 0) return 0;
     CUDA_TRY(launch_blocks_emit(sp, sp.bitmap, (const uint32_t*)db->d_span_cnt.p, nullptr, (const unsigned long long*)db->d_tile_off.p,
-                                nblocks, db->d_ctrl, true, pdl, (int)std::min<int64_t>(pr.grid_blocks_emit, (nblocks + 7) / 8),
-                                pr.blocks_emit_smem, db->stream));
+                                nblocks, db->d_ctrl, true, pdl, pr.blocks_emit, db->stream));
     run->note("blocks_emit(rowspace)");
     return 0;
 }
@@ -1166,7 +1040,6 @@ int launch_block_filter_front(imm3_db* db, const Prepared& pr, const ScanPlan& s
                               uint32_t* words, uint32_t* cnts) {
     const TableStore& t = *pr.table;
     const int64_t ntiles = sp.ntiles;
-    const bool lane = pr.block_filter == BlockFilter::kLane;
     const unsigned int* work = pr.prune ? (const unsigned int*)db->d_work.p : nullptr;
     if (pr.prune) {
         // whole blocks decided from their min / max; only the tiles a window edge cuts through reach the filter kernel
@@ -1175,16 +1048,10 @@ int launch_block_filter_front(imm3_db* db, const Prepared& pr, const ScanPlan& s
                                      (unsigned int*)db->d_work.p, db->num_sms, db->stream, grp_sum));
         run->note("blocks_prune");
     }
-    int filter_grid = phase_grid(pr, ntiles);
-    if (pr.block_filter != BlockFilter::kMini) {  // CTA tiles of 32 blocks (quad), 32 blocks per warp (lane)
-        const int64_t per_cta = 32 * (lane ? pr.lane_warps : 1);
-        filter_grid = (int)std::max<int64_t>(1, std::min<int64_t>(filter_grid, (nblocks + per_cta - 1) / per_cta));
-    }
-    CUDA_TRY(launch_blocks_filter(sp, words, cnts, (uint32_t*)db->d_tile_cnt.p,
-                                  (unsigned long long*)db->d_tile_off.p, db->d_ctrl, nblocks, filter_grid, pr.dyn_smem, pr.block_filter,
-                                  pr.lane_warps, work, db->stream, grp_sum));
-    run->note(lane ? "blocks_filter_lane/w=" + std::to_string(pr.lane_warps) + "/s=" + std::to_string(sp.stages)
-                   : with_stages(pr.block_filter == BlockFilter::kQuad ? "blocks_filter_quad" : "blocks_filter", sp.stages));
+    std::string route;
+    CUDA_TRY(launch_blocks_filter(sp, words, cnts, (uint32_t*)db->d_tile_cnt.p, (unsigned long long*)db->d_tile_off.p, db->d_ctrl, nblocks,
+                                  phase_grid(pr, ntiles), pr.block_filter, pr.front, work, grp_sum, db->stream, &route));
+    run->note(route);
     return (scan && !sp.scan_inline) ? launch_scan_kernel(db, sp, ntiles, run, true) : 0;
 }
 
@@ -1224,13 +1091,14 @@ int launch_blocks(imm3_db* db, const Prepared& pr, ScanPlan& sp, int64_t nblocks
     int rc;
     if ((rc = ensure_block_filter(db, pr, ntiles, nblocks)) || (merge && (rc = ensure_or_terms(db, pr, nblocks)))) return rc;
     int fused_grid = 0;  // > 0: blocks_scan_emit_kernel
-    int group_grid = 0, ngroups = 0;  // > 0: blocks_group_emit_kernel
+    int group_grid = 0;  // > 0: blocks_group_emit_kernel
     if (sp.nproj == 1 && sp.proj[0].pfor_slot >= 0 && !getenv("IMM3_NO_SCANEMIT")) {
-        if (lane && !merge && !getenv("IMM3_NO_GROUPEMIT")) CUDA_TRY(blocks_group_emit_grid(db->num_sms, nblocks, &group_grid, &ngroups));
+        size_t sum_bytes = 0;
+        if (lane && !merge && !getenv("IMM3_NO_GROUPEMIT")) CUDA_TRY(blocks_group_emit_grid(db->num_sms, nblocks, &group_grid, &sum_bytes));
         if (group_grid > 0) {
             if (!db->d_grp_sum.p) {
-                CUDA_TRY(cudaMalloc(&db->d_grp_sum.p, blocks_group_sum_bytes()));
-                db->d_grp_sum.cap = blocks_group_sum_bytes();
+                CUDA_TRY(cudaMalloc(&db->d_grp_sum.p, sum_bytes));
+                db->d_grp_sum.cap = sum_bytes;
                 CUDA_TRY(cudaMemsetAsync(db->d_grp_sum.p, 0, db->d_grp_sum.cap, db->stream));
             }
         } else {
@@ -1254,8 +1122,8 @@ int launch_blocks(imm3_db* db, const Prepared& pr, ScanPlan& sp, int64_t nblocks
         const bool pdl = !getenv("IMM3_NO_PDL");
         if ((rc = mark_mid(db, pdl, q))) return rc;
         if (group_grid > 0) {
-            CUDA_TRY(launch_blocks_group_emit(sp, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, grp_sum, nblocks, ngroups,
-                                              db->d_ctrl, pdl, group_grid, db->stream, pub, pub_seq));
+            CUDA_TRY(launch_blocks_group_emit(sp, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, grp_sum, nblocks, db->d_ctrl,
+                                              pdl, group_grid, db->stream, pub, pub_seq));
             run->note("blocks_group_emit/ctas=" + std::to_string(group_grid));
         } else {
             CUDA_TRY(launch_blocks_scan_emit(sp, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, (const uint32_t*)db->d_tile_cnt.p,
@@ -1270,8 +1138,7 @@ int launch_blocks(imm3_db* db, const Prepared& pr, ScanPlan& sp, int64_t nblocks
         if (sp.nproj > 0) {
             CUDA_TRY(launch_blocks_emit(sp, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p,
                                         sp.scan_inline ? nullptr : (const unsigned int*)db->d_tile_list.p,
-                                        (const unsigned long long*)db->d_tile_off.p, nblocks, db->d_ctrl, false, pdl,
-                                        (int)std::min<int64_t>(pr.grid_blocks_emit, (nblocks + 7) / 8), pr.blocks_emit_smem, db->stream));
+                                        (const unsigned long long*)db->d_tile_off.p, nblocks, db->d_ctrl, false, pdl, pr.blocks_emit, db->stream));
             run->note("blocks_emit(blocks)");
         }
     }
@@ -1294,7 +1161,7 @@ int run_scan_once(imm3_db* db, const Prepared& pr, const Extent& ex, Run* run, i
     case Pipeline::kBlocks: rc = launch_blocks(db, pr, sp, ex.nblocks, run, &q); break;
     case Pipeline::kSinglePass:
         CUDA_TRY(cudaEventRecord(db->ev0, db->stream));
-        CUDA_TRY(launch_scan_blocks(sp, db->d_ctrl, db->d_status, pr.grid, pr.dyn_smem, db->stream));
+        CUDA_TRY(launch_scan_blocks(sp, db->d_ctrl, db->d_status, pr.front.grid, pr.front.smem, db->stream));
         run->note("scan_blocks");
         break;
     }
@@ -1359,7 +1226,7 @@ int run_scan_once(imm3_db* db, const Prepared& pr, const Extent& ex, Run* run, i
         run->stage_ms[1] += b;
     }
     *total = (int64_t)db->h_ctrl->c.total;
-    if (pr.pipeline == Pipeline::kDense && sp.nproj > 0 && pr.emit_stage_bytes > 0)  // feedback for the next query of this shape
+    if (pr.pipeline == Pipeline::kDense && sp.nproj > 0 && pr.emit.stream.stage_bytes > 0)  // feedback for the next query of this shape
         db->emit_hint[pr.shape_key] = (db->h_ctrl->c.total > 0 && db->h_ctrl->c.dense_rows * 2 >= db->h_ctrl->c.total) ? 1 : 0;
     if (sp.trace) {
         unsigned long long h[64];
@@ -1498,6 +1365,7 @@ int imm3_open(const char* data_dir, const imm3_open_opts* opts, imm3_db** out) {
             cudaDeviceProp prop;
             CUDA_TRY(cudaGetDeviceProperties(&prop, db->device));
             if (prop.major < 10) return fail(IMM3_ERR_CUDA, "device %d is sm_%d%d; this library is built for sm_100a only", db->device, prop.major, prop.minor);
+            CUDA_TRY(configure_device());
             db->num_sms = prop.multiProcessorCount;
             if (const char* g = getenv("IMM3_L2_FETCH")) {  // experiment: DRAM->L2 fetch granularity hint (32 / 64 / 128 bytes)
                 CUDA_TRY(cudaDeviceSetLimit(cudaLimitMaxL2FetchGranularity, (size_t)atoi(g)));
@@ -1981,6 +1849,7 @@ struct AggQuery {
     bool has_sum = false;
     bool enc_filter = false;         // a predicate on a sorted-int-codec column: the block filter front decides it
     int smem_optin = 0;              // agg_blocks_kernel: the device's shared memory per CTA (cudaDevAttrMaxSharedMemoryPerBlockOptin)
+    size_t blocks_smem = 0;          // ... and what one of its CTAs needs (size_agg_blocks)
 };
 
 // Validation and plan of an aggregate, before any device work: group and aggregate columns, the result schema, the COUNT a
@@ -2108,10 +1977,9 @@ int check_agg_block_rows(const AggQuery& q) {
 }
 // ... and, once the slice is planned, agg_blocks_kernel's shared memory against the device's opt-in limit.
 int check_agg_smem(const AggQuery& q) {
-    const size_t smem = agg_blocks_smem_bytes(q.shape, q.ap.npfor, q.ap.blk_words_cap) + 1024;  // (1 KB: the kernel's static shared memory)
-    if (!q.shape.blocks || smem <= (size_t)q.smem_optin) return 0;
+    if (!q.shape.blocks || q.blocks_smem <= (size_t)q.smem_optin) return 0;
     return fail(IMM3_ERR_UNSUPPORTED, "aggregation over %d sorted-int-codec columns with %d aggregates needs %zu bytes of shared memory per CTA, the device has %d",
-                q.ap.npfor, q.ap.naggs, smem, q.smem_optin);
+                q.ap.npfor, q.ap.naggs, q.blocks_smem, q.smem_optin);
 }
 
 // The device plans of this rank's slice: the filter front, then the AggPlan's columns.  An encoded predicate: the block
@@ -2121,14 +1989,14 @@ int plan_agg_slice(imm3_db* db, AggQuery* q) {
     Prepared& pr = q->pr;
     ScanPlan& sp = pr.sp;
     const TableStore& t = *pr.table;
-    int occ = 0, rc = plan_columns(db, &pr);
+    int rc = plan_columns(db, &pr);
     if (rc) return rc;
     if (q->enc_filter) {
         pr.pipeline = Pipeline::kBlocks;  // (IMM3_PATH=fused and IMM3_NO_HYBRID choose Project pipelines only)
         choose_block_filter(&pr);
     }
-    rc = q->enc_filter ? size_block_front(&pr, &occ) : size_dense_filter(db, &pr, &occ);
-    if (rc || (rc = plan_grid(db, &pr, occ)) || (rc = q->enc_filter ? ensure_block_filter(db, pr, sp.ntiles, t.nblocks) : ensure_row_space(db, sp))) return rc;
+    rc = q->enc_filter ? size_block_front(&pr) : size_dense_filter(db, &pr);
+    if (rc || (rc = plan_grid(db, &pr)) || (rc = q->enc_filter ? ensure_block_filter(db, pr, sp.ntiles, t.nblocks) : ensure_row_space(db, sp))) return rc;
     sp.scan_inline = q->enc_filter ? block_scan_inline(pr, sp.ntiles) : 1;  // (row space: only the total matters here, the last CTA's scan provides it)
     AggPlan& ap = q->ap;
     ap.nrows = t.nrows;
@@ -2142,7 +2010,7 @@ int plan_agg_slice(imm3_db* db, AggQuery* q) {
             ap.pfor[i].word_off = c.d_word_off;
             words = std::max<int64_t>(words, c.max_block_words);
         }
-        ap.blk_words_cap = block_words_cap(words);
+        q->blocks_smem = size_agg_blocks(&ap, q->shape, words);
         ap.nblocks = t.nblocks;
         ap.row_start = t.d_row_start;
         CUDA_TRY(cudaDeviceGetAttribute(&q->smem_optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, db->device));
@@ -2163,9 +2031,10 @@ int launch_agg_local(imm3_db* db, const AggQuery* q, AggEntry* out, Run* run) {
                                                  (uint32_t*)db->d_span_cnt.p);
         if (rc) return rc;
     } else {
+        std::string route;
         CUDA_TRY(launch_filter(sp, (uint32_t*)db->d_bitmap.p, (uint32_t*)db->d_span_cnt.p, (uint32_t*)db->d_tile_cnt.p,
-                               (unsigned long long*)db->d_tile_off.p, db->d_ctrl, pr.grid, pr.dyn_smem, db->stream));
-        run->note(filter_route(sp));
+                               (unsigned long long*)db->d_tile_off.p, db->d_ctrl, pr.front.grid, pr.front.smem, db->stream, &route));
+        run->note(route);
     }
     CUDA_TRY(launch_agg(q->ap, q->shape, (const uint32_t*)db->d_bitmap.p, (const uint32_t*)db->d_span_cnt.p, table, counters, db->d_ctrl,
                         db->num_sms, db->stream));
